@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            our CUDA arm (one process per GPU)
     python bench.py --impl reference [--steps K] [--warmup W]      the reference's own CPU implementation
+    python bench.py ... --dump-outputs DIR                          also write the headline's outputs as DIR/<name>.npy
 
 Workload (config.workload): BASELINE.json configs[1] -- N=1M rows, D=256, q=16, 20% entries missing,
 FP64, masked ("mode B") VB-PCA, synthetic data generated on the device.  With --gpus N every rank owns
@@ -622,8 +623,44 @@ def bench_e2e(torch, dist, dev, eng, local, steps):
                     "(DMMA), summed; at N > 1 one NCCL all-reduce of the statistics"}
 
 
-def measure_config(torch, dist, dev, rank, world, local, lib, _cabi, cfg, steps, warmup, sampler, hbm, peak_tf, traffic_json):
-    """Build the engine of one configuration on this rank's shard, time `steps` sweeps, break the sweep down."""
+DUMP_ROW_BYTES = 32 << 20        # the sampled per-row outputs; the rest (W, mu, globals, bounds) is O(D q + steps)
+
+
+def dump_outputs(eng, slots, out_dir, seed=0):
+    """What a caller of the timed sweeps receives, as float64 .npy files: the bound of every timed sweep, the replicated
+    state (PlateEngine.get_state_small) and, for a fixed seeded sample of rows (its indices in `rows`), the rows' posterior
+    means and covariances in get_state()'s layout.  The sample keeps the files small at any N (about 32 MB of rows)."""
+    import numpy as np
+    import torch
+    from pyvb_b200.engine import tril_pack_index
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"elbo": eng.trace[slots].cpu().numpy()}
+    out.update(eng.get_state_small())
+    q = eng.q
+    n = min(eng.N, DUMP_ROW_BYTES // (8 * (q + q * q)))
+    rows = np.sort(np.random.RandomState(seed).choice(eng.N, n, replace=False))
+    dev = eng.Zbar.device
+    it = torch.as_tensor(rows, device=dev)
+    z = eng.Zbar[it].to(torch.float64)
+    ii, jj = tril_pack_index(q)
+    if eng.Sig is not None:
+        sp = eng.Sig[it]
+    else:
+        sp = eng.M2[it].to(torch.float64) - z[:, torch.as_tensor(ii, device=dev)] * z[:, torch.as_tensor(jj, device=dev)]
+    sp = sp.cpu().numpy()
+    Sig = np.zeros((n, q, q))
+    Sig[:, ii, jj] = sp
+    Sig[:, jj, ii] = sp
+    out.update(rows=rows, Zbar=z.cpu().numpy(), Sig=Sig)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
+    return sorted(out)
+
+
+def measure_config(torch, dist, dev, rank, world, local, lib, _cabi, cfg, steps, warmup, sampler, hbm, peak_tf, traffic_json,
+                   dump_dir=None):
+    """Build the engine of one configuration on this rank's shard, time `steps` sweeps, break the sweep down; with
+    `dump_dir` (rank 0) the outputs of the timed sweeps are written there before anything else runs on the engine."""
     from pyvb_b200 import PlateEngine
     N, D, q = cfg["N"], cfg["D"], cfg["q"]
     X = make_data(torch, N, D, q, cfg["missing"], 1234, dev, rank=rank)
@@ -635,6 +672,8 @@ def measure_config(torch, dist, dev, rank, world, local, lib, _cabi, cfg, steps,
         eng.distributed = False
     ms, slots, win = timed_sweeps(torch, dist, dev, eng, steps, warmup)
     eng.check()
+    if dump_dir is not None and rank == 0:
+        dump_outputs(eng, slots, dump_dir)
     elbo = [float(v) for v in eng.trace[slots].cpu().tolist()]
     kt = kernel_breakdown(torch, dev, eng, lib, _cabi, N)
     roof, table = rooflines(eng, kt, N, ms / steps, hbm, peak_tf, traffic_json)
@@ -677,7 +716,7 @@ def run_ours(a):
     # ---- headline: BASELINE.json configs[1] (or the --N/--D/--q override), one shard per GPU
     cfg = {"N": a.N, "D": a.D, "q": a.q, "missing": a.missing, "mode": a.mode, "algo": a.algo, "ard": a.ard}
     eng, head, win = measure_config(torch, dist, dev, rank, world, local, lib, _cabi, cfg, a.steps, a.warmup, sampler, hbm,
-                                    peak_tf, traffic_json)
+                                    peak_tf, traffic_json, dump_dir=a.dump_outputs)
     clocks = sampler.stop(*win) if sampler is not None else None
     e2e = bench_e2e(torch, dist, dev, eng, local, max(1, min(a.steps, 8))) if a.mode == "B" else None
 
@@ -784,7 +823,13 @@ def main():
     ap.add_argument("--quick", action="store_true", help="headline + e2e only (profiling runs)")
     ap.add_argument("--no-c4", dest="no_c4", action="store_true", help="skip the config-4-shape object (q = 64, ARD)")
     ap.add_argument("--ard", action="store_true", help="ARD Gamma precisions per latent column (config 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the headline's timed sweeps (last state, bounds) to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs is not None and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of our arm (--impl ours)")
     if a.impl == "reference":
         run_reference(a)
     else:

@@ -160,6 +160,44 @@ def test_zsums_buffer_covers_every_k2_kernel_and_configuration(monkeypatch):
                 assert need <= size, (q, N, env, need, size)
 
 
+class _DumpEngine(object):
+    """Stands in for PlateEngine in bench.dump_outputs (host tensors, keep_sigma=False layout)."""
+    def __init__(self, N, D, q, seed):
+        import torch
+        rng = np.random.RandomState(seed)
+        ii, jj = np.tril_indices(q)
+        self.N, self.q, self.Sig = N, q, None
+        self.Zbar = torch.as_tensor(rng.randn(N, q))
+        self.sig_packed = rng.rand(N, len(ii))
+        self.M2 = torch.as_tensor(self.sig_packed + self.Zbar.numpy()[:, ii] * self.Zbar.numpy()[:, jj])
+        self.trace = torch.as_tensor(rng.randn(16))
+        self.small = {"Wbar": rng.randn(D, q), "mu": rng.randn(D), "qb": 0.5, "alpha": np.ones(q)}
+
+    def get_state_small(self):
+        return self.small
+
+
+@pytest.mark.parametrize("N,q", [(50, 3), (20000, 64)])
+def test_bench_dump_outputs_writes_a_fixed_row_sample_in_float64(tmp_path, N, q):
+    import bench
+    e = _DumpEngine(N, 8, q, seed=1)
+    names = bench.dump_outputs(e, [5, 6, 7], str(tmp_path / "a"))
+    bench.dump_outputs(_DumpEngine(N, 8, q, seed=1), [5, 6, 7], str(tmp_path / "b"))
+    total = 0
+    for name in names:
+        a = np.load(str(tmp_path / "a" / (name + ".npy")))
+        assert a.dtype == np.float64 and np.array_equal(a, np.load(str(tmp_path / "b" / (name + ".npy")))), name
+        total += a.nbytes
+    assert total <= 64 << 20
+    rows = np.load(str(tmp_path / "a" / "rows.npy")).astype(np.int64)
+    assert len(rows) == min(N, bench.DUMP_ROW_BYTES // (8 * (q + q * q))) and np.all(np.diff(rows) > 0)
+    assert np.array_equal(np.load(str(tmp_path / "a" / "elbo.npy")), e.trace.numpy()[5:8])
+    assert np.array_equal(np.load(str(tmp_path / "a" / "Zbar.npy")), e.Zbar.numpy()[rows])
+    Sig = np.load(str(tmp_path / "a" / "Sig.npy"))
+    ii, jj = np.tril_indices(q)
+    assert np.allclose(Sig[:, ii, jj], e.sig_packed[rows], rtol=0, atol=1e-12) and np.array_equal(Sig, Sig.transpose(0, 2, 1))
+
+
 def test_engine_refuses_to_run_without_gpu():
     import torch
     if torch.cuda.is_available():
