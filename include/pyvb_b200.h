@@ -239,14 +239,17 @@ int pyvb_zstep_i8_f64(long long N, int D, int q, const double *X, long long ldx,
  * treats as optional: xcache (valid: the X-only sums of an earlier pyvb_stats_f64 call).  zsums: the K2 partials of the
  * Z step that produced these rows, or NULL (then logdet [N] is read and the MZ column sums take one more pass).
  *   maskT  pyvb_stats_i8_maskt_bytes(N, D) bytes, [n / 64][D][64] int8: pyvb_prepare_maskt_i8 (once per data set)
- *   ZI     pyvb_stats_i8_digits_bytes(N, q) bytes, scratch pyvb_stats_i8_scratch_len(q) doubles: per-call scratch; the
- *          caller ZEROES scratch once (its last 8 doubles are the guard's counters, kept from call to call)
+ *   ZI     pyvb_stats_i8_digits_bytes(N, q) bytes, per-call scratch; NULL is allowed where pyvb_stats_i8_fused(D, q) is 1
+ *          (D <= 256: the digit planes are made in shared memory; PYVB_I8_FUSED=0, read on every call, turns that off)
+ *   scratch pyvb_stats_i8_scratch_len(q) doubles: per-call scratch; the caller ZEROES it once (its last 8 doubles are the
+ *          guard's counters, kept from call to call)
  *   ws     pyvb_stats_i8_workspace_bytes(N, D, q)
  * Accuracy guard, as for pyvb_zstep_i8_f64: a data dimension d with cnt_d * max_c zscale_c * 2^-55 > 2^-38 * max_i T1[d][ii]
  * (outlier rows that d does not observe) sends the whole pass to the FP64 tensor cores, before the exchange. */
 int pyvb_stats_i8_supported(int D, int q);
 long long pyvb_stats_i8_npad(long long N);
 size_t pyvb_stats_i8_digits_bytes(long long N, int q);
+int pyvb_stats_i8_fused(int D, int q);
 size_t pyvb_stats_i8_maskt_bytes(long long N, int D);
 size_t pyvb_stats_i8_scratch_len(int q);
 size_t pyvb_stats_i8_guard_offset(int q);   /* scratch[off] = data dimensions that failed the guard in the last call, [off+1] = fall-backs so far */

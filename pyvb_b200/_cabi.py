@@ -52,6 +52,7 @@ SIGNATURES = {
     "pyvb_stats_i8_supported": (c_int, [c_int, c_int]),
     "pyvb_stats_i8_npad": (c_ll, [c_ll]),
     "pyvb_stats_i8_digits_bytes": (c_sz, [c_ll, c_int]),
+    "pyvb_stats_i8_fused": (c_int, [c_int, c_int]),
     "pyvb_stats_i8_maskt_bytes": (c_sz, [c_ll, c_int]),
     "pyvb_stats_i8_scratch_len": (c_sz, [c_int]),
     "pyvb_stats_i8_guard_offset": (c_sz, [c_int]),

@@ -384,6 +384,7 @@ int pyvb_zstep_i8_f64(long long N, int D, int q, const double *X, long long ldx,
 int pyvb_stats_i8_supported(int D, int q) { return (stats_i8_supported(D, q) && dmma_supported(D, q)) ? 1 : 0; }
 long long pyvb_stats_i8_npad(long long N) { return stats_i8_npad(N); }
 size_t pyvb_stats_i8_digits_bytes(long long N, int q) { return stats_i8_digits_bytes(N, q); }
+int pyvb_stats_i8_fused(int D, int q) { return (pyvb_stats_i8_supported(D, q) && stats_i8_fused(D)) ? 1 : 0; }
 size_t pyvb_stats_i8_maskt_bytes(long long N, int D) { return stats_i8_maskt_bytes(N, D); }
 size_t pyvb_stats_i8_scratch_len(int q) { return stats_i8_scratch_len(q, pyvb_mz_pitch(q)); }
 size_t pyvb_stats_i8_guard_offset(int q) {
@@ -424,7 +425,8 @@ int pyvb_stats_i8_f64(long long N, int D, int q, const double *X, long long ldx,
                                      peers ? peers->epoch : 0ULL, st);
         return e0 == cudaSuccess ? PYVB_OK : cuda_fail(e0, "stats_i8 (empty shard)");
     }
-    ARG(X && maskT && MZ && ZI && scratch && xcache, "null pointer (xcache is required)");
+    ARG(X && maskT && MZ && scratch && xcache, "null pointer (xcache is required)");
+    ARG(ZI || stats_i8_fused(D), "ZI is required where pyvb_stats_i8_fused(D, q) is 0");
     ARG(zsums || logdet, "zsums or logdet");
     ARG(logdet || k2_impl(q) >= 1, "logdet is needed when the K2 partials carry no column maxima");
     ARG(ldx >= D && (ldx % 2) == 0 && ldmz == pyvb_mz_pitch(q), "ldx, ldmz");

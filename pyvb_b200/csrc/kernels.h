@@ -149,6 +149,7 @@ double *stats_i8_guard(double *scratch, int q, int ldmz);   // [0] data dimensio
 cudaError_t launch_stats_i8_check(int D, int q, const double *ws, int nchunks, const double *xcache, double *scratch,
                                   int ldmz, double tol, cudaStream_t st);
 int stats_i8_nchunks(long long N, int D, int q);
+bool stats_i8_fused(int D);                                 // launch_stats_i8 makes the digit planes in shared memory (ZI unused)
 cudaError_t launch_prepare_maskT_i8(long long N, int D, const double *X, long long ldx, void *maskT, cudaStream_t st);
 cudaError_t launch_stats_i8(long long N, int D, int q, const void *maskT, const double *MZ, int ldmz, void *ZI,
                             double *scratch, double *ws, int nchunks, const double *zsums, int nzblk, int zkw, int trusted,

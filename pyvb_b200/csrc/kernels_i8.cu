@@ -1099,6 +1099,268 @@ stats_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     }
 }
 
+// K3-i8 with the digit planes made in shared memory (D <= 256: at most two blocks of 128 data dimensions).  digitize_kernel
+// writes 7 bytes per MZ entry to ZI and stats_i8_kernel reads them back (1.1 GB each way per sweep at N = 1M, q = 16), for
+// data that only ever feeds the MMA.  Here converter warps read the MZ rows with coalesced loads and write the digit tile
+// straight into the ring stage, byte for byte the SWIZZLE_64B image TMA delivered from ZI (oracle/i8_fused_oracle.py).
+// Work item = (column tile of 32, row chunk) over ALL blocks of data dimensions: each digit tile is made once and feeds
+// the MMAs of both blocks (two TMEM accumulators of 224 columns).  Same chunks and the same integer sums as
+// stats_i8_kernel, recombined by the same epilogue: bit-identical partials.
+// Warps: 0 TMA producer (the maskT tiles), 1 MMA issuer, 2-9 epilogue, 10-17 converters (two groups of four that take
+// alternate K steps, a warp = 16 rows of a 64-row step).  Ring stage = [maskT block 0 | maskT block 1 | digit tile].
+constexpr int SF_CONV = 8;
+constexpr int SF_NTHR = (2 + 8 + SF_CONV) * 32;
+constexpr int SF_STG = 2 * A_B + B_B;                    // 30 KB
+constexpr int SF_NSMAX = 8;
+
+int sf_stages(int q) {
+    const size_t fixed = 1024 + (size_t)stats_i8_ncols(q) * 8 + (size_t)(2 * SF_NSMAX + 2) * 8 + 16;
+    const int ns = (int)((227 * 1024 - fixed) / SF_STG);
+    return ns < SF_NSMAX ? ns : SF_NSMAX;
+}
+size_t sf_smem_bytes(int q, int ns) {
+    return 1024 + (size_t)ns * SF_STG + (size_t)stats_i8_ncols(q) * 8 + (size_t)(2 * ns + 2) * 8 + 16;
+}
+
+__global__ void __launch_bounds__(SF_NTHR, 1)
+stats_i8_fused_kernel(const __grid_constant__ CUtensorMap tmA, long long N, int D, int q, const double *__restrict__ MZ, int ldmz,
+                      const double *__restrict__ zscale, double *__restrict__ ws, long long rows_per_chunk, int nchunks,
+                      int ndb, int nct, int ns) {
+    extern __shared__ unsigned char smem_dyn[];
+    unsigned char *smem = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
+    const int P = i_tri(q), NCZ = nct * CT;
+    unsigned char *st_base = smem;                                             // [ns][A0 8 KB | A1 8 KB | B 14 KB]
+    double *fcol = reinterpret_cast<double *>(smem + (size_t)ns * SF_STG);    // [NCZ]: zscale_c * 2^-54
+    uint64_t *full = reinterpret_cast<uint64_t *>(fcol + NCZ);                // [ns]: producer (tx bytes) + 4 converter warps
+    uint64_t *empty = full + ns;                                               // [ns]: MMA commit
+    uint64_t *tfull = empty + ns;
+    uint64_t *tempty = tfull + 1;
+    uint32_t *tbase = reinterpret_cast<uint32_t *>(tempty + 1);
+
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int nitems = nct * nchunks;
+    for (int c = tid; c < NCZ; c += SF_NTHR) fcol[c] = zscale[c] * 5.5511151231257827e-17;   // 2^-54
+    if (tid == 0) {
+        tma_prefetch_desc(&tmA);
+        for (int s = 0; s < ns; ++s) {
+            mbar_init(&full[s], 1 + SF_CONV / 2);
+            mbar_init(&empty[s], 1);
+        }
+        mbar_init(tfull, 1);
+        mbar_init(tempty, 8);
+        mbar_fence_init();
+    }
+    if (warp == 1) umma::tmem_alloc(tbase, 512);
+    umma::fence_before_sync();
+    __syncthreads();
+    umma::fence_after_sync();
+    const uint32_t tmem = *tbase;
+
+    // item -> (chunk, column tile), chunk-major as in stats_i8_kernel; K steps of the chunk
+    auto item_geom = [&](int item, int &chunk, int &ct, long long &r0, int &nsteps) {
+        chunk = item / nct;
+        ct = item - chunk * nct;
+        r0 = (long long)chunk * rows_per_chunk;
+        long long r1 = r0 + rows_per_chunk;
+        if (r1 > N) r1 = N;
+        nsteps = (r1 > r0) ? (int)((r1 - r0 + BKB - 1) / BKB) : 0;
+    };
+
+    if (warp == 0) {
+        // TMA producer: the maskT tiles (128 data dimensions x 64 rows) of every block
+        const bool leader = elect_one();
+        int s = 0;
+        uint32_t ph = 0;
+        for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
+            int chunk, ct, nsteps;
+            long long r0;
+            item_geom(item, chunk, ct, r0, nsteps);
+            for (int k = 0; k < nsteps; ++k) {
+                umma::mbar_wait_bounded(&empty[s], ph ^ 1);
+                if (leader) {
+                    mbar_arrive_expect_tx(&full[s], (uint32_t)(ndb * A_B));
+                    const long long kb = r0 / BKB + k;
+                    for (int b = 0; b < ndb; ++b)
+                        tma_load_3d_i8(st_base + (size_t)s * SF_STG + b * A_B, &tmA, 0, (int)(kb * D + b * BM), 0, &full[s]);
+                }
+                __syncwarp();
+                if (++s == ns) {
+                    s = 0;
+                    ph ^= 1;
+                }
+            }
+        }
+    } else if (warp == 1) {
+        // MMA issuer: per K step two MMAs (K = 2 x 32 bytes) per block of data dimensions, on the same digit tile
+        const bool leader = elect_one();
+        const uint32_t idesc = umma::idesc_s8_s32(BM, NPL * CT);
+        const uint64_t adesc0 = umma::desc_kmajor_sw64(smem_u32(st_base), 0);
+        const uint64_t bdesc0 = umma::desc_kmajor_sw64(smem_u32(st_base + 2 * A_B), 0);
+        int s = 0, tl = 0;
+        uint32_t ph = 0;
+        for (int item = blockIdx.x; item < nitems; item += gridDim.x, ++tl) {
+            int chunk, ct, nsteps;
+            long long r0;
+            item_geom(item, chunk, ct, r0, nsteps);
+            umma::mbar_wait_bounded(tempty, (uint32_t)((tl & 1) ^ 1));       // the epilogue has drained the accumulators
+            umma::fence_after_sync();
+            for (int k = 0; k < nsteps; ++k) {
+                umma::mbar_wait_bounded(&full[s], ph);
+                umma::fence_after_sync();
+                if (leader) {
+                    const uint64_t off = (uint64_t)((s * SF_STG) >> 4);
+                    for (int b = 0; b < ndb; ++b) {
+                        const uint32_t dacc = tmem + (uint32_t)(b * 256);
+                        const uint64_t ad = adesc0 + off + (uint64_t)(b * (A_B >> 4));
+                        umma::mma_i8(dacc, ad, bdesc0 + off, idesc, k ? 1u : 0u);
+                        umma::mma_i8(dacc, ad + 2, bdesc0 + off + 2, idesc, 1u);
+                    }
+                    umma::mma_commit(&empty[s]);
+                }
+                __syncwarp();
+                if (++s == ns) {
+                    s = 0;
+                    ph ^= 1;
+                }
+            }
+            if (leader) umma::mma_commit(tfull);
+            __syncwarp();
+        }
+    } else if (warp < 10) {
+        // epilogue: the recombination of stats_i8_kernel, for each block of data dimensions
+        const StatLayout L(D, q);
+        const int wq = warp & 3, half = (warp - 2) >> 2;
+        int tl = 0;
+        for (int item = blockIdx.x; item < nitems; item += gridDim.x, ++tl) {
+            int chunk, ct, nsteps;
+            long long r0;
+            item_geom(item, chunk, ct, r0, nsteps);
+            const int c0 = ct * CT + half * 16;
+            double *out = ws + (size_t)chunk * L.len;
+            umma::mbar_wait_bounded(tfull, (uint32_t)(tl & 1));
+            umma::fence_after_sync();
+            for (int b = 0; b < ndb; ++b) {
+                const int d = b * BM + wq * 32 + lane;
+                const uint32_t taddr = tmem + (uint32_t)(b * 256 + half * 16) + ((uint32_t)(wq * 32) << 16);
+#pragma unroll
+                for (int ch = 0; ch < 2; ++ch) {
+                    uint32_t a[NPL][8];
+                    if (nsteps > 0) {                              // an empty chunk contributes zeros (nothing was accumulated)
+#pragma unroll
+                        for (int p = 0; p < NPL; ++p) tmem_ld8(taddr + (uint32_t)(p * CT + ch * 8), a[p]);
+                        umma::tmem_ld_wait();
+                    }
+#pragma unroll
+                    for (int k = 0; k < 8; ++k) {
+                        double v = 0.0;
+                        if (nsteps > 0) {
+#pragma unroll
+                            for (int p = NPL - 1; p >= 0; --p) v = fma(v, 256.0, i2d((int)a[p][k]));
+                        }
+                        const int c = c0 + ch * 8 + k;
+                        if (d < D) {
+                            if (c < P) out[L.t1 + (size_t)d * P + c] = fcol[c] * v;
+                            else if (c < P + q) out[L.bst + (size_t)d * q + (c - P)] = fcol[c] * v;
+                        }
+                    }
+                }
+            }
+            umma::fence_before_sync();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(tempty);
+        }
+    } else {
+        // converters: the arithmetic of digitize_kernel (2^54 / zscale_c, NaN / inf -> 0, zero past row N and column P + q,
+        // the BIAS / xor byte split), written as the SWIZZLE_64B image of the K-major tile: plane p, column l of the tile,
+        // row n of the step at byte (p * 32 + l) * 64 + (((n >> 4) ^ ((l >> 1) & 3)) << 4) + (n & 15).  Warp cw owns rows
+        // 16 (cw % 4) ... + 15 of every other step; a lane owns one column and puts four rows into one 32-bit word per
+        // plane.  Lane group l / 8 starts at row quad l / 8 of the warp's 16 rows (and cycles): with the swizzle the 32 words
+        // of every store instruction fall into 32 different banks.  The loads stay full 32-byte sectors (8 lanes x 8 bytes
+        // of one row per group).  The loads of a warp's next step are issued before it converts the current one: with one
+        // step in flight per warp (32 KB per SM) the HBM latency, not the bandwidth, set the pace.
+        const int cw = warp - 10, grp = cw >> 2, rq = cw & 3, rot = lane >> 3;
+        const int nvalid = P + q;
+        constexpr unsigned long long BIAS = 0x0080808080808080ULL;
+        const uint32_t wbase = (uint32_t)(lane * 64 + ((rq ^ ((lane >> 1) & 3)) << 4));
+        // position (item, K step of the item) of this warp's steps: the CTA's steps j = grp, grp + 2, ... in order
+        struct Pos {
+            int item, k, nsteps, ct;
+            long long r0;
+        };
+        auto settle = [&](Pos &p) {                            // past the end of an item: into the next non-empty one
+            while (p.item < nitems && p.k >= p.nsteps) {
+                p.k -= p.nsteps;
+                p.item += gridDim.x;
+                int chunk;
+                if (p.item < nitems) item_geom(p.item, chunk, p.ct, p.r0, p.nsteps);
+            }
+        };
+        auto load = [&](const Pos &p, double (&x)[16]) {
+            const int c = p.ct * CT + lane;
+            const bool cv = p.item < nitems && c < nvalid;
+            const long long nb = p.r0 + (long long)p.k * BKB + rq * 16;
+#pragma unroll
+            for (int g = 0; g < 4; ++g)
+#pragma unroll
+                for (int kk = 0; kk < 4; ++kk) {
+                    const long long n = nb + 4 * ((g + rot) & 3) + kk;
+                    x[g * 4 + kk] = (cv && n < N) ? __ldcs(MZ + n * ldmz + c) : 0.0;
+                }
+        };
+        Pos cur;
+        cur.item = blockIdx.x;
+        cur.k = grp;
+        cur.nsteps = 0;
+        {
+            int chunk;
+            if (cur.item < nitems) item_geom(cur.item, chunk, cur.ct, cur.r0, cur.nsteps);
+        }
+        settle(cur);
+        double xv[16], xn[16];
+        load(cur, xv);
+        for (int j = grp; cur.item < nitems; j += 2) {
+            Pos nxt = cur;
+            nxt.k += 2;
+            settle(nxt);
+            load(nxt, xn);                                     // in flight while this step is converted
+            const int s = j % ns;
+            umma::mbar_wait_bounded(&empty[s], (uint32_t)(((j / ns) & 1) ^ 1));
+            const int c = cur.ct * CT + lane;
+            const double inv = c < nvalid ? 18014398509481984.0 / zscale[c] : 0.0;    // 2^54 / scale
+            unsigned char *bt = st_base + (size_t)s * SF_STG + 2 * A_B;
+#pragma unroll
+            for (int g = 0; g < 4; ++g) {
+                const int qd = (g + rot) & 3;
+                unsigned int lo[4], hi[4];
+#pragma unroll
+                for (int kk = 0; kk < 4; ++kk) {
+                    double t = xv[g * 4 + kk] * inv;
+                    t = (fabs(t) <= 18014398509481984.0) ? t : 0.0;
+                    const unsigned long long u = ((unsigned long long)__double2ll_rn(t) + BIAS) ^ BIAS;
+                    lo[kk] = (unsigned int)u;
+                    hi[kk] = (unsigned int)(u >> 32);
+                }
+#pragma unroll
+                for (int p = 0; p < NPL; ++p) {
+                    const unsigned int *w = (p < 4) ? lo : hi;
+                    const unsigned int sel = (unsigned)(p & 3) | ((unsigned)(4 + (p & 3)) << 4);
+                    const unsigned int w01 = __byte_perm(w[0], w[1], sel), w23 = __byte_perm(w[2], w[3], sel);
+                    *reinterpret_cast<unsigned int *>(bt + p * (CT * BKB) + wbase + qd * 4) = __byte_perm(w01, w23, 0x5410);
+                }
+            }
+            fence_async_smem();                                 // generic-proxy stores before the MMA's async-proxy reads
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&full[s]);
+            cur = nxt;
+#pragma unroll
+            for (int i = 0; i < 16; ++i) xv[i] = xn[i];
+        }
+    }
+    umma::fence_before_sync();
+    __syncthreads();
+    if (warp == 1) umma::tmem_dealloc(tmem, 512);
+}
+
 
 // ---- microbenchmark: back-to-back tcgen05.mma on fixed shared-memory operands (no loads): the tensor-core rate of the
 // box for kind::i8 (kind = 0) or kind::f16 / bf16 (kind = 1) at M = 128, N = n, one K step of 32 bytes per instruction.
@@ -1353,7 +1615,15 @@ cudaError_t launch_prepare_maskT_i8(long long N, int D, const double *X, long lo
     return cudaGetLastError();
 }
 
+// PYVB_I8_FUSED=0 keeps digitize_kernel + stats_i8_kernel where the fused kernel applies.  Read on every call, so that one
+// process can compare the two paths.
+bool stats_i8_fused(int D) {
+    const char *e = getenv("PYVB_I8_FUSED");
+    return (D + BM - 1) / BM <= 2 && !(e && e[0] == '0');
+}
+
 // colmax -> zscale -> digit planes of the MZ rows -> T1, Bst partial sums of every row chunk in ws[chunk][stat layout]
+// (D <= 256: stats_i8_fused_kernel makes the digit planes in shared memory and ZI is not touched; it may be NULL)
 // zsums (nullable): K2's per-CTA partials [column sums | 4 scalars | bounds on the column maxima] (nzblk partials of zkw
 // doubles).  Without them (or when `trusted` is 0: a K2 kernel that leaves no maxima) one pass over the MZ rows builds the same
 // partials in `scratch` (logdet needed); *zs_out / *nzblk_out / *zkw_out say which partials the second stage must add up.
@@ -1380,27 +1650,45 @@ cudaError_t launch_stats_i8(long long N, int D, int q, const void *maskT, const 
     *nzblk_out = nzblk;
     *zkw_out = zkw;
     colmax_reduce_kernel<<<(NCZ + 7) / 8, 256, 0, st>>>(NCZ, P + q, zkw, zsums + orow + 4, nzblk, zscale);
-    dim3 gd((unsigned)((N + 127) / 128), (unsigned)nct);
-    digitize_kernel<<<gd, 256, 0, st>>>(N, npad, ldmz, P + q, MZ, zscale, static_cast<signed char *>(ZI));
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    CUtensorMap tmA, tmB;
-    {   // tile-major operands: maskT [npad / 64][D][64] (+ one box of slack), ZI [npad / 64][nct][224][64]
-        EncodeTiledFn enc = get_encode_i8();
-        if (!enc) return cudaErrorNotSupported;
-        const cuuint64_t nkb = (cuuint64_t)(npad / BKB);
-        if (nkb * (cuuint64_t)D + BM >= (1ULL << 31) || nkb * nct * (NPL * CT) >= (1ULL << 31)) return cudaErrorNotSupported;
-        cuuint32_t es[3] = {1, 1, 1};
+    const cuuint64_t nkb = (cuuint64_t)(npad / BKB);
+    EncodeTiledFn enc = get_encode_i8();
+    if (!enc) return cudaErrorNotSupported;
+    if (nkb * (cuuint64_t)D + BM >= (1ULL << 31) || nkb * nct * (NPL * CT) >= (1ULL << 31)) return cudaErrorNotSupported;
+    const cuuint32_t es[3] = {1, 1, 1};
+    CUtensorMap tmA;
+    {   // maskT [npad / 64][D][64] (+ one box of slack: the last block of data dimensions may reach past D)
         cuuint64_t da[3] = {BKB, nkb * D + BM, 1}, sa[2] = {BKB, (nkb * D + BM) * BKB};
         cuuint32_t ba[3] = {BKB, BM, 1};
         CUresult r = enc(&tmA, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void *>(maskT), da, sa, ba, es,
                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
+    }
+    const long long rpc = stats_i8_rows_per_chunk(N, nchunks);
+    if (stats_i8_fused(D)) {
+        const int ns = sf_stages(q);
+        const size_t smem = sf_smem_bytes(q, ns);
+        e = cudaFuncSetAttribute(stats_i8_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        const long long nitems = (long long)nct * nchunks;
+        const int grid = (int)(nitems < 148 ? nitems : 148);
+        stats_i8_fused_kernel<<<grid, SF_NTHR, smem, st>>>(tmA, N, D, q, MZ, ldmz, (const double *)zscale, ws, rpc, nchunks, ndb,
+                                                           nct, ns);
+        return cudaGetLastError();
+    }
+    if (ZI == nullptr) return cudaErrorInvalidValue;
+    dim3 gd((unsigned)((N + 127) / 128), (unsigned)nct);
+    digitize_kernel<<<gd, 256, 0, st>>>(N, npad, ldmz, P + q, MZ, zscale, static_cast<signed char *>(ZI));
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    CUtensorMap tmB;
+    {   // ZI [npad / 64][nct][224][64]
         cuuint64_t db[3] = {BKB, nkb * nct * (NPL * CT), 1}, sb[2] = {BKB, nkb * nct * (NPL * CT) * BKB};
         cuuint32_t bb[3] = {BKB, (cuuint32_t)(NPL * CT / i8_cluster_size()), 1};
-        r = enc(&tmB, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, ZI, db, sb, bb, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        CUresult r = enc(&tmB, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, ZI, db, sb, bb, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                         CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
     }
     const int cl = i8_cluster_size();
@@ -1418,8 +1706,8 @@ cudaError_t launch_stats_i8(long long N, int D, int q, const void *maskT, const 
         ks_env = ev ? atoi(ev) : 0;
     }
     const int ks = (ks_env >= 1 && ks_env <= 4) ? ks_env : 2;
-    return launch_cluster(kern, grid, NTHR, smem, cl, st, tmA, tmB, N, D, q, (const double *)zscale, ws,
-                          stats_i8_rows_per_chunk(N, nchunks), nchunks, ndb, nct, ks);
+    return launch_cluster(kern, grid, NTHR, smem, cl, st, tmA, tmB, N, D, q, (const double *)zscale, ws, rpc, nchunks, ndb,
+                          nct, ks);
 }
 
 }  // namespace pyvb

@@ -190,15 +190,18 @@ class PlateEngine(object):
         self.ws_bytes = int(self.lib.pyvb_stats_workspace_bytes(N, D, q, ALGO_F32 if self.f32 else self.algo))
         if self.use_i8_stats:
             # the digit planes cost 7 bytes per MZ entry: when they would take more than 40 % of the free memory (config 4
-            # at full size on one GPU) the statistics stay on the FP64 tensor cores
-            need = int(self.lib.pyvb_stats_i8_digits_bytes(N, q)) + int(self.lib.pyvb_stats_i8_maskt_bytes(N, D))
+            # at full size on one GPU) the statistics stay on the FP64 tensor cores.  At D <= 256 they are made in shared
+            # memory (pyvb_stats_i8_fused) and only the transposed mask is allocated.
+            fused = bool(self.lib.pyvb_stats_i8_fused(D, q))
+            need = int(self.lib.pyvb_stats_i8_maskt_bytes(N, D)) + (0 if fused else int(self.lib.pyvb_stats_i8_digits_bytes(N, q)))
             if need > 0.4 * torch.cuda.mem_get_info(dev)[0]:
                 self.use_i8_stats = False
         if self.use_i8_stats:
             try:
                 self.npad = int(self.lib.pyvb_stats_i8_npad(N))
                 self.maskT = torch.empty(int(self.lib.pyvb_stats_i8_maskt_bytes(N, D)), dtype=torch.int8, device=dev)
-                self.ZI = torch.empty(int(self.lib.pyvb_stats_i8_digits_bytes(N, q)), dtype=torch.int8, device=dev)
+                self.ZI = None if fused else torch.empty(int(self.lib.pyvb_stats_i8_digits_bytes(N, q)), dtype=torch.int8,
+                                                         device=dev)
                 # (zeros: the tail of the scratch is the guard block -- counters of the accuracy check -- see the header)
                 self.i8_scratch = torch.zeros(int(self.lib.pyvb_stats_i8_scratch_len(q)), dtype=f64, device=dev)
                 self.ws_bytes = max(self.ws_bytes, int(self.lib.pyvb_stats_i8_workspace_bytes(N, D, q)))
@@ -487,8 +490,11 @@ class PlateEngine(object):
                 _cabi.check(self.lib.pyvb_prepare_maskt_i8(self.N, self.D, self.X.data_ptr(), self.D,
                                                            self.maskT.data_ptr(), self._stream()), "pyvb_prepare_maskt_i8")
                 self._maskT_valid = True
+            if self.ZI is None and not self.lib.pyvb_stats_i8_fused(self.D, self.q):    # PYVB_I8_FUSED=0 set since
+                self.ZI = torch.empty(int(self.lib.pyvb_stats_i8_digits_bytes(self.N, self.q)), dtype=torch.int8,
+                                      device=self.MZ.device)
             rc = self.lib.pyvb_stats_i8_f64(self.N, self.D, self.q, self.X.data_ptr(), self.D, self.maskT.data_ptr(),
-                                            self.MZ.data_ptr(), self.ldmz, self.logdet.data_ptr(), self.ZI.data_ptr(),
+                                            self.MZ.data_ptr(), self.ldmz, self.logdet.data_ptr(), self._p(self.ZI),
                                             self.i8_scratch.data_ptr(), self.stats.data_ptr(), self.ws.data_ptr(),
                                             self.ws_bytes, self.xcache.data_ptr(),
                                             self.zsums.data_ptr() if (self.zsums is not None and self._zsums_valid) else 0,
