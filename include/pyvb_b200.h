@@ -293,6 +293,38 @@ int pyvb_stats_f32(long long N, long long nalloc, int D, int q, const void *plan
                    void *ws, size_t ws_bytes, double *xcache, const double *zsums, const pyvb_peers *peers /* host */,
                    void *stream);
 
+/* ---- sparse observations (mode B, FP64, q in {8, 16, 32, 64}, any D) ----
+ * The stored entries of a CSR matrix are the observations (a stored zero is an observed 0); everything not stored is
+ * missing.  The work of a sweep is per stored entry: the Z step gathers one Gw row per entry of its row, the statistics
+ * gather one MZ row per entry of their column.  The callers own and validate the layouts (pyvb_b200/sparse.py builds them):
+ * column indices in [0, D), sorted within a row, no duplicates, finite values.  Both calls are deterministic (fixed
+ * summation order, no atomics).
+ *   CSR       indptr int64 [N + 1] (the rows' own offsets: a row range [lo, hi) passes indptr + lo), indices int32,
+ *             values double
+ *   blocked   the same entries column-major per row block: nblk blocks of pyvb_csr_block_rows(N, D, q) consecutive
+ *   CSC       rows (pyvb_csr_stats_blocks(N, D, q) of them; any nblk >= 1 is valid, these sizes keep a block's MZ rows in
+ *             the L2).  colptr int64 [nblk * D + 1]: the entries of block b, column d are [colptr[b*D + d],
+ *             colptr[b*D + d + 1]) of rows int32 (row index within these N rows, increasing) / vals double
+ *   xcache    2*D + 2 doubles [cnt (D) | colsumX (D) | sum x^2 | number of stored entries] of these N rows, computed once by
+ *             the caller (the layout of pyvb_stats_f64's cache)
+ * pyvb_zstep_csr_f64: MZ rows [0, N) <- [qprec packed | 0 | eta] (rows without entries get the prior), then the batched
+ * solve in place as pyvb_zsolve_f64 (zsums, Sig nullable as there).
+ * pyvb_stats_csr_f64: T1 | Bst | Ast per row block, then the shared second stage with xcache and the optional peer exchange.
+ * zsums: the K2 partials of the pyvb_zstep_csr_f64 call that covered exactly these N rows, or NULL (then the MZ column sums
+ * and the log-det scalars take one pass each over MZ / logdet).  ws: pyvb_stats_csr_workspace_bytes(N, D, q, nblk).  An
+ * empty shard (N = 0) contributes zeros and still takes part in the exchange. */
+int pyvb_csr_supported(int D, int q);
+int pyvb_csr_stats_blocks(long long N, int D, int q);
+long long pyvb_csr_block_rows(long long N, int D, int q);
+size_t pyvb_stats_csr_workspace_bytes(long long N, int D, int q, int nblk);
+int pyvb_zstep_csr_f64(long long N, int D, int q, const long long *indptr, const int *indices, const double *values,
+                       const double *Gw, int ldg, const double *P0, const double *h0, double *gl, double *MZ,
+                       long long ldmz, double *Sig, double *logdet, double *zsums, void *stream);
+int pyvb_stats_csr_f64(long long N, int D, int q, int nblk, const long long *colptr, const int *rows, const double *vals,
+                       const double *MZ, long long ldmz, const double *logdet, double *stats, void *ws, size_t ws_bytes,
+                       const double *xcache, const double *zsums, const pyvb_peers *peers /* host, nullable */,
+                       void *stream);
+
 /* ---- VB smoother of a linear dynamic system, batched over B independent sequences (BASELINE config 5) ----
  * Replaces the sweep of examples/Linear_Dynamic_System.py:69-76 for every sequence: all X_t.update() forwards, all
  * backwards (nodes/gaussian.py:102-123 + nodes/node.py:203-227), the columns of A and C (nodes/nodes_todo.py:43-62),

@@ -70,6 +70,14 @@ SIGNATURES = {
     "pyvb_zsums_len_f32": (c_sz, [c_ll, c_int]),
     "pyvb_zstep_f32": (c_int, [c_ll, c_ll, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp]),
     "pyvb_stats_f32": (c_int, [c_ll, c_ll, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_sz, c_dp, c_dp, ctypes.POINTER(Peers), c_dp]),
+    "pyvb_csr_supported": (c_int, [c_int, c_int]),
+    "pyvb_csr_stats_blocks": (c_int, [c_ll, c_int, c_int]),
+    "pyvb_csr_block_rows": (c_ll, [c_ll, c_int, c_int]),
+    "pyvb_stats_csr_workspace_bytes": (c_sz, [c_ll, c_int, c_int, c_int]),
+    "pyvb_zstep_csr_f64": (c_int, [c_ll, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_int, c_dp, c_dp, c_dp, c_dp, c_ll, c_dp,
+                                   c_dp, c_dp, c_dp]),
+    "pyvb_stats_csr_f64": (c_int, [c_ll, c_int, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_ll, c_dp, c_dp, c_dp, c_sz, c_dp,
+                                   c_dp, ctypes.POINTER(Peers), c_dp]),
     "pyvb_lds_max_len": (c_int, []),
     "pyvb_lds_iterate_f64": (c_int, [c_int, c_int, c_int, c_int] + [c_dp] * 11 + [ctypes.c_double] * 3 + [c_int, c_dp, c_dp]),
     "pyvb_lds_iterate_known_f64": (c_int, [c_int, c_int, c_int, c_int] + [c_dp] * 12 + [ctypes.c_double] * 3 + [c_int, c_dp, c_dp]),

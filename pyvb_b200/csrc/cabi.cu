@@ -472,6 +472,79 @@ int pyvb_stats_i8_f64(long long N, int D, int q, const double *X, long long ldx,
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "stats_reduce");
 }
 
+int pyvb_csr_supported(int D, int q) { return (D >= 1 && csr_supported(q)) ? 1 : 0; }
+int pyvb_csr_stats_blocks(long long N, int D, int q) { return csr_stats_nblocks(N, D, q); }
+long long pyvb_csr_block_rows(long long N, int D, int q) { return csr_block_rows(N, D, q); }
+size_t pyvb_stats_csr_workspace_bytes(long long N, int D, int q, int nblk) {
+    const StatLayout L(D, q);
+    if (N <= 0) return align256((L.len + PYVB_NSCAL) * sizeof(double));
+    return align256((size_t)(nblk < 1 ? 1 : nblk) * L.len * sizeof(double)) +
+           align256((size_t)rowscalars_nblk(N) * PYVB_NSCAL * sizeof(double));
+}
+
+int pyvb_zstep_csr_f64(long long N, int D, int q, const long long *indptr, const int *indices, const double *values,
+                       const double *Gw, int ldg, const double *P0, const double *h0, double *gl, double *MZ,
+                       long long ldmz, double *Sig, double *logdet, double *zsums, void *stream) {
+    ARG(N >= 0 && D >= 1, "N, D");
+    if (!csr_supported(q)) return fail(PYVB_ENOSUP, "%s", "the CSR path needs q in {8, 16, 32, 64}");
+    if (N == 0) return PYVB_OK;
+    ARG(indptr && indices && values && Gw && P0 && h0 && gl && MZ && logdet, "null pointer");
+    ARG(ldg == pyvb_gw_pitch(q) && ldmz == pyvb_mz_pitch(q), "ldg / ldmz must equal pyvb_gw_pitch(q) / pyvb_mz_pitch(q)");
+    ARG((reinterpret_cast<uintptr_t>(Gw) & 15) == 0 && (reinterpret_cast<uintptr_t>(MZ) & 15) == 0,
+        "Gw and MZ must be 16-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = launch_zstep_csr(N, q, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, (int)ldmz, st);
+    if (e == cudaSuccess) e = launch_zsolve(N, q, MZ, Sig, logdet, gl, zsums, st);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zstep_csr");
+}
+
+int pyvb_stats_csr_f64(long long N, int D, int q, int nblk, const long long *colptr, const int *rows, const double *vals,
+                       const double *MZ, long long ldmz, const double *logdet, double *stats, void *ws, size_t ws_bytes,
+                       const double *xcache, const double *zsums, const pyvb_peers *peers, void *stream) {
+    ARG(N >= 0 && D >= 1, "N, D");
+    if (!csr_supported(q)) return fail(PYVB_ENOSUP, "%s", "the CSR path needs q in {8, 16, 32, 64}");
+    ARG(stats && ws, "null pointer");
+    ARG(peers == NULL || (peers->bufs != NULL && peers->world >= 1 && peers->rank >= 0 && peers->rank < peers->world &&
+                          peers->world <= 256 && peers->epoch >= 1),
+        "peers");
+    const StatLayout L(D, q);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (N == 0) {
+        // an empty shard contributes zeros, but still takes part in the exchange
+        ARG(ws_bytes >= (L.len + PYVB_NSCAL) * sizeof(double), "workspace too small");
+        cudaError_t e0 = cudaMemsetAsync(ws, 0, (L.len + PYVB_NSCAL) * sizeof(double), st);
+        if (e0 == cudaSuccess)
+            e0 = launch_stats_reduce(D, q, (const double *)ws, 1, (const double *)ws + L.len, 1, stats, NULL, 0, NULL, 0, 0,
+                                     peers ? peers->bufs : NULL, peers ? peers->world : 1, peers ? peers->rank : 0,
+                                     peers ? peers->epoch : 0ULL, st);
+        return e0 == cudaSuccess ? PYVB_OK : cuda_fail(e0, "stats_csr (empty shard)");
+    }
+    ARG(nblk >= 1 && colptr && rows && vals && MZ && xcache, "nblk, null pointer (xcache is required)");
+    ARG(zsums || logdet, "zsums or logdet");
+    ARG(ldmz == pyvb_mz_pitch(q) && (reinterpret_cast<uintptr_t>(MZ) & 15) == 0, "ldmz must equal pyvb_mz_pitch(q), MZ 16-byte aligned");
+    ARG(ws_bytes >= pyvb_stats_csr_workspace_bytes(N, D, q, nblk), "workspace too small");
+    double *ws_main = (double *)ws;
+    cudaError_t e = launch_stats_csc(D, q, nblk, colptr, rows, vals, MZ, (int)ldmz, ws_main, st);
+    if (e != cudaSuccess) return cuda_fail(e, "stats_csr");
+    int nzblk = 0, zkw = 0;
+    if (zsums) zsolve_partials(N, q, nzblk, zkw);
+    // without K2's partials: S, zsum from one pass over the MZ rows, the log-det scalars from the per-row pass (which reads
+    // no X with skip_x set)
+    double *ws_sc = NULL;
+    const int nsc = rowscalars_nblk(N);
+    if (nzblk == 0) {
+        ws_sc = (double *)((char *)ws + align256((size_t)nblk * L.len * sizeof(double)));
+        const int gz = gw_woff(q);
+        e = launch_mzsums(N, D, q, MZ + gz, ldmz, MZ, ldmz, ws_main, nblk, st);
+        if (e == cudaSuccess) e = launch_rowscalars(N, D, NULL, D, NULL, NULL, NULL, logdet, ws_sc, nsc, 1, st);
+        if (e != cudaSuccess) return cuda_fail(e, "stats_csr (row sums)");
+    }
+    e = launch_stats_reduce(D, q, ws_main, nblk, ws_sc, nsc, stats, const_cast<double *>(xcache), 1,
+                            nzblk > 0 ? zsums : NULL, nzblk, zkw, peers ? peers->bufs : NULL, peers ? peers->world : 1,
+                            peers ? peers->rank : 0, peers ? peers->epoch : 0ULL, st);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "stats_reduce");
+}
+
 int pyvb_f32_pitch(int q) { return f32_ncp(q); }
 int pyvb_f32_zoff(int q) { return f32_zoff(q); }
 int pyvb_f32_poff(int q) { return f32_poff(q); }

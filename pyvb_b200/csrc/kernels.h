@@ -157,6 +157,18 @@ cudaError_t launch_stats_i8(long long N, int D, int q, const void *maskT, const 
 cudaError_t launch_stats_x_dmma(long long N, int D, int q, const double *X, long long ldx, const double *MZ,
                                 double *ws_main, int nchunks, cudaStream_t st);
 
+// ---- sparse observations: CSR gather for the Z step, row-blocked CSC gather for the statistics (kernels_sparse.cu) ----
+bool csr_supported(int q);                                  // q in {8, 16, 32, 64} (the q of launch_zsolve)
+int csr_stats_nblocks(long long N, int D, int q);           // row blocks of the column-major layout (partials of K3-csc)
+long long csr_block_rows(long long N, int D, int q);        // rows per block (the last one may hold fewer)
+// MZ rows [0, N) <- [qprec packed | 0 | eta], the input of launch_zsolve
+cudaError_t launch_zstep_csr(long long N, int q, const long long *indptr, const int *indices, const double *values,
+                             const double *Gw, int ldg, const double *P0, const double *h0, const double *gl, double *MZ,
+                             int ldmz, cudaStream_t st);
+// T1 | Bst | Ast of every row block b into ws_main[b][statlen] (the other entries of the partials are not written)
+cudaError_t launch_stats_csc(int D, int q, int nblk, const long long *colptr, const int *rows, const double *vals,
+                             const double *MZ, int ldmz, double *ws_main, cudaStream_t st);
+
 // ---- LDS smoother, batched over sequences (kernels_lds.cu) ----
 size_t lds_smem_bytes(int T, int d);
 cudaError_t launch_lds_iterate(int B, int T, int q, int d, const double *Y, double *X, double *Xcov3, double *A,

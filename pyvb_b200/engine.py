@@ -23,6 +23,7 @@ import numpy as np
 import torch
 
 from . import _cabi
+from . import sparse as _sparse
 import os
 
 from .dist import PeerExchange, allreduce_stats
@@ -63,6 +64,9 @@ class PlateEngine(object):
     Parameters
     ----------
     X : (N, D) array or tensor, NaN = missing.  The local row shard.
+        Or a sparse matrix (scipy.sparse, any format; torch sparse CSR, host or device): the STORED entries are the
+        observations (a stored zero is an observed 0), everything not stored is missing.  Sparse input runs the CSR
+        gather kernels (kernels_sparse.cu): mode "B", precision "f64", q in {8, 16, 32, 64}, algo "auto", any D.
     q : latent dimension (<= 64)
     mode : "B" masked/marginalised (throughput path) or "A" reference-exact imputation
     distributed : all-reduce the statistics over torch.distributed's default group
@@ -89,6 +93,16 @@ class PlateEngine(object):
     def _construct(self, X, q, mode, alpha0, alpha_mu, a0, b0, ard, ard_a0, ard_b0, P0, m0, algo, keep_sigma,
                    distributed, row_offset, trace_len):
         self.mode, self.q, self.ard = mode, int(q), bool(ard)
+        self.sparse = _sparse.is_sparse(X)
+        if self.sparse:
+            if mode != "B":
+                raise ValueError("sparse input needs mode='B' (mode A imputes every missing entry: pass a dense array)")
+            if self.f32:
+                raise ValueError("sparse input needs precision='f64'")
+            if int(q) not in (8, 16, 32, 64):
+                raise ValueError("sparse input needs q in (8, 16, 32, 64), got %d" % int(q))
+            if algo != "auto":
+                raise ValueError("sparse input needs algo='auto' (the CSR kernels are the only sparse path)")
         # algo "i8": the mask contraction of the Z step on the INT8 tensor cores (exact, kernels_i8.cu); the rest as "dmma".
         # "auto" picks it when the shape allows (PYVB_I8=0 keeps the all-DMMA path)
         self.use_i8 = (algo == "i8")
@@ -101,10 +115,14 @@ class PlateEngine(object):
         self.row_offset = int(row_offset)
         f64 = torch.float64
         dev = self.device
-        Xt = torch.as_tensor(X)
-        assert Xt.dim() == 2
-        Xt = Xt.to(device=dev, dtype=f64).contiguous()
-        self.N, self.D = int(Xt.shape[0]), int(Xt.shape[1])
+        if self.sparse:
+            self.csr = _sparse.to_csr(X, device=dev)         # validated: finite values, no duplicates, columns in [0, D)
+            self.N, self.D = self.csr.N, self.csr.D
+        else:
+            Xt = torch.as_tensor(X)
+            assert Xt.dim() == 2
+            Xt = Xt.to(device=dev, dtype=f64).contiguous()
+            self.N, self.D = int(Xt.shape[0]), int(Xt.shape[1])
         N, D = self.N, self.D
         self.P = q * (q + 1) // 2
         self.L = StatLayout(D, q)
@@ -113,9 +131,15 @@ class PlateEngine(object):
         self.ard_a0, self.ard_b0 = float(ard_a0), float(ard_b0)
 
         # ---- data
-        obs = ~torch.isnan(Xt)
-        n_obs_local = int(obs.sum().item())
-        if self.f32:
+        obs = None if self.sparse else ~torch.isnan(Xt)
+        n_obs_local = int(self.csr.values.numel()) if self.sparse else int(obs.sum().item())
+        if self.sparse:
+            # the statistics read the entries column-major per row block (K3-csc); the X-only sums are taken once, here
+            self.csc = _sparse.block_csc(self.csr, int(self.lib.pyvb_csr_block_rows(N, D, q)))
+            self.xcache_sparse = _sparse.x_cache(self.csr).to(dev)
+            self.Xorig, self.X, self.V, self.qldX = None, None, None, None
+            n_eff_local = n_obs_local
+        elif self.f32:
             # FP32 variant (tcgen05): the data live as three bf16 planes (mask | x_h | x_m); the sums that depend on
             # X alone are taken once, here, in FP64
             if mode != "B" or not self.lib.pyvb_f32_supported(self.D, q) or q not in (16, 32):
@@ -144,7 +168,7 @@ class PlateEngine(object):
             self.qldX = None
             n_eff_local = n_obs_local
         del obs
-        i8_ok = bool(self.lib.pyvb_i8_supported(D, q)) and mode == "B" and not self.f32
+        i8_ok = bool(self.lib.pyvb_i8_supported(D, q)) and mode == "B" and not self.f32 and not self.sparse
         if self.use_i8 is None:
             self.use_i8 = i8_ok
         elif self.use_i8 and not i8_ok:
@@ -188,6 +212,8 @@ class PlateEngine(object):
         self.stats = torch.zeros(self.L.len, dtype=f64, device=dev)
         assert self.L.len == int(self.lib.pyvb_stats_len(D, q))
         self.ws_bytes = int(self.lib.pyvb_stats_workspace_bytes(N, D, q, ALGO_F32 if self.f32 else self.algo))
+        if self.sparse:
+            self.ws_bytes = int(self.lib.pyvb_stats_csr_workspace_bytes(N, D, q, self.csc.nblk))
         if self.use_i8_stats:
             # the digit planes cost 7 bytes per MZ entry: when they would take more than 40 % of the free memory (config 4
             # at full size on one GPU) the statistics stay on the FP64 tensor cores.  At D <= 256 they are made in shared
@@ -209,7 +235,12 @@ class PlateEngine(object):
                 self.maskT = self.ZI = self.i8_scratch = None
                 self.use_i8_stats = False
         self.ws = torch.empty(self.ws_bytes, dtype=torch.uint8, device=dev)
-        if self.f32:
+        if self.sparse:
+            self.xcache = self.xcache_sparse
+            self._xcache_valid = True
+            nz = int(self.lib.pyvb_zsums_len(N, q))
+            self.zsums = torch.zeros(nz, dtype=f64, device=dev) if nz > 0 else None
+        elif self.f32:
             self._xcache_valid = True
             nz = int(self.lib.pyvb_zsums_len_f32(N, q))
             self.zsums = torch.zeros(nz, dtype=f64, device=dev)
@@ -380,6 +411,9 @@ class PlateEngine(object):
     @_on_device
     def set_X(self, X):
         """Replace the (mode B) data shard, e.g. from pinned host memory; invalidates the cached X sums."""
+        if self.sparse:
+            raise NotImplementedError("set_X: a sparse engine keeps its entries in the layouts built at construction; "
+                                      "build a new engine for new data")
         assert self.mode == "B" and not self.f32
         self.X.copy_(X, non_blocking=True)
         self._xcache_valid = False
@@ -472,6 +506,20 @@ class PlateEngine(object):
     def _ensure_stats(self):
         if self._stats_fresh:
             return
+        if self.sparse:
+            c = self.csc
+            rc = self.lib.pyvb_stats_csr_f64(self.N, self.D, self.q, c.nblk, c.colptr.data_ptr(), c.rows.data_ptr(),
+                                             c.vals.data_ptr(), self.MZ.data_ptr(), self.ldmz, self.logdet.data_ptr(),
+                                             self.stats.data_ptr(), self.ws.data_ptr(), self.ws_bytes,
+                                             self.xcache.data_ptr(),
+                                             self.zsums.data_ptr() if (self.zsums is not None and self._zsums_valid) else 0,
+                                             self.peers.next() if (self.peers is not None and self.distributed) else None,
+                                             self._stream())
+            _cabi.check(rc, "pyvb_stats_csr_f64")
+            if self.distributed and self.peers is None:
+                allreduce_stats(self.stats)
+            self._stats_fresh = True
+            return
         if self.f32:
             if not self._zsums_valid and self.N > 0:
                 self._zsums_from_state()
@@ -538,6 +586,19 @@ class PlateEngine(object):
         self._ensure_gw()
         q, P, D = self.q, self.P, self.D
         sig = 0 if self.Sig is None else self.Sig.data_ptr() + lo * P * 8
+        if self.sparse:
+            # any row range: K1-csr owns whole rows, so [lo, hi) is a pointer offset into the row offsets
+            full = (lo == 0 and hi == self.N and self.zsums is not None)
+            self._zsums_valid = False
+            rc = self.lib.pyvb_zstep_csr_f64(hi - lo, D, q, self.csr.indptr.data_ptr() + lo * 8,
+                                             self.csr.indices.data_ptr(), self.csr.values.data_ptr(), self.Gw.data_ptr(),
+                                             self.ldg, self.P0.data_ptr(), self.h0.data_ptr(), self.gl.data_ptr(),
+                                             self.MZ.data_ptr() + lo * self.ldmz * 8, self.ldmz, sig,
+                                             self.logdet.data_ptr() + lo * 8, self.zsums.data_ptr() if full else 0,
+                                             self._stream())
+            _cabi.check(rc, "pyvb_zstep_csr_f64")
+            self._zsums_valid = full
+            return
         if self.f32:
             full = (lo == 0 and hi == self.N)
             if not full and not self._zsums_valid:
@@ -662,6 +723,9 @@ class PlateEngine(object):
         over rows: on the tensor-core paths every chunk's statistics are taken right behind its Z step and added up, so
         that only the last chunk's work is left when the upload ends.  Returns the trace slot of the bound (no host
         synchronisation)."""
+        if self.sparse:
+            raise NotImplementedError("iterate_from_host streams a dense host array; a sparse engine keeps its entries "
+                                      "on the device")
         assert self.mode == "B"
         assert not self.f32, "iterate_from_host: the FP32 variant keeps X as bf16 planes; use precision='f64'"
         N = self.N
