@@ -92,6 +92,22 @@ extern "C" {
 #define PYVB_GL_ALQB 80      /* [64] ARD Gamma qb_i */
 #define PYVB_GL_LEN 144
 
+/* per-dimension noise precisions (noise "diagonal", factor analysis): the nd block, PYVB_ND_LEN arrays of D doubles each;
+ * array k starts at nd + k * D (pyvb_nd_len(D) doubles in all) */
+#define PYVB_ND_TAU 0        /* tau_d = qa_d / qb_d                                  (state: updated by PYVB_OP_BETA) */
+#define PYVB_ND_QB 1         /* qb_d                                                 (state: updated by PYVB_OP_BETA) */
+#define PYVB_ND_QA 2         /* qa_d = a0_d + cnt_d / 2, cnt_d the GLOBAL observed count of column d   (constant)   */
+#define PYVB_ND_PSI_QA 3     /* digamma(qa_d)                                                           (constant)   */
+#define PYVB_ND_LGAM_QA 4    /* lgamma(qa_d)                                                            (constant)   */
+#define PYVB_ND_A0 5         /* prior Gamma(a0_d, b0_d)                                                 (constant)   */
+#define PYVB_ND_B0 6
+#define PYVB_ND_LGAM_A0 7    /* lgamma(a0_d)                                                            (constant)   */
+#define PYVB_ND_SXX 8        /* sum_n O_nd x_nd^2 over ALL rows (all ranks)                             (constant)   */
+#define PYVB_ND_R 9          /* out: r_d = sum_n O_nd <(x_nd - w_d z_n - mu_d)^2>                                    */
+#define PYVB_ND_EX 10        /* out: bound term of the X entries of column d                                         */
+#define PYVB_ND_EB 11        /* out: bound term of the Gamma of column d                                             */
+#define PYVB_ND_LEN 12
+
 /* pyvb_global_f64 op mask */
 #define PYVB_OP_MU 1
 #define PYVB_OP_BETA 2
@@ -199,6 +215,29 @@ int pyvb_global_f64(int D, int q, int ops, int col_lo, int col_hi, const double 
                     double *mu, double *muvar, double *gl, const double *P0, const double *h0,
                     const pyvb_consts *consts /* host */, double *elbo_out, void *stream);
 
+/* ---- per-dimension noise precisions (mode B, FP64; every Z-step path) ----
+ * x_nd ~ N(w_d . z_n + mu_d, 1 / tau_d) with one Gamma posterior per data dimension (DiagonalGamma, nodes/nodes_todo.py:159-204).
+ * nd: the block described at PYVB_ND_* (pyvb_nd_len(D) doubles, device).  The caller fills the constants once (qa_d needs the
+ * global observed counts, sxx_d the global sums of squares) and tau_d / qb_d with the initial state, and keeps
+ * gl[PYVB_GL_TAU] = 1: the per-dimension precisions then travel inside the Gw rows.
+ *   pyvb_pack_gw_nd_f64   Gw rows [tau_d G_d | pad | tau_d <w_d> | <mu_d>]: pyvb_zstep_f64 (every algo), pyvb_zstep_i8_f64 and
+ *                         pyvb_zstep_csr_f64 read them unchanged and compute qprec_n = P0 + sum_d O_nd tau_d G_d and
+ *                         eta_n = h0 + sum_d O_nd tau_d (x_nd - mu_d) <w_d>
+ *   pyvb_wupdate_nd_f64   pyvb_wupdate_f64 with tau_d in place of the shared tau
+ *   pyvb_global_nd_f64    pyvb_global_f64 for this model: PYVB_OP_MU updates Mu with the current tau_d, PYVB_OP_BETA every
+ *                         Gamma (qb_d, tau_d), PYVB_OP_BETA or PYVB_OP_ELBO write r_d and the per-d bound terms, PYVB_OP_ALPHA
+ *                         is unchanged, PYVB_OP_ELBO adds everything up (fixed order: deterministic).  gl[PYVB_GL_RESID2]
+ *                         receives sum_d r_d; gl[PYVB_GL_QA / QB / TAU] are not touched.  Mode B only (consts->mode_a = 0);
+ *                         consts->a0 / b0 / psi_qa / lgam_qa / lgam_a0 are not read (nd carries them per d). */
+size_t pyvb_nd_len(int D);
+int pyvb_pack_gw_nd_f64(int D, int q, const double *Wbar, const double *Wvar, const double *mu, const double *nd,
+                        double *Gw, int ldg, void *stream);
+int pyvb_wupdate_nd_f64(int D, int q, int col_lo, int col_hi, const double *stats, const double *mu, const double *nd,
+                        const double *gl, double *Wbar, double *Wvar, void *stream);
+int pyvb_global_nd_f64(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar,
+                       const double *Wvar, double *mu, double *muvar, double *gl, double *nd, const double *P0,
+                       const double *h0, const pyvb_consts *consts /* host */, double *elbo_out, void *stream);
+
 /* Mode A: x_hat = observed ? x : W zbar + mu, v = observed ? 0 : 1/tau for rows [0,N) that are not
  * fully observed (pointers already offset to the first row). */
 int pyvb_impute_f64(long long N, int D, int q, const double *Xorig, long long ldx, const double *Wbar,
@@ -221,7 +260,8 @@ int pyvb_impute_f64(long long N, int D, int q, const double *Xorig, long long ld
  * when tau * D * max_c scale_c * 2^-55 > 2^-38 * max_i qprec_ii for any row (gl[PYVB_GL_I8BAD] counts them), the whole
  * call is redone on the FP64 tensor cores by conditional launches that exit at once otherwise (gl[PYVB_GL_I8FALL] counts
  * the fall-backs).  The result is therefore accurate to 2^-38 of max_i qprec_ii per row for ANY input range; on the
- * normalised data of BASELINE.json's configurations the bound sits at ~2^-50 and the guard never fires. */
+ * normalised data of BASELINE.json's configurations the bound sits at ~2^-50 and the guard never fires.
+ * The digit planes are made from the packed G columns of Gw (which must be current), so Wbar / Wvar are not read. */
 int pyvb_i8_supported(int D, int q);
 size_t pyvb_i8_digits_bytes(int D, int q);
 int pyvb_i8_ncols(int q);

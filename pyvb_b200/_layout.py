@@ -12,6 +12,10 @@ GL_ALPHA = 16
 GL_ALQB = 80
 GL_LEN = 144
 
+# per-dimension noise block (noise="diagonal"): row k of the (ND_LEN, D) array
+ND_TAU, ND_QB, ND_QA, ND_PSI_QA, ND_LGAM_QA, ND_A0, ND_B0, ND_LGAM_A0, ND_SXX, ND_R, ND_EX, ND_EB = range(12)
+ND_LEN = 12
+
 OP_MU, OP_BETA, OP_ALPHA, OP_ELBO = 1, 2, 4, 8
 ALGO_AUTO, ALGO_GENERIC, ALGO_DMMA, ALGO_DMMA_K1, ALGO_F32 = 0, 1, 2, 3, 4
 QMAX = 64

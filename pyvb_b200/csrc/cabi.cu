@@ -178,8 +178,19 @@ int pyvb_pack_gw_f64(int D, int q, const double *Wbar, const double *Wvar, const
     ARG(D >= 1 && q >= 1 && q <= PYVB_QMAX, "D, q");
     ARG(Wbar && Wvar && mu && Gw, "null pointer");
     ARG(ldg >= gw_woff(q) + q + 1, "ldg");
-    cudaError_t e = launch_pack_gw(D, q, Wbar, Wvar, mu, Gw, ldg, (cudaStream_t)stream);
+    cudaError_t e = launch_pack_gw(D, q, Wbar, Wvar, mu, nullptr, Gw, ldg, (cudaStream_t)stream);
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "pack_gw");
+}
+
+size_t pyvb_nd_len(int D) { return D > 0 ? (size_t)PYVB_ND_LEN * D : 0; }
+
+int pyvb_pack_gw_nd_f64(int D, int q, const double *Wbar, const double *Wvar, const double *mu, const double *nd, double *Gw,
+                        int ldg, void *stream) {
+    ARG(D >= 1 && q >= 1 && q <= PYVB_QMAX, "D, q");
+    ARG(Wbar && Wvar && mu && nd && Gw, "null pointer");
+    ARG(ldg >= gw_woff(q) + q + 1, "ldg");
+    cudaError_t e = launch_pack_gw(D, q, Wbar, Wvar, mu, nd + (size_t)PYVB_ND_TAU * D, Gw, ldg, (cudaStream_t)stream);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "pack_gw_nd");
 }
 
 int pyvb_zstep_f64(long long N, int D, int q, const double *X, long long ldx, const double *Gw, int ldg,
@@ -286,8 +297,18 @@ int pyvb_wupdate_f64(int D, int q, int col_lo, int col_hi, const double *stats, 
     ARG(D >= 1 && q >= 1 && q <= PYVB_QMAX, "D, q");
     ARG(0 <= col_lo && col_lo <= col_hi && col_hi <= q, "column range");
     ARG(stats && mu && gl && Wbar && Wvar, "null pointer");
-    cudaError_t e = launch_wupdate(D, q, col_lo, col_hi, stats, mu, gl, Wbar, Wvar, (cudaStream_t)stream);
+    cudaError_t e = launch_wupdate(D, q, col_lo, col_hi, stats, mu, gl, nullptr, Wbar, Wvar, (cudaStream_t)stream);
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "wupdate");
+}
+
+int pyvb_wupdate_nd_f64(int D, int q, int col_lo, int col_hi, const double *stats, const double *mu, const double *nd,
+                        const double *gl, double *Wbar, double *Wvar, void *stream) {
+    ARG(D >= 1 && q >= 1 && q <= PYVB_QMAX, "D, q");
+    ARG(0 <= col_lo && col_lo <= col_hi && col_hi <= q, "column range");
+    ARG(stats && mu && nd && gl && Wbar && Wvar, "null pointer");
+    cudaError_t e = launch_wupdate(D, q, col_lo, col_hi, stats, mu, gl, nd + (size_t)PYVB_ND_TAU * D, Wbar, Wvar,
+                                   (cudaStream_t)stream);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "wupdate_nd");
 }
 
 int pyvb_global_f64(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar, const double *Wvar, double *mu,
@@ -296,9 +317,24 @@ int pyvb_global_f64(int D, int q, int ops, int col_lo, int col_hi, const double 
     ARG(D >= 1 && q >= 1 && q <= PYVB_QMAX, "D, q");
     ARG(stats && Wbar && Wvar && mu && muvar && gl && P0 && h0 && consts, "null pointer");
     ARG(0 <= col_lo && col_lo <= col_hi && col_hi <= q, "column range");
-    cudaError_t e =
-        launch_global(D, q, ops, col_lo, col_hi, stats, Wbar, Wvar, mu, muvar, gl, P0, h0, *consts, elbo_out, (cudaStream_t)stream);
+    cudaError_t e = launch_global(D, q, ops, col_lo, col_hi, stats, Wbar, Wvar, mu, muvar, gl, P0, h0, *consts, elbo_out,
+                                  nullptr, (cudaStream_t)stream);
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "global");
+}
+
+int pyvb_global_nd_f64(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar,
+                       const double *Wvar, double *mu, double *muvar, double *gl, double *nd, const double *P0,
+                       const double *h0, const pyvb_consts *consts, double *elbo_out, void *stream) {
+    ARG(D >= 1 && q >= 1 && q <= PYVB_QMAX, "D, q");
+    ARG(stats && Wbar && Wvar && mu && muvar && gl && nd && P0 && h0 && consts, "null pointer");
+    ARG(0 <= col_lo && col_lo <= col_hi && col_hi <= q, "column range");
+    ARG(!consts->mode_a, "per-dimension noise is a mode-B model (consts->mode_a must be 0)");
+    cudaStream_t st = (cudaStream_t)stream;
+    // Mu and the Gammas first: the Mu and X bound terms read what they leave
+    cudaError_t e = launch_noise_diag(D, q, ops, stats, Wbar, Wvar, mu, muvar, nd, consts->alpha_mu, st);
+    if (e == cudaSuccess)
+        e = launch_global(D, q, ops, col_lo, col_hi, stats, Wbar, Wvar, mu, muvar, gl, P0, h0, *consts, elbo_out, nd, st);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "global_nd");
 }
 
 int pyvb_impute_f64(long long N, int D, int q, const double *Xorig, long long ldx, const double *Wbar,
@@ -352,7 +388,7 @@ int pyvb_zstep_i8_f64(long long N, int D, int q, const double *X, long long ldx,
         st2 = aux->s;
     }
     if (k1_only != 3) {      // first: its CTAs take one slot per SM, the eta kernel's CTAs fill what is left
-        e = launch_pack_g_i8(D, q, Wbar, Wvar, GI, gscale, gl, st);
+        e = launch_pack_g_i8(D, q, Gw, ldg, GI, gscale, gl, st);
         if (e == cudaSuccess) e = launch_zstep_i8(N, D, q, mask, GI, P0, gscale, gl, MZ, (int)ldmz, st);
     }
     if (e == cudaSuccess && k1_only != 2) {

@@ -18,7 +18,8 @@ struct I8Check {
 };
 
 // ---- generic (any D, q <= 64) ------------------------------------------------
-cudaError_t launch_pack_gw(int D, int q, const double *Wbar, const double *Wvar, const double *mu,
+// tau_d (nullable): per-dimension noise precisions folded into the row (pyvb_pack_gw_nd_f64)
+cudaError_t launch_pack_gw(int D, int q, const double *Wbar, const double *Wvar, const double *mu, const double *tau_d,
                            double *Gw, int ldg, cudaStream_t st);
 cudaError_t launch_zstep_generic(long long N, int D, int q, const double *X, long long ldx, const double *Gw,
                                  int ldg, const double *P0, const double *h0, double *gl, double *Zbar,
@@ -45,10 +46,15 @@ cudaError_t launch_stats_reduce(int D, int q, const double *ws_main, int nchunks
                                 cudaStream_t st);
 size_t peer_buffer_bytes(size_t len);
 cudaError_t launch_wupdate(int D, int q, int col_lo, int col_hi, const double *stats, const double *mu,
-                           const double *gl, double *Wbar, double *Wvar, cudaStream_t st);
+                           const double *gl, const double *tau_d, double *Wbar, double *Wvar, cudaStream_t st);
+// nd (nullable): per-dimension noise mode -- Mu and the Gammas are left to launch_noise_diag, which must run first
 cudaError_t launch_global(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar, const double *Wvar,
                           double *mu, double *muvar, double *gl, const double *P0, const double *h0,
-                          const pyvb_consts &c, double *elbo_out, cudaStream_t st);
+                          const pyvb_consts &c, double *elbo_out, const double *nd, cudaStream_t st);
+// per-dimension noise precisions (kernels_noise.cu): Mu (PYVB_OP_MU), r_d, the Gamma of every d (PYVB_OP_BETA) and the per-d X
+// and Beta bound terms (PYVB_OP_BETA | PYVB_OP_ELBO) into the nd block; one warp per data dimension, no atomics
+cudaError_t launch_noise_diag(int D, int q, int ops, const double *stats, const double *Wbar, const double *Wvar, double *mu,
+                              double *muvar, double *nd, double alpha_mu, cudaStream_t st);
 cudaError_t launch_impute(long long N, int D, int q, const double *Xorig, long long ldx, const double *Wbar,
                           const double *mu, const double *Zbar, long long ldz, const double *gl, double *Xhat,
                           double *V, double *qldX, cudaStream_t st);
@@ -131,8 +137,8 @@ size_t i8_mask_bytes(long long N, int D);      // bytes of the tile-major int8 m
 int i8_ncols(int q);                           // packed columns rounded up to 32 (length of gscale)
 cudaError_t launch_prepare_mask_i8(long long N, int D, const double *X, long long ldx, void *mask, cudaStream_t st);
 // also clears gl[PYVB_GL_I8BAD] (the guard counter of the Z step that follows)
-cudaError_t launch_pack_g_i8(int D, int q, const double *Wbar, const double *Wvar, void *GI, double *gscale, double *gl,
-                             cudaStream_t st);
+// G is read from the packed Gw rows (pitch pyvb_gw_pitch(q)): with per-dimension noise they carry tau_d G_d
+cudaError_t launch_pack_g_i8(int D, int q, const double *Gw, int ldg, void *GI, double *gscale, double *gl, cudaStream_t st);
 cudaError_t launch_zstep_i8(long long N, int D, int q, const void *mask, const void *GI, const double *P0,
                             const double *gscale, const double *gl, double *MZ, int ldmz, cudaStream_t st);
 

@@ -16,33 +16,40 @@
 namespace pyvb {
 
 // =============================================================== pack Gw
+// ND: per-dimension noise precisions (include/pyvb_b200.h, "nd" block) folded into the row: [tau_d G_d | pad | tau_d wbar_d |
+// mu_d], so that every Z-step contraction computes sum_d O_nd tau_d G_d and sum_d O_nd (x_nd - mu_d) tau_d wbar_d unchanged
+template <bool ND>
 __global__ void pack_gw_kernel(int D, int q, const double *__restrict__ Wbar, const double *__restrict__ Wvar,
-                               const double *__restrict__ mu, double *__restrict__ Gw, int ldg) {
+                               const double *__restrict__ mu, const double *__restrict__ tau_d, double *__restrict__ Gw,
+                               int ldg) {
     const int d = blockIdx.x;
     if (d >= D) return;
     const int P = tri(q), Pp = gw_woff(q);
     const double *w = Wbar + (size_t)d * q;
     const double *v = Wvar + (size_t)d * q;
     double *g = Gw + (size_t)d * ldg;
+    const double t = ND ? tau_d[d] : 1.0;
     for (int idx = threadIdx.x; idx < q * q; idx += blockDim.x) {
         const int i = idx / q, j = idx % q;
         if (j <= i) {
             double val = w[i] * w[j];
             if (i == j) val += v[i];
+            if (ND) val *= t;
             g[tri(i) + j] = val;
         }
     }
     for (int c = P + threadIdx.x; c < ldg; c += blockDim.x) {
         double val = 0.0;
-        if (c >= Pp && c < Pp + q) val = w[c - Pp];
+        if (c >= Pp && c < Pp + q) val = ND ? t * w[c - Pp] : w[c - Pp];
         else if (c == Pp + q) val = mu[d];
         g[c] = val;
     }
 }
 
-cudaError_t launch_pack_gw(int D, int q, const double *Wbar, const double *Wvar, const double *mu, double *Gw,
-                           int ldg, cudaStream_t st) {
-    pack_gw_kernel<<<D, 128, 0, st>>>(D, q, Wbar, Wvar, mu, Gw, ldg);
+cudaError_t launch_pack_gw(int D, int q, const double *Wbar, const double *Wvar, const double *mu, const double *tau_d,
+                           double *Gw, int ldg, cudaStream_t st) {
+    if (tau_d) pack_gw_kernel<true><<<D, 128, 0, st>>>(D, q, Wbar, Wvar, mu, tau_d, Gw, ldg);
+    else pack_gw_kernel<false><<<D, 128, 0, st>>>(D, q, Wbar, Wvar, mu, nullptr, Gw, ldg);
     return cudaGetLastError();
 }
 
@@ -580,20 +587,21 @@ cudaError_t launch_stats_reduce(int D, int q, const double *ws_main, int nchunks
 }
 
 // =============================================================== W columns (Gauss-Seidel), thread per d
+// tau_d (nullable): per-dimension noise precisions; NULL reads the shared tau of gl
 // QT > 0: q known at compile time -- the loops unroll and w[] lives in registers (with a run-time q the array is indexed
 // dynamically, i.e. it sits in local memory, and every FMA of the q^2-long dependent chain waits for a local load: 36 us at
 // D = 256, q = 16); QT = 0: any q.
 template <int QT>
 __global__ void __launch_bounds__(128)
 wupdate_kernel(int D, int q_rt, int col_lo, int col_hi, const double *__restrict__ stats,
-               const double *__restrict__ mu, const double *__restrict__ gl, double *__restrict__ Wbar,
-               double *__restrict__ Wvar) {
+               const double *__restrict__ mu, const double *__restrict__ gl, const double *__restrict__ tau_d,
+               double *__restrict__ Wbar, double *__restrict__ Wvar) {
     const int d = blockIdx.x * blockDim.x + threadIdx.x;
     if (d >= D) return;
     const int q = QT > 0 ? QT : q_rt;
     const StatLayout L(D, q);
     const int P = L.P;
-    const double tau = gl[PYVB_GL_TAU];
+    const double tau = tau_d ? tau_d[d] : gl[PYVB_GL_TAU];
     const double *T1 = stats + L.t1 + (size_t)d * P;
     const double *Bst = stats + L.bst + (size_t)d * q;
     const double *Ast = stats + L.ast + (size_t)d * q;
@@ -631,13 +639,13 @@ wupdate_kernel(int D, int q_rt, int col_lo, int col_hi, const double *__restrict
 }
 
 cudaError_t launch_wupdate(int D, int q, int col_lo, int col_hi, const double *stats, const double *mu,
-                           const double *gl, double *Wbar, double *Wvar, cudaStream_t st) {
+                           const double *gl, const double *tau_d, double *Wbar, double *Wvar, cudaStream_t st) {
     const int blocks = (D + 63) / 64;
     switch (q) {
-        case 16: wupdate_kernel<16><<<blocks, 64, 0, st>>>(D, q, col_lo, col_hi, stats, mu, gl, Wbar, Wvar); break;
-        case 32: wupdate_kernel<32><<<blocks, 64, 0, st>>>(D, q, col_lo, col_hi, stats, mu, gl, Wbar, Wvar); break;
-        case 64: wupdate_kernel<64><<<blocks, 64, 0, st>>>(D, q, col_lo, col_hi, stats, mu, gl, Wbar, Wvar); break;
-        default: wupdate_kernel<0><<<(D + 127) / 128, 128, 0, st>>>(D, q, col_lo, col_hi, stats, mu, gl, Wbar, Wvar);
+        case 16: wupdate_kernel<16><<<blocks, 64, 0, st>>>(D, q, col_lo, col_hi, stats, mu, gl, tau_d, Wbar, Wvar); break;
+        case 32: wupdate_kernel<32><<<blocks, 64, 0, st>>>(D, q, col_lo, col_hi, stats, mu, gl, tau_d, Wbar, Wvar); break;
+        case 64: wupdate_kernel<64><<<blocks, 64, 0, st>>>(D, q, col_lo, col_hi, stats, mu, gl, tau_d, Wbar, Wvar); break;
+        default: wupdate_kernel<0><<<(D + 127) / 128, 128, 0, st>>>(D, q, col_lo, col_hi, stats, mu, gl, tau_d, Wbar, Wvar);
     }
     return cudaGetLastError();
 }
@@ -666,13 +674,16 @@ __device__ __forceinline__ void gk_store_remote(const double *local_smem, uint32
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(rank));
     asm volatile("st.shared::cluster.f64 [%0], %1;" ::"r"(r), "d"(v) : "memory");
 }
+// nd (nullable): the per-dimension noise block (include/pyvb_b200.h).  With it, noise_diag_kernel (kernels_noise.cu) has already
+// done Mu, the per-dimension Gammas and their bound terms: this kernel skips its scalar Mu / Beta and the contraction, and adds
+// the per-dimension X and Beta terms in a fixed order (one CTA).
 constexpr int GK_CLUSTER = 8;
 
 __global__ void __launch_bounds__(1024)
 global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__restrict__ stats, const double *__restrict__ Wbar,
               const double *__restrict__ Wvar, double *mu, double *muvar, double *gl,
               const double *__restrict__ P0, const double *__restrict__ h0, const pyvb_consts c,
-              double *elbo_out) {
+              double *elbo_out, const double *__restrict__ nd) {
     __shared__ double sh[33];
     __shared__ double cl_part[GK_CLUSTER];                              // the cluster's partial sums of the D x P contraction
     __shared__ unsigned short ijtab[PYVB_QMAX * (PYVB_QMAX + 1) / 2];   // packed index -> (i << 8) | j
@@ -695,7 +706,7 @@ global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__res
     double tau = gl[PYVB_GL_TAU];
     __syncthreads();
 
-    if ((ops & PYVB_OP_MU) && crank == 0) {
+    if ((ops & PYVB_OP_MU) && crank == 0 && !nd) {
         for (int d = tid; d < D; d += nt) {
             const double prec = c.alpha_mu + tau * cnt[d];
             double s = colx[d];
@@ -727,7 +738,7 @@ global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__res
         __syncthreads();
     }
     double resid2 = 0.0;
-    if (ops & (PYVB_OP_BETA | PYVB_OP_ELBO)) {
+    if ((ops & (PYVB_OP_BETA | PYVB_OP_ELBO)) && !nd) {
         // (d, p) advance incrementally and (i, j) come from a table: a 64-bit division and a square root per element made
         //  this loop 0.5 ms at D = 1024, q = 32); the cluster's CTAs take contiguous slices of the D x P index range
         double dot = 0.0;
@@ -836,16 +847,31 @@ global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__res
         const double eZ = nrows * (-0.5 * q * LN2PI + 0.5 * c.lndet_P0 - 0.5 * c.m0P0m0 + 0.5 * q * LN2PI + 0.5 * q) -
                           0.5 * trPS + zh + 0.5 * sc[PYVB_SC_QLDZ];
         // ---- X rows (nodes_todo.py:144-147 uses ln<tau>)
-        const double nE = sc[PYVB_SC_NE];
-        double eX = -0.5 * nE * LN2PI + 0.5 * nE * (log(qa) - log(qb)) - 0.5 * tau * resid2;
-        if (c.mode_a) {
-            eX -= sc[PYVB_SC_NLAT] * (-0.5 * D * LN2PI - 0.5 * D) - 0.5 * sc[PYVB_SC_LATQLD];
-            eX -= 0.5 * sc[PYVB_SC_PNMISS] * LN2PI - 0.5 * sc[PYVB_SC_PLNV] - 0.5 * sc[PYVB_SC_PNMISS];
+        double eX, eB;
+        if (nd) {
+            // per-dimension terms of noise_diag_kernel, summed in a fixed order
+            double px = 0.0, pb = 0.0, pr = 0.0;
+            for (int d = tid; d < D; d += nt) {
+                px += nd[(size_t)PYVB_ND_EX * D + d];
+                pb += nd[(size_t)PYVB_ND_EB * D + d];
+                pr += nd[(size_t)PYVB_ND_R * D + d];
+            }
+            eX = block_sum(px, sh);
+            eB = block_sum(pb, sh);
+            pr = block_sum(pr, sh);
+            if (tid == 0) gl[PYVB_GL_RESID2] = pr;
+        } else {
+            const double nE = sc[PYVB_SC_NE];
+            eX = -0.5 * nE * LN2PI + 0.5 * nE * (log(qa) - log(qb)) - 0.5 * tau * resid2;
+            if (c.mode_a) {
+                eX -= sc[PYVB_SC_NLAT] * (-0.5 * D * LN2PI - 0.5 * D) - 0.5 * sc[PYVB_SC_LATQLD];
+                eX -= 0.5 * sc[PYVB_SC_PNMISS] * LN2PI - 0.5 * sc[PYVB_SC_PLNV] - 0.5 * sc[PYVB_SC_PNMISS];
+            }
+            // ---- Gammas (nodes_todo.py:149-157)
+            const double El = c.psi_qa - log(qb);
+            eB = (c.a0 - 1.0) * El - c.lgam_a0 + c.a0 * log(c.b0) - c.b0 * (qa / qb) -
+                 ((qa - 1.0) * El - c.lgam_qa + qa * log(qb) - qa);
         }
-        // ---- Gammas (nodes_todo.py:149-157)
-        const double El = c.psi_qa - log(qb);
-        const double eB = (c.a0 - 1.0) * El - c.lgam_a0 + c.a0 * log(c.b0) - c.b0 * (qa / qb) -
-                          ((qa - 1.0) * El - c.lgam_qa + qa * log(qb) - qa);
         double eA = 0.0;
         if (c.ard) {
             for (int i = 0; i < q; ++i) {
@@ -871,9 +897,9 @@ global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__res
 
 cudaError_t launch_global(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar, const double *Wvar,
                           double *mu, double *muvar, double *gl, const double *P0, const double *h0,
-                          const pyvb_consts &c, double *elbo_out, cudaStream_t st) {
-    // one cluster; its size follows the work of the D x P contraction (small problems: one CTA)
-    const long long work = (long long)D * q * (q + 1) / 2;
+                          const pyvb_consts &c, double *elbo_out, const double *nd, cudaStream_t st) {
+    // one cluster; its size follows the work of the D x P contraction (small problems, or no contraction: one CTA)
+    const long long work = nd ? 0 : (long long)D * q * (q + 1) / 2;
     const int cl = work >= (1LL << 17) ? GK_CLUSTER : work >= (1LL << 15) ? 2 : 1;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)cl, 1, 1);
@@ -887,7 +913,8 @@ cudaError_t launch_global(int D, int q, int ops, int col_lo, int col_hi, const d
     at[0].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, global_kernel, D, q, ops, col_lo, col_hi, stats, Wbar, Wvar, mu, muvar, gl, P0, h0, c, elbo_out);
+    return cudaLaunchKernelEx(&cfg, global_kernel, D, q, ops, col_lo, col_hi, stats, Wbar, Wvar, mu, muvar, gl, P0, h0, c, elbo_out,
+                              nd);
 }
 
 // =============================================================== mode A imputation, warp per row

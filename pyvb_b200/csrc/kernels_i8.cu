@@ -75,24 +75,19 @@ prepare_mask_i8_kernel(long long N, int D, const double *__restrict__ X, long lo
 }
 
 // one CTA per output column c: scale_c = max_d |G[d][c]|, then the seven balanced base-256 digits of
-// round(G / scale_c * 2^54).  GI[kb][ct][plane][c % 32][64] (int8), kb = d / 64, ct = c / 32: the B tile of (kb, ct) is
+// round(G / scale_c * 2^54).  G[d][c] is column c of the packed Gw row d (pack_gw_kernel: the same w_i w_j (+ v_i) bits, or
+// tau_d times them with per-dimension noise).  GI[kb][ct][plane][c % 32][64] (int8), kb = d / 64, ct = c / 32: the B tile of (kb, ct) is
 // one contiguous [224 rows][64 bytes] block.
 __global__ void __launch_bounds__(256)
-pack_g_i8_kernel(int D, int q, const double *__restrict__ Wbar, const double *__restrict__ Wvar,
-                 signed char *__restrict__ GI, double *__restrict__ gscale, double *__restrict__ gl) {
+pack_g_i8_kernel(int D, int q, const double *__restrict__ Gw, int ldg, signed char *__restrict__ GI,
+                 double *__restrict__ gscale, double *__restrict__ gl) {
     __shared__ double sh[33];
     const int P = i_tri(q);
     const int c = blockIdx.x;
     if (c == 0 && threadIdx.x == 0) gl[PYVB_GL_I8BAD] = 0.0;           // guard counter of the Z step that follows (K2 adds to it)
-    int i = 0, j = 0;
-    if (c < P) unpack_p(c, i, j);
     double mx = 0.0;
     for (int d = threadIdx.x; d < D; d += blockDim.x) {
-        double g = 0.0;
-        if (c < P) {
-            g = Wbar[(size_t)d * q + i] * Wbar[(size_t)d * q + j];
-            if (i == j) g += Wvar[(size_t)d * q + i];
-        }
+        const double g = (c < P) ? Gw[(size_t)d * ldg + c] : 0.0;
         mx = fmax(mx, fabs(g));
     }
     for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
@@ -111,11 +106,7 @@ pack_g_i8_kernel(int D, int q, const double *__restrict__ Wbar, const double *__
     const double inv = 18014398509481984.0 / scale;                     // 2^54 / scale
     const int nct = gridDim.x / CT;
     for (int d = threadIdx.x; d < D; d += blockDim.x) {
-        double g = 0.0;
-        if (c < P) {
-            g = Wbar[(size_t)d * q + i] * Wbar[(size_t)d * q + j];
-            if (i == j) g += Wvar[(size_t)d * q + i];
-        }
+        const double g = (c < P) ? Gw[(size_t)d * ldg + c] : 0.0;
         long long v = __double2ll_rn(g * inv);
 #pragma unroll
         for (int t = 0; t < NPL; ++t) {
@@ -1461,9 +1452,8 @@ cudaError_t launch_prepare_mask_i8(long long N, int D, const double *X, long lon
     return cudaGetLastError();
 }
 
-cudaError_t launch_pack_g_i8(int D, int q, const double *Wbar, const double *Wvar, void *GI, double *gscale, double *gl,
-                             cudaStream_t st) {
-    pack_g_i8_kernel<<<i_nc8(q), 256, 0, st>>>(D, q, Wbar, Wvar, static_cast<signed char *>(GI), gscale, gl);
+cudaError_t launch_pack_g_i8(int D, int q, const double *Gw, int ldg, void *GI, double *gscale, double *gl, cudaStream_t st) {
+    pack_g_i8_kernel<<<i_nc8(q), 256, 0, st>>>(D, q, Gw, ldg, static_cast<signed char *>(GI), gscale, gl);
     return cudaGetLastError();
 }
 

@@ -23,6 +23,7 @@ import numpy as np
 import torch
 
 from . import _cabi
+from . import _layout
 from . import sparse as _sparse
 import os
 
@@ -71,11 +72,14 @@ class PlateEngine(object):
     mode : "B" masked/marginalised (throughput path) or "A" reference-exact imputation
     distributed : all-reduce the statistics over torch.distributed's default group
     row_offset : global index of local row 0 (mode A treats global row 0 specially)
+    noise : "scalar" -- one noise precision tau shared by every data dimension (Gamma(a0, b0)) -- or "diagonal" -- factor
+        analysis: x_nd ~ N(w_d z_n + mu_d, 1 / tau_d) with one Gamma(a0_d, b0_d) posterior per data dimension (DiagonalGamma);
+        a0 and b0 may then be scalars or length-D arrays.  "diagonal" runs on every FP64 mode-B path (dense and sparse).
     """
 
     def __init__(self, X, q, mode="B", alpha0=1e-3, alpha_mu=1e-3, a0=1e-3, b0=1e-3, ard=False,
                  ard_a0=1e-3, ard_b0=1e-3, P0=None, m0=None, device=None, algo="auto",
-                 keep_sigma=True, distributed=False, row_offset=0, trace_len=4096, precision="f64"):
+                 keep_sigma=True, distributed=False, row_offset=0, trace_len=4096, precision="f64", noise="scalar"):
         if not torch.cuda.is_available():
             raise RuntimeError("pyvb_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         self.lib = _cabi.lib()
@@ -83,6 +87,11 @@ class PlateEngine(object):
         assert 1 <= q <= QMAX, "latent dimension must be in [1, %d]" % QMAX
         assert precision in ("f64", "f32")
         self.f32 = (precision == "f32")
+        if noise not in ("scalar", "diagonal"):
+            raise ValueError("noise must be 'scalar' or 'diagonal', got %r" % (noise,))
+        self.diag = (noise == "diagonal")
+        if self.diag and (mode != "B" or self.f32):
+            raise ValueError("noise='diagonal' needs mode='B' and precision='f64'")
         self.device = torch.device(device if device is not None else "cuda:%d" % torch.cuda.current_device())
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
@@ -127,10 +136,30 @@ class PlateEngine(object):
         self.P = q * (q + 1) // 2
         self.L = StatLayout(D, q)
         self.alpha0, self.alpha_mu = float(alpha0), float(alpha_mu)
+        if self.diag:
+            a0v, b0v = self._per_dim(a0, "a0"), self._per_dim(b0, "b0")
+            a0 = b0 = 1.0                     # the scalar Gamma's constants below are not read in diagonal mode
         self.a0, self.b0 = float(a0), float(b0)
         self.ard_a0, self.ard_b0 = float(ard_a0), float(ard_b0)
 
         # ---- data
+        if self.diag:
+            # the data constants of the per-dimension Gammas: observed count and sum of squares of every column
+            if self.sparse:
+                cnt_d, _, sxx_d = (torch.as_tensor(a, dtype=f64, device=dev) for a in _sparse.column_sums(self.csr))
+            else:
+                cnt_d, sxx_d = torch.zeros(D, dtype=f64, device=dev), torch.zeros(D, dtype=f64, device=dev)
+                for lo in range(0, N, 1 << 16):
+                    x = Xt[lo:lo + (1 << 16)]
+                    o = ~torch.isnan(x)
+                    cnt_d += o.sum(0).to(f64)
+                    sxx_d += torch.where(o, x * x, torch.zeros((), dtype=f64, device=dev)).sum(0)
+                    del x, o
+            if self.distributed:
+                import torch.distributed as dist
+                both = torch.cat([cnt_d, sxx_d])
+                dist.all_reduce(both)
+                cnt_d, sxx_d = both[:D], both[D:]
         obs = None if self.sparse else ~torch.isnan(Xt)
         n_obs_local = int(self.csr.values.numel()) if self.sparse else int(obs.sum().item())
         if self.sparse:
@@ -280,6 +309,17 @@ class PlateEngine(object):
         c.ard, c.mode_a = int(self.ard), int(mode == "A")
         self.consts = c
         self.qa, self.al_qa = qa, al_qa
+        self.nd = None
+        if self.diag:
+            from scipy import special
+            cnt = cnt_d.cpu().numpy()
+            qa_d = a0v + 0.5 * cnt
+            nd = np.zeros((int(self.lib.pyvb_nd_len(D)) // D, D))
+            nd[_layout.ND_QA], nd[_layout.ND_PSI_QA], nd[_layout.ND_LGAM_QA] = qa_d, special.digamma(qa_d), special.gammaln(qa_d)
+            nd[_layout.ND_A0], nd[_layout.ND_B0], nd[_layout.ND_LGAM_A0] = a0v, b0v, special.gammaln(a0v)
+            nd[_layout.ND_SXX] = sxx_d.cpu().numpy()
+            self.nd = torch.as_tensor(nd, dtype=f64).to(dev).reshape(-1)
+            self.qa = qa_d
 
         # deterministic stand-in initialisation (SURVEY 8d); parity runs call set_state()
         self.set_state({"qb": 0.5, "al_qb": np.ones(q)})
@@ -296,6 +336,17 @@ class PlateEngine(object):
     # ------------------------------------------------------------------ plumbing
     def _stream(self):
         return torch.cuda.current_stream(self.device).cuda_stream
+
+    def _per_dim(self, v, name):
+        """A scalar or (D,) prior parameter of the per-dimension Gammas as a (D,) float64 array."""
+        a = np.asarray(v, dtype=np.float64)
+        if a.ndim == 0:
+            a = np.full(self.D, float(a))
+        if a.shape != (self.D,):
+            raise ValueError("%s must be a scalar or have shape (%d,), got %s" % (name, self.D, a.shape))
+        if not (np.all(np.isfinite(a)) and np.all(a > 0)):
+            raise ValueError("%s must be finite and positive" % name)
+        return a
 
     def _allreduce_scalar(self, v):
         if self.distributed:
@@ -343,11 +394,20 @@ class PlateEngine(object):
         if self.f32:
             self._resplit()
         gl = self.gl.cpu()
-        gl[GL_QA] = self.qa
         gl[GL_NONPD] = 0.0                      # a fresh state: earlier non-PD rows are history
-        if "qb" in st:
-            gl[GL_QB] = float(st["qb"])
-        gl[GL_TAU] = gl[GL_QA] / gl[GL_QB]
+        if self.diag:
+            # tau_d travels in the Gw rows and the W update reads it from nd: the shared tau stays 1
+            gl[GL_QA] = gl[GL_QB] = gl[GL_TAU] = 1.0
+            if "qb" in st:
+                qb = np.broadcast_to(np.asarray(st["qb"], dtype=np.float64), (self.D,))
+                nd = self.nd.view(-1, self.D)
+                nd[_layout.ND_QB] = torch.as_tensor(np.ascontiguousarray(qb)).to(dev)
+                nd[_layout.ND_TAU] = nd[_layout.ND_QA] / nd[_layout.ND_QB]
+        else:
+            gl[GL_QA] = self.qa
+            if "qb" in st:
+                gl[GL_QB] = float(st["qb"])
+            gl[GL_TAU] = gl[GL_QA] / gl[GL_QB]
         if self.ard:
             if "al_qb" in st:
                 gl[GL_ALQB:GL_ALQB + q] = torch.as_tensor(np.asarray(st["al_qb"], dtype=np.float64).reshape(q))
@@ -414,6 +474,9 @@ class PlateEngine(object):
         if self.sparse:
             raise NotImplementedError("set_X: a sparse engine keeps its entries in the layouts built at construction; "
                                       "build a new engine for new data")
+        if self.diag:
+            raise NotImplementedError("set_X: with noise='diagonal' the column sums of squares are constants of the data set; "
+                                      "build a new engine for new data")
         assert self.mode == "B" and not self.f32
         self.X.copy_(X, non_blocking=True)
         self._xcache_valid = False
@@ -441,10 +504,17 @@ class PlateEngine(object):
             out["Xhat"] = self.X.cpu().numpy()
             out["V"] = self.V.cpu().numpy()
         gl = self.gl.cpu().numpy()
-        out["qa"], out["qb"], out["tau"] = float(gl[GL_QA]), float(gl[GL_QB]), float(gl[GL_TAU])
+        out.update(self._noise_state(gl))
         out["alpha"] = gl[GL_ALPHA:GL_ALPHA + q].copy()
         out["al_qb"] = gl[GL_ALQB:GL_ALQB + q].copy()
         return out
+
+    def _noise_state(self, gl):
+        """qa, qb, tau: floats, or (D,) arrays with noise='diagonal'."""
+        if self.diag:
+            nd = self.nd.view(-1, self.D).cpu().numpy()
+            return {"qa": nd[_layout.ND_QA].copy(), "qb": nd[_layout.ND_QB].copy(), "tau": nd[_layout.ND_TAU].copy()}
+        return {"qa": float(gl[GL_QA]), "qb": float(gl[GL_QB]), "tau": float(gl[GL_TAU])}
 
     def get_row(self, i):
         """Host copy of ONE row of the plate (O(q^2 + D), no pass over the other rows): zbar_i, Sigma_i and, in mode A,
@@ -468,10 +538,11 @@ class PlateEngine(object):
     def get_state_small(self):
         """Host copy of the replicated (row-independent) state only."""
         gl = self.gl.cpu().numpy()
-        return {"Wbar": self.Wbar.cpu().numpy(), "Wvar": self.Wvar.cpu().numpy(), "mu": self.mu.cpu().numpy(),
-                "muvar": self.muvar.cpu().numpy(), "qa": float(gl[GL_QA]), "qb": float(gl[GL_QB]),
-                "tau": float(gl[GL_TAU]), "alpha": gl[GL_ALPHA:GL_ALPHA + self.q].copy(),
-                "al_qb": gl[GL_ALQB:GL_ALQB + self.q].copy()}
+        out = {"Wbar": self.Wbar.cpu().numpy(), "Wvar": self.Wvar.cpu().numpy(), "mu": self.mu.cpu().numpy(),
+               "muvar": self.muvar.cpu().numpy(), "alpha": gl[GL_ALPHA:GL_ALPHA + self.q].copy(),
+               "al_qb": gl[GL_ALQB:GL_ALQB + self.q].copy()}
+        out.update(self._noise_state(gl))
+        return out
 
     def check(self):
         """Raise LinAlgError if any posterior precision was not positive definite (gaussian.py:118)."""
@@ -495,6 +566,11 @@ class PlateEngine(object):
             rc = self.lib.pyvb_pack_gw_f32(self.D, self.q, self.Wbar.data_ptr(), self.Wvar.data_ptr(),
                                            self.mu.data_ptr(), self.GT.data_ptr(), self.WT.data_ptr(), self._stream())
             _cabi.check(rc, "pyvb_pack_gw_f32")
+            self._gw_fresh = True
+        if not self._gw_fresh and self.diag:
+            rc = self.lib.pyvb_pack_gw_nd_f64(self.D, self.q, self.Wbar.data_ptr(), self.Wvar.data_ptr(), self.mu.data_ptr(),
+                                              self.nd.data_ptr(), self.Gw.data_ptr(), self.ldg, self._stream())
+            _cabi.check(rc, "pyvb_pack_gw_nd_f64")
             self._gw_fresh = True
         if not self._gw_fresh:
             rc = self.lib.pyvb_pack_gw_f64(self.D, self.q, self.Wbar.data_ptr(), self.Wvar.data_ptr(),
@@ -571,6 +647,13 @@ class PlateEngine(object):
     def update_W(self, col_lo=0, col_hi=None):
         col_hi = self.q if col_hi is None else col_hi
         self._ensure_stats()
+        if self.diag:
+            rc = self.lib.pyvb_wupdate_nd_f64(self.D, self.q, col_lo, col_hi, self.stats.data_ptr(), self.mu.data_ptr(),
+                                              self.nd.data_ptr(), self.gl.data_ptr(), self.Wbar.data_ptr(),
+                                              self.Wvar.data_ptr(), self._stream())
+            _cabi.check(rc, "pyvb_wupdate_nd_f64")
+            self._gw_fresh = False
+            return
         rc = self.lib.pyvb_wupdate_f64(self.D, self.q, col_lo, col_hi, self.stats.data_ptr(), self.mu.data_ptr(),
                                        self.gl.data_ptr(), self.Wbar.data_ptr(), self.Wvar.data_ptr(),
                                        self._stream())
@@ -665,6 +748,15 @@ class PlateEngine(object):
     def _global(self, ops, elbo_out=0, col_lo=0, col_hi=None):
         self._ensure_stats()
         col_hi = self.q if col_hi is None else col_hi
+        if self.diag:
+            rc = self.lib.pyvb_global_nd_f64(self.D, self.q, ops, col_lo, col_hi, self.stats.data_ptr(), self.Wbar.data_ptr(),
+                                             self.Wvar.data_ptr(), self.mu.data_ptr(), self.muvar.data_ptr(),
+                                             self.gl.data_ptr(), self.nd.data_ptr(), self.P0.data_ptr(), self.h0.data_ptr(),
+                                             _cabi.ctypes.byref(self.consts), elbo_out, self._stream())
+            _cabi.check(rc, "pyvb_global_nd_f64")
+            if ops & (OP_MU | OP_BETA):             # mu_d and tau_d live in the Gw rows
+                self._gw_fresh = False
+            return
         rc = self.lib.pyvb_global_f64(self.D, self.q, ops, col_lo, col_hi, self.stats.data_ptr(), self.Wbar.data_ptr(),
                                       self.Wvar.data_ptr(), self.mu.data_ptr(), self.muvar.data_ptr(),
                                       self.gl.data_ptr(), self.P0.data_ptr(), self.h0.data_ptr(),
@@ -726,6 +818,9 @@ class PlateEngine(object):
         if self.sparse:
             raise NotImplementedError("iterate_from_host streams a dense host array; a sparse engine keeps its entries "
                                       "on the device")
+        if self.diag:
+            raise NotImplementedError("iterate_from_host: with noise='diagonal' the column sums of squares are constants of "
+                                      "the resident data set")
         assert self.mode == "B"
         assert not self.f32, "iterate_from_host: the FP32 variant keeps X as bf16 planes; use precision='f64'"
         N = self.N

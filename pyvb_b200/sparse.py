@@ -118,16 +118,23 @@ def block_csc(csr, rows_per_block):
     return BlockedCSC(colptr, row[perm].to(torch.int32).contiguous(), csr.values[perm].contiguous(), nblk, R)
 
 
-def x_cache(csr):
-    """[cnt (D) | colsumX (D) | sum x^2 | nnz] as a float64 CPU tensor.  Sequential sums in stored order (numpy bincount),
-    sum x^2 exactly rounded over its per-column parts: the same input always gives the same bits."""
+def column_sums(csr):
+    """Per column: stored entries, their sum and their sum of squares (float64 numpy arrays of length D).  Sequential sums in
+    stored order (numpy bincount): the same input always gives the same bits."""
     D = csr.D
     col = csr.indices.cpu().numpy().astype(np.int64, copy=False)
     val = csr.values.cpu().numpy()
     cnt = np.bincount(col, minlength=D).astype(np.float64)
     colx = np.bincount(col, weights=val, minlength=D)
-    sxx = math.fsum(np.bincount(col, weights=val * val, minlength=D).tolist())
-    out = np.concatenate([cnt, colx, [sxx, float(val.size)]])
+    colxx = np.bincount(col, weights=val * val, minlength=D)
+    return cnt, colx, colxx
+
+
+def x_cache(csr):
+    """[cnt (D) | colsumX (D) | sum x^2 | nnz] as a float64 CPU tensor, from column_sums; sum x^2 exactly rounded over its
+    per-column parts."""
+    cnt, colx, colxx = column_sums(csr)
+    out = np.concatenate([cnt, colx, [math.fsum(colxx.tolist()), float(csr.values.numel())]])
     return torch.as_tensor(out, dtype=torch.float64)
 
 
