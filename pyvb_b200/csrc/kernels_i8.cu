@@ -1092,53 +1092,87 @@ stats_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
 
 // K3-i8 with the digit planes made in shared memory (D <= 256: at most two blocks of 128 data dimensions).  digitize_kernel
 // writes 7 bytes per MZ entry to ZI and stats_i8_kernel reads them back (1.1 GB each way per sweep at N = 1M, q = 16), for
-// data that only ever feeds the MMA.  Here converter warps read the MZ rows with coalesced loads and write the digit tile
-// straight into the ring stage, byte for byte the SWIZZLE_64B image TMA delivered from ZI (oracle/i8_fused_oracle.py).
+// data that only ever feeds the MMA.  Here converter warps take the MZ rows from TMA tiles and write the digit tile straight
+// into the ring stage, byte for byte the SWIZZLE_64B image TMA delivered from ZI (oracle/i8_fused_oracle.py).
 // Work item = (column tile of 32, row chunk) over ALL blocks of data dimensions: each digit tile is made once and feeds
 // the MMAs of both blocks (two TMEM accumulators of 224 columns).  Same chunks and the same integer sums as
 // stats_i8_kernel, recombined by the same epilogue: bit-identical partials.
 // Warps: 0 TMA producer (the maskT tiles), 1 MMA issuer, 2-9 epilogue, 10-17 converters (two groups of four that take
-// alternate K steps, a warp = 16 rows of a 64-row step).  Ring stage = [maskT block 0 | maskT block 1 | digit tile].
+// alternate K steps, a warp = 16 rows of a 64-row step).  Ring stage = [maskT block 0 | maskT block 1 | digit tile]; each
+// converter warp also has its own ring of MZ tiles.
 constexpr int SF_CONV = 8;
 constexpr int SF_NTHR = (2 + 8 + SF_CONV) * 32;
 constexpr int SF_STG = 2 * A_B + B_B;                    // 30 KB
+constexpr int SF_ZB = 16 * CT * 8;                       // 4 KB: a converter warp's MZ values of one step (16 rows x 32 columns)
 constexpr int SF_NSMAX = 8;
+constexpr int SF_PROF = 24;                              // PYVB_I8_PROF clock slots per CTA
 
-int sf_stages(int q) {
-    const size_t fixed = 1024 + (size_t)stats_i8_ncols(q) * 8 + (size_t)(2 * SF_NSMAX + 2) * 8 + 16;
-    const int ns = (int)((227 * 1024 - fixed) / SF_STG);
-    return ns < SF_NSMAX ? ns : SF_NSMAX;
+size_t sf_smem_bytes(int q, int ns, int nz) {
+    return 1024 + (size_t)ns * SF_STG + (size_t)SF_CONV * nz * SF_ZB + (size_t)stats_i8_ncols(q) * 8 +
+           (size_t)(2 * ns + 2 + SF_CONV * nz) * 8 + 16;
 }
-size_t sf_smem_bytes(int q, int ns) {
-    return 1024 + (size_t)ns * SF_STG + (size_t)stats_i8_ncols(q) * 8 + (size_t)(2 * ns + 2) * 8 + 16;
+// Two MZ slots per converter warp (64 KB, 32 KB of it in flight while a step is converted), the rest of the 227 KB in ring
+// stages: at C2 (q = 16) 5 stages + 2 slots ran the kernel in 0.382 ms, 4 + 3 in 0.392, 3 + 4 in 0.409, 2 + 5 in 0.424 (one
+// B200, 1000 W).  The converters barely wait for their TMA loads at any depth; ring stages decouple them from the MMAs.
+constexpr int SF_NZ = 2;
+int sf_stages(int q) {
+    int ns = SF_NSMAX;
+    while (ns > 2 && sf_smem_bytes(q, ns, SF_NZ) > 227 * 1024) --ns;
+    return ns;
+}
+
+// 2-D tiled TMA load with an L2 cache policy (createpolicy)
+__device__ __forceinline__ void tma_load_2d_hint(const void *dst_smem, const void *tmap, int c0, int c1, uint64_t *bar,
+                                                 uint64_t policy) {
+    asm volatile(
+        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3}], [%4], "
+        "%5;" ::"r"(smem_u32(dst_smem)),
+        "l"(tmap), "r"(c0), "r"(c1), "r"(smem_u32(bar)), "l"(policy)
+        : "memory");
 }
 
 __global__ void __launch_bounds__(SF_NTHR, 1)
-stats_i8_fused_kernel(const __grid_constant__ CUtensorMap tmA, long long N, int D, int q, const double *__restrict__ MZ, int ldmz,
+stats_i8_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmZ, long long N, int D, int q,
                       const double *__restrict__ zscale, double *__restrict__ ws, long long rows_per_chunk, int nchunks,
-                      int ndb, int nct, int ns) {
+                      int ndb, int nct, int ns, int nz, long long *prof) {
+    long long w0 = 0, w1 = 0;                                  // PYVB_I8_PROF: clocks spent waiting, per role
+    const long long tstart = clock64();
+#define PROF_WAIT(acc, stmt)                    \
+    do {                                        \
+        if (prof) {                             \
+            const long long t_ = clock64();     \
+            stmt;                               \
+            acc += clock64() - t_;              \
+        } else {                                \
+            stmt;                               \
+        }                                       \
+    } while (0)
     extern __shared__ unsigned char smem_dyn[];
     unsigned char *smem = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
     const int P = i_tri(q), NCZ = nct * CT;
     unsigned char *st_base = smem;                                             // [ns][A0 8 KB | A1 8 KB | B 14 KB]
-    double *fcol = reinterpret_cast<double *>(smem + (size_t)ns * SF_STG);    // [NCZ]: zscale_c * 2^-54
+    unsigned char *zbuf = smem + (size_t)ns * SF_STG;                          // [SF_CONV][nz][16 rows x 32 doubles]
+    double *fcol = reinterpret_cast<double *>(zbuf + (size_t)SF_CONV * nz * SF_ZB);   // [NCZ]: zscale_c * 2^-54
     uint64_t *full = reinterpret_cast<uint64_t *>(fcol + NCZ);                // [ns]: producer (tx bytes) + 4 converter warps
     uint64_t *empty = full + ns;                                               // [ns]: MMA commit
     uint64_t *tfull = empty + ns;
     uint64_t *tempty = tfull + 1;
-    uint32_t *tbase = reinterpret_cast<uint32_t *>(tempty + 1);
+    uint64_t *zfull = tempty + 1;                                              // [SF_CONV][nz]: tmZ tx bytes
+    uint32_t *tbase = reinterpret_cast<uint32_t *>(zfull + SF_CONV * nz);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int nitems = nct * nchunks;
     for (int c = tid; c < NCZ; c += SF_NTHR) fcol[c] = zscale[c] * 5.5511151231257827e-17;   // 2^-54
     if (tid == 0) {
         tma_prefetch_desc(&tmA);
+        tma_prefetch_desc(&tmZ);
         for (int s = 0; s < ns; ++s) {
             mbar_init(&full[s], 1 + SF_CONV / 2);
             mbar_init(&empty[s], 1);
         }
         mbar_init(tfull, 1);
         mbar_init(tempty, 8);
+        for (int i = 0; i < SF_CONV * nz; ++i) mbar_init(&zfull[i], 1);
         mbar_fence_init();
     }
     if (warp == 1) umma::tmem_alloc(tbase, 512);
@@ -1167,7 +1201,7 @@ stats_i8_fused_kernel(const __grid_constant__ CUtensorMap tmA, long long N, int 
             long long r0;
             item_geom(item, chunk, ct, r0, nsteps);
             for (int k = 0; k < nsteps; ++k) {
-                umma::mbar_wait_bounded(&empty[s], ph ^ 1);
+                PROF_WAIT(w0, umma::mbar_wait_bounded(&empty[s], ph ^ 1));
                 if (leader) {
                     mbar_arrive_expect_tx(&full[s], (uint32_t)(ndb * A_B));
                     const long long kb = r0 / BKB + k;
@@ -1193,10 +1227,10 @@ stats_i8_fused_kernel(const __grid_constant__ CUtensorMap tmA, long long N, int 
             int chunk, ct, nsteps;
             long long r0;
             item_geom(item, chunk, ct, r0, nsteps);
-            umma::mbar_wait_bounded(tempty, (uint32_t)((tl & 1) ^ 1));       // the epilogue has drained the accumulators
+            PROF_WAIT(w1, umma::mbar_wait_bounded(tempty, (uint32_t)((tl & 1) ^ 1)));   // the epilogue has drained the accumulators
             umma::fence_after_sync();
             for (int k = 0; k < nsteps; ++k) {
-                umma::mbar_wait_bounded(&full[s], ph);
+                PROF_WAIT(w0, umma::mbar_wait_bounded(&full[s], ph));
                 umma::fence_after_sync();
                 if (leader) {
                     const uint64_t off = (uint64_t)((s * SF_STG) >> 4);
@@ -1228,7 +1262,7 @@ stats_i8_fused_kernel(const __grid_constant__ CUtensorMap tmA, long long N, int 
             item_geom(item, chunk, ct, r0, nsteps);
             const int c0 = ct * CT + half * 16;
             double *out = ws + (size_t)chunk * L.len;
-            umma::mbar_wait_bounded(tfull, (uint32_t)(tl & 1));
+            PROF_WAIT(w0, umma::mbar_wait_bounded(tfull, (uint32_t)(tl & 1)));
             umma::fence_after_sync();
             for (int b = 0; b < ndb; ++b) {
                 const int d = b * BM + wq * 32 + lane;
@@ -1261,18 +1295,24 @@ stats_i8_fused_kernel(const __grid_constant__ CUtensorMap tmA, long long N, int 
             if (lane == 0) mbar_arrive(tempty);
         }
     } else {
-        // converters: the arithmetic of digitize_kernel (2^54 / zscale_c, NaN / inf -> 0, zero past row N and column P + q,
-        // the BIAS / xor byte split), written as the SWIZZLE_64B image of the K-major tile: plane p, column l of the tile,
-        // row n of the step at byte (p * 32 + l) * 64 + (((n >> 4) ^ ((l >> 1) & 3)) << 4) + (n & 15).  Warp cw owns rows
-        // 16 (cw % 4) ... + 15 of every other step; a lane owns one column and puts four rows into one 32-bit word per
-        // plane.  Lane group l / 8 starts at row quad l / 8 of the warp's 16 rows (and cycles): with the swizzle the 32 words
-        // of every store instruction fall into 32 different banks.  The loads stay full 32-byte sectors (8 lanes x 8 bytes
-        // of one row per group).  The loads of a warp's next step are issued before it converts the current one: with one
-        // step in flight per warp (32 KB per SM) the HBM latency, not the bandwidth, set the pace.
+        // converters: the arithmetic of digitize_kernel (2^54 / zscale_c, NaN / inf -> 0, the BIAS / xor byte split), written
+        // as the SWIZZLE_64B image of the K-major tile: plane p, column l of the tile, row n of the step at byte
+        // (p * 32 + l) * 64 + (((n >> 4) ^ ((l >> 1) & 3)) << 4) + (n & 15).  Warp cw owns rows 16 (cw % 4) ... + 15 of every
+        // other step; a lane owns one column and puts four rows into one 32-bit word per plane.  Lane group l / 8 starts at
+        // row quad l / 8 of the warp's 16 rows (and cycles): with the swizzle the 32 words of every store instruction fall
+        // into 32 different banks.
+        // The MZ values arrive by TMA (tmZ: 16 rows x 32 columns, 4 KB) in a ring of nz slots private to the warp, nz steps
+        // ahead: rows >= N and columns >= P + q (the pitch past zbar among them) arrive as zeros, so no column past zbar is
+        // ever read.
         const int cw = warp - 10, grp = cw >> 2, rq = cw & 3, rot = lane >> 3;
         const int nvalid = P + q;
         constexpr unsigned long long BIAS = 0x0080808080808080ULL;
         const uint32_t wbase = (uint32_t)(lane * 64 + ((rq ^ ((lane >> 1) & 3)) << 4));
+        const double *zring = reinterpret_cast<const double *>(zbuf + (size_t)cw * nz * SF_ZB);
+        uint64_t *zb = zfull + cw * nz;
+        const bool zlead = elect_one();
+        uint64_t policy = 0;
+        if (zlead) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(policy));   // MZ is read once
         // position (item, K step of the item) of this warp's steps: the CTA's steps j = grp, grp + 2, ... in order
         struct Pos {
             int item, k, nsteps, ct;
@@ -1286,17 +1326,10 @@ stats_i8_fused_kernel(const __grid_constant__ CUtensorMap tmA, long long N, int 
                 if (p.item < nitems) item_geom(p.item, chunk, p.ct, p.r0, p.nsteps);
             }
         };
-        auto load = [&](const Pos &p, double (&x)[16]) {
-            const int c = p.ct * CT + lane;
-            const bool cv = p.item < nitems && c < nvalid;
-            const long long nb = p.r0 + (long long)p.k * BKB + rq * 16;
-#pragma unroll
-            for (int g = 0; g < 4; ++g)
-#pragma unroll
-                for (int kk = 0; kk < 4; ++kk) {
-                    const long long n = nb + 4 * ((g + rot) & 3) + kk;
-                    x[g * 4 + kk] = (cv && n < N) ? __ldcs(MZ + n * ldmz + c) : 0.0;
-                }
+        auto issue = [&](const Pos &p, int slot) {            // (elected lane) this warp's 16 rows of the step at p
+            mbar_arrive_expect_tx(&zb[slot], (uint32_t)SF_ZB);
+            tma_load_2d_hint(zring + slot * (SF_ZB / 8), &tmZ, p.ct * CT, (int)(p.r0 + (long long)p.k * BKB + rq * 16), &zb[slot],
+                             policy);
         };
         Pos cur;
         cur.item = blockIdx.x;
@@ -1307,17 +1340,38 @@ stats_i8_fused_kernel(const __grid_constant__ CUtensorMap tmA, long long N, int 
             if (cur.item < nitems) item_geom(cur.item, chunk, cur.ct, cur.r0, cur.nsteps);
         }
         settle(cur);
-        double xv[16], xn[16];
-        load(cur, xv);
-        for (int j = grp; cur.item < nitems; j += 2) {
-            Pos nxt = cur;
-            nxt.k += 2;
-            settle(nxt);
-            load(nxt, xn);                                     // in flight while this step is converted
+        Pos ahead = cur;                                       // the step whose values are loaded next
+        for (int i = 0; i < nz && ahead.item < nitems; ++i) {
+            if (zlead) issue(ahead, i);
+            ahead.k += 2;
+            settle(ahead);
+        }
+        int ict = -1;
+        double inv = 0.0;
+        for (int j = grp, zt = 0; cur.item < nitems; j += 2, ++zt) {
+            const int zs = zt % nz;
+            PROF_WAIT(w0, umma::mbar_wait_bounded(&zb[zs], (uint32_t)((zt / nz) & 1)));
+            double xv[16];
+            const double *zr = zring + zs * (SF_ZB / 8) + lane;   // row r of the slot: 32 contiguous doubles
+#pragma unroll
+            for (int g = 0; g < 4; ++g)
+#pragma unroll
+                for (int kk = 0; kk < 4; ++kk) xv[g * 4 + kk] = zr[(4 * ((g + rot) & 3) + kk) * CT];
+            // the slot is refilled: the generic-proxy reads of all lanes before the async-proxy write
+            __syncwarp();
+            fence_async_smem();
+            if (ahead.item < nitems) {
+                if (zlead) issue(ahead, zs);
+                ahead.k += 2;
+                settle(ahead);
+            }
+            if (cur.ct != ict) {
+                ict = cur.ct;
+                const int c = ict * CT + lane;
+                inv = c < nvalid ? 18014398509481984.0 / zscale[c] : 0.0;    // 2^54 / scale
+            }
             const int s = j % ns;
-            umma::mbar_wait_bounded(&empty[s], (uint32_t)(((j / ns) & 1) ^ 1));
-            const int c = cur.ct * CT + lane;
-            const double inv = c < nvalid ? 18014398509481984.0 / zscale[c] : 0.0;    // 2^54 / scale
+            PROF_WAIT(w1, umma::mbar_wait_bounded(&empty[s], (uint32_t)(((j / ns) & 1) ^ 1)));
             unsigned char *bt = st_base + (size_t)s * SF_STG + 2 * A_B;
 #pragma unroll
             for (int g = 0; g < 4; ++g) {
@@ -1342,10 +1396,24 @@ stats_i8_fused_kernel(const __grid_constant__ CUtensorMap tmA, long long N, int 
             fence_async_smem();                                 // generic-proxy stores before the MMA's async-proxy reads
             __syncwarp();
             if (lane == 0) mbar_arrive(&full[s]);
-            cur = nxt;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) xv[i] = xn[i];
+            cur.k += 2;
+            settle(cur);
         }
+    }
+#undef PROF_WAIT
+    // [producer: empty][MMA: full, tempty][epilogue warp 2: tfull][converters: loads 8][converters: empty 8][total]
+    if (prof && lane == 0 && (warp < 3 || warp >= 10)) {       // (all lanes of a role wait together: lane 0's clocks are the role's)
+        long long *o = prof + (size_t)blockIdx.x * SF_PROF;
+        if (warp < 2) {
+            o[warp] = w0;
+            if (warp == 1) o[2] = w1;
+        } else if (warp == 2) {
+            o[3] = w0;
+        } else {
+            o[4 + (warp - 10)] = w0;
+            o[12 + (warp - 10)] = w1;
+        }
+        if (warp == 0) o[20] = clock64() - tstart;
     }
     umma::fence_before_sync();
     __syncthreads();
@@ -1658,15 +1726,47 @@ cudaError_t launch_stats_i8(long long N, int D, int q, const void *maskT, const 
     }
     const long long rpc = stats_i8_rows_per_chunk(N, nchunks);
     if (stats_i8_fused(D)) {
-        const int ns = sf_stages(q);
-        const size_t smem = sf_smem_bytes(q, ns);
+        CUtensorMap tmZ;
+        {   // the MZ columns [0, P + q) as [N][P + q] doubles with the row pitch ldmz (16-byte aligned, C-ABI): 32-column x
+            // 16-row boxes, rows >= N and columns >= P + q zero-filled
+            cuuint64_t dz[2] = {(cuuint64_t)(P + q), (cuuint64_t)N}, sz[1] = {(cuuint64_t)ldmz * sizeof(double)};
+            cuuint32_t bz[2] = {CT, 16};
+            CUresult r = enc(&tmZ, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<double *>(MZ), dz, sz, bz, es,
+                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+            if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
+        }
+        const int ns = sf_stages(q), nz = SF_NZ;
+        const size_t smem = sf_smem_bytes(q, ns, nz);
         e = cudaFuncSetAttribute(stats_i8_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
         const long long nitems = (long long)nct * nchunks;
         const int grid = (int)(nitems < 148 ? nitems : 148);
-        stats_i8_fused_kernel<<<grid, SF_NTHR, smem, st>>>(tmA, N, D, q, MZ, ldmz, (const double *)zscale, ws, rpc, nchunks, ndb,
-                                                           nct, ns);
-        return cudaGetLastError();
+        static long long *prof = nullptr;
+        static int prof_on = -1;
+        if (prof_on < 0) {
+            prof_on = getenv("PYVB_I8_PROF") ? 1 : 0;
+            if (prof_on && cudaMalloc(&prof, 148 * SF_PROF * sizeof(long long)) != cudaSuccess) prof_on = 0;
+        }
+        stats_i8_fused_kernel<<<grid, SF_NTHR, smem, st>>>(tmA, tmZ, N, D, q, (const double *)zscale, ws, rpc, nchunks, ndb, nct,
+                                                           ns, nz, prof_on ? prof : (long long *)nullptr);
+        e = cudaGetLastError();
+        if (prof_on && e == cudaSuccess) {      // diagnosis only: synchronises
+            long long h[148 * SF_PROF];
+            cudaStreamSynchronize(st);
+            cudaMemcpy(h, prof, sizeof(h), cudaMemcpyDeviceToHost);
+            double a[SF_PROF] = {0};
+            for (int b = 0; b < grid; ++b)
+                for (int k = 0; k < SF_PROF; ++k) a[k] += (double)h[b * SF_PROF + k] / grid;
+            double cl = 0, ce = 0;
+            for (int w = 0; w < SF_CONV; ++w) {
+                cl += a[4 + w] / SF_CONV;
+                ce += a[12 + w] / SF_CONV;
+            }
+            fprintf(stderr, "[i8 stats prof] N=%lld D=%d q=%d ns=%d nz=%d total %.0f clk | producer: empty %.0f | mma: full %.0f tempty %.0f | epilogue(w2): tfull %.0f | converters: loads %.0f empty %.0f\n",
+                    N, D, q, ns, nz, a[20], a[0], a[1], a[2], a[3], cl, ce);
+        }
+        return e;
     }
     if (ZI == nullptr) return cudaErrorInvalidValue;
     dim3 gd((unsigned)((N + 127) / 128), (unsigned)nct);
