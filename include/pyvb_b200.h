@@ -156,8 +156,8 @@ int pyvb_gw_woff(int q);                               /* first <w_d> column of 
 int pyvb_mz_pitch(int q);                              /* doubles per row of the interleaved [M2 | zbar] array */
 size_t pyvb_stats_len(int D, int q);                   /* doubles */
 size_t pyvb_stats_workspace_bytes(long long N, int D, int q, int algo);
-size_t pyvb_zsums_len(long long N, int q);             /* doubles to allocate (the largest over the K2 kernels); 0 when K2 has no fast path for q */
-int pyvb_zsums_blocks(long long N, int q);             /* partials the K2 kernel in use writes: the first pyvb_zsums_blocks * pyvb_zsums_kw doubles */
+size_t pyvb_zsums_len(long long N, int q);             /* doubles to allocate: pyvb_zsums_blocks * pyvb_zsums_kw; 0 when K2 has no fast path for q */
+int pyvb_zsums_blocks(long long N, int q);             /* partials the K2 kernel of q writes (at most 148) */
 
 /* peer exchange buffers: cudaMalloc'd (zeroed) so that the CUDA IPC handle (64 bytes) names exactly this buffer */
 size_t pyvb_peer_bytes(size_t stats_len);
@@ -310,7 +310,7 @@ int pyvb_f32_pitch(int q);
 int pyvb_f32_zoff(int q);
 int pyvb_f32_poff(int q);
 int pyvb_f32_supported(int D, int q);
-size_t pyvb_zsums_len_f32(long long N, int q);        /* K2 partials of the FP32 path (always the blocked kernel) */
+size_t pyvb_zsums_len_f32(long long N, int q);        /* K2 partials of the FP32 path */
 int pyvb_prepare_x_f32(long long N, int D, const double *X, long long ldx, void *planes, void *stream);
 int pyvb_pack_gw_f32(int D, int q, const double *Wbar, const double *Wvar, const double *mu, void *GT, void *WT,
                      void *stream);

@@ -117,21 +117,7 @@ size_t pyvb_zsums_len_f32(long long N, int q) {
 
 int pyvb_zsums_kw(int q) { return 2 * (gw_woff(q) + q) + PYVB_ZS_EXTRA; }
 
-size_t pyvb_zsums_len(long long N, int q) {
-    size_t len = 0;                                     // the largest over the K2 implementations (PYVB_K2 is read per call)
-    for (int impl = 0; impl <= 5; ++impl) {
-        int nblk, kw;
-        zsolve_partials_of(impl, N, q, nblk, kw);
-        if ((size_t)nblk * kw > len) len = (size_t)nblk * kw;
-        // the Gauss-Jordan and blocked-sweep kernels run one CTA per SM at most, but how many rows a CTA takes depends on the
-        // configuration picked by PYVB_GJ / PYVB_SWEEP, which is also read per call: size for the worst case
-        if ((impl == 4 || impl == 5) && kw > 0) {
-            const size_t worst = (size_t)(N < 148 ? (N < 1 ? 1 : N) : 148) * kw;
-            if (worst > len) len = worst;
-        }
-    }
-    return len;
-}
+size_t pyvb_zsums_len(long long N, int q) { return (size_t)pyvb_zsums_blocks(N, q) * pyvb_zsums_kw(q); }
 
 int pyvb_zsums_blocks(long long N, int q) {
     int nblk, kw;
@@ -403,7 +389,7 @@ int pyvb_zstep_i8_f64(long long N, int D, int q, const double *X, long long ldx,
     if (e == cudaSuccess && !k1_only) {
         // K2 checks every finished qprec row against the fixed-point bound of K1-i8 (kernels.h: I8Check); when a row fails,
         // the whole step is redone on the FP64 tensor cores by two conditional launches that exit at once otherwise
-        const int guard = (k2_impl(q) == 0) ? 0 : i8_guard_mode();
+        const int guard = i8_guard_mode();
         I8Check chk;
         if (guard) {
             chk.gscale = gscale;
@@ -464,14 +450,13 @@ int pyvb_stats_i8_f64(long long N, int D, int q, const double *X, long long ldx,
     ARG(X && maskT && MZ && scratch && xcache, "null pointer (xcache is required)");
     ARG(ZI || stats_i8_fused(D), "ZI is required where pyvb_stats_i8_fused(D, q) is 0");
     ARG(zsums || logdet, "zsums or logdet");
-    ARG(logdet || k2_impl(q) >= 1, "logdet is needed when the K2 partials carry no column maxima");
     ARG(ldx >= D && (ldx % 2) == 0 && ldmz == pyvb_mz_pitch(q), "ldx, ldmz");
     ARG(ws_bytes >= pyvb_stats_i8_workspace_bytes(N, D, q), "workspace too small");
     int nzblk = 0, zkw = 0;
     if (zsums) zsolve_partials(N, q, nzblk, zkw);
     const int nch = stats_i8_nchunks(N, D, q);
-    // the default K2 kernels leave bounds on the column maxima behind their column sums: [sums OROW | 4 | maxima OROW]
-    const bool kmax = nzblk > 0 && k2_impl(q) >= 1;
+    // the K2 kernels leave bounds on the column maxima behind their column sums: [sums OROW | 4 | maxima OROW]
+    const bool kmax = nzblk > 0;
     AuxStream *aux = aux_stream();                              // Ast (FP64 tensor cores on X) next to digitize + the INT8 kernel
     cudaStream_t st2 = st;
     cudaError_t e = cudaSuccess;

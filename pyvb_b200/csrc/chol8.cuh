@@ -4,35 +4,6 @@
 
 namespace pyvb {
 
-// ---- per-LANE 8 x 8 Cholesky + triangular inverse in registers (thread-per-matrix kernel, kernels_k2t.cu; lane-parallel
-// diagonal blocks of the blocked kernel, kernels_k2m.cu).  Packed lower triangle A[c8_idx(i, j)], i >= j.
-// In: SPD block.  Out: X = chol(A)^-1 (lower triangular); lp *= prod_k 1/l_kk.  Straight-line code, no shuffles.
-__host__ __device__ constexpr int c8_idx(int i, int j) { return i * (i + 1) / 2 + j; }
-__device__ __forceinline__ void chol_inv8(double (&A)[36], double &lp) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        const double rinv = rsqrt(A[c8_idx(k, k)]);
-        lp *= rinv;
-        A[c8_idx(k, k)] = rinv;
-#pragma unroll
-        for (int i = k + 1; i < 8; ++i) A[c8_idx(i, k)] *= rinv;
-#pragma unroll
-        for (int j = k + 1; j < 8; ++j)
-#pragma unroll
-            for (int i = j; i < 8; ++i) A[c8_idx(i, j)] = fma(-A[c8_idx(i, k)], A[c8_idx(j, k)], A[c8_idx(i, j)]);
-    }
-    // in-place inverse of L (its diagonal already holds 1 / l_kk), column by column
-#pragma unroll
-    for (int j = 0; j < 8; ++j)
-#pragma unroll
-        for (int i = j + 1; i < 8; ++i) {
-            double s = A[c8_idx(i, j)] * A[c8_idx(j, j)];
-#pragma unroll
-            for (int k = j + 1; k < i; ++k) s = fma(A[c8_idx(i, k)], A[c8_idx(k, j)], s);
-            A[c8_idx(i, j)] = -s * A[c8_idx(i, i)];
-        }
-}
-
 // 8 x 8 diagonal blocks of MPW independent matrices, accumulator layout (lane l: row l/4, columns 2(l%4), 2(l%4)+1).
 // In: the SPD blocks A (lower triangle valid).  Out: X = chol(A)^-1 (lower triangular, exact zeros above the
 // diagonal); lprod[m] is multiplied by prod_k 1/l_kk.  Right-looking factorisation and right-looking inversion fused

@@ -68,42 +68,27 @@ int zstep_eta_pitch(int q);
 cudaError_t launch_zstep_eta_dmma(long long N, int D, int q, const double *X, long long ldx, const double *Gw,
                                   double *weta, const double *P0, const double *h0, double *gl, double *MZ,
                                   cudaStream_t st);
+// K2, the batched q x q solve in place on the MZ rows, one kernel per q: thread per matrix at q = 8 (kernels_k2t.cu), Gauss-Jordan
+// in registers at q = 16, 32 (kernels_k2g.cu), blocked symmetric sweep at q = 64 (kernels_k2s.cu).
 // cond (nullable, device): the kernel exits at once unless *cond > 0 (the conditional fall-back launches of the INT8 path)
 cudaError_t launch_zsolve(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
                           cudaStream_t st, const double *cond = nullptr, I8Check chk = I8Check());
 // K2 leaves nblk partials of kw doubles each in zsums (0, 0: no fast K2 for this q)
 void zsolve_partials(long long N, int q, int &nblk, int &kw);
-void zsolve_partials_of(int impl, long long N, int q, int &nblk, int &kw);
-// blocked tensor-core K2 (kernels_k2.cu): q in {8, 16, 32, 64}
-int zsolve_blocked_blocks(long long N, int q);
-int zsolve_blocked_kw(int q);
-cudaError_t launch_zsolve_blocked(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl,
-                                  double *zsums, cudaStream_t st, const double *cond = nullptr, I8Check chk = I8Check());
-// 0 register-resident, 1 blocked tensor-core, 2 thread per matrix, 3 blocked with lane-parallel diagonal blocks,
-// 4 Gauss-Jordan in registers, 5 blocked symmetric sweep (scalar panel + DMMA update) (PYVB_K2 overrides)
-int k2_impl(int q);
-int k2_impl_f32(int q);   // the FP32-row variant only exists for the blocked / thread-per-matrix kernels
-// blocked tensor-core K2 with lane-parallel 8 x 8 diagonal blocks, several matrices per warp (kernels_k2m.cu): q in {16, 32, 64}
-int zsolve_lanediag_blocks(long long N, int q);
-int zsolve_lanediag_kw(int q);
-cudaError_t launch_zsolve_lanediag(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
-                                   cudaStream_t st, const double *cond = nullptr, I8Check chk = I8Check());
-// Gauss-Jordan-in-registers K2 (kernels_k2g.cu): q in {16, 32}; same partial layout as the blocked kernel
-int zsolve_gj_blocks(long long N, int q);
+// the K2 kernels behind launch_zsolve; all of them leave the partial layout [column sums OROW | 4 scalars | column maxima OROW]
+int zsolve_gj_blocks(long long N, int q);         // q in {16, 32}
 int zsolve_gj_kw(int q);
 cudaError_t launch_zsolve_gj(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
                              cudaStream_t st, const double *cond = nullptr, I8Check chk = I8Check());
-// blocked symmetric sweep, scalar panel + DMMA trailing update, in place in the packed rows (kernels_k2s.cu): q in {16, 32, 64};
-// same partial layout as the blocked kernel
-int zsolve_sweep_blocks(long long N, int q);
+int zsolve_sweep_blocks(long long N, int q);      // q = 64
 int zsolve_sweep_kw(int q);
 cudaError_t launch_zsolve_sweep(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
                                 cudaStream_t st, const double *cond = nullptr, I8Check chk = I8Check());
-// thread-per-matrix K2 (kernels_k2t.cu): q in {8, 16}
-int zsolve_tpm_blocks(long long N, int q);
+int zsolve_tpm_blocks(long long N, int q);        // q in {8, 16} (q = 16: the FP32 rows)
 int zsolve_tpm_kw(int q);
 cudaError_t launch_zsolve_tpm(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
                               cudaStream_t st, const double *cond = nullptr, I8Check chk = I8Check());
+// K2 on the FP32 rows: thread per matrix at q = 16, blocked tensor-core kernel (kernels_k2.cu) at q = 32, 64
 cudaError_t launch_zsolve_tpm_f32(long long N, int q, float *MZ32, void *MP, double *Sig, double *logdet, double *gl,
                                   double *zsums, cudaStream_t st);
 cudaError_t launch_zsolve_f32(long long N, int q, float *MZ32, void *MP, double *Sig, double *logdet, double *gl,

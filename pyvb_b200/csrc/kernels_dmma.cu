@@ -2,9 +2,8 @@
 //
 //   zstep_dmma_kernel<Q>  K1: [O | O.(X-mu)] (rows x D)  @  Gw (D x (P+q))  -> per-row [qprec packed | eta],
 //                             written into the MZ row (one bulk store per row)
-//   zsolve_kernel<Q>      K2: per-row Cholesky / inverse / solve IN PLACE on the MZ rows with the matrix row
-//                             held in registers (lane i owns row i; q lanes per matrix):
-//                             [qprec | eta] -> [<zz^T> packed | zbar].  Separate kernel on purpose: K2 is a
+//   K2 (launch_zsolve below, kernels in kernels_k2*.cu): per-row q x q SPD inverse / solve IN PLACE on the MZ rows,
+//                             [qprec | eta] -> [<zz^T> packed | zbar].  Separate kernels on purpose: K2 is a
 //                             latency-bound DFMA chain; fused behind K1 it kept the CTA's registers and the
 //                             DMMA pipe idle half of the time (profiles/r01_ncu_*.md)
 //   stats_dmma_kernel<Q>  K3: [O | O.X]^T (D x rows) @ [<zz^T> | zbar] (rows x (P+q)) -> T1, Bst, Ast
@@ -19,7 +18,6 @@
 // four rows a half-warp touches differ in the swizzle bits, and row pitches of the non-swizzled tiles are
 // 32 or 96 bytes mod 128.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -136,137 +134,6 @@ template <int Q, bool ETA = false> struct ZT {
     static constexpr size_t SMEM = 1024 + (size_t)MAIN_B + (size_t)(P + Q) * 8 + 2 * ST * 8;
     static_assert(XT_B % 1024 == 0, "swizzled tiles must stay 1024-byte aligned");
 };
-
-// ------------------------------------------------------------------ K2: per-row Cholesky inverse in registers
-// Lane li of a Q-lane group owns row li of the matrix (registers, statically indexed: everything below is
-// fully unrolled).  Both passes are RIGHT-LOOKING so that the only serial dependence per step is
-// pivot -> rsqrt -> broadcast; all multiply-adds of a step are independent of each other:
-//   pass 1 (Cholesky):  l_ik = a_ik / sqrt(a_kk);  a_ij -= l_ik l_jk  for all j > k      (column k broadcast via smem)
-//   pass 2 (X = L^-1, lane j owns column j, fused with Sigma = X^T X):
-//                       x_k = (delta_jk - t_k) / l_kk;  t_i += l_ik x_k for all i > k;  Sigma_j. += x_k * (row k of X)
-// The factor is kept column-major in shared memory (packed: column k holds rows k..Q-1, its diagonal slot
-// holds 1/l_kk), which is exactly the order in which both passes broadcast it.
-__host__ __device__ constexpr int c_lcol(int k, int Q) { return k * Q - k * (k - 1) / 2 - k; }   // + i addresses (i,k), i >= k
-
-template <int Q, int MI>
-__device__ __forceinline__ void k2_solve(const double *const (&Arow)[MI], const double *const (&eta)[MI],
-                                         double *const (&Lc)[MI], double *xbuf, const int li,
-                                         double (&Sg)[MI][Q], double (&z)[MI], double (&ldet)[MI], bool (&ok)[MI]) {
-    const int lane = threadIdx.x & 31;
-    double Ar[MI][Q];
-#pragma unroll
-    for (int m = 0; m < MI; ++m) {
-#pragma unroll
-        for (int j = 0; j < Q; ++j) Ar[m][j] = (j <= li) ? Arow[m][j] : 0.0;   // row li of the lower triangle
-    }
-    // ---- pass 1: right-looking Cholesky
-#pragma unroll
-    for (int k = 0; k < Q; ++k) {
-#pragma unroll
-        for (int m = 0; m < MI; ++m) {
-            const double d = __shfl_sync(0xffffffffu, Ar[m][k], k, Q);
-            const double rinv = rsqrt(d);                 // d <= 0 -> NaN / inf, caught through the log-det below
-            const double l = Ar[m][k] * rinv;
-            Ar[m][k] = l;
-            if (li >= k) Lc[m][c_lcol(k, Q) + li] = (li == k) ? rinv : l;
-        }
-        __syncwarp();
-        if (k + 1 < Q) {
-#pragma unroll
-            for (int m = 0; m < MI; ++m) {
-                const double *col = Lc[m] + c_lcol(k, Q);
-                const double nl = -Ar[m][k];
-                constexpr int dummy = 0;
-                (void)dummy;
-                int j = k + 1;
-                if ((c_lcol(k, Q) + j) & 1) {   // compile-time parity: first element unaligned for a 16-byte load
-                    Ar[m][j] = fma(nl, col[j], Ar[m][j]);
-                    ++j;
-                }
-#pragma unroll
-                for (int jj = 0; jj < Q; jj += 2) {
-                    const int j2 = j + jj;
-                    if (j2 + 1 < Q) {
-                        const double2 l2 = *reinterpret_cast<const double2 *>(col + j2);
-                        Ar[m][j2] = fma(nl, l2.x, Ar[m][j2]);
-                        Ar[m][j2 + 1] = fma(nl, l2.y, Ar[m][j2 + 1]);
-                    } else if (j2 < Q) {
-                        Ar[m][j2] = fma(nl, col[j2], Ar[m][j2]);
-                    }
-                }
-            }
-        }
-    }
-    // ln prod diag chol = -sum_k ln(1/l_kk): lane li takes its own diagonal slot, the group adds up
-#pragma unroll
-    for (int m = 0; m < MI; ++m) {
-        double v = -log(Lc[m][c_lcol(0, Q) + li * Q - li * (li - 1) / 2]);
-#pragma unroll
-        for (int o = Q / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        ldet[m] = v;
-        ok[m] = (v - v == 0.0);                           // finite <=> every pivot was positive
-    }
-    // ---- pass 2: X = L^-1 (column li per lane) and Sigma = X^T X
-    double t[MI][Q];
-#pragma unroll
-    for (int m = 0; m < MI; ++m)
-#pragma unroll
-        for (int j = 0; j < Q; ++j) {
-            Sg[m][j] = 0.0;
-            t[m][j] = 0.0;
-        }
-#pragma unroll
-    for (int k = 0; k < Q; ++k) {
-        double xk[MI];
-        double *xb = xbuf + (k & 1) * (MI * 32);
-#pragma unroll
-        for (int m = 0; m < MI; ++m) {
-            const double *col = Lc[m] + c_lcol(k, Q);
-            xk[m] = (((li == k) ? 1.0 : 0.0) - t[m][k]) * col[k];
-            xb[m * 32 + lane] = xk[m];
-            int i = k + 1;
-            if (i < Q && ((c_lcol(k, Q) + i) & 1)) {
-                t[m][i] = fma(col[i], xk[m], t[m][i]);
-                ++i;
-            }
-#pragma unroll
-            for (int ii = 0; ii < Q; ii += 2) {
-                const int i2 = i + ii;
-                if (i2 + 1 < Q) {
-                    const double2 l2 = *reinterpret_cast<const double2 *>(col + i2);
-                    t[m][i2] = fma(l2.x, xk[m], t[m][i2]);
-                    t[m][i2 + 1] = fma(l2.y, xk[m], t[m][i2 + 1]);
-                } else if (i2 < Q) {
-                    t[m][i2] = fma(col[i2], xk[m], t[m][i2]);
-                }
-            }
-        }
-        __syncwarp();
-#pragma unroll
-        for (int m = 0; m < MI; ++m) {
-            const double *xrow = xb + m * 32 + (lane - li);       // row k of X: entries j <= k are non-zero
-#pragma unroll
-            for (int j = 0; j + 1 <= k; j += 2) {
-                const double2 x2 = *reinterpret_cast<const double2 *>(xrow + j);
-                Sg[m][j] = fma(xk[m], x2.x, Sg[m][j]);
-                Sg[m][j + 1] = fma(xk[m], x2.y, Sg[m][j + 1]);
-            }
-            if (!(k & 1)) Sg[m][k] = fma(xk[m], xrow[k], Sg[m][k]);
-        }
-    }
-    // ---- posterior mean: z = Sigma . eta
-#pragma unroll
-    for (int m = 0; m < MI; ++m) {
-        double z0 = 0.0, z1 = 0.0;
-#pragma unroll
-        for (int j = 0; j < Q; j += 2) {
-            const double2 e2 = *reinterpret_cast<const double2 *>(eta[m] + j);
-            z0 = fma(Sg[m][j], e2.x, z0);
-            z1 = fma(Sg[m][j + 1], e2.y, z1);
-        }
-        z[m] = z0 + z1;
-    }
-}
 
 // ------------------------------------------------------------------ Z step, part 1 (K1): tensor-core contraction
 // Persistent: every CTA walks over (row tile, column tile) pairs; the TMA pipeline runs CONTINUOUSLY across the
@@ -449,160 +316,6 @@ zstep_dmma_kernel(const __grid_constant__ CUtensorMap tmX, long long N, int D, c
     }
 }
 
-// ------------------------------------------------------------------ Z step, part 2 (K2): batched q x q solve
-template <int Q> struct KC2;
-template <> struct KC2<8>  { static constexpr int MI = 2, WARPS = 4, OCC = 3; };
-template <> struct KC2<16> { static constexpr int MI = 2, WARPS = 4, OCC = 3; };
-template <> struct KC2<32> { static constexpr int MI = 1, WARPS = 4, OCC = 3; };
-
-template <int Q> struct K2T {
-    static constexpr int P = c_tri(Q), PP = (P + 7) & ~7, OROW = PP + Q, LDG = c_gw_pitch(Q);
-    static constexpr int MI = KC2<Q>::MI, WARPS = KC2<Q>::WARPS;
-    static constexpr int G = 32 / Q, RPP = G * MI;           // rows per warp pass
-    // per warp: 2 x RPP rows (double buffered, solved in place), RPP packed column-major factors,
-    // broadcast scratch, 2 mbarriers
-    static constexpr int WARP_D = 2 * RPP * OROW + RPP * P + 2 * MI * 32 + 2 + OROW;
-    static constexpr size_t SMEM = (size_t)WARPS * WARP_D * 8 + 16;
-    static constexpr int KW = 2 * OROW + PYVB_ZS_EXTRA;       // doubles per CTA in the partials: [sums | 4 scalars | maxima (unused: 0)]
-    static_assert(WARP_D % 2 == 0 && OROW % 2 == 0 && P % 2 == 0, "16-byte alignment of the per-warp buffers");
-};
-
-// rows [0, N) of MZ hold [qprec packed | pad | eta]; they are replaced by [<zz^T> packed | 0 | zbar].
-// Each warp walks its own contiguous block of rows, RPP rows per pass; loads are bulk copies one pass ahead.
-template <int Q>
-__global__ void __launch_bounds__(32 * KC2<Q>::WARPS, KC2<Q>::OCC)
-zsolve_kernel(long long N, double *__restrict__ MZ, double *__restrict__ Sig, double *__restrict__ logdet,
-              double *gl, long long rows_per_warp, double *__restrict__ zsums) {
-    using T = K2T<Q>;
-    extern __shared__ __align__(16) double smem_k2[];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    double *base = smem_k2 + (size_t)warp * T::WARP_D;
-    double *raw = base;                                      // [2][RPP][OROW]
-    double *lcs = raw + 2 * T::RPP * T::OROW;                // [RPP][P]
-    double *xbuf = lcs + T::RPP * T::P;                      // [2][MI*32]
-    uint64_t *bar = reinterpret_cast<uint64_t *>(xbuf + 2 * T::MI * 32);   // [2]
-    double *csum = xbuf + 2 * T::MI * 32 + 2;                // [OROW] column sums of this warp's output rows
-    const int li = lane % Q, lg = lane / Q;
-    const long long wr0 = ((long long)blockIdx.x * T::WARPS + warp) * rows_per_warp;
-    long long wr1 = wr0 + rows_per_warp;
-    if (wr1 > N) wr1 = N;
-    if (lane == 0) {
-        mbar_init(&bar[0], 1);
-        mbar_init(&bar[1], 1);
-        mbar_fence_init();
-    }
-    for (int c = lane; c < T::OROW; c += 32) csum[c] = 0.0;
-    double s_qld = 0.0, s_ld = 0.0, s_n = 0.0;               // sum 0.5/logdet, sum logdet, rows (lanes with li == 0)
-    __syncwarp();
-    const int npass = (wr1 > wr0) ? (int)((wr1 - wr0 + T::RPP - 1) / T::RPP) : 0;
-
-    auto load = [&](int pass) {      // lane 0: bulk loads of the pass' rows into raw[pass & 1]
-        const int b = pass & 1;
-        const long long r0 = wr0 + (long long)pass * T::RPP;
-        const int nv = (wr1 - r0 < T::RPP) ? (int)(wr1 - r0) : T::RPP;
-        mbar_arrive_expect_tx(&bar[b], (uint32_t)(nv * T::OROW * 8));
-        for (int r = 0; r < nv; ++r)
-            bulk_g2s(raw + (size_t)(b * T::RPP + r) * T::OROW, MZ + (r0 + r) * T::LDG, T::OROW * 8, &bar[b]);
-    };
-    if (lane == 0 && npass > 0) load(0);
-    uint32_t ph[2] = {0, 0};
-    for (int pass = 0; pass < npass; ++pass) {
-        const int b = pass & 1;
-        if (lane == 0 && pass + 1 < npass) {
-            bulk_wait_read_all();    // the stores that read raw[b ^ 1] one pass ago have drained
-            load(pass + 1);
-        }
-        mbar_wait(&bar[b], ph[b]);
-        ph[b] ^= 1;
-        const long long r0 = wr0 + (long long)pass * T::RPP;
-        double *O[T::MI];
-        const double *Arow[T::MI];
-        const double *eta[T::MI];
-        double *Lc[T::MI];
-        long long nrow[T::MI];
-#pragma unroll
-        for (int m = 0; m < T::MI; ++m) {
-            const int r = lg * T::MI + m;
-            O[m] = raw + (size_t)(b * T::RPP + r) * T::OROW;
-            nrow[m] = r0 + r;
-            if (nrow[m] >= wr1) {     // tail of the block: solve the identity instead of stale shared memory
-#pragma unroll
-                for (int j = 0; j < Q; ++j)
-                    if (j <= li) O[m][c_tri(li) + j] = (j == li) ? 1.0 : 0.0;
-                O[m][T::PP + li] = 0.0;
-            }
-            Arow[m] = O[m] + c_tri(li);
-            eta[m] = O[m] + T::PP;
-            Lc[m] = lcs + (size_t)r * T::P;
-        }
-        __syncwarp();
-        double Sg[T::MI][Q], z[T::MI], ldet[T::MI];
-        bool ok[T::MI];
-        k2_solve<Q, T::MI>(Arow, eta, Lc, xbuf, li, Sg, z, ldet, ok);
-#pragma unroll
-        for (int m = 0; m < T::MI; ++m) xbuf[m * 32 + lane] = z[m];
-        __syncwarp();                // also: every lane has read eta before the row is overwritten
-#pragma unroll
-        for (int m = 0; m < T::MI; ++m) {
-            const bool valid = nrow[m] < wr1;
-            const double *zrow = xbuf + m * 32 + (lane - li);
-            double *orow = O[m] + c_tri(li);
-            double *sgl = (Sig != nullptr && valid) ? (Sig + nrow[m] * T::P + c_tri(li)) : nullptr;
-#pragma unroll
-            for (int j = 0; j < Q; ++j) {
-                if (j <= li) {
-                    orow[j] = fma(z[m], zrow[j], Sg[m][j]);
-                    if (sgl) sgl[j] = Sg[m][j];
-                }
-            }
-            O[m][T::PP + li] = z[m];
-            if (li == 0 && valid) {
-                logdet[nrow[m]] = ldet[m];
-                s_qld += 0.5 / ldet[m];
-                s_ld += ldet[m];
-                s_n += 1.0;
-                if (!ok[m]) atomicAdd(&gl[PYVB_GL_NONPD], 1.0);
-            }
-        }
-        fence_async_smem();
-        __syncwarp();
-        const int nv = (wr1 - r0 < T::RPP) ? (int)(wr1 - r0) : T::RPP;
-        if (lane == 0) {
-            for (int r = 0; r < nv; ++r)
-                bulk_s2g(MZ + (r0 + r) * T::LDG, raw + (size_t)(b * T::RPP + r) * T::OROW, T::OROW * 8);
-            bulk_commit();
-        }
-        // column sums of the finished rows (S = sum <zz^T>, zsum = sum zbar): saves a pass over MZ
-        for (int c = lane; c < T::OROW; c += 32) {
-            double a = csum[c];
-            for (int r = 0; r < nv; ++r) a += raw[(size_t)(b * T::RPP + r) * T::OROW + c];
-            csum[c] = a;
-        }
-        __syncwarp();                // all lanes are done with raw[b] before it is reloaded
-    }
-    if (lane == 0) bulk_wait_read_all();
-    if (zsums == nullptr) return;    // kernel-uniform
-    // ---- CTA partial of the column sums and of the per-row scalars, fixed order
-    s_qld = warp_sum(s_qld);
-    s_ld = warp_sum(s_ld);
-    s_n = warp_sum(s_n);
-    if (lane == 0) {
-        xbuf[0] = s_qld;
-        xbuf[1] = s_ld;
-        xbuf[2] = s_n;
-    }
-    __syncthreads();
-    double *out = zsums + (size_t)blockIdx.x * T::KW;
-    for (int c = threadIdx.x; c < T::KW; c += 32 * T::WARPS) {
-        double a = 0.0;
-        for (int w = 0; w < T::WARPS; ++w) {
-            const double *wb = smem_k2 + (size_t)w * T::WARP_D + 2 * T::RPP * T::OROW + T::RPP * T::P;   // xbuf of warp w
-            a += (c < T::OROW) ? wb[2 * T::MI * 32 + 2 + c] : ((c - T::OROW < 3) ? wb[c - T::OROW] : 0.0);
-        }
-        out[c] = a;
-    }
-}
-
 // pure-DMMA loop: the FP64 tensor roofline of the box (see pyvb_bench_dmma_f64)
 __global__ void __launch_bounds__(256) bench_dmma_kernel(double *out, int iters, double a, double b) {
     double c[8][2];
@@ -624,100 +337,6 @@ cudaError_t launch_bench_dmma(int blocks, int iters, double *scratch, cudaStream
 }
 
 bool dmma_supported(int D, int q) { return (q == 8 || q == 16 || q == 32 || q == 64) && D >= 16 && (D % 16) == 0; }
-
-// Grid of K2: two waves of CTAs over 148 SMs x OCC (every row costs the same), each warp owns a contiguous
-// block of rows (a multiple of the pass size).  Also the number of column-sum partials.
-template <int Q>
-static void zsolve_plan(long long N, long long &blocks, long long &rpw) {
-    using T = K2T<Q>;
-    const long long warps_target = 148LL * KC2<Q>::OCC * T::WARPS * 2;
-    rpw = (N + warps_target - 1) / warps_target;
-    rpw = ((rpw + T::RPP - 1) / T::RPP) * T::RPP;
-    if (rpw < 4 * T::RPP) rpw = 4 * T::RPP;
-    const long long nwarps = (N + rpw - 1) / rpw;
-    blocks = (nwarps + T::WARPS - 1) / T::WARPS;
-    if (blocks < 1) blocks = 1;
-}
-
-template <int Q>
-static cudaError_t launch_zsolve_q(long long N, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
-                                   cudaStream_t st) {
-    using T = K2T<Q>;
-    cudaError_t e = cudaFuncSetAttribute(zsolve_kernel<Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::SMEM);
-    if (e != cudaSuccess) return e;
-    long long blocks, rpw;
-    zsolve_plan<Q>(N, blocks, rpw);
-    zsolve_kernel<Q><<<(unsigned)blocks, 32 * T::WARPS, T::SMEM, st>>>(N, MZ, Sig, logdet, gl, rpw, zsums);
-    return cudaGetLastError();
-}
-
-// Which batched solve runs for this q: 0 = register-resident (lane per matrix row, above), 1 = blocked tensor-core
-// kernel (kernels_k2.cu), 2 = thread per matrix (kernels_k2t.cu), 3 = lane-parallel diagonal blocks (kernels_k2m.cu), 4 = Gauss-Jordan
-// (kernels_k2g.cu), 5 = blocked symmetric sweep (kernels_k2s.cu).  q = 64 exists blocked / lanediag / sweep.  PYVB_K2 = reg /
-// blocked / tpm / lanediag / gj / sweep overrides the default (measured per 1M rows, FP64: q = 16: 1.62 / 2.0 / see DESIGN ms; q = 32: 9.0 / 5.8).
-int k2_impl(int q) {
-    const char *e = getenv("PYVB_K2");               // read per call (tests flip it); callers size zsums with pyvb_zsums_len
-    int mode = (e && e[0] == 'b') ? 1 : (e && e[0] == 'r') ? 0 : (e && e[0] == 't') ? 2 : (e && e[0] == 'l') ? 3
-               : (e && e[0] == 'g') ? 4 : (e && e[0] == 's') ? 5 : -1;
-    if (q == 64 && (mode == 0 || mode == 2)) mode = -1;  // q = 64 only exists blocked
-    if (mode == 2 && q > 16) mode = -1;
-    if (mode == 3 && q < 16) mode = -1;
-    if (mode == 4 && q != 16 && q != 32) mode = -1;
-    if (mode == 5 && q != 16 && q != 32 && q != 64) mode = -1;
-    if (mode >= 0) return mode;
-    if (q == 16 || q == 32) return 4;
-    // q = 64: the blocked sweep on swizzled tiles (kernels_k2s.cu): 11.4 ms per 400k rows against 12.3 for the blocked Cholesky kernel,
-    // and it leaves the column sums / maxima, which saves the statistics' extra pass over the MZ rows: 24.1 -> 21.4 ms per sweep at the
-    // config-4 shape.  (q = 32: 6.0 vs 5.5 ms for the Gauss-Jordan kernel, q = 16: 1.4 vs 0.6: not there.)
-    if (q == 64) return 5;
-    return q >= 32 ? 1 : 2;      // (the lane-parallel-diagonal kernel, 3, is not faster: 7.7 vs 7.4 ms at q = 32; DESIGN.md 5)
-}
-int k2_impl_f32(int q) {
-    const int impl = k2_impl(q);
-    return (impl == 4 || impl == 5) ? (q >= 32 ? 1 : 2) : impl;
-}
-
-void zsolve_partials(long long N, int q, int &nblk, int &kw) { zsolve_partials_of(k2_impl(q), N, q, nblk, kw); }
-
-// the partials implementation `impl` leaves (pyvb_zsums_len sizes the buffer for the largest of them: PYVB_K2 may change
-// between the allocation and a later call)
-void zsolve_partials_of(int impl, long long N, int q, int &nblk, int &kw) {
-    long long b = 0, r = 0;
-    nblk = kw = 0;
-    if (N <= 0) return;
-    if (impl == 1) {
-        kw = zsolve_blocked_kw(q);
-        nblk = kw > 0 ? zsolve_blocked_blocks(N, q) : 0;
-        return;
-    }
-    if (impl == 2) {
-        kw = zsolve_tpm_kw(q);
-        nblk = zsolve_tpm_blocks(N, q);
-        return;
-    }
-    if (impl == 3) {
-        kw = zsolve_lanediag_kw(q);
-        nblk = kw > 0 ? zsolve_lanediag_blocks(N, q) : 0;
-        return;
-    }
-    if (impl == 4) {
-        kw = zsolve_gj_kw(q);
-        nblk = kw > 0 ? zsolve_gj_blocks(N, q) : 0;
-        return;
-    }
-    if (impl == 5) {
-        kw = zsolve_sweep_kw(q);
-        nblk = kw > 0 ? zsolve_sweep_blocks(N, q) : 0;
-        return;
-    }
-    switch (q) {
-        case 8: zsolve_plan<8>(N, b, r); kw = K2T<8>::KW; break;
-        case 16: zsolve_plan<16>(N, b, r); kw = K2T<16>::KW; break;
-        case 32: zsolve_plan<32>(N, b, r); kw = K2T<32>::KW; break;
-        default: return;
-    }
-    nblk = (int)b;
-}
 
 template <int Q, bool ETA>
 static cudaError_t launch_k1_q(long long N, int D, const double *X, long long ldx, const double *Gw, const double *P0,
@@ -794,22 +413,33 @@ cudaError_t launch_zstep_dmma(long long N, int D, int q, const double *X, long l
     return cudaErrorNotSupported;
 }
 
+// K2, one kernel per q (DESIGN.md 5 has the measurements behind the choice): thread per matrix at q = 8 (kernels_k2t.cu),
+// Gauss-Jordan in registers at q = 16, 32 (kernels_k2g.cu), blocked symmetric sweep on swizzled tiles at q = 64 (kernels_k2s.cu)
+void zsolve_partials(long long N, int q, int &nblk, int &kw) {
+    nblk = kw = 0;
+    if (N <= 0) return;
+    switch (q) {
+        case 8: kw = zsolve_tpm_kw(q), nblk = zsolve_tpm_blocks(N, q); break;
+        case 16:
+        case 32: kw = zsolve_gj_kw(q), nblk = zsolve_gj_blocks(N, q); break;
+        case 64: kw = zsolve_sweep_kw(q), nblk = zsolve_sweep_blocks(N, q); break;
+    }
+}
+
 cudaError_t launch_zsolve(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
                           cudaStream_t st, const double *cond, I8Check chk) {
     if (N <= 0) return cudaSuccess;
-    const int impl = k2_impl(q);
-    // the Gauss-Jordan kernel moves the rows with bulk copies: 16-byte aligned rows (the pitch is a multiple of 32 bytes)
-    if ((impl == 4 || impl == 5) && (reinterpret_cast<uintptr_t>(MZ) & 15) != 0) return cudaErrorMisalignedAddress;
-    if (impl == 1) return launch_zsolve_blocked(N, q, MZ, Sig, logdet, gl, zsums, st, cond, chk);
-    if (impl == 2) return launch_zsolve_tpm(N, q, MZ, Sig, logdet, gl, zsums, st, cond, chk);
-    if (impl == 3) return launch_zsolve_lanediag(N, q, MZ, Sig, logdet, gl, zsums, st, cond, chk);
-    if (impl == 4) return launch_zsolve_gj(N, q, MZ, Sig, logdet, gl, zsums, st, cond, chk);
-    if (impl == 5) return launch_zsolve_sweep(N, q, MZ, Sig, logdet, gl, zsums, st, cond, chk);
-    if (cond != nullptr || chk.gscale != nullptr) return cudaErrorNotSupported;   // the cross-check kernel has no guard
+    // the Gauss-Jordan and sweep kernels move the rows with bulk copies: 16-byte aligned rows (the pitch is a multiple of 32 bytes)
+    const bool aligned = (reinterpret_cast<uintptr_t>(MZ) & 15) == 0;
     switch (q) {
-        case 8: return launch_zsolve_q<8>(N, MZ, Sig, logdet, gl, zsums, st);
-        case 16: return launch_zsolve_q<16>(N, MZ, Sig, logdet, gl, zsums, st);
-        case 32: return launch_zsolve_q<32>(N, MZ, Sig, logdet, gl, zsums, st);
+        case 8: return launch_zsolve_tpm(N, q, MZ, Sig, logdet, gl, zsums, st, cond, chk);
+        case 16:
+        case 32:
+            if (!aligned) return cudaErrorMisalignedAddress;
+            return launch_zsolve_gj(N, q, MZ, Sig, logdet, gl, zsums, st, cond, chk);
+        case 64:
+            if (!aligned) return cudaErrorMisalignedAddress;
+            return launch_zsolve_sweep(N, q, MZ, Sig, logdet, gl, zsums, st, cond, chk);
     }
     return cudaErrorNotSupported;
 }

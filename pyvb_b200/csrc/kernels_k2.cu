@@ -1,7 +1,8 @@
 // K2, blocked: batched q x q SPD inverse / solve with the FP64 tensor cores (DMMA.8x8x4), one warp per matrix.
 //
 // Replaces, per row n, the reference's  cho_factor(qprec) / cho_solve(., I) / dot(qcov, .)  and
-// q_ln_det = .5/log(prod(diag(chol)))  (nodes/gaussian.py:117-123) for q in {8, 16, 32, 64}.
+// q_ln_det = .5/log(prod(diag(chol)))  (nodes/gaussian.py:117-123) for the FP32 rows at q = 32, 64 (the FP64 rows have a
+// faster kernel at every q: launch_zsolve, DESIGN.md 5).
 //
 // The matrix lives in shared memory as NB x NB lower-triangular storage of 8 x 8 blocks (NB = q/8, 64 doubles per
 // block, 32-byte chunks XOR-swizzled so that every DMMA fragment pattern -- row-wise, transposed, accumulator --
@@ -38,8 +39,6 @@ template <int Q> struct KBC;
 // MPW: matrices per warp, processed as interleaved instruction streams (the 8 x 8 diagonal blocks are a chain of
 // 8 dependent pivots each; a second matrix fills the latency)
 // (measured: MPW = 2 does not help -- the kernel is issue-bound, not latency-bound -- so MPW = 1 everywhere)
-template <> struct KBC<8>  { static constexpr int WARPS = 8,  OCC = 3, MPW = 1; static constexpr bool ZS = true; };
-template <> struct KBC<16> { static constexpr int WARPS = 8,  OCC = 2, MPW = 1; static constexpr bool ZS = true; };
 template <> struct KBC<32> { static constexpr int WARPS = 10, OCC = 2, MPW = 1; static constexpr bool ZS = true; };
 template <> struct KBC<64> { static constexpr int WARPS = 11, OCC = 1, MPW = 1; static constexpr bool ZS = false; };
 
@@ -449,77 +448,43 @@ zsolve_blocked_kernel(long long N, typename KIO<Q, F32>::type *__restrict__ MZ, 
     }
 }
 
-template <int Q, bool F32>
-cudaError_t launch_blocked_q(long long N, void *MZ, double *Sig, double *logdet, double *gl, double *zsums, void *MP,
-                             cudaStream_t st, const double *cond = nullptr, I8Check chk = I8Check()) {
+template <int Q>
+int blocked_blocks(long long N) {
     using T = KB<Q>;
-    cudaError_t e = cudaFuncSetAttribute(zsolve_blocked_kernel<Q, F32>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    long long b = (N + (long long)T::MPW * T::WARPS - 1) / ((long long)T::MPW * T::WARPS);
+    if (b > 148LL * T::OCC) b = 148LL * T::OCC;
+    if (b < 1) b = 1;
+    return (int)b;
+}
+
+template <int Q>
+cudaError_t launch_blocked_q(long long N, float *MZ32, void *MP, double *Sig, double *logdet, double *gl, double *zsums,
+                             cudaStream_t st) {
+    using T = KB<Q>;
+    cudaError_t e = cudaFuncSetAttribute(zsolve_blocked_kernel<Q, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)T::SMEM);
     if (e != cudaSuccess) return e;
-    const int blocks = zsolve_blocked_blocks(N, Q);
-    zsolve_blocked_kernel<Q, F32><<<blocks, 32 * T::WARPS, T::SMEM, st>>>(
-        N, static_cast<typename KIO<Q, F32>::type *>(MZ), Sig, logdet, gl, T::ZS ? zsums : nullptr,
-        static_cast<__nv_bfloat16 *>(MP), cond, chk);
+    zsolve_blocked_kernel<Q, true><<<blocked_blocks<Q>(N), 32 * T::WARPS, T::SMEM, st>>>(
+        N, MZ32, Sig, logdet, gl, T::ZS ? zsums : nullptr, static_cast<__nv_bfloat16 *>(MP), nullptr, I8Check());
     return cudaGetLastError();
 }
 
 }  // namespace
 
-int zsolve_blocked_blocks(long long N, int q) {
-    int warps = 8, occ = 2, mpw = 1;
-    switch (q) {
-        case 8: warps = KB<8>::WARPS; occ = KB<8>::OCC; mpw = KB<8>::MPW; break;
-        case 16: warps = KB<16>::WARPS; occ = KB<16>::OCC; mpw = KB<16>::MPW; break;
-        case 32: warps = KB<32>::WARPS; occ = KB<32>::OCC; mpw = KB<32>::MPW; break;
-        case 64: warps = KB<64>::WARPS; occ = KB<64>::OCC; mpw = KB<64>::MPW; break;
-        default: return 0;
-    }
-    long long b = (N + (long long)mpw * warps - 1) / ((long long)mpw * warps);
-    if (b > 148LL * occ) b = 148LL * occ;
-    if (b < 1) b = 1;
-    return (int)b;
-}
-
-int zsolve_blocked_kw(int q) {
-    switch (q) {
-        case 8: return KB<8>::KW;
-        case 16: return KB<16>::KW;
-        case 32: return KB<32>::KW;
-    }
-    return 0;   // q = 64: no column-sum partials (the statistics pass sums the MZ rows itself)
-}
-
-cudaError_t launch_zsolve_blocked(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl,
-                                  double *zsums, cudaStream_t st, const double *cond, I8Check chk) {
-    if (N <= 0) return cudaSuccess;
-    switch (q) {
-        case 8: return launch_blocked_q<8, false>(N, MZ, Sig, logdet, gl, zsums, nullptr, st, cond, chk);
-        case 16: return launch_blocked_q<16, false>(N, MZ, Sig, logdet, gl, zsums, nullptr, st, cond, chk);
-        case 32: return launch_blocked_q<32, false>(N, MZ, Sig, logdet, gl, zsums, nullptr, st, cond, chk);
-        case 64: return launch_blocked_q<64, false>(N, MZ, Sig, logdet, gl, zsums, nullptr, st, cond, chk);
-    }
-    return cudaErrorNotSupported;
-}
-
+// q = 16: the thread-per-matrix kernel (kernels_k2t.cu); q = 64: no column-sum partials (the statistics pass sums the rows itself)
 void zsolve_partials_f32(long long N, int q, int &nblk, int &kw) {
-    if (q == 16 && k2_impl_f32(q) == 2) {
-        kw = zsolve_tpm_kw(q);
-        nblk = N > 0 ? zsolve_tpm_blocks(N, q) : 0;
-        return;
-    }
-    kw = (q == 16 || q == 32) ? zsolve_blocked_kw(q) : 0;
-    nblk = (kw > 0 && N > 0) ? zsolve_blocked_blocks(N, q) : 0;
+    kw = (q == 16) ? zsolve_tpm_kw(q) : (q == 32) ? KB<32>::KW : 0;
+    nblk = (kw == 0 || N <= 0) ? 0 : (q == 16) ? zsolve_tpm_blocks(N, q) : blocked_blocks<32>(N);
 }
 
 // FP32 rows (see KIO): in place on MZ32, plus the bf16 x 3 split of the finished rows into MP [3][N][pitch]
 cudaError_t launch_zsolve_f32(long long N, int q, float *MZ32, void *MP, double *Sig, double *logdet, double *gl,
                               double *zsums, cudaStream_t st) {
     if (N <= 0) return cudaSuccess;
-    if (q == 16 && k2_impl_f32(q) == 2) return launch_zsolve_tpm_f32(N, q, MZ32, MP, Sig, logdet, gl, zsums, st);
     switch (q) {
-        case 16: return launch_blocked_q<16, true>(N, MZ32, Sig, logdet, gl, zsums, MP, st);
-        case 32: return launch_blocked_q<32, true>(N, MZ32, Sig, logdet, gl, zsums, MP, st);
-        case 64: return launch_blocked_q<64, true>(N, MZ32, Sig, logdet, gl, zsums, MP, st);
+        case 16: return launch_zsolve_tpm_f32(N, q, MZ32, MP, Sig, logdet, gl, zsums, st);
+        case 32: return launch_blocked_q<32>(N, MZ32, MP, Sig, logdet, gl, zsums, st);
+        case 64: return launch_blocked_q<64>(N, MZ32, MP, Sig, logdet, gl, zsums, st);
     }
     return cudaErrorNotSupported;
 }

@@ -22,9 +22,6 @@
 // use the same broadcast scheme.  The rows of a group (MPW matrices) travel as ONE bulk copy each way (global -> shared ->
 // registers ... registers -> shared -> global, in place), column sums / maxima bounds / log-det scalars per CTA as in the
 // other K2 kernels (zsums partial layout of the blocked kernel).
-#include <stdio.h>
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "kernels.h"
 #include "ptx.cuh"
@@ -389,6 +386,20 @@ zsolve_gj_kernel(long long N, double *__restrict__ MZ, double *__restrict__ Sig,
     }
 }
 
+// The configuration of each q (rows per lane, warps per CTA).  Measured per launch (B200): q = 16, N = 1M: (4, 8) 0.642 ms,
+// (2, 16) 0.79, (2, 12) 0.81, (2, 8) 0.89, (1, 16) 1.06; q = 32, N = 1.25M: (2, 8) 5.9 ms, (1, 12) 6.8, and 12 warps at two rows
+// per lane spill (168 registers) and serialise the broadcast loads.  More rows per lane = fewer broadcast loads per DFMA.
+using GJ16 = GJ<16, 4, 8>;
+using GJ32 = GJ<32, 2, 8>;
+
+template <typename T>
+int gj_blocks(long long N) {
+    long long b = (N + (long long)T::MPW * T::WARPS - 1) / ((long long)T::MPW * T::WARPS);
+    if (b > 148) b = 148;
+    if (b < 1) b = 1;
+    return (int)b;
+}
+
 template <int Q, int RPL, int WARPS>
 cudaError_t launch_gj_cfg(long long N, double *MZ, double *Sig, double *logdet, double *gl, double *zsums, cudaStream_t st,
                           const double *cond, I8Check chk) {
@@ -396,50 +407,21 @@ cudaError_t launch_gj_cfg(long long N, double *MZ, double *Sig, double *logdet, 
     cudaError_t e = cudaFuncSetAttribute(zsolve_gj_kernel<Q, RPL, WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)T::SMEM);
     if (e != cudaSuccess) return e;
-    zsolve_gj_kernel<Q, RPL, WARPS><<<zsolve_gj_blocks(N, Q), 32 * WARPS, T::SMEM, st>>>(N, MZ, Sig, logdet, gl, zsums, cond,
-                                                                                          chk);
+    zsolve_gj_kernel<Q, RPL, WARPS><<<gj_blocks<T>(N), 32 * WARPS, T::SMEM, st>>>(N, MZ, Sig, logdet, gl, zsums, cond, chk);
     return cudaGetLastError();
-}
-
-// (rows per lane, warps per CTA).  Measured per launch (B200, tools/gj_sweep.sh): q = 16, N = 1M: (4, 8) 0.642 ms, (2, 16) 0.79,
-// (2, 12) 0.81, (2, 8) 0.89, (1, 16) 1.06; q = 32, N = 1.25M: (2, 8) 5.9 ms, (1, 12) 6.8, and 12 warps at two rows per lane spill
-// (168 registers) and serialise the broadcast loads.  More rows per lane = fewer broadcast loads per DFMA; PYVB_GJ = "rpl,warps"
-// picks the other built configuration (measurements).
-void gj_config(int q, int &rpl, int &warps) {
-    rpl = (q == 16) ? 4 : 2;
-    warps = 8;
-    const char *e = getenv("PYVB_GJ");
-    int a = 0, b = 0;
-    if (e && sscanf(e, "%d,%d", &a, &b) == 2) {
-        if (q == 16 && a == 2 && b == 16) rpl = 2, warps = 16;
-        if (q == 32 && a == 1 && b == 12) rpl = 1, warps = 12;
-    }
 }
 
 }  // namespace
 
-int zsolve_gj_blocks(long long N, int q) {
-    if (q != 16 && q != 32) return 0;
-    int rpl, warps;
-    gj_config(q, rpl, warps);
-    const int mpw = 32 / (q / rpl);
-    long long b = (N + (long long)mpw * warps - 1) / ((long long)mpw * warps);
-    if (b > 148) b = 148;
-    if (b < 1) b = 1;
-    return (int)b;
-}
+int zsolve_gj_blocks(long long N, int q) { return q == 16 ? gj_blocks<GJ16>(N) : q == 32 ? gj_blocks<GJ32>(N) : 0; }
 
-int zsolve_gj_kw(int q) { return q == 16 ? GJ<16, 2, 8>::KW : q == 32 ? GJ<32, 2, 8>::KW : 0; }
+int zsolve_gj_kw(int q) { return q == 16 ? GJ16::KW : q == 32 ? GJ32::KW : 0; }
 
 cudaError_t launch_zsolve_gj(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
                              cudaStream_t st, const double *cond, I8Check chk) {
     if (N <= 0) return cudaSuccess;
-    int rpl, warps;
-    gj_config(q, rpl, warps);
-#define GJ_CASE(Q_, R_, W_) \
-    if (q == Q_ && rpl == R_ && warps == W_) return launch_gj_cfg<Q_, R_, W_>(N, MZ, Sig, logdet, gl, zsums, st, cond, chk);
-    GJ_CASE(16, 4, 8) GJ_CASE(16, 2, 16) GJ_CASE(32, 2, 8) GJ_CASE(32, 1, 12)
-#undef GJ_CASE
+    if (q == 16) return launch_gj_cfg<16, GJ16::RPL, GJ16::WARPS>(N, MZ, Sig, logdet, gl, zsums, st, cond, chk);
+    if (q == 32) return launch_gj_cfg<32, GJ32::RPL, GJ32::WARPS>(N, MZ, Sig, logdet, gl, zsums, st, cond, chk);
     return cudaErrorNotSupported;
 }
 

@@ -1,5 +1,5 @@
-// K2 as a BLOCKED symmetric sweep: 8 x 8 pivot tiles factored by scalar elimination, everything else on the FP64 tensor cores,
-// IN PLACE in the packed rows as they lie in HBM.
+// K2 at q = 64 as a BLOCKED symmetric sweep: 8 x 8 pivot tiles factored by scalar elimination, everything else on the FP64 tensor
+// cores, in place in shared memory on a tile-swizzled copy of the packed rows.
 //
 // Replaces cho_factor / cho_solve(., I) / dot(qcov, .) / q_ln_det of Gaussian.update (nodes/gaussian.py:117-123).
 //
@@ -9,9 +9,8 @@
 //
 //   M_KK <- -inv(M_KK),    M_IK <- M_IK inv(M_KK),    M_IJ <- M_IJ - M_IK inv(M_KK) M_KJ     (I, J != K),
 //
-// which keeps the state symmetric, so that only the lower triangle exists, every intermediate overwrites the slots of the block
-// it replaces (element (i, j), i >= j, at i (i + 1) / 2 + j: the HBM layout; a reader of the upper half swaps the indices) and
-// after q / 8 sweeps the row holds -Sigma.  inv(M_KK) is only ever applied in FACTORED form, M_KK = L D L^T, X = L^-1:
+// which keeps the state symmetric, so that only the lower tiles exist, every intermediate overwrites the tile it replaces, and
+// after q / 8 sweeps the tiles hold -Sigma.  inv(M_KK) is only ever applied in FACTORED form, M_KK = L D L^T, X = L^-1:
 //
 //   pivot   the 8 x 8 pivot tiles of the warp's MPW matrices together, lane (m, r) = row r of matrix m's tile: elimination without
 //           pivoting on [M_KK | I] gives D and X (one published column entry per lane and pivot, the pivot lane's row of X);
@@ -23,16 +22,17 @@
 // block LU, 4 - 22 x the error of the Cholesky route at q = 32 and cond 1e4 - 1e6, 1e-8 on a rank-deficient q = 64 case; a
 // recursive Schur-complement version with explicit 16 x 16 / 32 x 32 inverses was 400 x worse.  Both were found and measured in
 // the lane-level restatement, oracle/sweep_oracle.py, before / beside the GPU runs.)
-// Operand fragments are plain LDS.64 from the packed rows -- an A fragment of a tile is the B fragment of its transpose, so W^T
-// and the tiles above the pivot tile need no transposition pass -- accumulators go back with STS.64; W crosses shared memory
-// once (accumulator layout -> A fragments) through the panel slots it is about to vacate.
 //
-// ln prod diag chol = 1/2 sum ln(pivots): the pivots are those of the unblocked elimination.  zbar = Sigma eta: lane = row,
-// symmetric reads.  <zz^T> = Sigma + zbar zbar^T: tile by tile in the accumulator layout.  Column sums / maxima bounds /
-// log-det scalars per CTA as in the other K2 kernels (partial layout of the blocked kernel).
-#include <stdio.h>
-#include <stdlib.h>
-
+// Working layout: once its bulk copy has landed, every matrix is re-laid-out in place: lower tile (I, J) -> 64 doubles at
+// (I (I + 1) / 2 + J) 64, element (r, c) at the swizzled offset of the blocked Cholesky kernel,
+// r 8 + (((c >> 2) ^ ((r >> 1) & 1)) << 2) + (c & 3): accumulator-layout accesses are conflict-free 128-bit, A and B fragments
+// conflict-free 64-bit, and the diagonal tiles are kept whole (no mirror reads).  (The sweep used to run on the packed rows as they
+// lie in HBM; it was bound by shared-memory bandwidth, 45 % of its wavefronts bank conflicts of the packed triangle --
+// profiles/r02_k2_ncu.md, DESIGN.md 5.)  zbar = Sigma eta runs on the tensor core too (eta in column 0 of the B fragment), and the
+// <zz^T> pass puts the rows back into the packed order for the bulk store.
+//
+// ln prod diag chol = 1/2 sum ln(pivots): the pivots are those of the unblocked elimination.  Column sums / maxima bounds / log-det
+// scalars per CTA as in the other K2 kernels (partial layout of the blocked kernel).
 #include "common.cuh"
 #include "kernels.h"
 #include "ptx.cuh"
@@ -48,22 +48,6 @@ __host__ __device__ constexpr int s_pitch(int q) {          // == pyvb_mz_pitch(
     return p;
 }
 
-// MPW matrices per warp and stage (one bulk copy each way; 2 or 4), UM of them unrolled together in the tensor-core phases
-template <int Q, int MPW_, int WARPS_, int STAGES_, int UM_> struct SB {
-    static constexpr int MPW = MPW_, WARPS = WARPS_, STAGES = STAGES_, UM = UM_;
-    static constexpr int NBT = Q / 8;                          // tiles per dimension
-    static constexpr int P = s_tri(Q), PP = (P + 7) & ~7, OROW = PP + Q, PITCH = s_pitch(Q);
-    static constexpr int KW = 2 * OROW + PYVB_ZS_EXTRA;       // [column sums OROW | 4 scalars | bounds on the column maxima OROW]
-    static constexpr int STAGE_D = MPW * PITCH;               // the rows of a group as they lie in HBM
-    static constexpr int BC_D = 2 * MPW * 16;                 // published column + X row per pivot of the diagonal tiles, two parities
-    static constexpr int NTR = (Q > 32) ? Q / 32 : 1;         // rows of the maxima a lane tracks
-    static constexpr int WARP_D = STAGES * STAGE_D + BC_D + OROW + 4 + 2 * Q + 2;   // stages | .. | csum | scalars | maxima | mbarriers
-    static constexpr size_t SMEM = (size_t)WARPS * WARP_D * 8;
-    static_assert(MPW == 1 || MPW == 2 || MPW == 4, "the diagonal sweep spreads MPW x 8 tile rows over the lanes");
-    static_assert((STAGE_D % 2) == 0 && (OROW % 2) == 0 && (WARP_D % 2) == 0, "16-byte alignment of the per-warp arrays");
-    static_assert(STAGES == 1 || STAGES == 2, "one or two stages");
-};
-
 // 1 / d to the last bit or so: MUFU.RCP64H seed + two Newton steps (as kernels_k2g.cu)
 __device__ __forceinline__ double s_rcp(double d) {
     double r;
@@ -74,431 +58,6 @@ __device__ __forceinline__ double s_rcp(double d) {
     return fma(r, e, r);
 }
 
-// ---- 8 x 8 pivot tiles K of the warp's MPW matrices: M_KK = L D L^T by elimination without pivoting and X = L^-1 by the same
-// eliminations on the identity, lane (m, r) = row r of matrix m's tile (with MPW < 4 the other lanes shadow a lane of the same
-// row: same arithmetic, same stores).  Per pivot k every lane publishes its entry of column k (= row k of the reduced tile, by
-// symmetry) and the pivot lane its row of X; rows r > k subtract l_rk times both.  Out, in the slots of the tile's lower
-// triangle: X below the diagonal (its diagonal is 1), 1 / d on the diagonal.
-template <int K, typename T>
-__device__ __forceinline__ void s_pivot_tile(double *stg, double *bc, int lane, double &pr, bool &pos) {
-    constexpr int C0 = 8 * K;
-    const int m = (lane >> 3) % T::MPW, r = lane & 7;
-    double *st = stg + m * T::PITCH;
-    const int i = C0 + r;
-    double a[8], x[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-        a[j] = (j <= r) ? st[s_tri(i) + C0 + j] : st[s_tri(C0 + j) + i];
-        x[j] = 0.0;
-    }
-    double dinv = 1.0;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        double *b = bc + (k & 1) * (T::MPW * 16) + m * 16;      // [column k of the reduced tile (8) | row k of X (8)]
-        b[r] = a[k];
-        if (r == k) {
-#pragma unroll
-            for (int j = 0; j < k; ++j) b[8 + j] = x[j];
-        }
-        __syncwarp();
-        double B[8], XK[8];
-#pragma unroll
-        for (int j2 = k / 2; j2 < 4; ++j2) {
-            const double2 v = *reinterpret_cast<const double2 *>(b + 2 * j2);
-            B[2 * j2] = v.x;
-            B[2 * j2 + 1] = v.y;
-        }
-#pragma unroll
-        for (int j2 = 0; j2 < (k + 1) / 2; ++j2) {
-            const double2 v = *reinterpret_cast<const double2 *>(b + 8 + 2 * j2);
-            XK[2 * j2] = v.x;
-            XK[2 * j2 + 1] = v.y;
-        }
-        const double rc = s_rcp(B[k]);
-        dinv = (r == k) ? rc : dinv;
-        const double l = (r > k) ? a[k] * rc : 0.0;
-#pragma unroll
-        for (int j = k + 1; j < 8; ++j) a[j] = fma(-l, B[j], a[j]);
-#pragma unroll
-        for (int j = 0; j < k; ++j) x[j] = fma(-l, XK[j], x[j]);
-        x[k] = -l;
-    }
-    if ((lane >> 3) < T::MPW) {
-        pr *= dinv;                                             // 1 / d_r
-        pos = pos && (dinv > 0.0);
-    }
-#pragma unroll
-    for (int j = 0; j < 8; ++j)
-        if (j < r) st[s_tri(i) + C0 + j] = x[j];
-    st[s_tri(i) + i] = dinv;
-    __syncwarp();
-}
-
-// element (rr, cc) of the unit lower triangular X kept below the diagonal of pivot tile C0
-__device__ __forceinline__ double s_xfrag(const double *st, int C0, int rr, int cc) {
-    const int hi = rr > cc ? rr : cc, lo = rr > cc ? cc : rr;
-    const double v = st[s_tri(C0 + hi) + C0 + lo];
-    return rr > cc ? v : (rr == cc ? 1.0 : 0.0);
-}
-
-// ---- sweep of tile column K of the warp's MPW matrices, everything in place.  In: the symmetric sweep state M (lower triangle).
-// Out:   M_KK <- -inv(M_KK),   M_IK <- M_IK inv(M_KK),   M_IJ <- M_IJ - M_IK inv(M_KK) M_KJ      (I, J != K),
-// with inv(M_KK) only ever applied in its FACTORED form X^T D^-1 X (block Cholesky: as stable as the unblocked elimination):
-//   W_J = old_J X^T,    M_IJ -= (W_I D^-1) W_J^T,    M_JK <- (W_J D^-1) X,    M_KK <- -X^T D^-1 X.
-template <int K, typename T>
-__device__ __forceinline__ void s_sweep_tile(double *stg, double *bc, int lane, double &pr, bool &pos) {
-    constexpr int NBT = T::NBT, C0 = 8 * K;
-    const int gid = lane >> 2, qd = lane & 3;
-    s_pivot_tile<K, T>(stg, bc, lane, pr, pos);
-#pragma unroll(T::UM)
-    for (int m = 0; m < T::MPW; ++m) {
-        double *st = stg + m * T::PITCH;
-        // A fragments of the OLD panel tiles (J, K), J != K
-        double of[NBT][2];
-#pragma unroll
-        for (int J = 0; J < NBT; ++J)
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-                if (J == K) continue;
-                of[J][h] = (J > K) ? st[s_tri(8 * J + gid) + C0 + 4 * h + qd] : st[s_tri(C0 + 4 * h + qd) + 8 * J + gid];
-            }
-        // X[gid][4h + qd] (A fragment of X = B fragment of X^T), X[4h + qd][gid] (B fragment of X = A fragment of X^T), 1 / d_(4h + qd)
-        double xa[2], xb[2], dk[2];
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-            xa[h] = s_xfrag(st, C0, gid, 4 * h + qd);
-            xb[h] = s_xfrag(st, C0, 4 * h + qd, gid);
-            dk[h] = st[s_tri(C0 + 4 * h + qd) + C0 + 4 * h + qd];
-        }
-        // W_J = old_J X^T
-        double wt[NBT][2];
-#pragma unroll
-        for (int J = 0; J < NBT; ++J) {
-            if (J == K) continue;
-            wt[J][0] = wt[J][1] = 0.0;
-            dmma884(wt[J][0], wt[J][1], of[J][0], xa[0]);
-            dmma884(wt[J][0], wt[J][1], of[J][1], xa[1]);
-        }
-        // the pivot tile: X^T D^-1 X
-        double pv0 = 0.0, pv1 = 0.0;
-        dmma884(pv0, pv1, xb[0], xb[0] * dk[0]);
-        dmma884(pv0, pv1, xb[1], xb[1] * dk[1]);
-        __syncwarp();                                           // every lane has read the old panel and X
-        if (2 * qd <= gid) st[s_tri(C0 + gid) + C0 + 2 * qd] = -pv0;
-        if (2 * qd + 1 <= gid) st[s_tri(C0 + gid) + C0 + 2 * qd + 1] = -pv1;
-        // W through the panel slots (the change of layout), back as A fragments (== B fragments of W^T)
-#pragma unroll
-        for (int J = 0; J < NBT; ++J) {
-            if (J == K) continue;
-            if (J > K) {
-                double *o = st + s_tri(8 * J + gid) + C0 + 2 * qd;
-                o[0] = wt[J][0];
-                o[1] = wt[J][1];
-            } else {                                            // above the pivot tile: the slot of the transposed element
-                st[s_tri(C0 + 2 * qd) + 8 * J + gid] = wt[J][0];
-                st[s_tri(C0 + 2 * qd + 1) + 8 * J + gid] = wt[J][1];
-            }
-        }
-        __syncwarp();
-        double wa[NBT][2], wd[NBT][2];
-#pragma unroll
-        for (int I = 0; I < NBT; ++I)
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-                if (I == K) continue;
-                wa[I][h] = (I > K) ? st[s_tri(8 * I + gid) + C0 + 4 * h + qd] : st[s_tri(C0 + 4 * h + qd) + 8 * I + gid];
-                wd[I][h] = wa[I][h] * dk[h];
-            }
-        __syncwarp();                                           // every lane has read W
-        // the new panel (sweep convention): M_JK <- (W_J D^-1) X
-#pragma unroll
-        for (int J = 0; J < NBT; ++J) {
-            if (J == K) continue;
-            double t0 = 0.0, t1 = 0.0;
-            dmma884(t0, t1, wd[J][0], xb[0]);
-            dmma884(t0, t1, wd[J][1], xb[1]);
-            if (J > K) {
-                double *o = st + s_tri(8 * J + gid) + C0 + 2 * qd;
-                o[0] = t0;
-                o[1] = t1;
-            } else {
-                st[s_tri(C0 + 2 * qd) + 8 * J + gid] = t0;
-                st[s_tri(C0 + 2 * qd + 1) + 8 * J + gid] = t1;
-            }
-        }
-        // trailing update on the tensor cores: M_IJ -= (W_I D^-1) W_J^T for the lower tiles I >= J, I, J != K
-#pragma unroll
-        for (int I = 0; I < NBT; ++I) {
-            if (I == K) continue;
-            const double na0 = -wd[I][0], na1 = -wd[I][1];
-#pragma unroll
-            for (int J = 0; J <= I; ++J) {
-                if (J == K) continue;
-                double *o = st + s_tri(8 * I + gid) + 8 * J + 2 * qd;
-                double c0 = o[0], c1 = o[1];                    // (a diagonal tile: the upper half is junk that is never stored)
-                dmma884(c0, c1, na0, wa[J][0]);
-                dmma884(c0, c1, na1, wa[J][1]);
-                if (I > J || 2 * qd <= gid) o[0] = c0;
-                if (I > J || 2 * qd + 1 <= gid) o[1] = c1;
-            }
-        }
-    }
-    __syncwarp();
-}
-
-template <int K, typename T>
-__device__ __forceinline__ void s_sweep_all(double *stg, double *bc, int lane, double &pr, bool &pos) {
-    if constexpr (K < T::NBT) {
-        s_sweep_tile<K, T>(stg, bc, lane, pr, pos);
-        s_sweep_all<K + 1, T>(stg, bc, lane, pr, pos);
-    }
-}
-
-template <int Q, int MPW_, int WARPS_, int STAGES_, int UM_>
-__global__ void __launch_bounds__(32 * WARPS_, 1)
-zsolve_sweep_kernel(long long N, double *__restrict__ MZ, double *__restrict__ Sig, double *__restrict__ logdet, double *gl,
-                    double *__restrict__ zsums, const double *__restrict__ cond, const I8Check chk) {
-    using T = SB<Q, MPW_, WARPS_, STAGES_, UM_>;
-    constexpr int MPW = T::MPW, P = T::P, PP = T::PP, PITCH = T::PITCH, NBT = T::NBT, NTR = T::NTR;
-    constexpr int NPASS = MPW * Q / 32;                          // passes of the lane = row loops over the warp's 4 Q rows
-    if (cond != nullptr && !(*cond > 0.0)) return;               // conditional (fall-back) launch: nothing to redo
-    __shared__ double s_chk[T::WARPS + 1];
-    extern __shared__ __align__(16) double smem_sb[];
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int gid = lane >> 2, qd = lane & 3;
-    double *stage = smem_sb + (size_t)warp * T::WARP_D;
-    double *bc = stage + T::STAGES * T::STAGE_D;
-    double *csum = bc + T::BC_D;                                  // [OROW]
-    double *wsc = csum + T::OROW;                                 // [4]
-    double *wmx = wsc + 4;                                        // [2 Q]: max_n <z_i z_i>, max_n |<z_i>| of this warp's rows
-    uint64_t *bar = reinterpret_cast<uint64_t *>(wmx + 2 * Q);
-
-    for (int c = lane; c < T::OROW; c += 32) csum[c] = 0.0;
-    if (lane == 0) {
-        mbar_init(bar, 1);
-        mbar_init(bar + 1, 1);
-    }
-    // INT8 guard (kernels.h: I8Check): a row whose largest diagonal entry is below `thr` carries too much fixed-point rounding
-    if (chk.gscale != nullptr) {                                 // kernel-uniform
-        double mx = 0.0;
-        for (int c = tid; c < chk.ncols; c += 32 * T::WARPS) mx = fmax(mx, chk.gscale[c]);
-        for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-        if (lane == 0) s_chk[warp] = mx;
-    }
-    mbar_fence_init();
-    __syncthreads();
-    double thr = -1.0;
-    if (chk.gscale != nullptr) {
-        double mx = s_chk[0];
-        for (int w = 1; w < T::WARPS; ++w) mx = fmax(mx, s_chk[w]);
-        thr = gl[PYVB_GL_TAU] * chk.fac * mx;
-    }
-    if (cond != nullptr && blockIdx.x == 0 && tid == 0) gl[PYVB_GL_I8FALL] += 1.0;
-
-    double dmx[NTR], zmx[NTR], s_qld = 0.0, s_ld = 0.0, s_n = 0.0;
-#pragma unroll
-    for (int s = 0; s < NTR; ++s) dmx[s] = zmx[s] = 0.0;
-
-    const long long nwarps = (long long)gridDim.x * T::WARPS;
-    const long long ngroups = (N + MPW - 1) / MPW;
-    long long g = (long long)blockIdx.x * T::WARPS + warp;
-    if (g < ngroups && lane == 0) {                               // the first group of this warp
-        const long long left = N - g * MPW;
-        const uint32_t bytes = (uint32_t)((left < MPW ? left : MPW) * PITCH * 8);
-        mbar_arrive_expect_tx(bar, bytes);
-        bulk_g2s(stage, MZ + g * MPW * PITCH, bytes, bar);
-    }
-    for (int it = 0; g < ngroups; g += nwarps, ++it) {
-        const int sidx = (T::STAGES == 2) ? (it & 1) : 0;
-        double *stg = stage + sidx * T::STAGE_D;                  // this group's rows
-        const long long n0 = g * MPW;
-        const int nval = (N - n0 < MPW) ? (int)(N - n0) : MPW;
-        const long long gn = g + nwarps;                         // the warp's next group
-        if (T::STAGES == 2) {                                    // into the other stage now (its store has been read by then)
-            if (lane == 0 && gn < ngroups) {
-                bulk_wait_read_all();
-                const long long left = N - gn * MPW;
-                const uint32_t bytes = (uint32_t)((left < MPW ? left : MPW) * PITCH * 8);
-                mbar_arrive_expect_tx(bar + (sidx ^ 1), bytes);
-                bulk_g2s(stage + (sidx ^ 1) * T::STAGE_D, MZ + gn * MPW * PITCH, bytes, bar + (sidx ^ 1));
-            }
-            mbar_wait(bar + sidx, (uint32_t)((it >> 1) & 1));
-        } else {
-            mbar_wait(bar, (uint32_t)(it & 1));
-        }
-
-        {   // ---- the sweep; it leaves -Sigma in place.  Lane (m8, r8) = pivot-tile row r8 of matrix m8 (with MPW < 4: shadows)
-            const int m8 = lane >> 3, r8 = lane & 7;
-            if (thr >= 0.0) {                                    // INT8 guard: largest diagonal entry of qprec (kernel-uniform branch)
-                const double *st = stg + (m8 % MPW) * PITCH;
-                double dm = 0.0;
-#pragma unroll
-                for (int t = 0; t < NBT; ++t) dm = fmax(dm, st[s_tri(r8 + 8 * t) + r8 + 8 * t]);
-#pragma unroll
-                for (int o = 4; o > 0; o >>= 1) dm = fmax(dm, __shfl_xor_sync(0xffffffffu, dm, o));
-                if (r8 == 0 && m8 < nval && m8 < MPW && thr > dm) atomicAdd(&gl[PYVB_GL_I8BAD], 1.0);
-            }
-            // ln prod diag chol = -1/2 sum ln(1 / d_i); a pivot <= 0 (or NaN) poisons the logarithm
-            double pr = 1.0;
-            bool pos = true;
-            s_sweep_all<0, T>(stg, bc, lane, pr, pos);
-            double lg = pos ? log(pr) : __longlong_as_double(0x7ff8000000000000LL);
-#pragma unroll
-            for (int o = 4; o > 0; o >>= 1) lg += __shfl_xor_sync(0xffffffffu, lg, o);
-            const double ldsum = -0.5 * lg;
-            if (r8 == 0 && m8 < nval && m8 < MPW) {
-                logdet[n0 + m8] = ldsum;
-                s_qld += 0.5 / ldsum;
-                s_ld += ldsum;
-                s_n += 1.0;
-                if (!(ldsum - ldsum == 0.0)) atomicAdd(&gl[PYVB_GL_NONPD], 1.0);   // NaN / inf <=> a pivot was <= 0
-            }
-        }
-        if (Sig != nullptr) {                                    // kernel-uniform (the Sigma output is optional)
-            for (int m = 0; m < nval; ++m)
-                for (int c = lane; c < P; c += 32) Sig[(n0 + m) * P + c] = -stg[m * PITCH + c];
-        }
-
-        // ---- zbar = Sigma eta = -(state) eta: lane = row (pass p takes rows 32 p .. 32 p + 31 of the warp's MPW Q rows)
-        double z[NPASS];
-#pragma unroll
-        for (int p = 0; p < NPASS; ++p) {
-            const int idx = p * 32 + lane, m = idx / Q, i = idx % Q;
-            const double *st = stg + m * PITCH;
-            const double *rowp = st + s_tri(i), *colp = st + i;
-            double acc = 0.0;
-#pragma unroll
-            for (int j2 = 0; j2 < Q / 2; ++j2) {
-                const double2 E = *reinterpret_cast<const double2 *>(st + PP + 2 * j2);
-                const double v0 = (2 * j2 <= i) ? rowp[2 * j2] : colp[s_tri(2 * j2)];
-                const double v1 = (2 * j2 + 1 <= i) ? rowp[2 * j2 + 1] : colp[s_tri(2 * j2 + 1)];
-                acc = fma(v1, E.y, fma(v0, E.x, acc));
-            }
-            acc = -acc;
-            z[p] = acc;
-            if (m < nval) {
-                const int s = (NTR > 1) ? (p % NTR) : 0;
-                dmx[s] = fmax(dmx[s], fma(acc, acc, -rowp[i]));  // <z_i z_i> exactly as it is stored below
-                zmx[s] = fmax(zmx[s], fabs(acc));
-            }
-        }
-        __syncwarp();                                            // every lane has read eta
-#pragma unroll
-        for (int p = 0; p < NPASS; ++p) {
-            const int idx = p * 32 + lane, m = idx / Q, i = idx % Q;
-            stg[m * PITCH + PP + i] = z[p];                      // zbar takes eta's place
-        }
-        __syncwarp();
-        // ---- <zz^T> = Sigma + zbar zbar^T, tile by tile in the accumulator layout, packed in place
-#pragma unroll(T::UM)
-        for (int m = 0; m < MPW; ++m) {
-            double *st = stg + m * PITCH;
-            double zi[NBT];
-            double2 zj[NBT];
-#pragma unroll
-            for (int I = 0; I < NBT; ++I) {
-                zi[I] = st[PP + 8 * I + gid];
-                zj[I] = *reinterpret_cast<const double2 *>(st + PP + 8 * I + 2 * qd);
-            }
-#pragma unroll
-            for (int I = 0; I < NBT; ++I)
-#pragma unroll
-                for (int J = 0; J <= I; ++J) {
-                    double *o = st + s_tri(8 * I + gid) + 8 * J + 2 * qd;
-                    if (I > J || 2 * qd <= gid) o[0] = fma(zi[I], zj[J].x, -o[0]);
-                    if (I > J || 2 * qd + 1 <= gid) o[1] = fma(zi[I], zj[J].y, -o[1]);
-                }
-        }
-        fence_async_smem();
-        __syncwarp();
-        // ---- rows back to HBM (one bulk store), column sums of the finished rows, next group in
-        if (lane == 0) {
-            bulk_s2g(MZ + n0 * PITCH, stg, (uint32_t)(nval * PITCH * 8));
-            bulk_commit();
-        }
-        if (zsums != nullptr) {                                  // kernel-uniform
-            for (int c = lane; c < T::OROW; c += 32) {
-                double v = 0.0;
-#pragma unroll
-                for (int mm = 0; mm < MPW; ++mm)
-                    if (mm < nval) v += stg[mm * PITCH + c];
-                csum[c] += v;
-            }
-        }
-        __syncwarp();
-        if (T::STAGES == 1 && lane == 0 && gn < ngroups) {       // one stage: the store has to have read it first
-            bulk_wait_read_all();
-            const long long left = N - gn * MPW;
-            const uint32_t bytes = (uint32_t)((left < MPW ? left : MPW) * PITCH * 8);
-            mbar_arrive_expect_tx(bar, bytes);
-            bulk_g2s(stage, MZ + gn * MPW * PITCH, bytes, bar);
-        }
-    }
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-
-    if (zsums == nullptr) return;                                // kernel-uniform
-    // ---- CTA partial: [column sums | sum 0.5/logdet | sum logdet | rows | 0 | bounds on the column maxima]
-    s_qld = warp_sum(s_qld);
-    s_ld = warp_sum(s_ld);
-    s_n = warp_sum(s_n);
-    if (lane == 0) {
-        wsc[0] = s_qld;
-        wsc[1] = s_ld;
-        wsc[2] = s_n;
-        wsc[3] = 0.0;
-    }
-#pragma unroll
-    for (int s = 0; s < NTR; ++s) {
-#pragma unroll
-        for (int o = Q; o < 32; o <<= 1) {                        // q < 32: several lanes track the same row
-            dmx[s] = fmax(dmx[s], __shfl_xor_sync(0xffffffffu, dmx[s], o));
-            zmx[s] = fmax(zmx[s], __shfl_xor_sync(0xffffffffu, zmx[s], o));
-        }
-        if (lane < Q) {
-            wmx[s * 32 + lane] = dmx[s];
-            wmx[Q + s * 32 + lane] = zmx[s];
-        }
-    }
-    __syncthreads();
-    double *out = zsums + (size_t)blockIdx.x * T::KW;
-    const double *w0 = smem_sb + T::STAGES * T::STAGE_D + T::BC_D;    // csum of warp 0
-    for (int c = tid; c < T::OROW + 4; c += 32 * T::WARPS) {
-        double v = 0.0;
-        for (int w = 0; w < T::WARPS; ++w) v += w0[(size_t)w * T::WARP_D + c];   // [csum OROW | scalars 4] is contiguous
-        out[c] = v;
-    }
-    // CTA maxima of the diagonal second moments and of |z| (folded into warp 0's stage), then the column bounds:
-    // |<z_i z_j>| <= sqrt(<z_i z_i> <z_j z_j>) because <zz^T> is PSD
-    const double *m0 = w0 + T::OROW + 4;
-    double *fm = smem_sb;                                        // warp 0's stage is free now: [2 Q] folded maxima
-    for (int c = tid; c < 2 * Q; c += 32 * T::WARPS) {
-        double v = 0.0;
-        for (int w = 0; w < T::WARPS; ++w) v = fmax(v, m0[(size_t)w * T::WARP_D + c]);
-        fm[c] = v;
-    }
-    __syncthreads();
-    for (int c = tid; c < T::OROW; c += 32 * T::WARPS) {
-        double v = 0.0;
-        if (c < P) {
-            int i, j;
-            unpack_p(c, i, j);
-            v = sqrt(fm[i] * fm[j]);
-        } else if (c >= PP) {
-            v = fm[Q + c - PP];
-        }
-        out[T::OROW + 4 + c] = v;
-    }
-}
-
-// ================================================================================================================================
-// The same sweep on a TILE-SWIZZLED working layout.  ncu of the kernel above (profiles/r02_k2_ncu.md): it is bound by shared-memory
-// bandwidth, and 45 % of its wavefronts are bank conflicts of the packed triangle (rows start at i (i + 1) / 2, so the 8 rows of a
-// fragment land on arbitrary banks).  Here every matrix is re-laid-out once, in place, after its bulk copy has landed: lower tile
-// (I, J) -> 64 doubles at (I (I + 1) / 2 + J) 64, element (r, c) at the swizzled offset of the blocked Cholesky kernel,
-// r 8 + (((c >> 2) ^ ((r >> 1) & 1)) << 2) + (c & 3): accumulator-layout accesses are conflict-free 128-bit, A and B fragments
-// conflict-free 64-bit, and the diagonal tiles are kept whole (no mirror reads).  zbar = Sigma eta runs on the tensor core too (eta in
-// column 0 of the B fragment).  The rows are put back into the packed order for the bulk store by the <zz^T> pass.
-// ================================================================================================================================
 __host__ __device__ constexpr int s_sw(int r, int c) { return r * 8 + ((((c >> 2) ^ ((r >> 1) & 1))) << 2) + (c & 3); }
 __host__ __device__ constexpr int s_toff(int I, int J) { return (s_tri(I) + J) * 64; }
 
@@ -963,102 +522,32 @@ zsolve_tsweep_kernel(long long N, double *__restrict__ MZ, double *__restrict__ 
     }
 }
 
-template <int Q, int MPW, int WARPS, int STAGES, int UM>
-cudaError_t launch_sweep_cfg(long long N, double *MZ, double *Sig, double *logdet, double *gl, double *zsums, cudaStream_t st,
-                             const double *cond, I8Check chk) {
-    using T = SB<Q, MPW, WARPS, STAGES, UM>;
-    static_assert(T::SMEM <= 232448 - 1024, "shared memory of one CTA");
-    cudaError_t e = cudaFuncSetAttribute(zsolve_sweep_kernel<Q, MPW, WARPS, STAGES, UM>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::SMEM);
-    if (e != cudaSuccess) return e;
-    zsolve_sweep_kernel<Q, MPW, WARPS, STAGES, UM><<<zsolve_sweep_blocks(N, Q), 32 * WARPS, T::SMEM, st>>>(N, MZ, Sig, logdet, gl,
-                                                                                                            zsums, cond, chk);
-    return cudaGetLastError();
-}
-
-template <int Q, int MPW, int WARPS, int STAGES, int UM>
-cudaError_t launch_tsweep_cfg(long long N, double *MZ, double *Sig, double *logdet, double *gl, double *zsums, cudaStream_t st,
-                              const double *cond, I8Check chk) {
-    using T = SBT<Q, MPW, WARPS, STAGES, UM>;
-    static_assert(T::SMEM <= 232448 - 1024, "shared memory of one CTA");
-    cudaError_t e = cudaFuncSetAttribute(zsolve_tsweep_kernel<Q, MPW, WARPS, STAGES, UM>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::SMEM);
-    if (e != cudaSuccess) return e;
-    zsolve_tsweep_kernel<Q, MPW, WARPS, STAGES, UM><<<zsolve_sweep_blocks(N, Q), 32 * WARPS, T::SMEM, st>>>(N, MZ, Sig, logdet, gl,
-                                                                                                             zsums, cond, chk);
-    return cudaGetLastError();
-}
-
-// the tile-swizzled kernel and its built configurations
-#define SBT_CONFIGS(X) \
-    X(16, 4, 12, 2, 4) X(16, 4, 12, 2, 1) \
-    X(32, 4, 8, 1, 4) X(32, 4, 8, 1, 1) X(32, 2, 12, 1, 2) X(32, 2, 12, 1, 1) X(32, 2, 8, 2, 1) \
-    X(64, 2, 4, 1, 1) X(64, 1, 6, 1, 1) X(64, 1, 4, 2, 1)
-
-bool sweep_tiled() {                  // the default; PYVB_SWEEP_TILED=0 runs the sweep on the packed rows (the kernel above)
-    const char *e = getenv("PYVB_SWEEP_TILED");
-    return e == nullptr || e[0] != '0';
-}
-
-#define SB_CONFIGS(X) \
-    X(16, 4, 16, 2, 4) X(16, 4, 16, 2, 1) X(16, 2, 16, 2, 2) \
-    X(32, 4, 9, 1, 4) X(32, 4, 9, 1, 2) X(32, 4, 9, 1, 1) X(32, 2, 15, 1, 2) X(32, 2, 15, 1, 1) X(32, 2, 9, 2, 2) X(32, 4, 5, 2, 4) \
-    X(32, 2, 12, 1, 2) X(32, 4, 8, 1, 4) \
-    X(64, 1, 6, 1, 1) X(64, 1, 4, 2, 1) X(64, 2, 4, 1, 2) X(64, 2, 4, 1, 1)
-
-// built configurations (matrices per warp and stage, warps per CTA, stages, matrices unrolled together); PYVB_SWEEP =
-// "mpw,warps,stages,unroll" picks another built one (measurements)
-void sweep_config(int q, int &mpw, int &warps, int &stages, int &um) {
-    if (q == 16) mpw = 4, warps = 16, stages = 2, um = 4;
-    else if (q == 32) mpw = 4, warps = 8, stages = 1, um = 4;
-    else mpw = 2, warps = 4, stages = 1, um = 1;
-    const bool tiled = sweep_tiled();
-    if (tiled && q == 32) mpw = 4, warps = 8, stages = 1, um = 4;
-    if (tiled && q == 16) mpw = 4, warps = 12, stages = 2, um = 4;
-    const char *e = getenv("PYVB_SWEEP");
-    int a = 0, b = 0, c = 0, d = 0;
-    if (e && sscanf(e, "%d,%d,%d,%d", &a, &b, &c, &d) == 4) {
-#define SB_HAVE(Q_, M_, W_, S_, U_) if (q == Q_ && a == M_ && b == W_ && c == S_ && d == U_) mpw = a, warps = b, stages = c, um = d;
-        if (tiled) { SBT_CONFIGS(SB_HAVE) } else { SB_CONFIGS(SB_HAVE) }
-#undef SB_HAVE
-    }
-}
+// The configuration (matrices per warp and stage, warps per CTA, stages, matrices unrolled together).  Measured per launch (B200,
+// q = 64, 400k rows): (2, 4, 1, 1) 11.4 ms, (1, 6, 1, 1) 12.0 (profiles/r02_k2_sweep_v3_timings.txt)
+using SW64 = SBT<64, 2, 4, 1, 1>;
 
 }  // namespace
 
 int zsolve_sweep_blocks(long long N, int q) {
-    if (q != 16 && q != 32 && q != 64) return 0;
-    int mpw, warps, stages, um;
-    sweep_config(q, mpw, warps, stages, um);
-    long long b = (N + (long long)mpw * warps - 1) / ((long long)mpw * warps);
+    if (q != 64) return 0;
+    long long b = (N + (long long)SW64::MPW * SW64::WARPS - 1) / ((long long)SW64::MPW * SW64::WARPS);
     if (b > 148) b = 148;
     if (b < 1) b = 1;
     return (int)b;
 }
 
-int zsolve_sweep_kw(int q) {
-    return q == 16 ? SB<16, 4, 16, 2, 4>::KW : q == 32 ? SB<32, 4, 8, 1, 4>::KW : q == 64 ? SB<64, 2, 4, 1, 1>::KW : 0;
-}
+int zsolve_sweep_kw(int q) { return q == 64 ? SW64::KW : 0; }
 
 cudaError_t launch_zsolve_sweep(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
                                 cudaStream_t st, const double *cond, I8Check chk) {
     if (N <= 0) return cudaSuccess;
-    int mpw, warps, stages, um;
-    sweep_config(q, mpw, warps, stages, um);
-#define SB_CASE(Q_, M_, W_, S_, U_) \
-    if (q == Q_ && mpw == M_ && warps == W_ && stages == S_ && um == U_) \
-        return launch_sweep_cfg<Q_, M_, W_, S_, U_>(N, MZ, Sig, logdet, gl, zsums, st, cond, chk);
-    if (sweep_tiled()) {
-#define SBT_CASE(Q_, M_, W_, S_, U_) \
-    if (q == Q_ && mpw == M_ && warps == W_ && stages == S_ && um == U_) \
-        return launch_tsweep_cfg<Q_, M_, W_, S_, U_>(N, MZ, Sig, logdet, gl, zsums, st, cond, chk);
-        SBT_CONFIGS(SBT_CASE)
-#undef SBT_CASE
-        return cudaErrorNotSupported;
-    }
-    SB_CONFIGS(SB_CASE)
-#undef SB_CASE
-    return cudaErrorNotSupported;
+    if (q != 64) return cudaErrorNotSupported;
+    static_assert(SW64::SMEM <= 232448 - 1024, "shared memory of one CTA");
+    auto kernel = zsolve_tsweep_kernel<64, SW64::MPW, SW64::WARPS, SW64::STAGES, SW64::UM>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SW64::SMEM);
+    if (e != cudaSuccess) return e;
+    kernel<<<zsolve_sweep_blocks(N, q), 32 * SW64::WARPS, SW64::SMEM, st>>>(N, MZ, Sig, logdet, gl, zsums, cond, chk);
+    return cudaGetLastError();
 }
 
 }  // namespace pyvb

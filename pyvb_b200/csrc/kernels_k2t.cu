@@ -1,4 +1,5 @@
-// K2, thread per matrix (q = 8, 16): batched q x q SPD inverse / solve where every LANE owns one matrix.
+// K2, thread per matrix (FP64 rows at q = 8, FP32 rows at q = 16): batched q x q SPD inverse / solve where every LANE owns
+// one matrix.
 //
 // Replaces cho_factor / cho_solve(., I) / dot(qcov, .) / q_ln_det of Gaussian.update (nodes/gaussian.py:117-123).
 // A warp takes 32 consecutive rows of MZ.  The rows are loaded cooperatively (coalesced) into shared memory as
@@ -488,10 +489,7 @@ int zsolve_tpm_kw(int q) { return q == 8 ? TK<8>::KW : q == 16 ? TK<16>::KW : 0;
 cudaError_t launch_zsolve_tpm(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
                               cudaStream_t st, const double *cond, I8Check chk) {
     if (N <= 0) return cudaSuccess;
-    switch (q) {
-        case 8: return launch_tpm_q<8, false>(N, MZ, Sig, logdet, gl, zsums, nullptr, st, cond, chk);
-        case 16: return launch_tpm_q<16, false>(N, MZ, Sig, logdet, gl, zsums, nullptr, st, cond, chk);
-    }
+    if (q == 8) return launch_tpm_q<8, false>(N, MZ, Sig, logdet, gl, zsums, nullptr, st, cond, chk);
     return cudaErrorNotSupported;
 }
 cudaError_t launch_zsolve_tpm_f32(long long N, int q, float *MZ32, void *MP, double *Sig, double *logdet, double *gl,

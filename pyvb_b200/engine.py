@@ -698,9 +698,6 @@ class PlateEngine(object):
         full = (lo == 0 and hi == self.N and self.zsums is not None and self.algo in (ALGO_AUTO, ALGO_DMMA))
         # (_chunk_zsums: iterate_from_host takes the K2 partials of a row chunk for that chunk's statistics)
         zs = self.zsums.data_ptr() if ((full or _chunk_zsums) and self.zsums is not None) else 0
-        if zs and int(self.lib.pyvb_zsums_len(self.N, q)) > self.zsums.numel():
-            # (PYVB_K2 picks the batched-solve kernel per call; its partial layout must be the one this buffer was sized for)
-            raise RuntimeError("the K2 partial buffer was sized for another batched-solve kernel (PYVB_K2 changed?)")
         self._zsums_valid = False
         if self.use_i8 and lo % 128 == 0:                   # (the int8 mask is tiled by 128 rows: other offsets take the DMMA path)
             if not self._mask_valid:                        # the int8 mask follows X (static in mode B)

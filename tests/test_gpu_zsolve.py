@@ -1,9 +1,7 @@
 """K2 alone through the C-ABI (pyvb_zsolve_f64): batched q x q Cholesky / inverse / solve in place on MZ rows,
 against numpy/LAPACK -- the arithmetic of Gaussian.update, /root/reference/src/pyvb/nodes/gaussian.py:117-123
-(cho_factor, cho_solve(., I), dot(qcov, .), q_ln_det from prod(diag(chol))).  Both implementations: the
-register-resident kernel (q <= 32) and the blocked tensor-core kernel (q <= 64)."""
-import os
-
+(cho_factor, cho_solve(., I), dot(qcov, .), q_ln_det from prod(diag(chol))).  One kernel per q: thread per matrix
+(q = 8), Gauss-Jordan in registers (q = 16, 32), blocked symmetric sweep (q = 64)."""
 import numpy as np
 import pytest
 
@@ -24,7 +22,7 @@ def _case(N, q, seed, cond):
     return A, eta
 
 
-def _run(impl, q, A, eta, want_sig=True):
+def _run(q, A, eta, want_sig=True):
     import torch
     from pyvb_b200 import _cabi
     lib = _cabi.lib()
@@ -40,41 +38,22 @@ def _run(impl, q, A, eta, want_sig=True):
     sig = torch.zeros(N, P, dtype=torch.float64, device=dev)
     logdet = torch.zeros(N, dtype=torch.float64, device=dev)
     gl = torch.zeros(144, dtype=torch.float64, device=dev)
-    old = os.environ.get("PYVB_K2")
-    os.environ["PYVB_K2"] = impl
-    try:
-        nz = int(lib.pyvb_zsums_len(N, q))                 # what to allocate: the largest over the K2 kernels
-        nblk = int(lib.pyvb_zsums_blocks(N, q))            # what the kernel in use writes
-        zs = torch.full((max(nz, 1),), float("nan"), dtype=torch.float64, device=dev)
-        _cabi.check(lib.pyvb_zsolve_f64(N, q, mz.data_ptr(), ld, sig.data_ptr() if want_sig else 0,
-                                        logdet.data_ptr(), gl.data_ptr(), zs.data_ptr() if nz else 0,
-                                        torch.cuda.current_stream(dev).cuda_stream), "zsolve")
-        torch.cuda.synchronize()
-    finally:
-        if old is None:
-            os.environ.pop("PYVB_K2")
-        else:
-            os.environ["PYVB_K2"] = old
+    nz = int(lib.pyvb_zsums_len(N, q))
+    nblk = int(lib.pyvb_zsums_blocks(N, q))
+    zs = torch.full((max(nz, 1),), float("nan"), dtype=torch.float64, device=dev)
+    _cabi.check(lib.pyvb_zsolve_f64(N, q, mz.data_ptr(), ld, sig.data_ptr() if want_sig else 0,
+                                    logdet.data_ptr(), gl.data_ptr(), zs.data_ptr() if nz else 0,
+                                    torch.cuda.current_stream(dev).cuda_stream), "zsolve")
+    torch.cuda.synchronize()
     kw = int(lib.pyvb_zsums_kw(q))
     return (mz.cpu().numpy(), sig.cpu().numpy(), logdet.cpu().numpy(), gl.cpu().numpy(),
             zs.cpu().numpy()[:nblk * kw] if nblk else None, zoff)
 
 
-@pytest.mark.parametrize("impl", ["reg", "blocked", "tpm", "lanediag", "gj", "sweep"])
 @pytest.mark.parametrize("q,N", [(8, 1000), (16, 1), (16, 4099), (32, 2500), (32, 3), (64, 700), (64, 1)])
-def test_zsolve_matches_lapack(impl, q, N):
-    if impl == "reg" and q == 64:
-        pytest.skip("q = 64 only has the blocked kernels")
-    if impl == "tpm" and q > 16:
-        pytest.skip("the thread-per-matrix kernel covers q <= 16")
-    if impl == "lanediag" and q < 16:
-        pytest.skip("the lane-parallel-diagonal kernel covers q >= 16")
-    if impl == "gj" and q not in (16, 32):
-        pytest.skip("the Gauss-Jordan kernel covers q = 16, 32")
-    if impl == "sweep" and q not in (16, 32, 64):
-        pytest.skip("the blocked-sweep kernel covers q = 16, 32, 64")
+def test_zsolve_matches_lapack(q, N):
     A, eta = _case(N, q, seed=q + N, cond=1e4)
-    out, sig, logdet, gl, zs, zoff = _run(impl, q, A, eta)
+    out, sig, logdet, gl, zs, zoff = _run(q, A, eta)
     ii, jj = np.tril_indices(q)
     P = q * (q + 1) // 2
     Sg = np.linalg.inv(A)
@@ -89,26 +68,25 @@ def test_zsolve_matches_lapack(impl, q, N):
         kw = 2 * (zoff + q) + 4                         # [column sums | 4 scalars | column maxima of |.|]
         part = zs.reshape(-1, kw)
         tot = part[:, :zoff + q + 4].sum(0)
-        if impl != "reg":                               # the default kernels also leave (bounds on) the column maxima
-            mx = part[:, zoff + q + 4:].max(0)
-            true = np.abs(out).max(0)
-            cols = list(range(P)) + list(range(zoff, zoff + q))
-            assert np.all(mx[cols] >= true[cols] * (1 - 1e-12))
-            if impl == "tpm":
-                assert np.allclose(mx[cols], true[cols], rtol=2e-6)        # high-word maxima, rounded up
-            else:                                       # PSD bound sqrt(max <z_i z_i> max <z_j z_j>): tight on the diagonal
-                di = [i * (i + 1) // 2 + i for i in range(q)]
-                assert np.allclose(mx[di], true[di], rtol=1e-12)
+        mx = part[:, zoff + q + 4:].max(0)              # (bounds on) the column maxima
+        true = np.abs(out).max(0)
+        cols = list(range(P)) + list(range(zoff, zoff + q))
+        assert np.all(mx[cols] >= true[cols] * (1 - 1e-12))
+        if q == 8:                                      # thread per matrix
+            assert np.allclose(mx[cols], true[cols], rtol=2e-6)        # high-word maxima, rounded up
+        else:                                           # PSD bound sqrt(max <z_i z_i> max <z_j z_j>): tight on the diagonal
+            di = [i * (i + 1) // 2 + i for i in range(q)]
+            assert np.allclose(mx[di], true[di], rtol=1e-12)
         assert tensor_rel(tot[:P], out[:, :P].sum(0)) < 1e-12
         assert tensor_rel(tot[zoff:zoff + q], out[:, zoff:zoff + q].sum(0)) < 1e-12
         assert tot[zoff + q + 2] == N
         assert abs(tot[zoff + q + 1] - logdet.sum()) <= 1e-12 * abs(logdet.sum())
 
 
-@pytest.mark.parametrize("impl", ["reg", "blocked", "tpm", "lanediag", "gj", "sweep"])
-def test_zsolve_flags_non_pd(impl):
-    q, N = 16, 64
+@pytest.mark.parametrize("q", [8, 16, 32, 64])
+def test_zsolve_flags_non_pd(q):
+    N = 64
     A, eta = _case(N, q, seed=5, cond=10.0)
     A[17] -= 50.0 * np.eye(q)           # indefinite
-    out, sig, logdet, gl, zs, zoff = _run(impl, q, A, eta, want_sig=False)
+    out, sig, logdet, gl, zs, zoff = _run(q, A, eta, want_sig=False)
     assert float(gl[11]) == 1.0
