@@ -25,42 +25,17 @@ static int cuda_fail(cudaError_t e, const char *where) {
 
 static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
-// Helper stream of the INT8 path: the FP64-tensor kernels on X (eta, Ast) are independent of the INT8 kernels on the mask and
-// bound by different units, so they can run next to them (fork / join with two events around the pair).  Created on first
-// use, one per device.  OFF unless PYVB_I8_OVERLAP=1: measured, the pairs do not overlap in practice (C2: 0.824 vs 0.838 ms for
-// the K1 pair, the sweep unchanged) and the fork / join slows the chunked end-to-end path down.
-struct AuxStream {
-    cudaStream_t s = nullptr;
-    cudaEvent_t fork = nullptr, join = nullptr;
-    int state = 0;   // 0 not tried, 1 ready, -1 unavailable
-};
-static AuxStream *aux_stream() {
-    static AuxStream aux[64];
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
-    AuxStream &a = aux[dev];
-    if (a.state == 0) {
-        const char *e = getenv("PYVB_I8_OVERLAP");
-        a.state = -1;
-        if ((e && e[0] == '1') && cudaStreamCreateWithFlags(&a.s, cudaStreamNonBlocking) == cudaSuccess &&
-            cudaEventCreateWithFlags(&a.fork, cudaEventDisableTiming) == cudaSuccess &&
-            cudaEventCreateWithFlags(&a.join, cudaEventDisableTiming) == cudaSuccess)
-            a.state = 1;
-    }
-    return a.state == 1 ? &a : nullptr;
-}
-
 // Accuracy guard of the INT8 path (DESIGN.md 5a): relative accuracy (max norm, per row of qprec / per data dimension of T1)
-// below which the fixed-point contraction is redone on the FP64 tensor cores.  PYVB_I8_GUARD=0 switches the guard off
-// (measurement only), PYVB_I8_GUARD=force makes every call fall back (tests of the fall-back plumbing).
+// below which the fixed-point contraction is redone on the FP64 tensor cores.  PYVB_I8_GUARD=force makes every call fall
+// back (tests of the fall-back plumbing).
 static const double I8_TOL = 3.637978807091713e-12;     // 2^-38
-static int i8_guard_mode() {
-    static int mode = -1;
-    if (mode < 0) {
+static bool i8_guard_forced() {
+    static int forced = -1;
+    if (forced < 0) {
         const char *e = getenv("PYVB_I8_GUARD");
-        mode = (e && e[0] == '0') ? 0 : (e && e[0] == 'f') ? 2 : 1;
+        forced = (e && e[0] == 'f') ? 1 : 0;
     }
-    return mode;
+    return forced;
 }
 
 static int pick_algo(int algo, int D, int q) {
@@ -365,39 +340,23 @@ int pyvb_zstep_i8_f64(long long N, int D, int q, const double *X, long long ldx,
     cudaStream_t st = (cudaStream_t)stream;
     // k1_only: 0 whole Z step, 1 contraction only (INT8 qprec + DMMA eta), 2 INT8 part only, 3 eta part only
     cudaError_t e = cudaSuccess;
-    AuxStream *aux = (k1_only < 2) ? aux_stream() : nullptr;     // both parts wanted: the eta kernel runs next to the INT8 kernel
-    cudaStream_t st2 = st;
-    if (aux) {
-        e = cudaEventRecord(aux->fork, st);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(aux->s, aux->fork, 0);
-        if (e != cudaSuccess) return cuda_fail(e, "zstep_i8 (fork)");
-        st2 = aux->s;
-    }
-    if (k1_only != 3) {      // first: its CTAs take one slot per SM, the eta kernel's CTAs fill what is left
+    if (k1_only != 3) {
         e = launch_pack_g_i8(D, q, Gw, ldg, GI, gscale, gl, st);
         if (e == cudaSuccess) e = launch_zstep_i8(N, D, q, mask, GI, P0, gscale, gl, MZ, (int)ldmz, st);
     }
     if (e == cudaSuccess && k1_only != 2) {
         double *weta = (double *)((char *)GI + align256(i8_digits_bytes(D, q)));
-        e = launch_zstep_eta_dmma(N, D, q, X, ldx, Gw, weta, P0, h0, gl, MZ, st2);
-    }
-    if (aux) {
-        cudaError_t e2 = cudaEventRecord(aux->join, aux->s);
-        if (e2 == cudaSuccess) e2 = cudaStreamWaitEvent(st, aux->join, 0);
-        if (e == cudaSuccess) e = e2;
+        e = launch_zstep_eta_dmma(N, D, q, X, ldx, Gw, weta, P0, h0, gl, MZ, st);
     }
     if (e == cudaSuccess && !k1_only) {
         // K2 checks every finished qprec row against the fixed-point bound of K1-i8 (kernels.h: I8Check); when a row fails,
         // the whole step is redone on the FP64 tensor cores by two conditional launches that exit at once otherwise
-        const int guard = i8_guard_mode();
         I8Check chk;
-        if (guard) {
-            chk.gscale = gscale;
-            chk.ncols = q * (q + 1) / 2;
-            chk.fac = (guard == 2) ? 1e300 : (double)D * 2.7755575615628914e-17 / I8_TOL;     // D * 2^-55 / tol
-        }
+        chk.gscale = gscale;
+        chk.ncols = q * (q + 1) / 2;
+        chk.fac = i8_guard_forced() ? 1e300 : (double)D * 2.7755575615628914e-17 / I8_TOL;     // D * 2^-55 / tol
         e = launch_zsolve(N, q, MZ, Sig, logdet, gl, zsums, st, nullptr, chk);
-        if (e == cudaSuccess && guard)
+        if (e == cudaSuccess)
             e = launch_zstep_dmma(N, D, q, X, ldx, Gw, ldg, P0, h0, gl, MZ, Sig, logdet, zsums, 0, st, gl + PYVB_GL_I8BAD);
     }
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zstep_i8");
@@ -457,36 +416,20 @@ int pyvb_stats_i8_f64(long long N, int D, int q, const double *X, long long ldx,
     const int nch = stats_i8_nchunks(N, D, q);
     // the K2 kernels leave bounds on the column maxima behind their column sums: [sums OROW | 4 | maxima OROW]
     const bool kmax = nzblk > 0;
-    AuxStream *aux = aux_stream();                              // Ast (FP64 tensor cores on X) next to digitize + the INT8 kernel
-    cudaStream_t st2 = st;
-    cudaError_t e = cudaSuccess;
-    if (aux) {
-        e = cudaEventRecord(aux->fork, st);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(aux->s, aux->fork, 0);
-        if (e != cudaSuccess) return cuda_fail(e, "stats_i8 (fork)");
-        st2 = aux->s;
-    }
     // K2's partials when they carry the maxima, else one pass over the MZ rows builds the same partials in `scratch`
     const double *zs = NULL;
     int zn = 0, zk = 0;
-    e = launch_stats_i8(N, D, q, maskT, MZ, (int)ldmz, ZI, scratch, (double *)ws, nch, zsums, nzblk, zkw, kmax ? 1 : 0, logdet,
-                        &zs, &zn, &zk, st);
-    if (e == cudaSuccess) e = launch_stats_x_dmma(N, D, q, X, ldx, MZ, (double *)ws, nch, st2);
-    if (aux) {
-        cudaError_t e2 = cudaEventRecord(aux->join, aux->s);
-        if (e2 == cudaSuccess) e2 = cudaStreamWaitEvent(st, aux->join, 0);
-        if (e == cudaSuccess) e = e2;
-    }
+    cudaError_t e = launch_stats_i8(N, D, q, maskT, MZ, (int)ldmz, ZI, scratch, (double *)ws, nch, zsums, nzblk, zkw,
+                                    kmax ? 1 : 0, logdet, &zs, &zn, &zk, st);
+    if (e == cudaSuccess) e = launch_stats_x_dmma(N, D, q, X, ldx, MZ, (double *)ws, nch, st);
     if (e != cudaSuccess) return cuda_fail(e, "stats_i8");
-    if (i8_guard_mode()) {
-        // the same guard for T1 / Bst: a data dimension whose sums are not accurate to I8_TOL sends the whole pass to the
-        // FP64 tensor cores (one conditional launch that exits at once otherwise); both before the exchange
-        double *guard = stats_i8_guard(scratch, q, (int)ldmz);
-        e = launch_stats_i8_check(D, q, (const double *)ws, nch, xcache, scratch, (int)ldmz,
-                                  i8_guard_mode() == 2 ? 0.0 : I8_TOL, st);      // (tol = 0: every observed dimension fails)
-        if (e == cudaSuccess) e = launch_stats_dmma(N, D, q, X, ldx, MZ, (double *)ws, nch, st, guard);
-        if (e != cudaSuccess) return cuda_fail(e, "stats_i8 (guard)");
-    }
+    // the same guard for T1 / Bst: a data dimension whose sums are not accurate to I8_TOL sends the whole pass to the
+    // FP64 tensor cores (one conditional launch that exits at once otherwise); both before the exchange
+    double *guard = stats_i8_guard(scratch, q, (int)ldmz);
+    e = launch_stats_i8_check(D, q, (const double *)ws, nch, xcache, scratch, (int)ldmz,
+                              i8_guard_forced() ? 0.0 : I8_TOL, st);      // (tol = 0: every observed dimension fails)
+    if (e == cudaSuccess) e = launch_stats_dmma(N, D, q, X, ldx, MZ, (double *)ws, nch, st, guard);
+    if (e != cudaSuccess) return cuda_fail(e, "stats_i8 (guard)");
     e = launch_stats_reduce(D, q, (const double *)ws, nch, NULL, 0, stats, const_cast<double *>(xcache), 1, zs, zn, zk,
                             peers ? peers->bufs : NULL, peers ? peers->world : 1, peers ? peers->rank : 0,
                             peers ? peers->epoch : 0ULL, st);

@@ -237,21 +237,7 @@ int i8_stages(int D, int q, int hstage, int pair = 0, int adbl = 0) {  // digit-
         if (i8_smem_bytes(D, q, nst, hstage, pair, adbl) <= 227 * 1024) return nst;
     return 0;
 }
-int i8_pair_mode() {                                     // PYVB_I8_PAIR = 0 | 1 (default 1): tcgen05.mma.cta_group::2 in K1-i8 / K3-i8
-    static int m = -1;
-    if (m < 0) {
-        const char *e = getenv("PYVB_I8_PAIR");
-        m = (e && e[0] == '0') ? 0 : 1;
-    }
-    return m;
-}
 int i8_hstage(int D, int q) {                            // half staging only where it buys a stage and stages are scarce
-    static int force = -2;
-    if (force == -2) {
-        const char *e = getenv("PYVB_I8_HSTAGE");
-        force = e ? atoi(e) : -1;
-    }
-    if (force == 0 || force == 1) return force;
     const int full = i8_stages(D, q, 0);
     return (full < 6 && i8_stages(D, q, 1) > full) ? 1 : 0;
 }
@@ -608,15 +594,7 @@ cudaError_t launch_cluster(void (*kern)(KArgs...), int grid, int block, size_t s
     cfg.numAttrs = cl > 1 ? 1 : 0;
     return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
-int i8_cluster_size() {                     // PYVB_I8_CLUSTER = 1 | 2 | 4 (default 2)
-    static int cl = 0;
-    if (!cl) {
-        const char *e = getenv("PYVB_I8_CLUSTER");
-        cl = e ? atoi(e) : 2;
-        if (cl != 1 && cl != 2 && cl != 4) cl = 2;
-    }
-    return cl;
-}
+constexpr int I8_CL = 2;                    // CTAs per cluster of K1-i8 (1 for tiny problems) and K3-i8
 
 // =====================================================================================================================
 // K3-i8: the mask-type sufficient statistics  T1 = O^T vec<zz^T>,  Bst = O^T Zbar  (hstack, nodes/nodes_todo.py:50-61)
@@ -636,40 +614,6 @@ constexpr int SST = 9;                                   // stages of the K3-i8 
 constexpr int SST_PAIR = 13;                             // ... with cta_group::2 (15 KB each: half of the digit tile per CTA)
 constexpr int CM_BLOCKS = 148 * 4;                       // partial column maxima
 
-// column maxima of |MZ| over a block of rows: pm[blk][ldmz].  Warp per row, lane l owns the columns l, l + 32, ...
-// (KPL of them, in registers): every row is KPL independent coalesced loads.
-template <int KPL>
-__global__ void __launch_bounds__(256)
-colmax_kernel(long long N, int ldmz, const double *__restrict__ MZ, double *__restrict__ pm, long long rows_per_blk) {
-    extern __shared__ double cm_sh[];                       // [ldmz]
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const long long r0 = (long long)blockIdx.x * rows_per_blk;
-    long long r1 = r0 + rows_per_blk;
-    if (r1 > N) r1 = N;
-    double m[KPL];
-#pragma unroll
-    for (int k = 0; k < KPL; ++k) m[k] = 0.0;
-#pragma unroll 2
-    for (long long n = r0 + warp; n < r1; n += 8) {
-        const double *row = MZ + n * ldmz;
-#pragma unroll
-        for (int k = 0; k < KPL; ++k) {
-            const int c = lane + 32 * k;
-            if (c < ldmz) m[k] = fmax(m[k], fabs(row[c]));
-        }
-    }
-    for (int w = 0; w < 8; ++w) {
-        if (warp == w) {
-#pragma unroll
-            for (int k = 0; k < KPL; ++k) {
-                const int c = lane + 32 * k;
-                if (c < ldmz) cm_sh[c] = (w == 0) ? m[k] : fmax(cm_sh[c], m[k]);
-            }
-        }
-        __syncthreads();
-    }
-    for (int c = threadIdx.x; c < ldmz; c += 256) pm[(size_t)blockIdx.x * ldmz + c] = cm_sh[c];
-}
 // The partials K2 would have left for a block of rows -- [column sums (ldmz - 4) | sum 0.5/logdet, sum logdet, rows, 0 |
 // column maxima of |.| (ldmz - 4)] -- in ONE pass over the MZ rows, for the cases where K2 leaves none (q = 64, or rows
 // written from outside the kernels): replaces three passes (column sums, per-row scalars, column maxima).  A warp takes
@@ -1531,8 +1475,7 @@ cudaError_t launch_zstep_i8(long long N, int D, int q, const void *mask, const v
     if (!i8_supported(D, q)) return cudaErrorNotSupported;
     const I8Geom g(q);
     const long long nrb = (N + BM - 1) / BM;
-    int cl = i8_cluster_size();
-    while (cl > 1 && nrb < 2LL * cl) cl >>= 1;               // tiny problems: no point in pairing
+    const int cl = (nrb < 2LL * I8_CL) ? 1 : I8_CL;          // tiny problems: no point in pairing
     CUtensorMap tmA, tmB;
     const uint64_t nk = (uint64_t)(D / BKB);
     if ((uint64_t)nrb * nk * BM >= (1ULL << 31)) return cudaErrorNotSupported;
@@ -1554,29 +1497,17 @@ cudaError_t launch_zstep_i8(long long N, int D, int q, const void *mask, const v
     // tcgen05.mma.cta_group::2 where digit stages are scarce (D = 1024: 5 stages of 14 KB next to the 128 KB mask block -> 10 of
     // 7 KB; K1 4.49 -> 4.19 ms on the config-3 shard).  Where eight full stages fit anyway (D <= 512) the pair only couples the
     // two CTAs' epilogues (D = 256: 0.43 -> 0.54 ms): plain clusters with multicast there.
-    const int pair = (cl == 2 && i8_pair_mode() && i8_stages(D, q, i8_hstage(D, q), 0) < 8) ? 1 : 0;
+    const int pair = (cl == 2 && i8_stages(D, q, i8_hstage(D, q), 0) < 8) ? 1 : 0;
     const int hstage = pair ? ((i8_stages(D, q, 0, 1) < 12 && i8_stages(D, q, 1, 1) > i8_stages(D, q, 0, 1)) ? 1 : 0) : i8_hstage(D, q);
-    // a second mask block where it costs no digit stage (D <= 256): PYVB_I8_ADBL=0 switches it off
-    static int adbl_on = -1;
-    if (adbl_on < 0) {
-        const char *ev = getenv("PYVB_I8_ADBL");
-        adbl_on = (ev && ev[0] == '0') ? 0 : 1;
-    }
-    const int adbl = (adbl_on && !pair && i8_stages(D, q, hstage, 0, 1) >= ST / 2) ? 1 : 0;
+    // a second mask block where it costs no digit stage (D <= 256)
+    const int adbl = (!pair && i8_stages(D, q, hstage, 0, 1) >= ST / 2) ? 1 : 0;
     int nst = i8_stages(D, q, hstage, pair, adbl);
     if (nst < 2) return cudaErrorNotSupported;
     const size_t smem = i8_smem_bytes(D, q, nst, hstage, pair, adbl);
     // two K chunks per ring stage: half as many barrier round trips, TMA arms and commits per MMA -- with one tile per stage the
     // producer's and the issuer's per-stage latency (~300 clocks each) was as long as the tile's two MMAs (257 clocks).  Measured
     // under ncu on one box: config-3 shard 5.07 -> 4.02 ms, config 2 0.450 -> 0.388 ms, D = 512 / q = 64 unchanged.
-    // PYVB_I8_KS = 1 | 2 overrides.
-    static int ks_env = -1;
-    if (ks_env < 0) {
-        const char *ev = getenv("PYVB_I8_KS");
-        ks_env = ev ? atoi(ev) : 0;
-    }
-    int ks = (ks_env == 1 || ks_env == 2) ? ks_env : 2;
-    if ((nk % 2) != 0 || nst < 4) ks = 1;
+    const int ks = ((nk % 2) != 0 || nst < 4) ? 1 : 2;
     if (ks == 2) nst /= 2;                                   // same bytes: the ring keeps its depth in K chunks
     CUtensorMap tmO8;
     {   // the same rows as 8-column x 32-row boxes (64-byte rows, SWIZZLE_64B) for the half-staging epilogue
@@ -1590,7 +1521,7 @@ cudaError_t launch_zstep_i8(long long N, int D, int q, const void *mask, const v
     }
     long long gl_ = (nrb + cl - 1) / cl * cl;
     const int grid = (int)(gl_ < 148 ? gl_ : 148 / cl * cl);
-    auto kern = cl == 4 ? zstep_i8_kernel<4> : cl == 2 ? (pair ? zstep_i8_kernel<2, true> : zstep_i8_kernel<2>) : zstep_i8_kernel<1>;
+    auto kern = pair ? zstep_i8_kernel<I8_CL, true> : cl == I8_CL ? zstep_i8_kernel<I8_CL> : zstep_i8_kernel<1>;
     e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     static long long *prof = nullptr;
@@ -1634,18 +1565,10 @@ cudaError_t launch_stats_i8_check(int D, int q, const double *ws, int nchunks, c
     return cudaGetLastError();
 }
 
-static int stats_pair_min_d() {                          // PYVB_I8_STATS_PAIR_D: smallest D that uses the CTA-pair MMA in K3-i8
-    static int d = -1;
-    if (d < 0) {
-        const char *e = getenv("PYVB_I8_STATS_PAIR_D");
-        d = e ? atoi(e) : 512;
-    }
-    return d;
-}
 static long long gcd_ll(long long a, long long b) { return b ? gcd_ll(b, a % b) : a; }
 // chunks: items = ndb * nct * nchunks a whole number of rounds over 148 CTAs, chunks of >= 32 K steps, <= 2^23 rows
 int stats_i8_nchunks(long long N, int D, int q) {
-    const int cl = i8_cluster_size();
+    const int cl = I8_CL;
     const long long ncl = 148 / cl;
     const long long per = (long long)(((D + BM - 1) / BM + cl - 1) / cl) * (stats_i8_ncols(q) / CT);   // items of a cluster per chunk
     const long long step = ncl / gcd_ll(ncl, per);
@@ -1776,26 +1699,21 @@ cudaError_t launch_stats_i8(long long N, int D, int q, const void *maskT, const 
     CUtensorMap tmB;
     {   // ZI [npad / 64][nct][224][64]
         cuuint64_t db[3] = {BKB, nkb * nct * (NPL * CT), 1}, sb[2] = {BKB, nkb * nct * (NPL * CT) * BKB};
-        cuuint32_t bb[3] = {BKB, (cuuint32_t)(NPL * CT / i8_cluster_size()), 1};
+        cuuint32_t bb[3] = {BKB, (cuuint32_t)(NPL * CT / I8_CL), 1};
         CUresult r = enc(&tmB, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, ZI, db, sb, bb, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                          CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
     }
-    const int cl = i8_cluster_size();
-    const int pair = (cl == 2 && i8_pair_mode() && ndb >= 2 && D >= stats_pair_min_d()) ? 1 : 0;   // tcgen05.mma.cta_group::2
+    const int cl = I8_CL;
+    const int pair = (cl == 2 && ndb >= 2 && D >= 512) ? 1 : 0;   // tcgen05.mma.cta_group::2
     const size_t smem = si8_smem_bytes(q, pair);
-    auto kern = cl == 4 ? stats_i8_kernel<4> : cl == 2 ? (pair ? stats_i8_kernel<2, true> : stats_i8_kernel<2>) : stats_i8_kernel<1>;
+    auto kern = pair ? stats_i8_kernel<I8_CL, true> : stats_i8_kernel<I8_CL>;
     e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     const long long nitems = (long long)((ndb + cl - 1) / cl) * nct * nchunks;
     const int grid = (int)(nitems < 148 / cl ? nitems : 148 / cl) * cl;
     // K steps per ring stage (as in K1-i8; ncu on one box: config-3 shard 4.17 -> 3.34 ms, config 2 284 -> 265 us; 3 and 4 are slower)
-    static int ks_env = -1;                                    // PYVB_I8_STATS_KS = 1 .. 4 (default 2)
-    if (ks_env < 0) {
-        const char *ev = getenv("PYVB_I8_STATS_KS");
-        ks_env = ev ? atoi(ev) : 0;
-    }
-    const int ks = (ks_env >= 1 && ks_env <= 4) ? ks_env : 2;
+    const int ks = 2;
     return launch_cluster(kern, grid, NTHR, smem, cl, st, tmA, tmB, N, D, q, (const double *)zscale, ws, rpc, nchunks, ndb,
                           nct, ks);
 }

@@ -113,11 +113,11 @@ class PlateEngine(object):
             if algo != "auto":
                 raise ValueError("sparse input needs algo='auto' (the CSR kernels are the only sparse path)")
         # algo "i8": the mask contraction of the Z step on the INT8 tensor cores (exact, kernels_i8.cu); the rest as "dmma".
-        # "auto" picks it when the shape allows (PYVB_I8=0 keeps the all-DMMA path)
+        # "auto" picks it when the shape allows ("dmma" keeps the all-DMMA path)
         self.use_i8 = (algo == "i8")
         if algo == "i8":
             algo = "dmma"
-        elif algo == "auto" and mode == "B" and not self.f32 and os.environ.get("PYVB_I8", "1") != "0":
+        elif algo == "auto" and mode == "B" and not self.f32:
             self.use_i8 = None                                  # decided below, once D is known
         self.algo = _ALGOS[algo] if isinstance(algo, str) else int(algo)
         self.distributed = bool(distributed)
@@ -208,8 +208,7 @@ class PlateEngine(object):
             self.gscale = torch.empty(int(self.lib.pyvb_i8_ncols(q)), dtype=f64, device=dev)
         self._mask_valid = False
         # ... and the mask-type statistics (K3-i8): transposed mask + digit planes of the MZ rows
-        self.use_i8_stats = bool(self.use_i8 and self.lib.pyvb_stats_i8_supported(D, q)
-                                 and os.environ.get("PYVB_I8_STATS", "1") != "0")
+        self.use_i8_stats = bool(self.use_i8 and self.lib.pyvb_stats_i8_supported(D, q))
         self._maskT_valid = False
         n_eff = self._allreduce_scalar(float(n_eff_local))
         self.n_rows_total = int(self._allreduce_scalar(float(N)))
