@@ -300,7 +300,9 @@ int pyvb_stats_i8_f64(long long N, int D, int q, const double *X, long long ldx,
                       size_t ws_bytes, const double *xcache, const double *zsums, const pyvb_peers *peers, void *stream);
 
 /* ---- FP32 variant of the Z-step contraction (tcgen05 tensor cores, TMEM accumulators, TMA-staged bf16 x 3 splits) ----
- * Same reference arithmetic as pyvb_zstep_f64's K1 (nodes/node.py:203-227).  q in {16, 32, 64}, D % 32 == 0.
+ * Same reference arithmetic as pyvb_zstep_f64's K1 (nodes/node.py:203-227).  D % 32 == 0; q in {16, 32, 64} for the
+ * Z step (pyvb_f32_supported), q in {16, 32} for pyvb_stats_f32: it reads the column sums of the rows from K2's partials,
+ * and K2 leaves none at q = 64 (pyvb_zsums_len_f32(N, 64) = 0).
  *   planes  bf16 [3][N][D]    mask | x_h | x_m  (x = x_h + x_m to 16 bits; zeros where not observed); static over sweeps
  *   GT      bf16 [3][NCP][D]  three-way split of [-mu_d <w_d> (q) | G_d packed (P) | pad]^T,  NCP = pyvb_f32_pitch(q)
  *   WT      bf16 [3][q][D]    three-way split of <W>^T
@@ -309,8 +311,8 @@ int pyvb_stats_i8_f64(long long N, int D, int q, const double *X, long long ldx,
 int pyvb_f32_pitch(int q);
 int pyvb_f32_zoff(int q);
 int pyvb_f32_poff(int q);
-int pyvb_f32_supported(int D, int q);
-size_t pyvb_zsums_len_f32(long long N, int q);        /* K2 partials of the FP32 path */
+int pyvb_f32_supported(int D, int q);                 /* the Z step; the statistics also need q != 64 */
+size_t pyvb_zsums_len_f32(long long N, int q);        /* K2 partials of the FP32 path (0 at q = 64) */
 int pyvb_prepare_x_f32(long long N, int D, const double *X, long long ldx, void *planes, void *stream);
 int pyvb_pack_gw_f32(int D, int q, const double *Wbar, const double *Wvar, const double *mu, void *GT, void *WT,
                      void *stream);
@@ -328,7 +330,8 @@ int pyvb_zstep_f32(long long N, long long nalloc, int D, int q, const void *plan
 
 /* FP32 statistics: T1, Bst, Ast partial sums on the tensor cores (MN-major bf16 tiles, FP32 accumulation per row
  * chunk, FP64 across chunks), then the shared fixed-order second stage (+ the peer exchange).  The sums that depend
- * on X alone (xcache) and K2's column sums (zsums) must be valid: the FP32 path has no other source for them. */
+ * on X alone (xcache) and K2's column sums (zsums) must be valid: the FP32 path has no other source for them, hence
+ * q in {16, 32} (PYVB_EINVAL at q = 64). */
 int pyvb_stats_f32(long long N, long long nalloc, int D, int q, const void *planes, const void *MP, double *stats,
                    void *ws, size_t ws_bytes, double *xcache, const double *zsums, const pyvb_peers *peers /* host */,
                    void *stream);

@@ -545,7 +545,7 @@ int pyvb_zstep_f32(long long N, long long nalloc, int D, int q, const void *plan
     if (N == 0) return PYVB_OK;
     ARG(planes && GT && WT && P0 && h0 && gl && MZ32 && MP && logdet, "null pointer");
     cudaError_t e = launch_zstep_f32(N, nalloc, D, q, planes, GT, WT, P0, h0, gl, MZ32, (cudaStream_t)stream);
-    if (e == cudaSuccess) e = launch_zsolve_f32(N, q, MZ32, MP, Sig, logdet, gl, zsums, (cudaStream_t)stream);
+    if (e == cudaSuccess) e = launch_zsolve_f32(N, nalloc, q, MZ32, MP, Sig, logdet, gl, zsums, (cudaStream_t)stream);
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zstep_f32");
 }
 

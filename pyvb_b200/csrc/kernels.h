@@ -88,11 +88,12 @@ int zsolve_tpm_blocks(long long N, int q);        // q in {8, 16} (q = 16: the F
 int zsolve_tpm_kw(int q);
 cudaError_t launch_zsolve_tpm(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
                               cudaStream_t st, const double *cond = nullptr, I8Check chk = I8Check());
-// K2 on the FP32 rows: thread per matrix at q = 16, blocked tensor-core kernel (kernels_k2.cu) at q = 32, 64
-cudaError_t launch_zsolve_tpm_f32(long long N, int q, float *MZ32, void *MP, double *Sig, double *logdet, double *gl,
-                                  double *zsums, cudaStream_t st);
-cudaError_t launch_zsolve_f32(long long N, int q, float *MZ32, void *MP, double *Sig, double *logdet, double *gl,
-                              double *zsums, cudaStream_t st);
+// K2 on the FP32 rows: thread per matrix at q = 16, blocked tensor-core kernel (kernels_k2.cu) at q = 32, 64.
+// MP: bf16 [3][nalloc][pitch] (N <= nalloc, already offset to the first row: a row range keeps the plane stride)
+cudaError_t launch_zsolve_tpm_f32(long long N, long long nalloc, int q, float *MZ32, void *MP, double *Sig, double *logdet,
+                                  double *gl, double *zsums, cudaStream_t st);
+cudaError_t launch_zsolve_f32(long long N, long long nalloc, int q, float *MZ32, void *MP, double *Sig, double *logdet,
+                              double *gl, double *zsums, cudaStream_t st);
 int stats_dmma_nchunks(long long N, int D, int q);
 cudaError_t launch_stats_dmma(long long N, int D, int q, const double *X, long long ldx, const double *MZ,
                               double *ws_main, int nchunks, cudaStream_t st, const double *cond = nullptr);

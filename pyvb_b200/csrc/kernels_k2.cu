@@ -58,7 +58,8 @@ template <int Q> struct KB {
 // Row format of the batched solve.  FP64: the interleaved MZ rows [packed (P) | pad | eta/zbar (q)], pitch
 // pyvb_mz_pitch(q).  FP32 variant: float rows [eta/zbar (q) | packed (P) | pad] of pitch pyvb_f32_pitch(q); the
 // arithmetic stays FP64 (the rows are converted on load / store), and the finished row is also written as a
-// three-way bf16 split (planes [3][N][pitch]) -- the B operand of the FP32 statistics kernel.
+// three-way bf16 split (planes [3][nalloc][pitch], nalloc >= N: a row range keeps the plane stride of the whole
+// allocation) -- the B operand of the FP32 statistics kernel.
 template <int Q, bool F32> struct KIO;
 template <int Q> struct KIO<Q, false> {
     using type = double;
@@ -83,7 +84,7 @@ template <int Q, bool F32>
 __global__ void __launch_bounds__(32 * KB<Q>::WARPS, KB<Q>::OCC)
 zsolve_blocked_kernel(long long N, typename KIO<Q, F32>::type *__restrict__ MZ, double *__restrict__ Sig,
                       double *__restrict__ logdet, double *gl, double *__restrict__ zsums,
-                      __nv_bfloat16 *__restrict__ MP, const double *__restrict__ cond, const I8Check chk) {
+                      __nv_bfloat16 *__restrict__ MP, long long nalloc, const double *__restrict__ cond, const I8Check chk) {
     using T = KB<Q>;
     if (cond != nullptr && !(*cond > 0.0)) return;               // conditional (fall-back) launch: nothing to redo
     __shared__ double s_chk[T::WARPS + 1];
@@ -376,7 +377,7 @@ zsolve_blocked_kernel(long long N, typename KIO<Q, F32>::type *__restrict__ MZ, 
                 const double s = blk[m][t & 0xfff];
                 const double mm = fma(zv[m][(t >> 12) & 63], zv[m][t >> 18], s);
                 row[m][IO::POFF + p] = (io_t)mm;
-                if (F32) store_split3(MP + n * IO::PITCH + IO::POFF + p, (size_t)N * IO::PITCH, (float)mm);
+                if (F32) store_split3(MP + n * IO::PITCH + IO::POFF + p, (size_t)nalloc * IO::PITCH, (float)mm);
                 if (sg) sg[p] = s;
                 if (T::ZS) csum[p] += mm;
             }
@@ -386,7 +387,7 @@ zsolve_blocked_kernel(long long N, typename KIO<Q, F32>::type *__restrict__ MZ, 
                 if (c >= Q) continue;
                 const double z = zv[m][c];
                 row[m][IO::ZOFF + c] = (io_t)z;
-                if (F32) store_split3(MP + n * IO::PITCH + IO::ZOFF + c, (size_t)N * IO::PITCH, (float)z);
+                if (F32) store_split3(MP + n * IO::PITCH + IO::ZOFF + c, (size_t)nalloc * IO::PITCH, (float)z);
                 if (T::ZS) {
                     csum[T::PP + c] += z;
                     // <z_c z_c> = Sigma_cc + z_c^2: with the diagonal maxima, |<z_i z_j>| <= sqrt(<z_i z_i> <z_j z_j>) bounds
@@ -458,33 +459,34 @@ int blocked_blocks(long long N) {
 }
 
 template <int Q>
-cudaError_t launch_blocked_q(long long N, float *MZ32, void *MP, double *Sig, double *logdet, double *gl, double *zsums,
-                             cudaStream_t st) {
+cudaError_t launch_blocked_q(long long N, long long nalloc, float *MZ32, void *MP, double *Sig, double *logdet, double *gl,
+                             double *zsums, cudaStream_t st) {
     using T = KB<Q>;
     cudaError_t e = cudaFuncSetAttribute(zsolve_blocked_kernel<Q, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)T::SMEM);
     if (e != cudaSuccess) return e;
     zsolve_blocked_kernel<Q, true><<<blocked_blocks<Q>(N), 32 * T::WARPS, T::SMEM, st>>>(
-        N, MZ32, Sig, logdet, gl, T::ZS ? zsums : nullptr, static_cast<__nv_bfloat16 *>(MP), nullptr, I8Check());
+        N, MZ32, Sig, logdet, gl, T::ZS ? zsums : nullptr, static_cast<__nv_bfloat16 *>(MP), nalloc, nullptr, I8Check());
     return cudaGetLastError();
 }
 
 }  // namespace
 
-// q = 16: the thread-per-matrix kernel (kernels_k2t.cu); q = 64: no column-sum partials (the statistics pass sums the rows itself)
+// q = 16: the thread-per-matrix kernel (kernels_k2t.cu); q = 64: no column-sum partials, so pyvb_stats_f32 (which has no
+// other source for the sums over the rows) rejects q = 64
 void zsolve_partials_f32(long long N, int q, int &nblk, int &kw) {
     kw = (q == 16) ? zsolve_tpm_kw(q) : (q == 32) ? KB<32>::KW : 0;
     nblk = (kw == 0 || N <= 0) ? 0 : (q == 16) ? zsolve_tpm_blocks(N, q) : blocked_blocks<32>(N);
 }
 
-// FP32 rows (see KIO): in place on MZ32, plus the bf16 x 3 split of the finished rows into MP [3][N][pitch]
-cudaError_t launch_zsolve_f32(long long N, int q, float *MZ32, void *MP, double *Sig, double *logdet, double *gl,
-                              double *zsums, cudaStream_t st) {
+// FP32 rows (see KIO): in place on MZ32, plus the bf16 x 3 split of the finished rows into MP [3][nalloc][pitch]
+cudaError_t launch_zsolve_f32(long long N, long long nalloc, int q, float *MZ32, void *MP, double *Sig, double *logdet,
+                              double *gl, double *zsums, cudaStream_t st) {
     if (N <= 0) return cudaSuccess;
     switch (q) {
-        case 16: return launch_zsolve_tpm_f32(N, q, MZ32, MP, Sig, logdet, gl, zsums, st);
-        case 32: return launch_blocked_q<32>(N, MZ32, MP, Sig, logdet, gl, zsums, st);
-        case 64: return launch_blocked_q<64>(N, MZ32, MP, Sig, logdet, gl, zsums, st);
+        case 16: return launch_zsolve_tpm_f32(N, nalloc, q, MZ32, MP, Sig, logdet, gl, zsums, st);
+        case 32: return launch_blocked_q<32>(N, nalloc, MZ32, MP, Sig, logdet, gl, zsums, st);
+        case 64: return launch_blocked_q<64>(N, nalloc, MZ32, MP, Sig, logdet, gl, zsums, st);
     }
     return cudaErrorNotSupported;
 }

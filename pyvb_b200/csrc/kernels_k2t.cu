@@ -115,11 +115,13 @@ __device__ __forceinline__ void split3_store(__nv_bfloat16 *dst, size_t plane, f
     dst[2 * plane] = __float2bfloat16(r1 - __bfloat162float(m));
 }
 
+// MP (FP32 rows only): bf16 [3][nalloc][PITCH], already offset to the first row; a row range keeps the plane stride of
+// the whole allocation
 template <int Q, bool F32>
 __global__ void __launch_bounds__(32 * TK<Q>::WARPS, 1)
 zsolve_tpm_kernel(long long N, typename TIO<Q, F32>::type *__restrict__ MZ, double *__restrict__ Sig,
                   double *__restrict__ logdet, double *gl, double *__restrict__ zsums, __nv_bfloat16 *__restrict__ MP,
-                  const double *__restrict__ cond, const I8Check chk) {
+                  long long nalloc, const double *__restrict__ cond, const I8Check chk) {
     using T = TK<Q>;
     if (cond != nullptr && !(*cond > 0.0)) return;                 // conditional (fall-back) launch: nothing to redo
     __shared__ double s_chk[T::WARPS + 1];
@@ -409,7 +411,7 @@ zsolve_tpm_kernel(long long N, typename TIO<Q, F32>::type *__restrict__ MZ, doub
                 if (e < P) {
                     const double v = sm[e * LP + m];
                     row[IO::POFF + e] = (io_t)v;
-                    if (F32) split3_store(MP + (n0 + m) * IO::PITCH + IO::POFF + e, (size_t)N * IO::PITCH, (float)v);
+                    if (F32) split3_store(MP + (n0 + m) * IO::PITCH + IO::POFF + e, (size_t)nalloc * IO::PITCH, (float)v);
                     cs[u] += v;
                     if (!F32) cm[u] = max(cm[u], __double2hiint(v) & 0x7fffffff);
                 }
@@ -417,7 +419,7 @@ zsolve_tpm_kernel(long long N, typename TIO<Q, F32>::type *__restrict__ MZ, doub
             if (lane < Q) {
                 const double v = sm[(P + lane) * LP + m];
                 row[IO::ZOFF + lane] = (io_t)v;
-                if (F32) split3_store(MP + (n0 + m) * IO::PITCH + IO::ZOFF + lane, (size_t)N * IO::PITCH, (float)v);
+                if (F32) split3_store(MP + (n0 + m) * IO::PITCH + IO::ZOFF + lane, (size_t)nalloc * IO::PITCH, (float)v);
                 cz += v;
                 if (!F32) czm = max(czm, __double2hiint(v) & 0x7fffffff);
             }
@@ -462,7 +464,7 @@ zsolve_tpm_kernel(long long N, typename TIO<Q, F32>::type *__restrict__ MZ, doub
 
 template <int Q, bool F32>
 cudaError_t launch_tpm_q(long long N, void *MZ, double *Sig, double *logdet, double *gl, double *zsums, void *MP,
-                         cudaStream_t st, const double *cond = nullptr, I8Check chk = I8Check()) {
+                         long long nalloc, cudaStream_t st, const double *cond = nullptr, I8Check chk = I8Check()) {
     using T = TK<Q>;
     cudaError_t e =
         cudaFuncSetAttribute(zsolve_tpm_kernel<Q, F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::SMEM);
@@ -470,7 +472,7 @@ cudaError_t launch_tpm_q(long long N, void *MZ, double *Sig, double *logdet, dou
     const int blocks = zsolve_tpm_blocks(N, Q);
     zsolve_tpm_kernel<Q, F32><<<blocks, 32 * T::WARPS, T::SMEM, st>>>(N, static_cast<typename TIO<Q, F32>::type *>(MZ), Sig,
                                                                     logdet, gl, zsums, static_cast<__nv_bfloat16 *>(MP),
-                                                                    cond, chk);
+                                                                    nalloc, cond, chk);
     return cudaGetLastError();
 }
 
@@ -489,13 +491,13 @@ int zsolve_tpm_kw(int q) { return q == 8 ? TK<8>::KW : q == 16 ? TK<16>::KW : 0;
 cudaError_t launch_zsolve_tpm(long long N, int q, double *MZ, double *Sig, double *logdet, double *gl, double *zsums,
                               cudaStream_t st, const double *cond, I8Check chk) {
     if (N <= 0) return cudaSuccess;
-    if (q == 8) return launch_tpm_q<8, false>(N, MZ, Sig, logdet, gl, zsums, nullptr, st, cond, chk);
+    if (q == 8) return launch_tpm_q<8, false>(N, MZ, Sig, logdet, gl, zsums, nullptr, 0, st, cond, chk);
     return cudaErrorNotSupported;
 }
-cudaError_t launch_zsolve_tpm_f32(long long N, int q, float *MZ32, void *MP, double *Sig, double *logdet, double *gl,
-                                  double *zsums, cudaStream_t st) {
+cudaError_t launch_zsolve_tpm_f32(long long N, long long nalloc, int q, float *MZ32, void *MP, double *Sig, double *logdet,
+                                  double *gl, double *zsums, cudaStream_t st) {
     if (N <= 0) return cudaSuccess;
-    if (q == 16) return launch_tpm_q<16, true>(N, MZ32, Sig, logdet, gl, zsums, MP, st);
+    if (q == 16) return launch_tpm_q<16, true>(N, MZ32, Sig, logdet, gl, zsums, MP, nalloc, st);
     return cudaErrorNotSupported;
 }
 
