@@ -87,6 +87,8 @@ extern "C" {
 #define PYVB_GL_RESID2 10
 #define PYVB_GL_NONPD 11     /* rows whose posterior precision was not positive definite (as a double) */
 #define PYVB_GL_I8BAD 12     /* INT8 path: rows of the LAST Z step whose qprec failed the accuracy guard (then redone on DMMA) */
+#define PYVB_GL_LNS 13       /* weighted data: 1/2 sum of ln s_nd over the observed entries of positive weight, ALL rows (all
+                                ranks); set by the caller, read by pyvb_global_w_f64 only */
 #define PYVB_GL_I8FALL 14    /* INT8 path: Z steps that fell back to the FP64 tensor cores so far (diagnostic) */
 #define PYVB_GL_ALPHA 16     /* [64] <alpha_i>  (constant prior precision when ARD is off) */
 #define PYVB_GL_ALQB 80      /* [64] ARD Gamma qb_i */
@@ -238,6 +240,35 @@ int pyvb_global_nd_f64(int D, int q, int ops, int col_lo, int col_hi, const doub
                        const double *Wvar, double *mu, double *muvar, double *gl, double *nd, const double *P0,
                        const double *h0, const pyvb_consts *consts /* host */, double *elbo_out, void *stream);
 
+/* ---- per-entry observation weights (mode B, FP64; the DMMA, generic and sparse paths) ----
+ * x_nd ~ N(w_d . z_n + mu_d, 1 / (tau s_nd)) for every entry with x_nd not NaN and s_nd > 0, s_nd >= 0 a KNOWN weight (inverse
+ * variances, repeat counts, confidences); s_nd = 0 is a missing entry, as a NaN is.  Lambda_n = tau diag(s_n) replaces
+ * tau diag(mask_n) in every contraction:  qprec_n = P0 + tau sum_d s_nd G_d,  eta_n = h0 + tau sum_d s_nd (x_nd - mu_d) <w_d>,
+ * T1 = (S.O)^T vec<zz^T>,  Bst = (S.O)^T Zbar,  Ast = (S.O.X)^T Zbar.  The weight of an entry whose x is NaN is never read.
+ *   S       [N][lds] doubles, the layout of X (the DMMA path: lds even, S 16-byte aligned); a row range passes S + lo * lds
+ *   weights the sparse paths: one double per stored entry, in the order of values (CSR) / vals (blocked CSC)
+ * The statistics' X-only sums become cnt_d = sum_n s_nd, colsumX_d = sum_n s_nd x_nd, sum s x^2 -- but scal[PYVB_SC_NE] stays
+ * the NUMBER of observed entries of positive weight: the caller's Gamma shape qa = a0 + nE / 2 (global) reads it.  xcache and
+ * the sparse xcache hold the same weighted sums.
+ *   pyvb_zstep_w_f64      pyvb_zstep_f64 with weights (algo generic or DMMA)
+ *   pyvb_stats_w_f64      pyvb_stats_f64 with weights, mode B (no V / Xorig / qldX)
+ *   pyvb_zstep_csr_w_f64, pyvb_stats_csr_w_f64   the CSR gathers with weights
+ *   pyvb_global_w_f64     pyvb_global_f64 (nd = NULL) or pyvb_global_nd_f64 (nd != NULL) for weighted data: the X bound term
+ *                         adds gl[PYVB_GL_LNS]; with nd, ncnt [D] (device) holds the NUMBER of observed entries of positive
+ *                         weight of every column (global), which the per-dimension bound terms read in place of cnt_d.
+ * pyvb_wupdate_f64 / pyvb_wupdate_nd_f64 / pyvb_pack_gw_*_f64 read only the statistics and the state: they serve both. */
+int pyvb_zstep_w_f64(long long N, int D, int q, const double *X, long long ldx, const double *S, long long lds,
+                     const double *Gw, int ldg, const double *P0, const double *h0, double *gl, double *Zbar, long long ldz,
+                     double *M2, long long ldm, double *Sig, double *logdet, double *zsums, int algo, void *stream);
+int pyvb_stats_w_f64(long long N, int D, int q, const double *X, long long ldx, const double *S, long long lds,
+                     const double *Zbar, long long ldz, const double *M2, long long ldm, const double *logdet, double *stats,
+                     void *ws, size_t ws_bytes, double *xcache, int xcache_valid, const double *zsums, int zsums_valid,
+                     const pyvb_peers *peers /* host, nullable */, int algo, void *stream);
+int pyvb_global_w_f64(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar,
+                      const double *Wvar, double *mu, double *muvar, double *gl, double *nd /* nullable */,
+                      const double *ncnt /* nullable without nd */, const double *P0, const double *h0,
+                      const pyvb_consts *consts /* host */, double *elbo_out, void *stream);
+
 /* Mode A: x_hat = observed ? x : W zbar + mu, v = observed ? 0 : 1/tau for rows [0,N) that are not
  * fully observed (pointers already offset to the first row). */
 int pyvb_impute_f64(long long N, int D, int q, const double *Xorig, long long ldx, const double *Wbar,
@@ -367,6 +398,15 @@ int pyvb_stats_csr_f64(long long N, int D, int q, int nblk, const long long *col
                        const double *MZ, long long ldmz, const double *logdet, double *stats, void *ws, size_t ws_bytes,
                        const double *xcache, const double *zsums, const pyvb_peers *peers /* host, nullable */,
                        void *stream);
+/* the same with per-entry observation weights (see "per-entry observation weights" above): weights [nnz] in the order of
+ * values, wts [nnz] in the order of vals; xcache then holds [sum s (D) | sum s x (D) | sum s x^2 | number of entries s > 0] */
+int pyvb_zstep_csr_w_f64(long long N, int D, int q, const long long *indptr, const int *indices, const double *values,
+                         const double *weights, const double *Gw, int ldg, const double *P0, const double *h0, double *gl,
+                         double *MZ, long long ldmz, double *Sig, double *logdet, double *zsums, void *stream);
+int pyvb_stats_csr_w_f64(long long N, int D, int q, int nblk, const long long *colptr, const int *rows, const double *vals,
+                         const double *wts, const double *MZ, long long ldmz, const double *logdet, double *stats, void *ws,
+                         size_t ws_bytes, const double *xcache, const double *zsums,
+                         const pyvb_peers *peers /* host, nullable */, void *stream);
 
 /* ---- VB smoother of a linear dynamic system, batched over B independent sequences (BASELINE config 5) ----
  * Replaces the sweep of examples/Linear_Dynamic_System.py:69-76 for every sequence: all X_t.update() forwards, all

@@ -39,6 +39,12 @@ SIGNATURES = {
     "pyvb_zsums_blocks": (c_int, [c_ll, c_int]),
     "pyvb_zstep_f64": (c_int, [c_ll, c_int, c_int, c_dp, c_ll, c_dp, c_int, c_dp, c_dp, c_dp,
                                c_dp, c_ll, c_dp, c_ll, c_dp, c_dp, c_dp, c_int, c_dp]),
+    "pyvb_zstep_w_f64": (c_int, [c_ll, c_int, c_int, c_dp, c_ll, c_dp, c_ll, c_dp, c_int, c_dp, c_dp, c_dp,
+                                 c_dp, c_ll, c_dp, c_ll, c_dp, c_dp, c_dp, c_int, c_dp]),
+    "pyvb_stats_w_f64": (c_int, [c_ll, c_int, c_int, c_dp, c_ll, c_dp, c_ll, c_dp, c_ll, c_dp, c_ll, c_dp,
+                                 c_dp, c_dp, c_sz, c_dp, c_int, c_dp, c_int, ctypes.POINTER(Peers), c_int, c_dp]),
+    "pyvb_global_w_f64": (c_int, [c_int, c_int, c_int, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp,
+                                  c_dp, ctypes.POINTER(Consts), c_dp, c_dp]),
     "pyvb_zsolve_f64": (c_int, [c_ll, c_int, c_dp, c_ll, c_dp, c_dp, c_dp, c_dp, c_dp]),
     "pyvb_stats_f64": (c_int, [c_ll, c_int, c_int, c_dp, c_ll, c_dp, c_dp, c_dp, c_dp, c_ll, c_dp, c_ll, c_dp,
                                c_dp, c_dp, c_sz, c_dp, c_int, c_dp, c_int, ctypes.POINTER(Peers), c_int, c_dp]),
@@ -78,6 +84,10 @@ SIGNATURES = {
                                    c_dp, c_dp, c_dp]),
     "pyvb_stats_csr_f64": (c_int, [c_ll, c_int, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_ll, c_dp, c_dp, c_dp, c_sz, c_dp,
                                    c_dp, ctypes.POINTER(Peers), c_dp]),
+    "pyvb_zstep_csr_w_f64": (c_int, [c_ll, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_dp, c_int, c_dp, c_dp, c_dp, c_dp, c_ll,
+                                     c_dp, c_dp, c_dp, c_dp]),
+    "pyvb_stats_csr_w_f64": (c_int, [c_ll, c_int, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_dp, c_ll, c_dp, c_dp, c_dp, c_sz,
+                                     c_dp, c_dp, ctypes.POINTER(Peers), c_dp]),
     "pyvb_lds_max_len": (c_int, []),
     "pyvb_lds_iterate_f64": (c_int, [c_int, c_int, c_int, c_int] + [c_dp] * 11 + [ctypes.c_double] * 3 + [c_int, c_dp, c_dp]),
     "pyvb_lds_iterate_known_f64": (c_int, [c_int, c_int, c_int, c_int] + [c_dp] * 12 + [ctypes.c_double] * 3 + [c_int, c_dp, c_dp]),

@@ -7,6 +7,7 @@ GL_QA, GL_QB, GL_TAU, GL_ELBO, GL_ELBO_W, GL_ELBO_MU, GL_ELBO_Z, GL_ELBO_X, GL_E
 GL_RESID2 = 10
 GL_NONPD = 11
 GL_I8BAD = 12
+GL_LNS = 13         # weighted data: 1/2 sum ln s_nd over the observed entries of positive weight (all rows, all ranks)
 GL_I8FALL = 14
 GL_ALPHA = 16
 GL_ALQB = 80

@@ -44,6 +44,16 @@ static int pick_algo(int algo, int D, int q) {
     return algo;
 }
 
+// the implementations behind the plain and the weighted (*_w_*) entry points: S / weights = NULL is the unweighted model
+static int zstep_impl(long long N, int D, int q, const double *X, long long ldx, const double *S, long long lds,
+                      const double *Gw, int ldg, const double *P0, const double *h0, double *gl, double *Zbar, long long ldz,
+                      double *M2, long long ldm, double *Sig, double *logdet, double *zsums, int algo, void *stream);
+static int stats_impl(long long N, int D, int q, const double *X, long long ldx, const double *S, long long lds,
+                      const double *V, const double *Xorig, const double *qldX, const double *Zbar, long long ldz,
+                      const double *M2, long long ldm, const double *logdet, double *stats, void *ws, size_t ws_bytes,
+                      double *xcache, int xcache_valid, const double *zsums, int zsums_valid, const pyvb_peers *peers,
+                      int algo, void *stream);
+
 extern "C" {
 
 int pyvb_version(void) { return 100; }
@@ -157,6 +167,20 @@ int pyvb_pack_gw_nd_f64(int D, int q, const double *Wbar, const double *Wvar, co
 int pyvb_zstep_f64(long long N, int D, int q, const double *X, long long ldx, const double *Gw, int ldg,
                    const double *P0, const double *h0, double *gl, double *Zbar, long long ldz, double *M2,
                    long long ldm, double *Sig, double *logdet, double *zsums, int algo, void *stream) {
+    return zstep_impl(N, D, q, X, ldx, NULL, 0, Gw, ldg, P0, h0, gl, Zbar, ldz, M2, ldm, Sig, logdet, zsums, algo, stream);
+}
+
+int pyvb_zstep_w_f64(long long N, int D, int q, const double *X, long long ldx, const double *S, long long lds,
+                     const double *Gw, int ldg, const double *P0, const double *h0, double *gl, double *Zbar, long long ldz,
+                     double *M2, long long ldm, double *Sig, double *logdet, double *zsums, int algo, void *stream) {
+    ARG(N == 0 || (S != NULL && lds >= D), "S, lds");
+    return zstep_impl(N, D, q, X, ldx, S, lds, Gw, ldg, P0, h0, gl, Zbar, ldz, M2, ldm, Sig, logdet, zsums, algo, stream);
+}
+}  // extern "C"
+
+static int zstep_impl(long long N, int D, int q, const double *X, long long ldx, const double *S, long long lds,
+                      const double *Gw, int ldg, const double *P0, const double *h0, double *gl, double *Zbar, long long ldz,
+                      double *M2, long long ldm, double *Sig, double *logdet, double *zsums, int algo, void *stream) {
     ARG(N >= 0 && D >= 1 && q >= 1 && q <= PYVB_QMAX, "N, D, q");
     if (N == 0) return PYVB_OK;                      // an empty row block (e.g. an empty shard): nothing to update
     ARG(X && Gw && P0 && h0 && gl && Zbar && M2 && logdet, "null pointer");
@@ -168,18 +192,22 @@ int pyvb_zstep_f64(long long N, int D, int q, const double *X, long long ldx, co
         if (!dmma_supported(D, q)) return fail(PYVB_ENOSUP, "%s", "DMMA path needs q in {8,16,32,64}, D % 16 == 0");
         ARG(ldg == pyvb_gw_pitch(q), "ldg must equal pyvb_gw_pitch(q) for the DMMA path");
         ARG((ldx % 2) == 0, "ldx must be even for the DMMA path");
+        ARG(S == NULL || ((lds % 2) == 0 && (reinterpret_cast<uintptr_t>(S) & 15) == 0),
+            "S: lds must be even and S 16-byte aligned for the DMMA path");
         ARG(ldz == pyvb_mz_pitch(q) && ldm == ldz && Zbar == M2 + gw_woff(q),
             "the DMMA path needs the interleaved MZ layout (see pyvb_mz_pitch)");
         e = launch_zstep_dmma(N, D, q, X, ldx, Gw, ldg, P0, h0, gl, M2, Sig, logdet, zsums,
-                              algo == PYVB_ALGO_DMMA_K1, (cudaStream_t)stream);
+                              algo == PYVB_ALGO_DMMA_K1, (cudaStream_t)stream, nullptr, S, lds);
     } else if (a == PYVB_ALGO_GENERIC) {
         e = launch_zstep_generic(N, D, q, X, ldx, Gw, ldg, P0, h0, gl, Zbar, ldz, M2, ldm, Sig, logdet,
-                                 (cudaStream_t)stream);
+                                 (cudaStream_t)stream, S, lds);
     } else {
         return fail(PYVB_EINVAL, "%s", "unknown algo");
     }
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zstep");
 }
+
+extern "C" {
 
 int pyvb_zsolve_f64(long long N, int q, double *MZ, long long ldmz, double *Sig, double *logdet, double *gl,
                     double *zsums, void *stream) {
@@ -196,6 +224,25 @@ int pyvb_stats_f64(long long N, int D, int q, const double *X, long long ldx, co
                    long long ldm, const double *logdet, double *stats, void *ws, size_t ws_bytes, double *xcache,
                    int xcache_valid, const double *zsums, int zsums_valid, const pyvb_peers *peers, int algo,
                    void *stream) {
+    return stats_impl(N, D, q, X, ldx, NULL, 0, V, Xorig, qldX, Zbar, ldz, M2, ldm, logdet, stats, ws, ws_bytes, xcache,
+                      xcache_valid, zsums, zsums_valid, peers, algo, stream);
+}
+
+int pyvb_stats_w_f64(long long N, int D, int q, const double *X, long long ldx, const double *S, long long lds,
+                     const double *Zbar, long long ldz, const double *M2, long long ldm, const double *logdet, double *stats,
+                     void *ws, size_t ws_bytes, double *xcache, int xcache_valid, const double *zsums, int zsums_valid,
+                     const pyvb_peers *peers, int algo, void *stream) {
+    ARG(N == 0 || (S != NULL && lds >= D), "S, lds");
+    return stats_impl(N, D, q, X, ldx, S, lds, NULL, NULL, NULL, Zbar, ldz, M2, ldm, logdet, stats, ws, ws_bytes, xcache,
+                      xcache_valid, zsums, zsums_valid, peers, algo, stream);
+}
+}  // extern "C"
+
+static int stats_impl(long long N, int D, int q, const double *X, long long ldx, const double *S, long long lds,
+                      const double *V, const double *Xorig, const double *qldX, const double *Zbar, long long ldz,
+                      const double *M2, long long ldm, const double *logdet, double *stats, void *ws, size_t ws_bytes,
+                      double *xcache, int xcache_valid, const double *zsums, int zsums_valid, const pyvb_peers *peers,
+                      int algo, void *stream) {
     ARG(N >= 0 && D >= 1 && q >= 1 && q <= PYVB_QMAX, "N, D, q");
     ARG(stats && ws, "null pointer");
     if (N == 0) {
@@ -224,17 +271,19 @@ int pyvb_stats_f64(long long N, int D, int q, const double *X, long long ldx, co
     if (a == PYVB_ALGO_DMMA) {
         if (!dmma_supported(D, q)) return fail(PYVB_ENOSUP, "%s", "DMMA path needs q in {8,16,32,64}, D % 16 == 0");
         ARG((ldx % 2) == 0, "ldx must be even for the DMMA path");
+        ARG(S == NULL || ((lds % 2) == 0 && (reinterpret_cast<uintptr_t>(S) & 15) == 0),
+            "S: lds must be even and S 16-byte aligned for the DMMA path");
         ARG(ldz == pyvb_mz_pitch(q) && ldm == ldz && Zbar == M2 + gw_woff(q),
             "the DMMA path needs the interleaved MZ layout (see pyvb_mz_pitch)");
         nch = stats_dmma_nchunks(N, D, q);
         use_x = (xcache != NULL && xcache_valid) ? 1 : 0;
         if (zsums != NULL && zsums_valid) zsolve_partials(N, q, nzblk, zkw);
-        e = launch_stats_dmma(N, D, q, X, ldx, M2, ws_main, nch, st);
+        e = launch_stats_dmma(N, D, q, X, ldx, M2, ws_main, nch, st, nullptr, S, lds);
         if (e == cudaSuccess && nzblk == 0) e = launch_mzsums(N, D, q, Zbar, ldz, M2, ldm, ws_main, nch, st);
-        if (e == cudaSuccess && !use_x) e = launch_colsums(N, D, q, X, ldx, ws_main, nch, st);
+        if (e == cudaSuccess && !use_x) e = launch_colsums(N, D, q, X, ldx, ws_main, nch, st, S, lds);
     } else if (a == PYVB_ALGO_GENERIC) {
         nch = stats_generic_nchunks(N);
-        e = launch_stats_generic(N, D, q, X, ldx, Zbar, ldz, M2, ldm, ws_main, nch, st);
+        e = launch_stats_generic(N, D, q, X, ldx, Zbar, ldz, M2, ldm, ws_main, nch, st, S, lds);
     } else {
         return fail(PYVB_EINVAL, "%s", "unknown algo");
     }
@@ -244,7 +293,7 @@ int pyvb_stats_f64(long long N, int D, int q, const double *X, long long ldx, co
     // mode B with cached X sums and K2's partials: nothing is left for the per-row scalar pass
     const int need_rows = !(use_x && Xorig == NULL && nzblk > 0);
     if (need_rows) {
-        e = launch_rowscalars(N, D, X, ldx, V, Xorig, qldX, logdet, ws_sc, nblk, use_x && Xorig == NULL, st);
+        e = launch_rowscalars(N, D, X, ldx, V, Xorig, qldX, logdet, ws_sc, nblk, use_x && Xorig == NULL, st, S, lds);
         if (e != cudaSuccess) return cuda_fail(e, "rowscalars");
     }
     e = launch_stats_reduce(D, q, ws_main, nch, need_rows ? ws_sc : NULL, nblk, stats, xcache, use_x,
@@ -252,6 +301,8 @@ int pyvb_stats_f64(long long N, int D, int q, const double *X, long long ldx, co
                             peers ? peers->rank : 0, peers ? peers->epoch : 0ULL, st);
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "stats_reduce");
 }
+
+extern "C" {
 
 int pyvb_wupdate_f64(int D, int q, int col_lo, int col_hi, const double *stats, const double *mu, const double *gl,
                      double *Wbar, double *Wvar, void *stream) {
@@ -296,6 +347,22 @@ int pyvb_global_nd_f64(int D, int q, int ops, int col_lo, int col_hi, const doub
     if (e == cudaSuccess)
         e = launch_global(D, q, ops, col_lo, col_hi, stats, Wbar, Wvar, mu, muvar, gl, P0, h0, *consts, elbo_out, nd, st);
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "global_nd");
+}
+
+int pyvb_global_w_f64(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar,
+                      const double *Wvar, double *mu, double *muvar, double *gl, double *nd, const double *ncnt,
+                      const double *P0, const double *h0, const pyvb_consts *consts, double *elbo_out, void *stream) {
+    ARG(D >= 1 && q >= 1 && q <= PYVB_QMAX, "D, q");
+    ARG(stats && Wbar && Wvar && mu && muvar && gl && P0 && h0 && consts, "null pointer");
+    ARG(0 <= col_lo && col_lo <= col_hi && col_hi <= q, "column range");
+    ARG(!consts->mode_a, "observation weights are a mode-B model (consts->mode_a must be 0)");
+    ARG(nd == NULL || ncnt != NULL, "per-dimension noise with weights needs the per-column counts ncnt");
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = cudaSuccess;
+    if (nd) e = launch_noise_diag(D, q, ops, stats, Wbar, Wvar, mu, muvar, nd, consts->alpha_mu, st, ncnt);
+    if (e == cudaSuccess)
+        e = launch_global(D, q, ops, col_lo, col_hi, stats, Wbar, Wvar, mu, muvar, gl, P0, h0, *consts, elbo_out, nd, st, true);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "global_w");
 }
 
 int pyvb_impute_f64(long long N, int D, int q, const double *Xorig, long long ldx, const double *Wbar,
@@ -449,6 +516,13 @@ size_t pyvb_stats_csr_workspace_bytes(long long N, int D, int q, int nblk) {
 int pyvb_zstep_csr_f64(long long N, int D, int q, const long long *indptr, const int *indices, const double *values,
                        const double *Gw, int ldg, const double *P0, const double *h0, double *gl, double *MZ,
                        long long ldmz, double *Sig, double *logdet, double *zsums, void *stream) {
+    return pyvb_zstep_csr_w_f64(N, D, q, indptr, indices, values, NULL, Gw, ldg, P0, h0, gl, MZ, ldmz, Sig, logdet, zsums,
+                                stream);
+}
+
+int pyvb_zstep_csr_w_f64(long long N, int D, int q, const long long *indptr, const int *indices, const double *values,
+                         const double *weights, const double *Gw, int ldg, const double *P0, const double *h0, double *gl,
+                         double *MZ, long long ldmz, double *Sig, double *logdet, double *zsums, void *stream) {
     ARG(N >= 0 && D >= 1, "N, D");
     if (!csr_supported(q)) return fail(PYVB_ENOSUP, "%s", "the CSR path needs q in {8, 16, 32, 64}");
     if (N == 0) return PYVB_OK;
@@ -457,7 +531,7 @@ int pyvb_zstep_csr_f64(long long N, int D, int q, const long long *indptr, const
     ARG((reinterpret_cast<uintptr_t>(Gw) & 15) == 0 && (reinterpret_cast<uintptr_t>(MZ) & 15) == 0,
         "Gw and MZ must be 16-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
-    cudaError_t e = launch_zstep_csr(N, q, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, (int)ldmz, st);
+    cudaError_t e = launch_zstep_csr(N, q, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, (int)ldmz, st, weights);
     if (e == cudaSuccess) e = launch_zsolve(N, q, MZ, Sig, logdet, gl, zsums, st);
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zstep_csr");
 }
@@ -465,6 +539,14 @@ int pyvb_zstep_csr_f64(long long N, int D, int q, const long long *indptr, const
 int pyvb_stats_csr_f64(long long N, int D, int q, int nblk, const long long *colptr, const int *rows, const double *vals,
                        const double *MZ, long long ldmz, const double *logdet, double *stats, void *ws, size_t ws_bytes,
                        const double *xcache, const double *zsums, const pyvb_peers *peers, void *stream) {
+    return pyvb_stats_csr_w_f64(N, D, q, nblk, colptr, rows, vals, NULL, MZ, ldmz, logdet, stats, ws, ws_bytes, xcache, zsums,
+                                peers, stream);
+}
+
+int pyvb_stats_csr_w_f64(long long N, int D, int q, int nblk, const long long *colptr, const int *rows, const double *vals,
+                         const double *wts, const double *MZ, long long ldmz, const double *logdet, double *stats, void *ws,
+                         size_t ws_bytes, const double *xcache, const double *zsums, const pyvb_peers *peers,
+                         void *stream) {
     ARG(N >= 0 && D >= 1, "N, D");
     if (!csr_supported(q)) return fail(PYVB_ENOSUP, "%s", "the CSR path needs q in {8, 16, 32, 64}");
     ARG(stats && ws, "null pointer");
@@ -488,7 +570,7 @@ int pyvb_stats_csr_f64(long long N, int D, int q, int nblk, const long long *col
     ARG(ldmz == pyvb_mz_pitch(q) && (reinterpret_cast<uintptr_t>(MZ) & 15) == 0, "ldmz must equal pyvb_mz_pitch(q), MZ 16-byte aligned");
     ARG(ws_bytes >= pyvb_stats_csr_workspace_bytes(N, D, q, nblk), "workspace too small");
     double *ws_main = (double *)ws;
-    cudaError_t e = launch_stats_csc(D, q, nblk, colptr, rows, vals, MZ, (int)ldmz, ws_main, st);
+    cudaError_t e = launch_stats_csc(D, q, nblk, colptr, rows, vals, MZ, (int)ldmz, ws_main, st, wts);
     if (e != cudaSuccess) return cuda_fail(e, "stats_csr");
     int nzblk = 0, zkw = 0;
     if (zsums) zsolve_partials(N, q, nzblk, zkw);

@@ -21,22 +21,25 @@ struct I8Check {
 // tau_d (nullable): per-dimension noise precisions folded into the row (pyvb_pack_gw_nd_f64)
 cudaError_t launch_pack_gw(int D, int q, const double *Wbar, const double *Wvar, const double *mu, const double *tau_d,
                            double *Gw, int ldg, cudaStream_t st);
+// S (nullable, here and below): per-entry observation weights [N][lds] of a mode-B data set (the weight of an entry whose x is
+// NaN is not read); every observed entry then counts with its weight, the statistics' cnt is the weight sum and nE the number
+// of observed entries of positive weight
 cudaError_t launch_zstep_generic(long long N, int D, int q, const double *X, long long ldx, const double *Gw,
                                  int ldg, const double *P0, const double *h0, double *gl, double *Zbar,
                                  long long ldz, double *M2, long long ldm, double *Sig, double *logdet,
-                                 cudaStream_t st);
+                                 cudaStream_t st, const double *S = nullptr, long long lds = 0);
 // main statistics: partial sums for `nchunks` row chunks into ws_main[nchunks][statlen]
 int stats_generic_nchunks(long long N);
 cudaError_t launch_stats_generic(long long N, int D, int q, const double *X, long long ldx, const double *Zbar,
                                  long long ldz, const double *M2, long long ldm, double *ws_main, int nchunks,
-                                 cudaStream_t st);
+                                 cudaStream_t st, const double *S = nullptr, long long lds = 0);
 cudaError_t launch_colsums(long long N, int D, int q, const double *X, long long ldx, double *ws_main, int nchunks,
-                           cudaStream_t st);
+                           cudaStream_t st, const double *S = nullptr, long long lds = 0);
 // per-row scalars: partial sums into ws_sc[nblk][PYVB_NSCAL]
 int rowscalars_nblk(long long N);
 cudaError_t launch_rowscalars(long long N, int D, const double *X, long long ldx, const double *V,
                               const double *Xorig, const double *qldX, const double *logdet, double *ws_sc,
-                              int nblk, int skip_x, cudaStream_t st);
+                              int nblk, int skip_x, cudaStream_t st, const double *S = nullptr, long long lds = 0);
 // column sums of the [M2 | zbar] rows -> S, zsum partials (DMMA path)
 cudaError_t launch_mzsums(long long N, int D, int q, const double *Zbar, long long ldz, const double *M2,
                           long long ldm, double *ws_main, int nchunks, cudaStream_t st);
@@ -48,22 +51,28 @@ size_t peer_buffer_bytes(size_t len);
 cudaError_t launch_wupdate(int D, int q, int col_lo, int col_hi, const double *stats, const double *mu,
                            const double *gl, const double *tau_d, double *Wbar, double *Wvar, cudaStream_t st);
 // nd (nullable): per-dimension noise mode -- Mu and the Gammas are left to launch_noise_diag, which must run first
+// weighted: the X bound term also carries gl[PYVB_GL_LNS]
 cudaError_t launch_global(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar, const double *Wvar,
                           double *mu, double *muvar, double *gl, const double *P0, const double *h0,
-                          const pyvb_consts &c, double *elbo_out, const double *nd, cudaStream_t st);
+                          const pyvb_consts &c, double *elbo_out, const double *nd, cudaStream_t st, bool weighted = false);
 // per-dimension noise precisions (kernels_noise.cu): Mu (PYVB_OP_MU), r_d, the Gamma of every d (PYVB_OP_BETA) and the per-d X
 // and Beta bound terms (PYVB_OP_BETA | PYVB_OP_ELBO) into the nd block; one warp per data dimension, no atomics
+// ncnt (nullable): weighted data -- the number of observed entries of every column, which the bound reads (stats' cnt is then
+// the weight sum)
 cudaError_t launch_noise_diag(int D, int q, int ops, const double *stats, const double *Wbar, const double *Wvar, double *mu,
-                              double *muvar, double *nd, double alpha_mu, cudaStream_t st);
+                              double *muvar, double *nd, double alpha_mu, cudaStream_t st, const double *ncnt = nullptr);
 cudaError_t launch_impute(long long N, int D, int q, const double *Xorig, long long ldx, const double *Wbar,
                           const double *mu, const double *Zbar, long long ldz, const double *gl, double *Xhat,
                           double *V, double *qldX, cudaStream_t st);
 
 // ---- FP64 tensor-core (DMMA) + TMA-bulk kernels -------------------------------
 bool dmma_supported(int D, int q);
+// S (nullable): per-entry observation weights, [N][lds] like X (lds even, 16-byte aligned): the contractions become
+// [S.O | S.O.(X - mu)] (K1) and [S.O | S.O.X] (K3); the weight of an entry whose x is NaN is not read
 cudaError_t launch_zstep_dmma(long long N, int D, int q, const double *X, long long ldx, const double *Gw,
                               int ldg, const double *P0, const double *h0, double *gl, double *MZ, double *Sig,
-                              double *logdet, double *zsums, int k1_only, cudaStream_t st, const double *cond = nullptr);
+                              double *logdet, double *zsums, int k1_only, cudaStream_t st, const double *cond = nullptr,
+                              const double *S = nullptr, long long lds = 0);
 int zstep_eta_pitch(int q);
 cudaError_t launch_zstep_eta_dmma(long long N, int D, int q, const double *X, long long ldx, const double *Gw,
                                   double *weta, const double *P0, const double *h0, double *gl, double *MZ,
@@ -96,7 +105,8 @@ cudaError_t launch_zsolve_f32(long long N, long long nalloc, int q, float *MZ32,
                               double *gl, double *zsums, cudaStream_t st);
 int stats_dmma_nchunks(long long N, int D, int q);
 cudaError_t launch_stats_dmma(long long N, int D, int q, const double *X, long long ldx, const double *MZ,
-                              double *ws_main, int nchunks, cudaStream_t st, const double *cond = nullptr);
+                              double *ws_main, int nchunks, cudaStream_t st, const double *cond = nullptr,
+                              const double *S = nullptr, long long lds = 0);
 
 // ---- FP32 variant: tcgen05 / TMEM contraction on bf16 x 3 splits (kernels_f32.cu) ----
 int f32_ncp(int q);                 // floats per MZ32 row
@@ -153,13 +163,14 @@ cudaError_t launch_stats_x_dmma(long long N, int D, int q, const double *X, long
 bool csr_supported(int q);                                  // q in {8, 16, 32, 64} (the q of launch_zsolve)
 int csr_stats_nblocks(long long N, int D, int q);           // row blocks of the column-major layout (partials of K3-csc)
 long long csr_block_rows(long long N, int D, int q);        // rows per block (the last one may hold fewer)
-// MZ rows [0, N) <- [qprec packed | 0 | eta], the input of launch_zsolve
+// MZ rows [0, N) <- [qprec packed | 0 | eta], the input of launch_zsolve.  weights (nullable): per entry, in the order of values
 cudaError_t launch_zstep_csr(long long N, int q, const long long *indptr, const int *indices, const double *values,
                              const double *Gw, int ldg, const double *P0, const double *h0, const double *gl, double *MZ,
-                             int ldmz, cudaStream_t st);
-// T1 | Bst | Ast of every row block b into ws_main[b][statlen] (the other entries of the partials are not written)
+                             int ldmz, cudaStream_t st, const double *weights = nullptr);
+// T1 | Bst | Ast of every row block b into ws_main[b][statlen] (the other entries of the partials are not written).
+// wts (nullable): per entry, in the order of vals
 cudaError_t launch_stats_csc(int D, int q, int nblk, const long long *colptr, const int *rows, const double *vals,
-                             const double *MZ, int ldmz, double *ws_main, cudaStream_t st);
+                             const double *MZ, int ldmz, double *ws_main, cudaStream_t st, const double *wts = nullptr);
 
 // ---- LDS smoother, batched over sequences (kernels_lds.cu) ----
 size_t lds_smem_bytes(int T, int d);

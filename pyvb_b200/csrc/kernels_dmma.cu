@@ -2,11 +2,13 @@
 //
 //   zstep_dmma_kernel<Q>  K1: [O | O.(X-mu)] (rows x D)  @  Gw (D x (P+q))  -> per-row [qprec packed | eta],
 //                             written into the MZ row (one bulk store per row)
+//                             (WT: per-entry observation weights S, a second TMA tile next to X: [S.O | S.O.(X-mu)])
 //   K2 (launch_zsolve below, kernels in kernels_k2*.cu): per-row q x q SPD inverse / solve IN PLACE on the MZ rows,
 //                             [qprec | eta] -> [<zz^T> packed | zbar].  Separate kernels on purpose: K2 is a
 //                             latency-bound DFMA chain; fused behind K1 it kept the CTA's registers and the
 //                             DMMA pipe idle half of the time (profiles/r01_ncu_*.md)
 //   stats_dmma_kernel<Q>  K3: [O | O.X]^T (D x rows) @ [<zz^T> | zbar] (rows x (P+q)) -> T1, Bst, Ast
+//                             (WT: [S.O | S.O.X]^T, the S sub-tiles next to the X sub-tiles)
 //
 // Reference arithmetic: nodes/node.py:203-227 (K1), nodes/gaussian.py:117-123 (K2), nodes/nodes_todo.py:50-61 (K3).
 //
@@ -106,14 +108,16 @@ __host__ __device__ constexpr int c_pitch4(int need) {      // smallest pitch >=
 
 // ETA = true: only the eta column groups [NGO, NG) (the O.(X - mu) @ <W> part); all warps line up along the rows.
 // Used together with the int8 mask contraction (kernels_i8.cu), which produces the qprec columns.
-template <int Q, bool ETA = false> struct ZT {
+// WT = true: per-entry weights S (same layout as X) -- every stage carries an S tile of the X tile's box and swizzle, and the
+// A operand becomes [S.O | S.O.(X - mu)]; at q = 8 (two 4-warp CTAs per SM) the doubled stages leave room for two of them.
+template <int Q, bool ETA = false, bool WT = false> struct ZT {
     using C = ZC<Q>;
     static constexpr int P = c_tri(Q), PP = (P + 7) & ~7, NGO = PP / 8, NGE = Q / 8, NG = NGO + NGE;
     // ETA: 2 x Q / 8 tensor-core instructions per 4 x 8 data entries -- the kernel streams X at HBM speed only with many
     // small stages in flight (8 stages, 2 CTAs per SM: > 100 KB outstanding per SM)
     // (ETA always takes 16 data dimensions per stage: its Gw tile is tiny, and half as many barrier round trips per byte)
     static constexpr int WM = ETA ? C::WM * C::WN : C::WM, WN = ETA ? 1 : C::WN, RGW = C::RGW, KC = ETA ? 16 : C::KC;
-    static constexpr int ST = ETA ? (Q <= 16 ? 8 : 5) : C::ST, OCC = ETA ? 2 : C::OCC;
+    static constexpr int ST = ETA ? (Q <= 16 ? 8 : 5) : ((WT && Q == 8) ? 2 : C::ST), OCC = ETA ? 2 : C::OCC;
     static constexpr int NCT = ETA ? 1 : C::NCT;
     static constexpr bool TILED = ETA || NCT > 1;
     static constexpr int CG0 = ETA ? NGO : 0;          // first column group this kernel computes
@@ -127,12 +131,14 @@ template <int Q, bool ETA = false> struct ZT {
     static constexpr int GP = TILED ? c_pitch4(NGT * 8 + 2) : LDG;   // pitch of the Gw tile in shared memory
     static constexpr int MUL = TILED ? NGT * 8 : MUCOL;              // where mu sits in a shared-memory Gw row
     static constexpr int XT_B = R * KC * 8;     // swizzled X tile (bytes), multiple of 1024
+    static constexpr int XS_B = WT ? 2 * XT_B : XT_B;   // data bytes of a stage: the X tile (+ the S tile behind it)
     static constexpr int GS_B = KC * GP * 8;
     static constexpr int OROW = NGT * 8;        // doubles per output row (segment) [packed | pad | eta]
     static constexpr int SROW = c_srow(OROW);   // staging pitch
-    static constexpr int MAIN_B = (ST * (XT_B + GS_B) + 15) & ~15;
+    static constexpr int MAIN_B = (ST * (XS_B + GS_B) + 15) & ~15;
     static constexpr size_t SMEM = 1024 + (size_t)MAIN_B + (size_t)(P + Q) * 8 + 2 * ST * 8;
     static_assert(XT_B % 1024 == 0, "swizzled tiles must stay 1024-byte aligned");
+    static_assert(!WT || OCC * (SMEM + 1024) <= 228 * 1024, "the weighted CTAs of an SM must fit its shared memory");
 };
 
 // ------------------------------------------------------------------ Z step, part 1 (K1): tensor-core contraction
@@ -140,19 +146,21 @@ template <int Q, bool ETA = false> struct ZT {
 // tiles (the copies of the next tile are in flight while the current one finishes), and the accumulators leave
 // straight from registers with 16-byte stores (8 rows x 64 contiguous bytes per warp instruction), so there is no
 // staging buffer, no per-tile prologue and no pipeline drain between tiles.
-template <int Q, bool ETA>
-__global__ void __launch_bounds__(ZT<Q, ETA>::NTHR, ZT<Q, ETA>::OCC)
+template <int Q, bool ETA, bool WT>
+__global__ void __launch_bounds__(ZT<Q, ETA, WT>::NTHR, ZT<Q, ETA, WT>::OCC)
 zstep_dmma_kernel(const __grid_constant__ CUtensorMap tmX, long long N, int D, const double *__restrict__ Gw,
                   const double *__restrict__ P0, const double *__restrict__ h0, const double *__restrict__ gl,
-                  double *__restrict__ MZ, long long ntiles, const double *__restrict__ cond) {
-    using T = ZT<Q, ETA>;
+                  double *__restrict__ MZ, long long ntiles, const double *__restrict__ cond,
+                  const __grid_constant__ CUtensorMap tmS) {
+    using T = ZT<Q, ETA, WT>;
     if (cond != nullptr && !(*cond > 0.0)) return;              // conditional (fall-back) launch of the INT8 path
     extern __shared__ unsigned char smem_dyn[];
     // 1024-byte aligned base (swizzled TMA tiles); pointer arithmetic on the __shared__ array keeps the
     // shared address space so that fragment loads compile to LDS, not generic LD
     unsigned char *smem = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
     unsigned char *xs_base = smem;                              // ST swizzled X tiles
-    unsigned char *gs_base = smem + T::ST * T::XT_B;            // ST Gw chunks
+    unsigned char *ss_base = smem + T::ST * T::XT_B;            // WT: ST swizzled S tiles
+    unsigned char *gs_base = smem + T::ST * T::XS_B;            // ST Gw chunks
     double *p0v = reinterpret_cast<double *>(smem + T::MAIN_B);
     double *h0s = p0v + T::P;
     uint64_t *full = reinterpret_cast<uint64_t *>(h0s + Q);
@@ -172,6 +180,7 @@ zstep_dmma_kernel(const __grid_constant__ CUtensorMap tmX, long long N, int D, c
     if (tid < Q) h0s[tid] = h0[tid];
     if (tid == 0) {
         tma_prefetch_desc(&tmX);
+        if (WT) tma_prefetch_desc(&tmS);
         for (int s = 0; s < T::ST; ++s) {
             mbar_init(&full[s], 1);
             mbar_init(&empty[s], T::NCW);
@@ -199,15 +208,17 @@ zstep_dmma_kernel(const __grid_constant__ CUtensorMap tmX, long long N, int D, c
         if (!T::TILED || ETA) {
             // ETA: Gw is the compact [wbar (Q) | mu | pad] array with row pitch GP (pack_weta_kernel): the chunk is one copy
             if (elect_one()) {
-                mbar_arrive_expect_tx(&full[s], (uint32_t)(T::XT_B + T::GS_B));
+                mbar_arrive_expect_tx(&full[s], (uint32_t)(T::XS_B + T::GS_B));
                 tma_load_2d(xs_base + s * T::XT_B, &tmX, kc * T::KC, (int)row0, &full[s]);   // rows past N: zero fill
+                if (WT) tma_load_2d(ss_base + s * T::XT_B, &tmS, kc * T::KC, (int)row0, &full[s]);
                 bulk_g2s(gs_base + s * T::GS_B, Gw + (size_t)kc * T::KC * (ETA ? T::GP : T::LDG), T::GS_B, &full[s]);
             }
         } else {
             // one Gw row segment per lane (+ the mu pair for the tile that holds the eta columns)
             if (elect_one()) {
-                mbar_arrive_expect_tx(&full[s], (uint32_t)(T::XT_B + T::KC * (ngt * 64 + (need_mu ? 16 : 0))));
+                mbar_arrive_expect_tx(&full[s], (uint32_t)(T::XS_B + T::KC * (ngt * 64 + (need_mu ? 16 : 0))));
                 tma_load_2d(xs_base + s * T::XT_B, &tmX, kc * T::KC, (int)row0, &full[s]);
+                if (WT) tma_load_2d(ss_base + s * T::XT_B, &tmS, kc * T::KC, (int)row0, &full[s]);
             }
             __syncwarp();
             if (lane < T::KC) {
@@ -259,6 +270,7 @@ zstep_dmma_kernel(const __grid_constant__ CUtensorMap tmX, long long N, int D, c
             if (warp == 0 && p_it < total_it) produce();       // keeps the pipeline ST - 1 steps ahead
             mbar_wait(&full[s], ph);
             const unsigned char *xs = xs_base + s * T::XT_B;
+            const unsigned char *ss = ss_base + s * T::XT_B;
             const double *gs = reinterpret_cast<const double *>(gs_base + s * T::GS_B) + qd * T::GP;
 #pragma unroll
             for (int kk = 0; kk < T::KC / 4; ++kk) {
@@ -270,8 +282,14 @@ zstep_dmma_kernel(const __grid_constant__ CUtensorMap tmX, long long N, int D, c
                     // rows of group rg sit 8 tile rows further: +8 rows keeps (row & 7) and ((row >> 1) & 3)
                     const double x = *reinterpret_cast<const double *>(xs + xo[kk] + rg * 8 * T::KC * 8);
                     const bool ob = (x == x);          // NaN = not observed
-                    ao[rg] = ob ? 1.0 : 0.0;
-                    ax[rg] = ob ? (x - muv) : 0.0;
+                    if (WT) {                          // (the weight of an unobserved entry is not read: it may be NaN)
+                        const double w = *reinterpret_cast<const double *>(ss + xo[kk] + rg * 8 * T::KC * 8);
+                        ao[rg] = ob ? w : 0.0;
+                        ax[rg] = ob ? w * (x - muv) : 0.0;
+                    } else {
+                        ao[rg] = ob ? 1.0 : 0.0;
+                        ax[rg] = ob ? (x - muv) : 0.0;
+                    }
                 }
 #pragma unroll
                 for (int j = 0; j < T::NGW; ++j) {
@@ -346,11 +364,12 @@ static cudaError_t launch_k1_q(long long N, int D, const double *X, long long ld
     cudaError_t e = make_map(&tmX, X, (uint64_t)D, (uint64_t)N, (uint64_t)ldx, T::KC, T::R,
                              T::KC == 16 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(zstep_dmma_kernel<Q, ETA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::SMEM);
+    e = cudaFuncSetAttribute(zstep_dmma_kernel<Q, ETA, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::SMEM);
     if (e != cudaSuccess) return e;
     const long long ntiles = ((N + T::R - 1) / T::R) * T::NCT;
     const long long blocks = ntiles < 148LL * T::OCC ? ntiles : 148LL * T::OCC;
-    zstep_dmma_kernel<Q, ETA><<<(unsigned)blocks, T::NTHR, T::SMEM, st>>>(tmX, N, D, Gw, P0, h0, gl, MZ, ntiles, nullptr);
+    zstep_dmma_kernel<Q, ETA, false><<<(unsigned)blocks, T::NTHR, T::SMEM, st>>>(tmX, N, D, Gw, P0, h0, gl, MZ, ntiles, nullptr,
+                                                                               tmX);
     return cudaGetLastError();
 }
 
@@ -380,35 +399,48 @@ cudaError_t launch_zstep_eta_dmma(long long N, int D, int q, const double *X, lo
     return cudaErrorNotSupported;
 }
 
-template <int Q>
-static cudaError_t launch_zstep_q(long long N, int D, const double *X, long long ldx, const double *Gw,
-                                  const double *P0, const double *h0, double *gl, double *MZ, double *Sig,
-                                  double *logdet, double *zsums, int k1_only, cudaStream_t st, const double *cond) {
-    using T = ZT<Q>;
-    CUtensorMap tmX;
-    cudaError_t e = make_map(&tmX, X, (uint64_t)D, (uint64_t)N, (uint64_t)ldx, T::KC, T::R,
-                             T::KC == 16 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B);
+template <int Q, bool WT>
+static cudaError_t launch_k1w_q(long long N, int D, const double *X, long long ldx, const double *S, long long lds,
+                                const double *Gw, const double *P0, const double *h0, double *gl, double *MZ,
+                                cudaStream_t st, const double *cond) {
+    using T = ZT<Q, false, WT>;
+    const CUtensorMapSwizzle sw = T::KC == 16 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
+    CUtensorMap tmX, tmS;
+    cudaError_t e = make_map(&tmX, X, (uint64_t)D, (uint64_t)N, (uint64_t)ldx, T::KC, T::R, sw);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(zstep_dmma_kernel<Q, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::SMEM);
+    tmS = tmX;                                                  // (not read without weights)
+    if (WT) e = make_map(&tmS, S, (uint64_t)D, (uint64_t)N, (uint64_t)lds, T::KC, T::R, sw);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(zstep_dmma_kernel<Q, false, WT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::SMEM);
     if (e != cudaSuccess) return e;
     const long long ntiles = ((N + T::R - 1) / T::R) * T::NCT;
     const long long blocks = ntiles < 148LL * ZC<Q>::OCC ? ntiles : 148LL * ZC<Q>::OCC;
-    zstep_dmma_kernel<Q, false><<<(unsigned)blocks, T::NTHR, T::SMEM, st>>>(tmX, N, D, Gw, P0, h0, gl, MZ, ntiles, cond);
-    e = cudaGetLastError();
+    zstep_dmma_kernel<Q, false, WT><<<(unsigned)blocks, T::NTHR, T::SMEM, st>>>(tmX, N, D, Gw, P0, h0, gl, MZ, ntiles, cond,
+                                                                              tmS);
+    return cudaGetLastError();
+}
+
+template <int Q>
+static cudaError_t launch_zstep_q(long long N, int D, const double *X, long long ldx, const double *S, long long lds,
+                                  const double *Gw, const double *P0, const double *h0, double *gl, double *MZ, double *Sig,
+                                  double *logdet, double *zsums, int k1_only, cudaStream_t st, const double *cond) {
+    cudaError_t e = S ? launch_k1w_q<Q, true>(N, D, X, ldx, S, lds, Gw, P0, h0, gl, MZ, st, cond)
+                      : launch_k1w_q<Q, false>(N, D, X, ldx, S, lds, Gw, P0, h0, gl, MZ, st, cond);
     if (e != cudaSuccess || k1_only) return e;
     return launch_zsolve(N, Q, MZ, Sig, logdet, gl, zsums, st, cond);
 }
 
 cudaError_t launch_zstep_dmma(long long N, int D, int q, const double *X, long long ldx, const double *Gw, int ldg,
                               const double *P0, const double *h0, double *gl, double *MZ, double *Sig,
-                              double *logdet, double *zsums, int k1_only, cudaStream_t st, const double *cond) {
+                              double *logdet, double *zsums, int k1_only, cudaStream_t st, const double *cond,
+                              const double *S, long long lds) {
     if (N <= 0) return cudaSuccess;
     if (ldg != c_gw_pitch(q)) return cudaErrorInvalidValue;
     switch (q) {
-        case 8: return launch_zstep_q<8>(N, D, X, ldx, Gw, P0, h0, gl, MZ, Sig, logdet, zsums, k1_only, st, cond);
-        case 16: return launch_zstep_q<16>(N, D, X, ldx, Gw, P0, h0, gl, MZ, Sig, logdet, zsums, k1_only, st, cond);
-        case 32: return launch_zstep_q<32>(N, D, X, ldx, Gw, P0, h0, gl, MZ, Sig, logdet, zsums, k1_only, st, cond);
-        case 64: return launch_zstep_q<64>(N, D, X, ldx, Gw, P0, h0, gl, MZ, Sig, logdet, zsums, k1_only, st, cond);
+        case 8: return launch_zstep_q<8>(N, D, X, ldx, S, lds, Gw, P0, h0, gl, MZ, Sig, logdet, zsums, k1_only, st, cond);
+        case 16: return launch_zstep_q<16>(N, D, X, ldx, S, lds, Gw, P0, h0, gl, MZ, Sig, logdet, zsums, k1_only, st, cond);
+        case 32: return launch_zstep_q<32>(N, D, X, ldx, S, lds, Gw, P0, h0, gl, MZ, Sig, logdet, zsums, k1_only, st, cond);
+        case 64: return launch_zstep_q<64>(N, D, X, ldx, S, lds, Gw, P0, h0, gl, MZ, Sig, logdet, zsums, k1_only, st, cond);
     }
     return cudaErrorNotSupported;
 }
@@ -454,7 +486,9 @@ template <> struct SC<64> { static constexpr int WM = 2, WN = 4, RGW = 2, KC = 8
 // XO = true: only the X-type statistics Ast = (O.X)^T Zbar (the mask-type ones come from the INT8 kernel, kernels_i8.cu):
 // all warps line up along the data dimensions, the MZ tile is just the zbar columns (+ the 4 pad columns that follow
 // them, which keeps the shared-memory pitch = 4 (mod 8): conflict-free B fragments)
-template <int Q, bool XO = false> struct STT {
+// WT = true: per-entry weights S (same layout as X): every stage carries the S sub-tiles behind the X sub-tiles, and the A
+// operand becomes [S.O | S.O.X]
+template <int Q, bool XO = false, bool WT = false> struct STT {
     using C = SC<Q>;
     static constexpr int P = c_tri(Q), PP = (P + 7) & ~7;
     static constexpr int NGO = XO ? 0 : (PP + Q) / 8, NGX = Q / 8, NG = NGO + NGX;   // O-type: [<zz^T> | pad | zbar]; X-type: zbar
@@ -472,26 +506,29 @@ template <int Q, bool XO = false> struct STT {
     static constexpr bool BTILE = XO || VP <= 256;    // MZ tile through one tensor copy (box dims are limited to 256)
     static constexpr int SUB_B = KC * 128;
     static constexpr int AS_B = NSUB * SUB_B, VS_B = KC * VPS * 8;
-    static constexpr size_t SMEM = 1024 + (size_t)ST * (AS_B + VS_B) + 2 * ST * 8;
+    static constexpr int AW_B = WT ? 2 * AS_B : AS_B;   // data bytes of a stage: the X sub-tiles (+ the S sub-tiles)
+    static constexpr size_t SMEM = 1024 + (size_t)ST * (AW_B + VS_B) + 2 * ST * 8;
+    static_assert(SMEM <= 227 * 1024, "one CTA must fit the shared memory of an SM");
     static_assert(DT % 16 == 0 && SUB_B % 1024 == 0, "sub-tiles must stay 1024-byte aligned");
 };
 
 // grid.x = number of d tiles, grid.y = row chunks.  Partial sums go to ws[chunk][stat layout]; a second
 // kernel adds the chunks in a fixed order (deterministic).
-template <int Q, bool XO>
-__global__ void __launch_bounds__(STT<Q, XO>::NTHR, SC<Q>::OCC)
+template <int Q, bool XO, bool WT>
+__global__ void __launch_bounds__(STT<Q, XO, WT>::NTHR, SC<Q>::OCC)
 stats_dmma_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmV, long long N, int D,
                   const double *__restrict__ MZ, double *__restrict__ ws, long long rows_per_chunk,
-                  const double *__restrict__ cond) {
-    using T = STT<Q, XO>;
+                  const double *__restrict__ cond, const __grid_constant__ CUtensorMap tmS) {
+    using T = STT<Q, XO, WT>;
     if (cond != nullptr && !(*cond > 0.0)) return;              // conditional (fall-back) launch of the INT8 statistics
     extern __shared__ unsigned char smem_dyn[];
     // 1024-byte aligned base (swizzled TMA tiles); pointer arithmetic on the __shared__ array keeps the
     // shared address space so that fragment loads compile to LDS, not generic LD
     unsigned char *smem = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
     unsigned char *as_base = smem;                          // ST x NSUB swizzled X sub-tiles
-    unsigned char *vs_base = smem + T::ST * T::AS_B;        // ST MZ tiles [KC][VP]
-    uint64_t *full = reinterpret_cast<uint64_t *>(smem + T::ST * (T::AS_B + T::VS_B));
+    unsigned char *ws_base = smem + T::ST * T::AS_B;        // WT: ST x NSUB swizzled S sub-tiles
+    unsigned char *vs_base = smem + T::ST * T::AW_B;        // ST MZ tiles [KC][VP]
+    uint64_t *full = reinterpret_cast<uint64_t *>(smem + T::ST * (T::AW_B + T::VS_B));
     uint64_t *empty = full + T::ST;
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -513,6 +550,7 @@ stats_dmma_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant
     if (tid == 0) {
         tma_prefetch_desc(&tmX);
         tma_prefetch_desc(&tmV);
+        if (WT) tma_prefetch_desc(&tmS);
         for (int s = 0; s < T::ST; ++s) {
             mbar_init(&full[s], 1);
             mbar_init(&empty[s], T::NCW);
@@ -530,9 +568,12 @@ stats_dmma_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant
         double *vs = reinterpret_cast<double *>(vs_base + s * T::VS_B);   // zero filled by the tensor copies
         if (T::BTILE) {
             if (elect_one()) {        // (not `lane == 0`: that wraps every TMA instruction in an election loop)
-                mbar_arrive_expect_tx(&full[s], (uint32_t)(nsub * T::SUB_B + T::VS_B));
+                mbar_arrive_expect_tx(&full[s], (uint32_t)((WT ? 2 : 1) * nsub * T::SUB_B + T::VS_B));
                 for (int t = 0; t < nsub; ++t)
                     tma_load_2d(as_base + s * T::AS_B + t * T::SUB_B, &tmX, d0 + t * 16, (int)nb, &full[s]);
+                if (WT)
+                    for (int t = 0; t < nsub; ++t)
+                        tma_load_2d(ws_base + s * T::AS_B + t * T::SUB_B, &tmS, d0 + t * 16, (int)nb, &full[s]);
                 tma_load_2d(vs, &tmV, 0, (int)nb, &full[s]);
             }
         } else {
@@ -542,9 +583,12 @@ stats_dmma_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant
                 for (int c = lane; c < T::VPS; c += 32) vs[r * T::VPS + c] = 0.0;
             __syncwarp();
             if (elect_one()) {
-                mbar_arrive_expect_tx(&full[s], (uint32_t)(nsub * T::SUB_B + nval * wcols * 8));
+                mbar_arrive_expect_tx(&full[s], (uint32_t)((WT ? 2 : 1) * nsub * T::SUB_B + nval * wcols * 8));
                 for (int t = 0; t < nsub; ++t)
                     tma_load_2d(as_base + s * T::AS_B + t * T::SUB_B, &tmX, d0 + t * 16, (int)nb, &full[s]);
+                if (WT)
+                    for (int t = 0; t < nsub; ++t)
+                        tma_load_2d(ws_base + s * T::AS_B + t * T::SUB_B, &tmS, d0 + t * 16, (int)nb, &full[s]);
             }
             __syncwarp();
             if (lane < nval)
@@ -587,6 +631,7 @@ stats_dmma_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant
             mbar_wait(&full[s], ph);
             if (active) {
                 const unsigned char *as = as_base + s * T::AS_B;
+                const unsigned char *wsb = ws_base + s * T::AS_B;
                 const double *vs = reinterpret_cast<const double *>(vs_base + s * T::VS_B) + qd * T::VPS + gid;
 #pragma unroll
                 for (int kk = 0; kk < T::KC / 4; ++kk) {
@@ -602,8 +647,14 @@ stats_dmma_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant
                             const int off = aoff[rg] + row * 128 + ((((dl[rg] >> 1) ^ (row & 7))) << 4);
                             const double x = *reinterpret_cast<const double *>(as + off);   // stale data if !in
                             const bool ob = in && (x == x);
-                            ao[rg] = ob ? 1.0 : 0.0;
-                            ax[rg] = ob ? x : 0.0;
+                            if (WT) {
+                                const double w = *reinterpret_cast<const double *>(wsb + off);
+                                ao[rg] = ob ? w : 0.0;
+                                ax[rg] = ob ? w * x : 0.0;
+                            } else {
+                                ao[rg] = ob ? 1.0 : 0.0;
+                                ax[rg] = ob ? x : 0.0;
+                            }
                         }
                     }
 #pragma unroll
@@ -680,12 +731,16 @@ int stats_dmma_nchunks(long long N, int D, int q) {
     return (int)c;
 }
 
-template <int Q, bool XO = false>
+template <int Q, bool XO = false, bool WT = false>
 static cudaError_t launch_stats_q(long long N, int D, const double *X, long long ldx, const double *MZ, double *ws,
-                                  int nchunks, cudaStream_t st, const double *cond = nullptr) {
-    using T = STT<Q, XO>;
-    CUtensorMap tmX, tmV;
+                                  int nchunks, cudaStream_t st, const double *cond = nullptr, const double *S = nullptr,
+                                  long long lds = 0) {
+    using T = STT<Q, XO, WT>;
+    CUtensorMap tmX, tmV, tmS;
     cudaError_t e = make_map(&tmX, X, (uint64_t)D, (uint64_t)N, (uint64_t)ldx, 16, T::KC, CU_TENSOR_MAP_SWIZZLE_128B);
+    if (e != cudaSuccess) return e;
+    tmS = tmX;                                                  // (not read without weights)
+    if (WT) e = make_map(&tmS, S, (uint64_t)D, (uint64_t)N, (uint64_t)lds, 16, T::KC, CU_TENSOR_MAP_SWIZZLE_128B);
     if (e != cudaSuccess) return e;
     if (XO) {   // the zbar columns [PP, PP + Q) and the 4 pad columns behind them
         e = make_map(&tmV, MZ + T::PP, (uint64_t)(Q + 4), (uint64_t)N, (uint64_t)T::VP, Q + 4, T::KC, CU_TENSOR_MAP_SWIZZLE_NONE);
@@ -696,14 +751,14 @@ static cudaError_t launch_stats_q(long long N, int D, const double *X, long long
     } else {
         tmV = tmX;   // unused
     }
-    e = cudaFuncSetAttribute(stats_dmma_kernel<Q, XO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::SMEM);
+    e = cudaFuncSetAttribute(stats_dmma_kernel<Q, XO, WT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::SMEM);
     if (e != cudaSuccess) return e;
     long long rpc = (N + nchunks - 1) / nchunks;
     rpc = ((rpc + T::KC - 1) / T::KC) * T::KC;                 // chunk boundaries on pipeline-step boundaries
     if (rpc < T::KC) rpc = T::KC;
     const int ndt = ((D + T::DT - 1) / T::DT) * T::NCT;
     dim3 grid((unsigned)ndt, (unsigned)nchunks);
-    stats_dmma_kernel<Q, XO><<<grid, T::NTHR, T::SMEM, st>>>(tmX, tmV, N, D, MZ, ws, rpc, cond);
+    stats_dmma_kernel<Q, XO, WT><<<grid, T::NTHR, T::SMEM, st>>>(tmX, tmV, N, D, MZ, ws, rpc, cond, tmS);
     return cudaGetLastError();
 }
 
@@ -720,8 +775,18 @@ cudaError_t launch_stats_x_dmma(long long N, int D, int q, const double *X, long
 }
 
 cudaError_t launch_stats_dmma(long long N, int D, int q, const double *X, long long ldx, const double *MZ,
-                              double *ws_main, int nchunks, cudaStream_t st, const double *cond) {
+                              double *ws_main, int nchunks, cudaStream_t st, const double *cond, const double *S,
+                              long long lds) {
     if (N <= 0) return cudaSuccess;
+    if (S) {
+        switch (q) {
+            case 8: return launch_stats_q<8, false, true>(N, D, X, ldx, MZ, ws_main, nchunks, st, cond, S, lds);
+            case 16: return launch_stats_q<16, false, true>(N, D, X, ldx, MZ, ws_main, nchunks, st, cond, S, lds);
+            case 32: return launch_stats_q<32, false, true>(N, D, X, ldx, MZ, ws_main, nchunks, st, cond, S, lds);
+            case 64: return launch_stats_q<64, false, true>(N, D, X, ldx, MZ, ws_main, nchunks, st, cond, S, lds);
+        }
+        return cudaErrorNotSupported;
+    }
     switch (q) {
         case 8: return launch_stats_q<8>(N, D, X, ldx, MZ, ws_main, nchunks, st, cond);
         case 16: return launch_stats_q<16>(N, D, X, ldx, MZ, ws_main, nchunks, st, cond);

@@ -57,13 +57,15 @@ cudaError_t launch_pack_gw(int D, int q, const double *Wbar, const double *Wvar,
 // K2 follows the reference literally (nodes/gaussian.py:118-123): Cholesky factor of qprec, then
 // cho_solve against the identity (two triangular solves per column; lane j owns column j), then
 // qmu = qcov . (pprec.pmu + sum m2).  ln prod diag chol comes from the factor's diagonal.
-template <int NT, int WPB>
+// WT: per-entry observation weights S [N][lds]: qprec_n = P0 + tau sum_d s_nd G_d, eta_n = h0 + tau sum_d s_nd (x_nd - mu_d) wbar_d
+// (an entry of weight 0 is skipped, as a NaN)
+template <int NT, int WPB, bool WT>
 __global__ void __launch_bounds__(32 * WPB)
 zstep_generic_kernel(long long N, int D, int q, const double *__restrict__ X, long long ldx,
                      const double *__restrict__ Gw, int ldg, const double *__restrict__ P0,
                      const double *__restrict__ h0, double *gl, double *__restrict__ Zbar, long long ldz,
                      double *__restrict__ M2, long long ldm, double *__restrict__ Sig,
-                     double *__restrict__ logdet) {
+                     double *__restrict__ logdet, const double *__restrict__ S, long long lds) {
     extern __shared__ double smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int P = tri(q), Pp = gw_woff(q), C = P + q;
@@ -84,11 +86,24 @@ zstep_generic_kernel(long long N, int D, int q, const double *__restrict__ X, lo
         for (int d0 = 0; d0 < D; d0 += 32) {
             const int d = d0 + lane;
             const double xv = (d < D) ? xr[d] : qnan;
+            const double sv = (WT && d < D) ? S[n * lds + d] : 1.0;
             const int dmax = min(32, D - d0);
             for (int dd = 0; dd < dmax; ++dd) {
                 const double x = __shfl_sync(0xffffffffu, xv, dd);
                 if (x != x) continue;  // not observed: warp-uniform
                 const double *g = Gw + (size_t)(d0 + dd) * ldg;
+                if (WT) {
+                    const double w = __shfl_sync(0xffffffffu, sv, dd);
+                    if (w == 0.0) continue;
+                    const double xm = w * (x - g[Pp + q]);
+#pragma unroll
+                    for (int t = 0; t < NT; ++t) {
+                        const int c = lane + 32 * t;
+                        if (c < P) acc[t] = fma(w, g[c], acc[t]);
+                        else if (c < C) acc[t] = fma(xm, g[c - P + Pp], acc[t]);
+                    }
+                    continue;
+                }
                 const double xm = x - g[Pp + q];
 #pragma unroll
                 for (int t = 0; t < NT; ++t) {
@@ -168,7 +183,7 @@ zstep_generic_kernel(long long N, int D, int q, const double *__restrict__ X, lo
 cudaError_t launch_zstep_generic(long long N, int D, int q, const double *X, long long ldx, const double *Gw,
                                  int ldg, const double *P0, const double *h0, double *gl, double *Zbar,
                                  long long ldz, double *M2, long long ldm, double *Sig, double *logdet,
-                                 cudaStream_t st) {
+                                 cudaStream_t st, const double *S, long long lds) {
     if (N <= 0) return cudaSuccess;
     const int C = tri(q) + q;
     const int nt = (C + 31) / 32;
@@ -176,13 +191,18 @@ cudaError_t launch_zstep_generic(long long N, int D, int q, const double *X, lon
     const size_t smem = (size_t)wpb * (2 * q * (q + 1) + 2 * q) * sizeof(double);
     long long blocks = (N + wpb - 1) / wpb;
     if (blocks > 148 * 16) blocks = 148 * 16;
-#define PYVB_LAUNCH_Z(NT, WPB)                                                                                 \
+#define PYVB_LAUNCH_ZW(NT, WPB, WT)                                                                            \
     do {                                                                                                       \
-        cudaError_t e = cudaFuncSetAttribute(zstep_generic_kernel<NT, WPB>,                                    \
+        cudaError_t e = cudaFuncSetAttribute(zstep_generic_kernel<NT, WPB, WT>,                                \
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);          \
         if (e != cudaSuccess) return e;                                                                        \
-        zstep_generic_kernel<NT, WPB><<<(unsigned)blocks, 32 * WPB, smem, st>>>(                               \
-            N, D, q, X, ldx, Gw, ldg, P0, h0, gl, Zbar, ldz, M2, ldm, Sig, logdet);                            \
+        zstep_generic_kernel<NT, WPB, WT><<<(unsigned)blocks, 32 * WPB, smem, st>>>(                           \
+            N, D, q, X, ldx, Gw, ldg, P0, h0, gl, Zbar, ldz, M2, ldm, Sig, logdet, S, lds);                    \
+    } while (0)
+#define PYVB_LAUNCH_Z(NT, WPB)                                                                                 \
+    do {                                                                                                       \
+        if (S) PYVB_LAUNCH_ZW(NT, WPB, true);                                                                  \
+        else PYVB_LAUNCH_ZW(NT, WPB, false);                                                                   \
     } while (0)
     if (nt <= 1) PYVB_LAUNCH_Z(1, 4);
     else if (nt <= 2) PYVB_LAUNCH_Z(2, 4);
@@ -190,16 +210,20 @@ cudaError_t launch_zstep_generic(long long N, int D, int q, const double *X, lon
     else if (nt <= 18) PYVB_LAUNCH_Z(18, 4);
     else PYVB_LAUNCH_Z(67, 2);
 #undef PYVB_LAUNCH_Z
+#undef PYVB_LAUNCH_ZW
     return cudaGetLastError();
 }
 
 // =============================================================== statistics (K3), generic
 // One thread per output element, rows of a chunk in the inner loop.  Outputs are per-chunk partial
-// sums (deterministic two-stage reduction).
+// sums (deterministic two-stage reduction).  WT: every observed entry counts with its weight s_nd (S [N][lds]): T1, Bst, Ast,
+// cnt = sum s, colx = sum s x.
+template <bool WT>
 __global__ void __launch_bounds__(256)
 stats_generic_kernel(long long N, int D, int q, const double *__restrict__ X, long long ldx,
                      const double *__restrict__ Zbar, long long ldz, const double *__restrict__ M2,
-                     long long ldm, double *__restrict__ ws, long long rows_per_chunk) {
+                     long long ldm, double *__restrict__ ws, long long rows_per_chunk, const double *__restrict__ S,
+                     long long lds) {
     const StatLayout L(D, q);
     const int P = L.P;
     const int CT = P + 2 * q + 2;
@@ -216,33 +240,33 @@ stats_generic_kernel(long long N, int D, int q, const double *__restrict__ X, lo
             if (c < P) {
                 for (long long n = r0; n < r1; ++n) {
                     const double x = X[n * ldx + d];
-                    if (x == x) acc += M2[n * ldm + c];
+                    if (x == x) acc = WT ? fma(S[n * lds + d], M2[n * ldm + c], acc) : acc + M2[n * ldm + c];
                 }
                 dest = L.t1 + (size_t)d * P + c;
             } else if (c < P + q) {
                 const int i = c - P;
                 for (long long n = r0; n < r1; ++n) {
                     const double x = X[n * ldx + d];
-                    if (x == x) acc += Zbar[n * ldz + i];
+                    if (x == x) acc = WT ? fma(S[n * lds + d], Zbar[n * ldz + i], acc) : acc + Zbar[n * ldz + i];
                 }
                 dest = L.bst + (size_t)d * q + i;
             } else if (c < P + 2 * q) {
                 const int i = c - P - q;
                 for (long long n = r0; n < r1; ++n) {
                     const double x = X[n * ldx + d];
-                    if (x == x) acc = fma(x, Zbar[n * ldz + i], acc);
+                    if (x == x) acc = fma(WT ? S[n * lds + d] * x : x, Zbar[n * ldz + i], acc);
                 }
                 dest = L.ast + (size_t)d * q + i;
             } else if (c == P + 2 * q) {
                 for (long long n = r0; n < r1; ++n) {
                     const double x = X[n * ldx + d];
-                    if (x == x) acc += 1.0;
+                    if (x == x) acc += WT ? S[n * lds + d] : 1.0;
                 }
                 dest = L.cnt + d;
             } else {
                 for (long long n = r0; n < r1; ++n) {
                     const double x = X[n * ldx + d];
-                    if (x == x) acc += x;
+                    if (x == x) acc = WT ? fma(S[n * lds + d], x, acc) : acc + x;
                 }
                 dest = L.colx + d;
             }
@@ -269,23 +293,28 @@ int stats_generic_nchunks(long long N) {
 
 cudaError_t launch_stats_generic(long long N, int D, int q, const double *X, long long ldx, const double *Zbar,
                                  long long ldz, const double *M2, long long ldm, double *ws_main, int nchunks,
-                                 cudaStream_t st) {
+                                 cudaStream_t st, const double *S, long long lds) {
     const int P = tri(q);
     const long long nout = (long long)D * (P + 2 * q + 2) + P + q;
     long long bx = (nout + 255) / 256;
     if (bx > 4096) bx = 4096;
     const long long rpc = (N + nchunks - 1) / nchunks;
     dim3 grid((unsigned)bx, (unsigned)nchunks);
-    stats_generic_kernel<<<grid, 256, 0, st>>>(N, D, q, X, ldx, Zbar, ldz, M2, ldm, ws_main, rpc > 0 ? rpc : 1);
+    if (S)
+        stats_generic_kernel<true><<<grid, 256, 0, st>>>(N, D, q, X, ldx, Zbar, ldz, M2, ldm, ws_main, rpc > 0 ? rpc : 1, S, lds);
+    else
+        stats_generic_kernel<false><<<grid, 256, 0, st>>>(N, D, q, X, ldx, Zbar, ldz, M2, ldm, ws_main, rpc > 0 ? rpc : 1,
+                                                          nullptr, 0);
     return cudaGetLastError();
 }
 
 // =============================================================== column sums of the mask and of O.X
 // (the DMMA statistics kernel leaves cnt / colsumX to this HBM-bound pass)
-template <int ROWS>
+// WT: weighted sums, cnt = sum s, colsumX = sum s x (S [N][lds])
+template <int ROWS, bool WT>
 __global__ void __launch_bounds__(128)
 colsums2_kernel(long long N, int D, int q, const double *__restrict__ X, long long ldx, double *__restrict__ ws,
-                long long rows_per_chunk) {
+                long long rows_per_chunk, const double *__restrict__ S, long long lds) {
     const StatLayout L(D, q);
     const int d = blockIdx.x * blockDim.x + threadIdx.x;
     const long long r0 = (long long)blockIdx.y * rows_per_chunk;
@@ -301,16 +330,28 @@ colsums2_kernel(long long N, int D, int q, const double *__restrict__ X, long lo
         for (int u = 0; u < ROWS; ++u) {
             const double x = X[(n + u) * ldx + d];
             if (x == x) {
-                c[u] += 1.0;
-                s[u] += x;
+                if (WT) {
+                    const double w = S[(n + u) * lds + d];
+                    c[u] += w;
+                    s[u] = fma(w, x, s[u]);
+                } else {
+                    c[u] += 1.0;
+                    s[u] += x;
+                }
             }
         }
     }
     for (; n < r1; ++n) {
         const double x = X[n * ldx + d];
         if (x == x) {
-            c[0] += 1.0;
-            s[0] += x;
+            if (WT) {
+                const double w = S[n * lds + d];
+                c[0] += w;
+                s[0] = fma(w, x, s[0]);
+            } else {
+                c[0] += 1.0;
+                s[0] += x;
+            }
         }
     }
     double ct = 0.0, stot = 0.0;
@@ -325,11 +366,12 @@ colsums2_kernel(long long N, int D, int q, const double *__restrict__ X, long lo
 }
 
 cudaError_t launch_colsums(long long N, int D, int q, const double *X, long long ldx, double *ws_main, int nchunks,
-                           cudaStream_t st) {
+                           cudaStream_t st, const double *S, long long lds) {
     long long rpc = (N + nchunks - 1) / nchunks;
     if (rpc < 1) rpc = 1;
     dim3 grid((unsigned)((D + 127) / 128), (unsigned)nchunks);
-    colsums2_kernel<8><<<grid, 128, 0, st>>>(N, D, q, X, ldx, ws_main, rpc);
+    if (S) colsums2_kernel<8, true><<<grid, 128, 0, st>>>(N, D, q, X, ldx, ws_main, rpc, S, lds);
+    else colsums2_kernel<8, false><<<grid, 128, 0, st>>>(N, D, q, X, ldx, ws_main, rpc, nullptr, 0);
     return cudaGetLastError();
 }
 
@@ -374,10 +416,13 @@ cudaError_t launch_mzsums(long long N, int D, int q, const double *Zbar, long lo
 }
 
 // =============================================================== per-row scalars (K4)
+// WT (mode B): sxx = sum s x^2 over the observed entries, nE = the NUMBER of observed entries of positive weight
+template <bool WT>
 __global__ void __launch_bounds__(256)
 rowscalars_kernel(long long N, int D, const double *__restrict__ X, long long ldx, const double *__restrict__ V,
                   const double *__restrict__ Xorig, const double *__restrict__ qldX,
-                  const double *__restrict__ logdet, double *__restrict__ ws_sc, int skip_x) {
+                  const double *__restrict__ logdet, double *__restrict__ ws_sc, int skip_x, const double *__restrict__ S,
+                  long long lds) {
     __shared__ double sh[33];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
     double sxx = 0, sumv = 0, ne = 0, qz = 0, ldz = 0, latq = 0, nlat = 0, pnm = 0, plnv = 0, nrows = 0;
@@ -388,8 +433,14 @@ rowscalars_kernel(long long N, int D, const double *__restrict__ X, long long ld
         for (int d = lane; d < D && !skip_x; d += 32) {
             const double x = xr[d];
             if (x == x) {
-                sxx = fma(x, x, sxx);
-                ne += 1.0;
+                if (WT) {
+                    const double w = S[n * lds + d];
+                    sxx = fma(w * x, x, sxx);
+                    ne += (w > 0.0) ? 1.0 : 0.0;
+                } else {
+                    sxx = fma(x, x, sxx);
+                    ne += 1.0;
+                }
                 if (V) sumv += V[n * (long long)D + d];
             }
             if (Xorig) {
@@ -444,8 +495,9 @@ int rowscalars_nblk(long long N) {
 
 cudaError_t launch_rowscalars(long long N, int D, const double *X, long long ldx, const double *V,
                               const double *Xorig, const double *qldX, const double *logdet, double *ws_sc,
-                              int nblk, int skip_x, cudaStream_t st) {
-    rowscalars_kernel<<<nblk, 256, 0, st>>>(N, D, X, ldx, V, Xorig, qldX, logdet, ws_sc, skip_x);
+                              int nblk, int skip_x, cudaStream_t st, const double *S, long long lds) {
+    if (S) rowscalars_kernel<true><<<nblk, 256, 0, st>>>(N, D, X, ldx, V, Xorig, qldX, logdet, ws_sc, skip_x, S, lds);
+    else rowscalars_kernel<false><<<nblk, 256, 0, st>>>(N, D, X, ldx, V, Xorig, qldX, logdet, ws_sc, skip_x, nullptr, 0);
     return cudaGetLastError();
 }
 
@@ -677,8 +729,10 @@ __device__ __forceinline__ void gk_store_remote(const double *local_smem, uint32
 // nd (nullable): the per-dimension noise block (include/pyvb_b200.h).  With it, noise_diag_kernel (kernels_noise.cu) has already
 // done Mu, the per-dimension Gammas and their bound terms: this kernel skips its scalar Mu / Beta and the contraction, and adds
 // the per-dimension X and Beta terms in a fixed order (one CTA).
+// WT: weighted data (pyvb_global_w_f64): the X bound term also carries the data constant gl[PYVB_GL_LNS] = 1/2 sum ln s_nd.
 constexpr int GK_CLUSTER = 8;
 
+template <bool WT>
 __global__ void __launch_bounds__(1024)
 global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__restrict__ stats, const double *__restrict__ Wbar,
               const double *__restrict__ Wvar, double *mu, double *muvar, double *gl,
@@ -872,6 +926,7 @@ global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__res
             eB = (c.a0 - 1.0) * El - c.lgam_a0 + c.a0 * log(c.b0) - c.b0 * (qa / qb) -
                  ((qa - 1.0) * El - c.lgam_qa + qa * log(qb) - qa);
         }
+        if (WT) eX += gl[PYVB_GL_LNS];
         double eA = 0.0;
         if (c.ard) {
             for (int i = 0; i < q; ++i) {
@@ -897,7 +952,7 @@ global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__res
 
 cudaError_t launch_global(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar, const double *Wvar,
                           double *mu, double *muvar, double *gl, const double *P0, const double *h0,
-                          const pyvb_consts &c, double *elbo_out, const double *nd, cudaStream_t st) {
+                          const pyvb_consts &c, double *elbo_out, const double *nd, cudaStream_t st, bool weighted) {
     // one cluster; its size follows the work of the D x P contraction (small problems, or no contraction: one CTA)
     const long long work = nd ? 0 : (long long)D * q * (q + 1) / 2;
     const int cl = work >= (1LL << 17) ? GK_CLUSTER : work >= (1LL << 15) ? 2 : 1;
@@ -913,8 +968,8 @@ cudaError_t launch_global(int D, int q, int ops, int col_lo, int col_hi, const d
     at[0].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, global_kernel, D, q, ops, col_lo, col_hi, stats, Wbar, Wvar, mu, muvar, gl, P0, h0, c, elbo_out,
-                              nd);
+    return cudaLaunchKernelEx(&cfg, weighted ? global_kernel<true> : global_kernel<false>, D, q, ops, col_lo, col_hi, stats, Wbar,
+                              Wvar, mu, muvar, gl, P0, h0, c, elbo_out, nd);
 }
 
 // =============================================================== mode A imputation, warp per row

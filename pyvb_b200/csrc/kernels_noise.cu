@@ -8,6 +8,8 @@
 //          + cnt_d (mu_d^2 + muvar_d) + sum_p g_dp T1[d][p]        (the per-d slice of global_kernel's D x P contraction)
 //   Gamma  qb_d = b0_d + r_d / 2, tau_d = qa_d / qb_d                                          (DiagonalGamma.update)
 //   bound  eX_d = -cnt_d/2 ln 2pi + cnt_d/2 (ln qa_d - ln qb_d) - tau_d r_d / 2   (ln<tau> as the scalar path)
+// WT (per-entry observation weights): the statistics' cnt_d is the weight sum sum_n s_nd, which Mu and r_d read; the bound reads
+// the NUMBER of observed entries of column d from ncnt[d] instead.
 //          eB_d = the Gamma bound of entry d                                       (DiagonalGamma.log_lower_bound)
 // global_kernel then adds eX_d and eB_d over d in a fixed order.  No atomics: replicas on several GPUs stay bit-identical.
 #include "common.cuh"
@@ -17,10 +19,11 @@ namespace pyvb {
 
 constexpr int ND_WARPS = 8;
 
+template <bool WT>
 __global__ void __launch_bounds__(32 * ND_WARPS)
 noise_diag_kernel(int D, int q, int ops, const double *__restrict__ stats, const double *__restrict__ Wbar,
                   const double *__restrict__ Wvar, double *__restrict__ mu, double *__restrict__ muvar, double *__restrict__ nd,
-                  double alpha_mu) {
+                  double alpha_mu, const double *__restrict__ ncnt) {
     __shared__ unsigned short ijtab[PYVB_QMAX * (PYVB_QMAX + 1) / 2];   // packed index -> (i << 8) | j
     const StatLayout L(D, q);
     const int P = L.P;
@@ -79,16 +82,20 @@ noise_diag_kernel(int D, int q, int ops, const double *__restrict__ stats, const
     const double a0 = nd[(size_t)PYVB_ND_A0 * D + d], b0 = nd[(size_t)PYVB_ND_B0 * D + d];
     const double El = nd[(size_t)PYVB_ND_PSI_QA * D + d] - log(b);
     nd[(size_t)PYVB_ND_R * D + d] = r;
-    nd[(size_t)PYVB_ND_EX * D + d] = -0.5 * cnt * LN2PI + 0.5 * cnt * (log(qa) - log(b)) - 0.5 * t * r;
+    const double nobs = WT ? ncnt[d] : cnt;
+    nd[(size_t)PYVB_ND_EX * D + d] = -0.5 * nobs * LN2PI + 0.5 * nobs * (log(qa) - log(b)) - 0.5 * t * r;
     nd[(size_t)PYVB_ND_EB * D + d] = (a0 - 1.0) * El - nd[(size_t)PYVB_ND_LGAM_A0 * D + d] + a0 * log(b0) - b0 * t -
                                      ((qa - 1.0) * El - nd[(size_t)PYVB_ND_LGAM_QA * D + d] + qa * log(b) - qa);
 }
 
 cudaError_t launch_noise_diag(int D, int q, int ops, const double *stats, const double *Wbar, const double *Wvar, double *mu,
-                              double *muvar, double *nd, double alpha_mu, cudaStream_t st) {
+                              double *muvar, double *nd, double alpha_mu, cudaStream_t st, const double *ncnt) {
     if (!(ops & (PYVB_OP_MU | PYVB_OP_BETA | PYVB_OP_ELBO))) return cudaSuccess;
-    noise_diag_kernel<<<(D + ND_WARPS - 1) / ND_WARPS, 32 * ND_WARPS, 0, st>>>(D, q, ops, stats, Wbar, Wvar, mu, muvar, nd,
-                                                                               alpha_mu);
+    const unsigned blocks = (D + ND_WARPS - 1) / ND_WARPS;
+    if (ncnt)
+        noise_diag_kernel<true><<<blocks, 32 * ND_WARPS, 0, st>>>(D, q, ops, stats, Wbar, Wvar, mu, muvar, nd, alpha_mu, ncnt);
+    else
+        noise_diag_kernel<false><<<blocks, 32 * ND_WARPS, 0, st>>>(D, q, ops, stats, Wbar, Wvar, mu, muvar, nd, alpha_mu, nullptr);
     return cudaGetLastError();
 }
 

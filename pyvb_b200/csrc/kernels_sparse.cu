@@ -37,20 +37,22 @@ template <int Q> struct SpT {
 // acc  += the packed columns of the gathered rows, and on the vector columns:
 //   K3 = false (Z step):      acc  += (x - row[PP + Q]) * row      (row[PP + Q] is mu_d in a Gw row)
 //   K3 = true  (statistics):  acc  += row,  accx += x * row
-template <int Q, bool K3, typename IDX>
+// WT: every entry's row counts with the entry's weight wt[e] (an array in the order of val): acc += w row, the x terms times w
+template <int Q, bool K3, bool WT, typename IDX>
 __device__ __forceinline__ void gather_rows(const double *__restrict__ src, long long ld, const IDX *__restrict__ idx,
-                                            const double *__restrict__ val, long long e0, long long e1, int t0,
-                                            double2 (&acc)[SpT<Q>::NT], double2 (&accx)[SpT<Q>::NX]) {
+                                            const double *__restrict__ val, const double *__restrict__ wt, long long e0,
+                                            long long e1, int t0, double2 (&acc)[SpT<Q>::NT], double2 (&accx)[SpT<Q>::NX]) {
     using T = SpT<Q>;
     for (long long e = e0; e < e1; e += T::U) {
         long long r[T::U];
-        double x[T::U], m[T::U];
+        double x[T::U], m[T::U], w[T::U];
         double2 v[T::U][T::NT];
 #pragma unroll
         for (int u = 0; u < T::U; ++u) {
             const bool ok = e + u < e1;
             r[u] = ok ? (long long)__ldg(idx + e + u) : -1;
             x[u] = ok ? __ldg(val + e + u) : 0.0;
+            w[u] = (WT && ok) ? __ldg(wt + e + u) : 1.0;
         }
 #pragma unroll
         for (int u = 0; u < T::U; ++u) {
@@ -67,18 +69,28 @@ __device__ __forceinline__ void gather_rows(const double *__restrict__ src, long
 #pragma unroll
         for (int u = 0; u < T::U; ++u) {
             if (r[u] < 0) continue;
-            const double xm = K3 ? x[u] : x[u] - m[u];
+            const double xm = WT ? w[u] * (K3 ? x[u] : x[u] - m[u]) : (K3 ? x[u] : x[u] - m[u]);
 #pragma unroll
             for (int t = 0; t < T::NT; ++t) {
                 const int k = t0 + t * T::G;
                 if (k >= T::NPAIR) continue;
                 if (2 * k < T::P) {
-                    acc[t].x += v[u][t].x;
-                    acc[t].y += v[u][t].y;
-                } else if (2 * k >= T::PP) {
-                    if (K3) {
+                    if (WT) {
+                        acc[t].x = fma(w[u], v[u][t].x, acc[t].x);
+                        acc[t].y = fma(w[u], v[u][t].y, acc[t].y);
+                    } else {
                         acc[t].x += v[u][t].x;
                         acc[t].y += v[u][t].y;
+                    }
+                } else if (2 * k >= T::PP) {
+                    if (K3) {
+                        if (WT) {
+                            acc[t].x = fma(w[u], v[u][t].x, acc[t].x);
+                            acc[t].y = fma(w[u], v[u][t].y, acc[t].y);
+                        } else {
+                            acc[t].x += v[u][t].x;
+                            acc[t].y += v[u][t].y;
+                        }
                         if (t >= T::TX) {
                             accx[t - T::TX].x = fma(xm, v[u][t].x, accx[t - T::TX].x);
                             accx[t - T::TX].y = fma(xm, v[u][t].y, accx[t - T::TX].y);
@@ -95,11 +107,13 @@ __device__ __forceinline__ void gather_rows(const double *__restrict__ src, long
 
 // ------------------------------------------------------------------ K1-csr: one group per row
 // indptr: the rows' own offsets into indices / values (indptr[0] need not be 0: a row range is a pointer offset)
-template <int Q>
+// WT: weights [nnz] in the order of values
+template <int Q, bool WT>
 __global__ void __launch_bounds__(SP_THREADS, SpT<Q>::MINB)
 zstep_csr_kernel(long long N, const long long *__restrict__ indptr, const int *__restrict__ indices,
                  const double *__restrict__ values, const double *__restrict__ Gw, int ldg, const double *__restrict__ P0,
-                 const double *__restrict__ h0, const double *__restrict__ gl, double *__restrict__ MZ, int ldmz) {
+                 const double *__restrict__ h0, const double *__restrict__ gl, double *__restrict__ MZ, int ldmz,
+                 const double *__restrict__ weights) {
     using T = SpT<Q>;
     __shared__ double prior[T::PP + Q];                  // [P0 packed | 0 | h0]: the row of an empty observation set
     for (int c = threadIdx.x; c < T::PP + Q; c += blockDim.x) {
@@ -121,7 +135,7 @@ zstep_csr_kernel(long long N, const long long *__restrict__ indptr, const int *_
     double2 acc[T::NT], accx[T::NX];
 #pragma unroll
     for (int t = 0; t < T::NT; ++t) acc[t] = make_double2(0.0, 0.0);
-    gather_rows<Q, false>(Gw, ldg, indices, values, indptr[n], indptr[n + 1], t0, acc, accx);
+    gather_rows<Q, false, WT>(Gw, ldg, indices, values, weights, indptr[n], indptr[n + 1], t0, acc, accx);
     double2 *out = reinterpret_cast<double2 *>(MZ + n * ldmz);
 #pragma unroll
     for (int t = 0; t < T::NT; ++t) {
@@ -133,12 +147,12 @@ zstep_csr_kernel(long long N, const long long *__restrict__ indptr, const int *_
 
 // ------------------------------------------------------------------ K3-csc: one group per (row block, column)
 // colptr [nblk * D + 1]: entries of item b * D + d are [colptr[b * D + d], colptr[b * D + d + 1]) of rows / vals, the rows
-// in increasing order; rows are row indices of the shard (MZ row r at MZ + r * ldmz)
-template <int Q>
+// in increasing order; rows are row indices of the shard (MZ row r at MZ + r * ldmz).  WT: weights in the order of vals
+template <int Q, bool WT>
 __global__ void __launch_bounds__(SP_THREADS, SpT<Q>::MINB)
 stats_csc_kernel(long long nitems, int D, const long long *__restrict__ colptr, const int *__restrict__ rows,
                  const double *__restrict__ vals, const double *__restrict__ MZ, int ldmz, double *__restrict__ ws,
-                 size_t statlen) {
+                 size_t statlen, const double *__restrict__ wts) {
     using T = SpT<Q>;
     const long long item = (long long)blockIdx.x * (SP_THREADS / T::G) + threadIdx.x / T::G;
     if (item >= nitems) return;
@@ -150,7 +164,7 @@ stats_csc_kernel(long long nitems, int D, const long long *__restrict__ colptr, 
     for (int t = 0; t < T::NT; ++t) acc[t] = make_double2(0.0, 0.0);
 #pragma unroll
     for (int t = 0; t < T::NX; ++t) accx[t] = make_double2(0.0, 0.0);
-    gather_rows<Q, true>(MZ, ldmz, rows, vals, colptr[item], colptr[item + 1], t0, acc, accx);
+    gather_rows<Q, true, WT>(MZ, ldmz, rows, vals, wts, colptr[item], colptr[item + 1], t0, acc, accx);
     const StatLayout L(D, Q);
     double *out = ws + (size_t)b * statlen;
 #pragma unroll
@@ -202,45 +216,54 @@ long long csr_block_rows(long long N, int D, int q) {
 template <int Q>
 static cudaError_t launch_zstep_csr_q(long long N, const long long *indptr, const int *indices, const double *values,
                                       const double *Gw, int ldg, const double *P0, const double *h0, const double *gl,
-                                      double *MZ, int ldmz, cudaStream_t st) {
+                                      double *MZ, int ldmz, cudaStream_t st, const double *weights) {
     constexpr int GPB = SP_THREADS / SpT<Q>::G;
     const long long blocks = (N + GPB - 1) / GPB;
-    zstep_csr_kernel<Q><<<(unsigned)blocks, SP_THREADS, 0, st>>>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, ldmz);
+    if (weights)
+        zstep_csr_kernel<Q, true><<<(unsigned)blocks, SP_THREADS, 0, st>>>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ,
+                                                                            ldmz, weights);
+    else
+        zstep_csr_kernel<Q, false><<<(unsigned)blocks, SP_THREADS, 0, st>>>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ,
+                                                                             ldmz, nullptr);
     return cudaGetLastError();
 }
 
 cudaError_t launch_zstep_csr(long long N, int q, const long long *indptr, const int *indices, const double *values,
                              const double *Gw, int ldg, const double *P0, const double *h0, const double *gl, double *MZ,
-                             int ldmz, cudaStream_t st) {
+                             int ldmz, cudaStream_t st, const double *weights) {
     if (N <= 0) return cudaSuccess;
     switch (q) {
-        case 8: return launch_zstep_csr_q<8>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, ldmz, st);
-        case 16: return launch_zstep_csr_q<16>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, ldmz, st);
-        case 32: return launch_zstep_csr_q<32>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, ldmz, st);
-        case 64: return launch_zstep_csr_q<64>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, ldmz, st);
+        case 8: return launch_zstep_csr_q<8>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, ldmz, st, weights);
+        case 16: return launch_zstep_csr_q<16>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, ldmz, st, weights);
+        case 32: return launch_zstep_csr_q<32>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, ldmz, st, weights);
+        case 64: return launch_zstep_csr_q<64>(N, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, ldmz, st, weights);
     }
     return cudaErrorNotSupported;
 }
 
 template <int Q>
 static cudaError_t launch_stats_csc_q(int D, int nblk, const long long *colptr, const int *rows, const double *vals,
-                                      const double *MZ, int ldmz, double *ws_main, cudaStream_t st) {
+                                      const double *MZ, int ldmz, double *ws_main, cudaStream_t st, const double *wts) {
     constexpr int GPB = SP_THREADS / SpT<Q>::G;
     const long long nitems = (long long)nblk * D;
     const long long blocks = (nitems + GPB - 1) / GPB;
-    stats_csc_kernel<Q><<<(unsigned)blocks, SP_THREADS, 0, st>>>(nitems, D, colptr, rows, vals, MZ, ldmz, ws_main,
-                                                                  StatLayout(D, Q).len);
+    if (wts)
+        stats_csc_kernel<Q, true><<<(unsigned)blocks, SP_THREADS, 0, st>>>(nitems, D, colptr, rows, vals, MZ, ldmz, ws_main,
+                                                                            StatLayout(D, Q).len, wts);
+    else
+        stats_csc_kernel<Q, false><<<(unsigned)blocks, SP_THREADS, 0, st>>>(nitems, D, colptr, rows, vals, MZ, ldmz, ws_main,
+                                                                             StatLayout(D, Q).len, nullptr);
     return cudaGetLastError();
 }
 
 cudaError_t launch_stats_csc(int D, int q, int nblk, const long long *colptr, const int *rows, const double *vals,
-                             const double *MZ, int ldmz, double *ws_main, cudaStream_t st) {
+                             const double *MZ, int ldmz, double *ws_main, cudaStream_t st, const double *wts) {
     if (nblk <= 0) return cudaSuccess;
     switch (q) {
-        case 8: return launch_stats_csc_q<8>(D, nblk, colptr, rows, vals, MZ, ldmz, ws_main, st);
-        case 16: return launch_stats_csc_q<16>(D, nblk, colptr, rows, vals, MZ, ldmz, ws_main, st);
-        case 32: return launch_stats_csc_q<32>(D, nblk, colptr, rows, vals, MZ, ldmz, ws_main, st);
-        case 64: return launch_stats_csc_q<64>(D, nblk, colptr, rows, vals, MZ, ldmz, ws_main, st);
+        case 8: return launch_stats_csc_q<8>(D, nblk, colptr, rows, vals, MZ, ldmz, ws_main, st, wts);
+        case 16: return launch_stats_csc_q<16>(D, nblk, colptr, rows, vals, MZ, ldmz, ws_main, st, wts);
+        case 32: return launch_stats_csc_q<32>(D, nblk, colptr, rows, vals, MZ, ldmz, ws_main, st, wts);
+        case 64: return launch_stats_csc_q<64>(D, nblk, colptr, rows, vals, MZ, ldmz, ws_main, st, wts);
     }
     return cudaErrorNotSupported;
 }

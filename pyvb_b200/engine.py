@@ -31,7 +31,7 @@ from .dist import PeerExchange, allreduce_stats
 import functools
 
 from ._layout import (ALGO_AUTO, ALGO_DMMA, ALGO_F32, ALGO_GENERIC, GL_ALPHA, GL_ALQB, GL_ELBO, GL_I8BAD, GL_I8FALL, GL_LEN,
-                      GL_NONPD, GL_QA, GL_QB, GL_TAU, OP_ALPHA, OP_BETA, OP_ELBO, OP_MU, QMAX, StatLayout)
+                      GL_LNS, GL_NONPD, GL_QA, GL_QB, GL_TAU, OP_ALPHA, OP_BETA, OP_ELBO, OP_MU, QMAX, StatLayout)
 
 _ALGOS = {"auto": ALGO_AUTO, "generic": ALGO_GENERIC, "dmma": ALGO_DMMA}
 
@@ -75,11 +75,18 @@ class PlateEngine(object):
     noise : "scalar" -- one noise precision tau shared by every data dimension (Gamma(a0, b0)) -- or "diagonal" -- factor
         analysis: x_nd ~ N(w_d z_n + mu_d, 1 / tau_d) with one Gamma(a0_d, b0_d) posterior per data dimension (DiagonalGamma);
         a0 and b0 may then be scalars or length-D arrays.  "diagonal" runs on every FP64 mode-B path (dense and sparse).
+    weights : known per-entry observation weights s_nd >= 0 (inverse variances, repeat counts, confidences):
+        x_nd ~ N(w_d z_n + mu_d, 1 / (tau s_nd)) (1 / (tau_d s_nd) with noise "diagonal").  An entry with s_nd = 0 is missing,
+        as a NaN is; a NaN x_nd is missing whatever its weight.  Dense X: an (N, D) array or tensor; sparse X: a sparse matrix
+        or tensor storing exactly the entries X stores.  Mode "B", precision "f64", the DMMA, generic and sparse paths
+        ("auto" picks DMMA where the shape allows it, else generic; "i8" is refused: its mask contraction is exact only for
+        0/1 weights).  None (the default): every observed entry has weight 1, the unweighted model.
     """
 
     def __init__(self, X, q, mode="B", alpha0=1e-3, alpha_mu=1e-3, a0=1e-3, b0=1e-3, ard=False,
                  ard_a0=1e-3, ard_b0=1e-3, P0=None, m0=None, device=None, algo="auto",
-                 keep_sigma=True, distributed=False, row_offset=0, trace_len=4096, precision="f64", noise="scalar"):
+                 keep_sigma=True, distributed=False, row_offset=0, trace_len=4096, precision="f64", noise="scalar",
+                 weights=None):
         if not torch.cuda.is_available():
             raise RuntimeError("pyvb_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         self.lib = _cabi.lib()
@@ -92,15 +99,18 @@ class PlateEngine(object):
         self.diag = (noise == "diagonal")
         if self.diag and (mode != "B" or self.f32):
             raise ValueError("noise='diagonal' needs mode='B' and precision='f64'")
+        self.weighted = weights is not None
+        if self.weighted and (mode != "B" or self.f32 or algo == "i8"):
+            raise ValueError("weights need mode='B', precision='f64' and algo 'auto', 'dmma' or 'generic'")
         self.device = torch.device(device if device is not None else "cuda:%d" % torch.cuda.current_device())
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
         with torch.cuda.device(self.device):
             self._construct(X, q, mode, alpha0, alpha_mu, a0, b0, ard, ard_a0, ard_b0, P0, m0, algo, keep_sigma,
-                            distributed, row_offset, trace_len)
+                            distributed, row_offset, trace_len, weights)
 
     def _construct(self, X, q, mode, alpha0, alpha_mu, a0, b0, ard, ard_a0, ard_b0, P0, m0, algo, keep_sigma,
-                   distributed, row_offset, trace_len):
+                   distributed, row_offset, trace_len, weights):
         self.mode, self.q, self.ard = mode, int(q), bool(ard)
         self.sparse = _sparse.is_sparse(X)
         if self.sparse:
@@ -117,7 +127,7 @@ class PlateEngine(object):
         self.use_i8 = (algo == "i8")
         if algo == "i8":
             algo = "dmma"
-        elif algo == "auto" and mode == "B" and not self.f32:
+        elif algo == "auto" and mode == "B" and not self.f32 and not self.weighted:
             self.use_i8 = None                                  # decided below, once D is known
         self.algo = _ALGOS[algo] if isinstance(algo, str) else int(algo)
         self.distributed = bool(distributed)
@@ -133,6 +143,49 @@ class PlateEngine(object):
             Xt = Xt.to(device=dev, dtype=f64).contiguous()
             self.N, self.D = int(Xt.shape[0]), int(Xt.shape[1])
         N, D = self.N, self.D
+        # ---- per-entry weights: S (dense, zero where x is missing) or the CSR-ordered `wcsr`; the NUMBER of observed entries of
+        # positive weight (per column `ncnt`: the per-dimension Gammas) and 1/2 sum ln s, both constants of the data set
+        self.S = self.wcsr = self.ncnt = None
+        self.lns = 0.0
+        if self.weighted:
+            if self.sparse:
+                self.wcsr = _sparse.weights_csr(weights, self.csr)
+                pos = self.wcsr > 0
+                ncnt = torch.bincount(self.csr.indices.to(torch.int64)[pos], minlength=D).to(f64)
+                lns = torch.log(self.wcsr[pos]).sum()
+                del pos
+            else:
+                if _sparse.is_sparse(weights):
+                    raise ValueError("weights of dense X must be a dense (N, D) array")
+                W = torch.as_tensor(weights)
+                if tuple(W.shape) != (N, D):
+                    raise ValueError("weights must have the shape of X, %s; got %s" % ((N, D), tuple(W.shape)))
+                # row chunks: the checks and the constants need no N x D temporaries
+                self.S = torch.empty(N, D, dtype=f64, device=dev)
+                ncnt, lns = torch.zeros(D, dtype=f64, device=dev), torch.zeros((), dtype=f64, device=dev)
+                zero, one = torch.zeros((), dtype=f64, device=dev), torch.ones((), dtype=f64, device=dev)
+                for lo in range(0, N, 1 << 16):
+                    w = W[lo:lo + (1 << 16)].to(device=dev, dtype=f64)
+                    o = ~torch.isnan(Xt[lo:lo + (1 << 16)])
+                    if not bool(torch.where(o, torch.isfinite(w), True).all()):
+                        raise ValueError("weights must be finite on the observed entries")
+                    if bool((o & (w < 0)).any()):
+                        raise ValueError("weights must be >= 0 on the observed entries")
+                    s = torch.where(o, w, zero)
+                    self.S[lo:lo + (1 << 16)] = s
+                    pos = s > 0
+                    ncnt += pos.sum(0).to(f64)
+                    lns += torch.log(torch.where(pos, s, one)).sum()
+                    del w, o, s, pos
+                del W
+            n_pos_local = int(ncnt.sum().item())        # the observations of positive weight
+            lns = 0.5 * float(lns.item())
+            if self.distributed:
+                import torch.distributed as dist
+                both = torch.cat([ncnt, torch.tensor([lns], dtype=f64, device=dev)])
+                dist.all_reduce(both)
+                ncnt, lns = both[:D].contiguous(), float(both[D].item())
+            self.ncnt, self.lns = ncnt, lns
         self.P = q * (q + 1) // 2
         self.L = StatLayout(D, q)
         self.alpha0, self.alpha_mu = float(alpha0), float(alpha_mu)
@@ -146,26 +199,33 @@ class PlateEngine(object):
         if self.diag:
             # the data constants of the per-dimension Gammas: observed count and sum of squares of every column
             if self.sparse:
-                cnt_d, _, sxx_d = (torch.as_tensor(a, dtype=f64, device=dev) for a in _sparse.column_sums(self.csr))
+                cnt_d, _, sxx_d = (torch.as_tensor(a, dtype=f64, device=dev)
+                                   for a in _sparse.column_sums(self.csr, self.wcsr))
             else:
+                # (with weights: sum s x^2; the counts of qa_d are ncnt)
                 cnt_d, sxx_d = torch.zeros(D, dtype=f64, device=dev), torch.zeros(D, dtype=f64, device=dev)
                 for lo in range(0, N, 1 << 16):
                     x = Xt[lo:lo + (1 << 16)]
                     o = ~torch.isnan(x)
                     cnt_d += o.sum(0).to(f64)
-                    sxx_d += torch.where(o, x * x, torch.zeros((), dtype=f64, device=dev)).sum(0)
-                    del x, o
+                    xx = x * x if self.S is None else self.S[lo:lo + (1 << 16)] * x * x
+                    sxx_d += torch.where(o, xx, torch.zeros((), dtype=f64, device=dev)).sum(0)
+                    del x, o, xx
             if self.distributed:
                 import torch.distributed as dist
                 both = torch.cat([cnt_d, sxx_d])
                 dist.all_reduce(both)
                 cnt_d, sxx_d = both[:D], both[D:]
+            if self.weighted:
+                cnt_d = self.ncnt                 # qa_d counts the observations; the weight sums enter through the statistics
         obs = None if self.sparse else ~torch.isnan(Xt)
         n_obs_local = int(self.csr.values.numel()) if self.sparse else int(obs.sum().item())
+        if self.weighted:
+            n_obs_local = n_pos_local
         if self.sparse:
             # the statistics read the entries column-major per row block (K3-csc); the X-only sums are taken once, here
-            self.csc = _sparse.block_csc(self.csr, int(self.lib.pyvb_csr_block_rows(N, D, q)))
-            self.xcache_sparse = _sparse.x_cache(self.csr).to(dev)
+            self.csc = _sparse.block_csc(self.csr, int(self.lib.pyvb_csr_block_rows(N, D, q)), self.wcsr)
+            self.xcache_sparse = _sparse.x_cache(self.csr, self.wcsr).to(dev)
             self.Xorig, self.X, self.V, self.qldX = None, None, None, None
             n_eff_local = n_obs_local
         elif self.f32:
@@ -394,6 +454,7 @@ class PlateEngine(object):
             self._resplit()
         gl = self.gl.cpu()
         gl[GL_NONPD] = 0.0                      # a fresh state: earlier non-PD rows are history
+        gl[GL_LNS] = self.lns                   # (read by the weighted bound only)
         if self.diag:
             # tau_d travels in the Gw rows and the W update reads it from nd: the shared tau stays 1
             gl[GL_QA] = gl[GL_QB] = gl[GL_TAU] = 1.0
@@ -476,6 +537,8 @@ class PlateEngine(object):
         if self.diag:
             raise NotImplementedError("set_X: with noise='diagonal' the column sums of squares are constants of the data set; "
                                       "build a new engine for new data")
+        if self.weighted:
+            raise NotImplementedError("set_X: the weights belong to the data set; build a new engine for new data")
         assert self.mode == "B" and not self.f32
         self.X.copy_(X, non_blocking=True)
         self._xcache_valid = False
@@ -583,14 +646,14 @@ class PlateEngine(object):
             return
         if self.sparse:
             c = self.csc
-            rc = self.lib.pyvb_stats_csr_f64(self.N, self.D, self.q, c.nblk, c.colptr.data_ptr(), c.rows.data_ptr(),
-                                             c.vals.data_ptr(), self.MZ.data_ptr(), self.ldmz, self.logdet.data_ptr(),
-                                             self.stats.data_ptr(), self.ws.data_ptr(), self.ws_bytes,
-                                             self.xcache.data_ptr(),
-                                             self.zsums.data_ptr() if (self.zsums is not None and self._zsums_valid) else 0,
-                                             self.peers.next() if (self.peers is not None and self.distributed) else None,
-                                             self._stream())
-            _cabi.check(rc, "pyvb_stats_csr_f64")
+            rc = self.lib.pyvb_stats_csr_w_f64(self.N, self.D, self.q, c.nblk, c.colptr.data_ptr(), c.rows.data_ptr(),
+                                               c.vals.data_ptr(), self._p(c.wts), self.MZ.data_ptr(), self.ldmz,
+                                               self.logdet.data_ptr(), self.stats.data_ptr(), self.ws.data_ptr(),
+                                               self.ws_bytes, self.xcache.data_ptr(),
+                                               self.zsums.data_ptr() if (self.zsums is not None and self._zsums_valid) else 0,
+                                               self.peers.next() if (self.peers is not None and self.distributed) else None,
+                                               self._stream())
+            _cabi.check(rc, "pyvb_stats_csr_w_f64")
             if self.distributed and self.peers is None:
                 allreduce_stats(self.stats)
             self._stats_fresh = True
@@ -629,14 +692,24 @@ class PlateEngine(object):
                 allreduce_stats(self.stats)
             self._stats_fresh = True
             return
-        rc = self.lib.pyvb_stats_f64(self.N, self.D, self.q, self.X.data_ptr(), self.D, self._p(self.V),
-                                     self._p(self.Xorig), self._p(self.qldX), self.Zbar.data_ptr(), self.ldmz,
-                                     self.M2.data_ptr(), self.ldmz, self.logdet.data_ptr(), self.stats.data_ptr(),
-                                     self.ws.data_ptr(), self.ws_bytes, self._p(self.xcache),
-                                     int(self._xcache_valid), self._p(self.zsums), int(self._zsums_valid),
-                                     self.peers.next() if (self.peers is not None and self.distributed) else None,
-                                     self.algo, self._stream())
-        _cabi.check(rc, "pyvb_stats_f64")
+        if self.weighted:
+            rc = self.lib.pyvb_stats_w_f64(self.N, self.D, self.q, self.X.data_ptr(), self.D, self.S.data_ptr(), self.D,
+                                           self.Zbar.data_ptr(), self.ldmz, self.M2.data_ptr(), self.ldmz,
+                                           self.logdet.data_ptr(), self.stats.data_ptr(), self.ws.data_ptr(), self.ws_bytes,
+                                           self.xcache.data_ptr(), int(self._xcache_valid), self._p(self.zsums),
+                                           int(self._zsums_valid),
+                                           self.peers.next() if (self.peers is not None and self.distributed) else None,
+                                           self.algo, self._stream())
+            _cabi.check(rc, "pyvb_stats_w_f64")
+        else:
+            rc = self.lib.pyvb_stats_f64(self.N, self.D, self.q, self.X.data_ptr(), self.D, self._p(self.V),
+                                         self._p(self.Xorig), self._p(self.qldX), self.Zbar.data_ptr(), self.ldmz,
+                                         self.M2.data_ptr(), self.ldmz, self.logdet.data_ptr(), self.stats.data_ptr(),
+                                         self.ws.data_ptr(), self.ws_bytes, self._p(self.xcache),
+                                         int(self._xcache_valid), self._p(self.zsums), int(self._zsums_valid),
+                                         self.peers.next() if (self.peers is not None and self.distributed) else None,
+                                         self.algo, self._stream())
+            _cabi.check(rc, "pyvb_stats_f64")
         self._xcache_valid = self.xcache is not None
         if self.distributed and self.peers is None:
             allreduce_stats(self.stats)          # fallback exchange: NCCL all-reduce
@@ -672,13 +745,13 @@ class PlateEngine(object):
             # any row range: K1-csr owns whole rows, so [lo, hi) is a pointer offset into the row offsets
             full = (lo == 0 and hi == self.N and self.zsums is not None)
             self._zsums_valid = False
-            rc = self.lib.pyvb_zstep_csr_f64(hi - lo, D, q, self.csr.indptr.data_ptr() + lo * 8,
-                                             self.csr.indices.data_ptr(), self.csr.values.data_ptr(), self.Gw.data_ptr(),
-                                             self.ldg, self.P0.data_ptr(), self.h0.data_ptr(), self.gl.data_ptr(),
-                                             self.MZ.data_ptr() + lo * self.ldmz * 8, self.ldmz, sig,
-                                             self.logdet.data_ptr() + lo * 8, self.zsums.data_ptr() if full else 0,
-                                             self._stream())
-            _cabi.check(rc, "pyvb_zstep_csr_f64")
+            rc = self.lib.pyvb_zstep_csr_w_f64(hi - lo, D, q, self.csr.indptr.data_ptr() + lo * 8,
+                                               self.csr.indices.data_ptr(), self.csr.values.data_ptr(), self._p(self.wcsr),
+                                               self.Gw.data_ptr(), self.ldg, self.P0.data_ptr(), self.h0.data_ptr(),
+                                               self.gl.data_ptr(), self.MZ.data_ptr() + lo * self.ldmz * 8, self.ldmz, sig,
+                                               self.logdet.data_ptr() + lo * 8, self.zsums.data_ptr() if full else 0,
+                                               self._stream())
+            _cabi.check(rc, "pyvb_zstep_csr_w_f64")
             self._zsums_valid = full
             return
         if self.f32:
@@ -713,12 +786,20 @@ class PlateEngine(object):
             _cabi.check(rc, "pyvb_zstep_i8_f64")
             self._zsums_valid = full
             return
-        rc = self.lib.pyvb_zstep_f64(hi - lo, D, q, self.X.data_ptr() + lo * D * 8, D, self.Gw.data_ptr(),
-                                     self.ldg, self.P0.data_ptr(), self.h0.data_ptr(), self.gl.data_ptr(),
-                                     self.Zbar.data_ptr() + lo * self.ldmz * 8, self.ldmz,
-                                     self.M2.data_ptr() + lo * self.ldmz * 8, self.ldmz, sig,
-                                     self.logdet.data_ptr() + lo * 8, zs, self.algo, self._stream())
-        _cabi.check(rc, "pyvb_zstep_f64")
+        if self.weighted:
+            rc = self.lib.pyvb_zstep_w_f64(hi - lo, D, q, self.X.data_ptr() + lo * D * 8, D, self.S.data_ptr() + lo * D * 8,
+                                           D, self.Gw.data_ptr(), self.ldg, self.P0.data_ptr(), self.h0.data_ptr(),
+                                           self.gl.data_ptr(), self.Zbar.data_ptr() + lo * self.ldmz * 8, self.ldmz,
+                                           self.M2.data_ptr() + lo * self.ldmz * 8, self.ldmz, sig,
+                                           self.logdet.data_ptr() + lo * 8, zs, self.algo, self._stream())
+            _cabi.check(rc, "pyvb_zstep_w_f64")
+        else:
+            rc = self.lib.pyvb_zstep_f64(hi - lo, D, q, self.X.data_ptr() + lo * D * 8, D, self.Gw.data_ptr(),
+                                         self.ldg, self.P0.data_ptr(), self.h0.data_ptr(), self.gl.data_ptr(),
+                                         self.Zbar.data_ptr() + lo * self.ldmz * 8, self.ldmz,
+                                         self.M2.data_ptr() + lo * self.ldmz * 8, self.ldmz, sig,
+                                         self.logdet.data_ptr() + lo * 8, zs, self.algo, self._stream())
+            _cabi.check(rc, "pyvb_zstep_f64")
         self._zsums_valid = full
         self._stats_fresh = False
 
@@ -744,6 +825,15 @@ class PlateEngine(object):
     def _global(self, ops, elbo_out=0, col_lo=0, col_hi=None):
         self._ensure_stats()
         col_hi = self.q if col_hi is None else col_hi
+        if self.weighted:
+            rc = self.lib.pyvb_global_w_f64(self.D, self.q, ops, col_lo, col_hi, self.stats.data_ptr(), self.Wbar.data_ptr(),
+                                            self.Wvar.data_ptr(), self.mu.data_ptr(), self.muvar.data_ptr(),
+                                            self.gl.data_ptr(), self._p(self.nd), self._p(self.ncnt), self.P0.data_ptr(),
+                                            self.h0.data_ptr(), _cabi.ctypes.byref(self.consts), elbo_out, self._stream())
+            _cabi.check(rc, "pyvb_global_w_f64")
+            if ops & (OP_MU | (OP_BETA if self.diag else 0)):   # mu_d (and tau_d) live in the Gw rows
+                self._gw_fresh = False
+            return
         if self.diag:
             rc = self.lib.pyvb_global_nd_f64(self.D, self.q, ops, col_lo, col_hi, self.stats.data_ptr(), self.Wbar.data_ptr(),
                                              self.Wvar.data_ptr(), self.mu.data_ptr(), self.muvar.data_ptr(),
@@ -817,6 +907,8 @@ class PlateEngine(object):
         if self.diag:
             raise NotImplementedError("iterate_from_host: with noise='diagonal' the column sums of squares are constants of "
                                       "the resident data set")
+        if self.weighted:
+            raise NotImplementedError("iterate_from_host: the weights are constants of the resident data set")
         assert self.mode == "B"
         assert not self.f32, "iterate_from_host: the FP32 variant keeps X as bf16 planes; use precision='f64'"
         N = self.N

@@ -8,6 +8,10 @@ stored is missing.  This module turns scipy.sparse matrices / arrays (any format
     CSC       `rows_per_block` consecutive rows, blocks one after the other                     (the statistics, K3-csc)
     xcache    float64 [cnt (D) | colsumX (D) | sum x^2 | number of stored entries]              (stats_reduce's X-only sums)
 
+Per-entry observation weights (PlateEngine(..., weights=...)) travel with the values: one float64 per stored entry, in CSR order
+and through the same permutation into the blocked CSC (`wts`); the X-only sums then become [sum s | sum s x | sum s x^2 | number
+of entries with s > 0].
+
 (include/pyvb_b200.h, "sparse observations").  Everything here is construction-time plumbing on torch / numpy: it runs
 without a GPU (on the CPU, or on the device where the input already lives) and is not on the per-sweep path.
 """
@@ -18,7 +22,7 @@ import numpy as np
 import torch
 
 CSR = collections.namedtuple("CSR", "indptr indices values N D")
-BlockedCSC = collections.namedtuple("BlockedCSC", "colptr rows vals nblk rows_per_block")
+BlockedCSC = collections.namedtuple("BlockedCSC", "colptr rows vals nblk rows_per_block wts", defaults=(None,))
 
 
 def is_sparse(X):
@@ -96,18 +100,39 @@ def to_csr(X, device=None):
     return CSR(indptr.contiguous(), col.to(torch.int32).contiguous(), val.contiguous(), N, D)
 
 
-def block_csc(csr, rows_per_block):
+def weights_csr(W, csr):
+    """The per-entry weights of the sparse observations `csr` as a float64 array in CSR order.  W: a sparse matrix / tensor
+    (any format to_csr accepts) whose stored pattern is exactly that of the observations.  Raises ValueError for a different
+    shape or pattern and for a negative or non-finite weight."""
+    if not is_sparse(W):
+        raise ValueError("weights of sparse observations must be a sparse matrix with the observations' stored pattern")
+    row, col, val, N, D = _coo_of(W, csr.indptr.device)
+    if (N, D) != (csr.N, csr.D):
+        raise ValueError("weights have shape %s, the observations %s" % ((N, D), (csr.N, csr.D)))
+    if val.numel() and not bool(torch.isfinite(val).all()):
+        raise ValueError("weights must be finite on the observed entries")
+    w = to_csr(W, device=csr.indptr.device)
+    if not (torch.equal(w.indptr, csr.indptr) and torch.equal(w.indices, csr.indices)):
+        raise ValueError("weights must store exactly the entries the observations store (same sparse pattern)")
+    if w.values.numel() and bool((w.values < 0).any()):
+        raise ValueError("weights must be >= 0 on the observed entries")
+    return w.values
+
+
+def block_csc(csr, rows_per_block, weights=None):
     """The row-blocked column-major copy of `csr`: rows cut into blocks of `rows_per_block` (the last may hold fewer);
-    within block b the entries of column d are colptr[b*D + d] .. colptr[b*D + d + 1], rows increasing."""
+    within block b the entries of column d are colptr[b*D + d] .. colptr[b*D + d + 1], rows increasing.  weights (optional,
+    CSR order): carried through the same permutation into `wts`."""
     N, D = csr.N, csr.D
     R = max(1, int(rows_per_block))
     nblk = max(1, (N + R - 1) // R)
     dev = csr.indptr.device
     nnz = int(csr.values.numel())
     if nnz == 0:
+        empty = torch.zeros(0, dtype=torch.float64, device=dev)
         return BlockedCSC(torch.zeros(nblk * D + 1, dtype=torch.int64, device=dev),
-                          torch.zeros(0, dtype=torch.int32, device=dev), torch.zeros(0, dtype=torch.float64, device=dev),
-                          nblk, R)
+                          torch.zeros(0, dtype=torch.int32, device=dev), empty, nblk, R,
+                          None if weights is None else empty)
     row = torch.repeat_interleave(torch.arange(N, device=dev, dtype=torch.int64), csr.indptr[1:] - csr.indptr[:-1])
     key = (row // R) * D + csr.indices.to(torch.int64)
     # the CSR order is (row, column): a stable sort on (block, column) keeps the rows increasing within a column
@@ -115,26 +140,35 @@ def block_csc(csr, rows_per_block):
     counts = torch.bincount(key, minlength=nblk * D)
     colptr = torch.zeros(nblk * D + 1, dtype=torch.int64, device=dev)
     colptr[1:] = torch.cumsum(counts, 0)
-    return BlockedCSC(colptr, row[perm].to(torch.int32).contiguous(), csr.values[perm].contiguous(), nblk, R)
+    return BlockedCSC(colptr, row[perm].to(torch.int32).contiguous(), csr.values[perm].contiguous(), nblk, R,
+                      None if weights is None else weights[perm].contiguous())
 
 
-def column_sums(csr):
-    """Per column: stored entries, their sum and their sum of squares (float64 numpy arrays of length D).  Sequential sums in
-    stored order (numpy bincount): the same input always gives the same bits."""
+def column_sums(csr, weights=None):
+    """Per column: stored entries, their sum and their sum of squares (float64 numpy arrays of length D); with weights (CSR
+    order) the weighted sums sum s, sum s x, sum s x^2.  Sequential sums in stored order (numpy bincount): the same input
+    always gives the same bits."""
     D = csr.D
     col = csr.indices.cpu().numpy().astype(np.int64, copy=False)
     val = csr.values.cpu().numpy()
-    cnt = np.bincount(col, minlength=D).astype(np.float64)
-    colx = np.bincount(col, weights=val, minlength=D)
-    colxx = np.bincount(col, weights=val * val, minlength=D)
+    if weights is None:
+        cnt = np.bincount(col, minlength=D).astype(np.float64)
+        sv = val
+    else:
+        s = weights.cpu().numpy()
+        cnt = np.bincount(col, weights=s, minlength=D)
+        sv = s * val
+    colx = np.bincount(col, weights=sv, minlength=D)
+    colxx = np.bincount(col, weights=sv * val, minlength=D)
     return cnt, colx, colxx
 
 
-def x_cache(csr):
-    """[cnt (D) | colsumX (D) | sum x^2 | nnz] as a float64 CPU tensor, from column_sums; sum x^2 exactly rounded over its
-    per-column parts."""
-    cnt, colx, colxx = column_sums(csr)
-    out = np.concatenate([cnt, colx, [math.fsum(colxx.tolist()), float(csr.values.numel())]])
+def x_cache(csr, weights=None):
+    """[cnt (D) | colsumX (D) | sum x^2 | entries] as a float64 CPU tensor, from column_sums; sum x^2 exactly rounded over its
+    per-column parts.  entries: the stored entries, or with weights those of positive weight."""
+    cnt, colx, colxx = column_sums(csr, weights)
+    n = csr.values.numel() if weights is None else int((weights > 0).sum())
+    out = np.concatenate([cnt, colx, [math.fsum(colxx.tolist()), float(n)]])
     return torch.as_tensor(out, dtype=torch.float64)
 
 
