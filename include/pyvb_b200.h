@@ -185,7 +185,8 @@ int pyvb_zstep_f64(long long N, int D, int q, const double *X, long long ldx, co
                    double *zsums, int algo, void *stream);
 
 /* K2 alone (DMMA-path layout): rows of MZ = [qprec packed | pad | eta] are replaced in place by
- * [<zz^T> packed | 0 | zbar]; batched q x q SPD inverse / solve, q in {8,16,32,64}.  Sig may be NULL.
+ * [<zz^T> packed | pad | zbar]; batched q x q SPD inverse / solve, q in {8,16,32,64}.  Sig may be NULL.  Only the packed
+ * and zbar columns are written: the pad [P, Pp) and the columns past Pp + q are passed through (no reader of the rows uses them).
  * MZ must be 16-byte aligned (the rows travel as bulk copies; the pitch is a multiple of 32 bytes). */
 int pyvb_zsolve_f64(long long N, int q, double *MZ, long long ldmz, double *Sig, double *logdet, double *gl,
                     double *zsums, void *stream);

@@ -453,9 +453,10 @@ zsolve_tsweep_kernel(long long N, double *__restrict__ MZ, double *__restrict__ 
         }
         fence_async_smem();
         __syncwarp();
-        // ---- rows back to HBM (one bulk store per row), column sums of the finished rows, next group in
+        // ---- rows back to HBM (one bulk store per row), column sums of the finished rows, next group in.  Only the OROW used
+        //      columns go back: the slot's doubles past them hold tile data, not the row's pitch tail
         if (lane == 0) {
-            for (int m = 0; m < nval; ++m) bulk_s2g(MZ + (n0 + m) * PITCH, stg + m * TS, (uint32_t)(PITCH * 8));
+            for (int m = 0; m < nval; ++m) bulk_s2g(MZ + (n0 + m) * PITCH, stg + m * TS, (uint32_t)(T::OROW * 8));
             bulk_commit();
         }
         if (zsums != nullptr) {                                  // kernel-uniform

@@ -29,6 +29,35 @@ def tensor_rel(a, b):
     return float(np.max(np.abs(a - b))) / den
 
 
+def refined_inverse(A, steps=3):
+    """Inverses of a batch of float64 SPD matrices [.., q, q] in extended precision (np.longdouble): a float64 inverse of the
+    equilibrated matrix, refined by Newton steps X <- X + X (I - A X) in long double.  The equilibration keeps the start
+    inside Newton's region of convergence for matrices whose diagonal spans many orders of magnitude."""
+    A = np.asarray(A, dtype=np.float64)
+    q = A.shape[-1]
+    d = 1.0 / np.sqrt(np.diagonal(A, axis1=-2, axis2=-1).astype(np.longdouble))
+    Al = d[..., :, None] * A.astype(np.longdouble) * d[..., None, :]
+    X = np.linalg.inv(Al.astype(np.float64)).astype(np.longdouble)
+    eye = np.eye(q, dtype=np.longdouble)
+    for _ in range(steps):
+        X = X + X @ (eye - Al @ X)
+    return d[..., :, None] * X * d[..., None, :]
+
+
+def half_logdet_ld(A):
+    """ln prod diag chol(A) = 0.5 ln det A of a batch of float64 SPD matrices, by a Cholesky factorisation in long double."""
+    L = np.array(A, dtype=np.longdouble)
+    q = L.shape[-1]
+    out = np.zeros(L.shape[:-2], dtype=np.longdouble)
+    for k in range(q):
+        piv = np.sqrt(L[..., k, k])
+        out += np.log(piv)
+        col = L[..., k + 1:, k] / piv[..., None]
+        L[..., k + 1:, k + 1:] -= col[..., :, None] * col[..., None, :]
+        L[..., k + 1:, k] = col
+    return out
+
+
 def oracle_from_golden(g, mode="A"):
     o = PlateOracle(g["X"], int(g["q"]), mode=mode, ard=bool(int(g.get("ard", 0))))
     o.load_state(golden_state(g, "init_"))

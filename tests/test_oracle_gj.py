@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 from scipy.linalg import cho_factor, cho_solve
 
-from helpers import tensor_rel
+from helpers import refined_inverse, tensor_rel
 from oracle.gj_oracle import gj_solve
 
 
@@ -22,10 +22,7 @@ def _case(N, q, seed, cond):
 @pytest.mark.parametrize("cond", [1e2, 1e4, 1e6])
 def test_gauss_jordan_is_as_accurate_as_the_cholesky_route(q, cond):
     A, eta = _case(60, q, seed=q, cond=cond)
-    Al = A.astype(np.longdouble)
-    X = np.linalg.inv(A).astype(np.longdouble)
-    for _ in range(3):                                   # Newton refinement in extended precision
-        X = X + X @ (np.eye(q, dtype=np.longdouble) - Al @ X)
+    X = refined_inverse(A)
     ref = np.stack([cho_solve(cho_factor(a), np.eye(q)) for a in A])
     Sg, z, ld = gj_solve(A, eta)
     e_ref, e_gj = tensor_rel(ref, X), tensor_rel(Sg, X)

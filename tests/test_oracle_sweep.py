@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 from scipy.linalg import cho_factor, cho_solve
 
-from helpers import tensor_rel
+from helpers import refined_inverse, tensor_rel
 from oracle.sweep_oracle import sweep_solve
 from oracle.tsweep_oracle import tsweep_solve
 
@@ -30,10 +30,7 @@ def _case(N, q, seed, cond):
 @pytest.mark.parametrize("cond", [1e2, 1e4, 1e6])
 def test_blocked_sweep_is_as_accurate_as_the_cholesky_route(q, cond, layout):
     A, eta = _case(9, q, seed=q, cond=cond)                      # (9: the last group is ragged)
-    Al = A.astype(np.longdouble)
-    X = np.linalg.inv(A).astype(np.longdouble)
-    for _ in range(3):                                           # Newton refinement in extended precision
-        X = X + X @ (np.eye(q, dtype=np.longdouble) - Al @ X)
+    X = refined_inverse(A)
     ref = np.stack([cho_solve(cho_factor(a), np.eye(q)) for a in A])
     Sg, z, ld, M2 = (sweep_solve if layout == "packed" else tsweep_solve)(A, eta, mpw=(1 if layout == "packed" else 2) if q == 64 else 4)
     e_ref, e_s = tensor_rel(ref, X), tensor_rel(Sg, X)
