@@ -270,6 +270,33 @@ int pyvb_global_w_f64(int D, int q, int ops, int col_lo, int col_hi, const doubl
                       const double *ncnt /* nullable without nd */, const double *P0, const double *h0,
                       const pyvb_consts *consts /* host */, double *elbo_out, void *stream);
 
+/* ---- row-wise W posterior (mode B, FP64, q in {8, 16, 32, 64}: the q of pyvb_zsolve_f64) ----
+ * q(W) = prod_d N(w_d | wbar_d, Sigma_d), one full q x q covariance per data dimension, in place of the q column nodes with
+ * diagonal covariances (pyvb_wupdate_f64).  The W step solves each row's block outright:
+ *   Lambda_d = diag(<alpha>) + tau_d T1_d,   eta_d = tau_d (Ast_d - mu_d Bst_d),   Sigma_d = Lambda_d^-1,   wbar_d = Sigma_d eta_d
+ * (tau_d = gl[PYVB_GL_TAU], or nd[PYVB_ND_TAU * D + d] with per-dimension noise; weighted statistics need nothing else).
+ *   WM   [D][ldwm] scratch rows, ldwm = pyvb_mz_pitch(q), 16-byte aligned: the K2 row [Lambda_d packed | 0 | eta_d | 0] is
+ *        assembled there and left as [<w_d w_d^T> packed | 0 | wbar_d | 0]
+ *   Wcov [D][P]  packed Sigma_d (state: pyvb_pack_gw_rows_f64 and pyvb_global_rows_f64 read it)
+ *   Wld  [D]     ln prod diag chol(Lambda_d) (= -1/2 ln det Sigma_d), the convention of the Z rows' logdet
+ *   Wbar, Wvar [D][q]  wbar_d and diag Sigma_d (the ARD update and the bound's prior term read them)
+ * A row whose Lambda_d is not positive definite is counted into gl[PYVB_GL_NONPD], as Z rows are.
+ *   pyvb_wupdate_rows_f64   the W step above (every row; there is no column subset)
+ *   pyvb_pack_gw_rows_f64   Gw rows with G_d = wbar_d wbar_d^T + Sigma_d (times tau_d with nd): every Z-step path reads them
+ *   pyvb_global_rows_f64    pyvb_global_f64 / _nd_f64 / _w_f64 in one: nd and ncnt nullable as in pyvb_global_w_f64, weighted
+ *                           != 0 adds gl[PYVB_GL_LNS] to the X term.  The residual contraction reads g = wbar_i wbar_j +
+ *                           Sigma_d,ij; the W bound term keeps its prior part, sum_i [-D/2 ln 2pi + 1/2 ln det(alpha_i I) -
+ *                           alpha_i/2 sum_d <w_di^2>], and takes the entropy of D row nodes with the reference's
+ *                           q_ln_det = .5 / ln prod diag chol quirk per node: sum_d [q/2 ln 2pi + 1/2 (0.5 / Wld_d) + q/2]. */
+int pyvb_wupdate_rows_f64(int D, int q, const double *stats, const double *mu, double *gl, const double *nd /* nullable */,
+                          double *WM, int ldwm, double *Wbar, double *Wvar, double *Wcov, double *Wld, void *stream);
+int pyvb_pack_gw_rows_f64(int D, int q, const double *Wbar, const double *Wcov, const double *mu,
+                          const double *nd /* nullable */, double *Gw, int ldg, void *stream);
+int pyvb_global_rows_f64(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar,
+                         const double *Wvar, const double *Wcov, const double *Wld, double *mu, double *muvar, double *gl,
+                         double *nd /* nullable */, const double *ncnt /* nullable */, int weighted, const double *P0,
+                         const double *h0, const pyvb_consts *consts /* host */, double *elbo_out, void *stream);
+
 /* Mode A: x_hat = observed ? x : W zbar + mu, v = observed ? 0 : 1/tau for rows [0,N) that are not
  * fully observed (pointers already offset to the first row). */
 int pyvb_impute_f64(long long N, int D, int q, const double *Xorig, long long ldx, const double *Wbar,

@@ -105,6 +105,10 @@ SIGNATURES = {
     "pyvb_wupdate_nd_f64": (c_int, [c_int, c_int, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp]),
     "pyvb_global_nd_f64": (c_int, [c_int, c_int, c_int, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp,
                                    ctypes.POINTER(Consts), c_dp, c_dp]),
+    "pyvb_wupdate_rows_f64": (c_int, [c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_dp, c_int, c_dp, c_dp, c_dp, c_dp, c_dp]),
+    "pyvb_pack_gw_rows_f64": (c_int, [c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_dp, c_int, c_dp]),
+    "pyvb_global_rows_f64": (c_int, [c_int, c_int, c_int, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp,
+                                     c_dp, c_int, c_dp, c_dp, ctypes.POINTER(Consts), c_dp, c_dp]),
     "pyvb_bench_dmma_f64": (c_int, [c_int, c_int, c_dp, c_dp]),
     "pyvb_bench_umma": (c_int, [c_int, c_int, c_int, c_int, c_int, c_dp, c_dp, c_dp]),
     "pyvb_impute_f64": (c_int, [c_ll, c_int, c_int, c_dp, c_ll, c_dp, c_dp, c_dp, c_ll, c_dp, c_dp, c_dp, c_dp, c_dp]),

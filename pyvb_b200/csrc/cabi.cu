@@ -365,6 +365,48 @@ int pyvb_global_w_f64(int D, int q, int ops, int col_lo, int col_hi, const doubl
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "global_w");
 }
 
+static bool k2_q(int q) { return q == 8 || q == 16 || q == 32 || q == 64; }
+
+int pyvb_wupdate_rows_f64(int D, int q, const double *stats, const double *mu, double *gl, const double *nd, double *WM, int ldwm,
+                          double *Wbar, double *Wvar, double *Wcov, double *Wld, void *stream) {
+    ARG(D >= 1 && k2_q(q), "D, q (8, 16, 32 or 64)");
+    ARG(stats && mu && gl && WM && Wbar && Wvar && Wcov && Wld, "null pointer");
+    ARG(ldwm == pyvb_mz_pitch(q), "ldwm must equal pyvb_mz_pitch(q)");
+    ARG((reinterpret_cast<uintptr_t>(WM) & 15) == 0, "WM must be 16-byte aligned");
+    cudaError_t e = launch_wupdate_rows(D, q, stats, mu, gl, nd ? nd + (size_t)PYVB_ND_TAU * D : nullptr, WM, ldwm, Wbar, Wvar,
+                                        Wcov, Wld, (cudaStream_t)stream);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "wupdate_rows");
+}
+
+int pyvb_pack_gw_rows_f64(int D, int q, const double *Wbar, const double *Wcov, const double *mu, const double *nd, double *Gw,
+                          int ldg, void *stream) {
+    ARG(D >= 1 && k2_q(q), "D, q (8, 16, 32 or 64)");
+    ARG(Wbar && Wcov && mu && Gw, "null pointer");
+    ARG(ldg >= gw_woff(q) + q + 1, "ldg");
+    cudaError_t e = launch_pack_gw(D, q, Wbar, nullptr, mu, nd ? nd + (size_t)PYVB_ND_TAU * D : nullptr, Gw, ldg,
+                                   (cudaStream_t)stream, Wcov);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "pack_gw_rows");
+}
+
+int pyvb_global_rows_f64(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar,
+                         const double *Wvar, const double *Wcov, const double *Wld, double *mu, double *muvar, double *gl,
+                         double *nd, const double *ncnt, int weighted, const double *P0, const double *h0,
+                         const pyvb_consts *consts, double *elbo_out, void *stream) {
+    ARG(D >= 1 && k2_q(q), "D, q (8, 16, 32 or 64)");
+    ARG(stats && Wbar && Wvar && Wcov && Wld && mu && muvar && gl && P0 && h0 && consts, "null pointer");
+    ARG(0 <= col_lo && col_lo <= col_hi && col_hi <= q, "column range");
+    ARG(!consts->mode_a, "the row-wise W posterior is a mode-B model (consts->mode_a must be 0)");
+    ARG(!(weighted && nd) || ncnt != NULL, "per-dimension noise with weights needs the per-column counts ncnt");
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = cudaSuccess;
+    if (nd) e = launch_noise_diag(D, q, ops, stats, Wbar, Wvar, mu, muvar, nd, consts->alpha_mu, st, weighted ? ncnt : nullptr,
+                                  Wcov);
+    if (e == cudaSuccess)
+        e = launch_global(D, q, ops, col_lo, col_hi, stats, Wbar, Wvar, mu, muvar, gl, P0, h0, *consts, elbo_out, nd, st,
+                          weighted != 0, Wcov, Wld);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "global_rows");
+}
+
 int pyvb_impute_f64(long long N, int D, int q, const double *Xorig, long long ldx, const double *Wbar,
                     const double *mu, const double *Zbar, long long ldz, const double *gl, double *Xhat, double *V,
                     double *qldX, void *stream) {

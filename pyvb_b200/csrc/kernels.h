@@ -19,8 +19,9 @@ struct I8Check {
 
 // ---- generic (any D, q <= 64) ------------------------------------------------
 // tau_d (nullable): per-dimension noise precisions folded into the row (pyvb_pack_gw_nd_f64)
+// Wcov (nullable): row-wise W posterior, packed Sigma_d [D][P] in place of diag(Wvar) (Wvar is then not read)
 cudaError_t launch_pack_gw(int D, int q, const double *Wbar, const double *Wvar, const double *mu, const double *tau_d,
-                           double *Gw, int ldg, cudaStream_t st);
+                           double *Gw, int ldg, cudaStream_t st, const double *Wcov = nullptr);
 // S (nullable, here and below): per-entry observation weights [N][lds] of a mode-B data set (the weight of an entry whose x is
 // NaN is not read); every observed entry then counts with its weight, the statistics' cnt is the weight sum and nE the number
 // of observed entries of positive weight
@@ -50,17 +51,25 @@ cudaError_t launch_stats_reduce(int D, int q, const double *ws_main, int nchunks
 size_t peer_buffer_bytes(size_t len);
 cudaError_t launch_wupdate(int D, int q, int col_lo, int col_hi, const double *stats, const double *mu,
                            const double *gl, const double *tau_d, double *Wbar, double *Wvar, cudaStream_t st);
+// row-wise W posterior: Lambda_d, eta_d into the K2 rows WM [D][ldwm], launch_zsolve, then wbar_d, diag Sigma_d into Wbar, Wvar.
+// Wcov [D][P] receives Sigma_d, Wld [D] ln prod diag chol(Lambda_d); non-PD rows are counted into gl[PYVB_GL_NONPD]
+cudaError_t launch_wupdate_rows(int D, int q, const double *stats, const double *mu, double *gl, const double *tau_d,
+                                double *WM, int ldwm, double *Wbar, double *Wvar, double *Wcov, double *Wld, cudaStream_t st);
 // nd (nullable): per-dimension noise mode -- Mu and the Gammas are left to launch_noise_diag, which must run first
 // weighted: the X bound term also carries gl[PYVB_GL_LNS]
+// Wcov, Wld (nullable, both or neither): row-wise W posterior -- the contraction reads Sigma_d, the W entropy term Wld
 cudaError_t launch_global(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar, const double *Wvar,
                           double *mu, double *muvar, double *gl, const double *P0, const double *h0,
-                          const pyvb_consts &c, double *elbo_out, const double *nd, cudaStream_t st, bool weighted = false);
+                          const pyvb_consts &c, double *elbo_out, const double *nd, cudaStream_t st, bool weighted = false,
+                          const double *Wcov = nullptr, const double *Wld = nullptr);
 // per-dimension noise precisions (kernels_noise.cu): Mu (PYVB_OP_MU), r_d, the Gamma of every d (PYVB_OP_BETA) and the per-d X
 // and Beta bound terms (PYVB_OP_BETA | PYVB_OP_ELBO) into the nd block; one warp per data dimension, no atomics
 // ncnt (nullable): weighted data -- the number of observed entries of every column, which the bound reads (stats' cnt is then
 // the weight sum)
+// Wcov (nullable): row-wise W posterior, r_d reads Sigma_d
 cudaError_t launch_noise_diag(int D, int q, int ops, const double *stats, const double *Wbar, const double *Wvar, double *mu,
-                              double *muvar, double *nd, double alpha_mu, cudaStream_t st, const double *ncnt = nullptr);
+                              double *muvar, double *nd, double alpha_mu, cudaStream_t st, const double *ncnt = nullptr,
+                              const double *Wcov = nullptr);
 cudaError_t launch_impute(long long N, int D, int q, const double *Xorig, long long ldx, const double *Wbar,
                           const double *mu, const double *Zbar, long long ldz, const double *gl, double *Xhat,
                           double *V, double *qldX, cudaStream_t st);

@@ -8,6 +8,7 @@
 //   zstep   : nodes/node.py:203-227 (m1, m2 for requester z) + nodes/gaussian.py:117-123
 //   stats   : nodes/nodes_todo.py:50-61 (hstack sums), nodes/nodes_todo.py:136-138 (Gamma traces)
 //   wupdate : nodes/nodes_todo.py:53-62 + nodes/gaussian.py:117-123 (diagonal precision)
+//   wrows   : the row-wise W posterior (DESIGN 5e), one q x q block per data dimension solved by K2
 //   global  : nodes/node.py:105-109 (Mu), nodes/nodes_todo.py:130-157, nodes/gaussian.py:136-151
 //   impute  : nodes/gaussian.py:125-134
 #include "common.cuh"
@@ -18,10 +19,11 @@ namespace pyvb {
 // =============================================================== pack Gw
 // ND: per-dimension noise precisions (include/pyvb_b200.h, "nd" block) folded into the row: [tau_d G_d | pad | tau_d wbar_d |
 // mu_d], so that every Z-step contraction computes sum_d O_nd tau_d G_d and sum_d O_nd (x_nd - mu_d) tau_d wbar_d unchanged
-template <bool ND>
+// WR: row-wise W posterior -- G_d = wbar_d wbar_d^T + Sigma_d with the packed row covariances Wcov [D][P] (Wvar is not read)
+template <bool ND, bool WR = false>
 __global__ void pack_gw_kernel(int D, int q, const double *__restrict__ Wbar, const double *__restrict__ Wvar,
                                const double *__restrict__ mu, const double *__restrict__ tau_d, double *__restrict__ Gw,
-                               int ldg) {
+                               int ldg, const double *__restrict__ Wcov = nullptr) {
     const int d = blockIdx.x;
     if (d >= D) return;
     const int P = tri(q), Pp = gw_woff(q);
@@ -33,7 +35,8 @@ __global__ void pack_gw_kernel(int D, int q, const double *__restrict__ Wbar, co
         const int i = idx / q, j = idx % q;
         if (j <= i) {
             double val = w[i] * w[j];
-            if (i == j) val += v[i];
+            if (WR) val += Wcov[(size_t)d * P + tri(i) + j];
+            else if (i == j) val += v[i];
             if (ND) val *= t;
             g[tri(i) + j] = val;
         }
@@ -47,8 +50,11 @@ __global__ void pack_gw_kernel(int D, int q, const double *__restrict__ Wbar, co
 }
 
 cudaError_t launch_pack_gw(int D, int q, const double *Wbar, const double *Wvar, const double *mu, const double *tau_d,
-                           double *Gw, int ldg, cudaStream_t st) {
-    if (tau_d) pack_gw_kernel<true><<<D, 128, 0, st>>>(D, q, Wbar, Wvar, mu, tau_d, Gw, ldg);
+                           double *Gw, int ldg, cudaStream_t st, const double *Wcov) {
+    if (Wcov) {
+        if (tau_d) pack_gw_kernel<true, true><<<D, 128, 0, st>>>(D, q, Wbar, nullptr, mu, tau_d, Gw, ldg, Wcov);
+        else pack_gw_kernel<false, true><<<D, 128, 0, st>>>(D, q, Wbar, nullptr, mu, nullptr, Gw, ldg, Wcov);
+    } else if (tau_d) pack_gw_kernel<true><<<D, 128, 0, st>>>(D, q, Wbar, Wvar, mu, tau_d, Gw, ldg);
     else pack_gw_kernel<false><<<D, 128, 0, st>>>(D, q, Wbar, Wvar, mu, nullptr, Gw, ldg);
     return cudaGetLastError();
 }
@@ -702,6 +708,53 @@ cudaError_t launch_wupdate(int D, int q, int col_lo, int col_hi, const double *s
     return cudaGetLastError();
 }
 
+// =============================================================== W rows (row-wise posterior), warp per d
+// q(W) = prod_d N(w_d | wbar_d, Sigma_d): Lambda_d = diag(<alpha>) + tau_d T1_d, eta_d = tau_d (Ast_d - mu_d Bst_d).  The
+// assemble kernel writes the K2 input row [Lambda_d packed | 0 | eta_d | 0] (pitch pyvb_mz_pitch(q)); launch_zsolve turns it
+// into [<w_d w_d^T> packed | 0 | wbar_d | 0] with Sigma_d and ln prod diag chol(Lambda_d) beside it; the finish kernel copies
+// wbar_d and diag Sigma_d into Wbar / Wvar, which the ARD update, the bound's prior term and the state read.
+// tau_d (nullable): per-dimension noise precisions; NULL reads the shared tau of gl
+__global__ void __launch_bounds__(256)
+wrows_assemble_kernel(int D, int q, const double *__restrict__ stats, const double *__restrict__ mu,
+                      const double *__restrict__ gl, const double *__restrict__ tau_d, double *__restrict__ WM, int ldwm) {
+    const int lane = threadIdx.x & 31;
+    const int d = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (d >= D) return;
+    const StatLayout L(D, q);
+    const int P = L.P, Pp = gw_woff(q);
+    const double tau = tau_d ? tau_d[d] : gl[PYVB_GL_TAU];
+    const double *T1 = stats + L.t1 + (size_t)d * P;
+    const double *Bst = stats + L.bst + (size_t)d * q, *Ast = stats + L.ast + (size_t)d * q;
+    const double m = mu[d];
+    double *r = WM + (size_t)d * ldwm;
+    for (int p = lane; p < P; p += 32) {
+        int i, j;
+        unpack_p(p, i, j);
+        r[p] = (i == j) ? fma(tau, T1[p], gl[PYVB_GL_ALPHA + i]) : tau * T1[p];
+    }
+    for (int c = P + lane; c < ldwm; c += 32) r[c] = (c >= Pp && c < Pp + q) ? tau * fma(-m, Bst[c - Pp], Ast[c - Pp]) : 0.0;
+}
+
+__global__ void __launch_bounds__(256)
+wrows_finish_kernel(int D, int q, const double *__restrict__ WM, int ldwm, const double *__restrict__ Wcov,
+                    double *__restrict__ Wbar, double *__restrict__ Wvar) {
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= D * q) return;
+    const int d = idx / q, i = idx - d * q;
+    Wbar[idx] = WM[(size_t)d * ldwm + gw_woff(q) + i];
+    Wvar[idx] = Wcov[(size_t)d * tri(q) + tri(i) + i];
+}
+
+cudaError_t launch_wupdate_rows(int D, int q, const double *stats, const double *mu, double *gl, const double *tau_d,
+                                double *WM, int ldwm, double *Wbar, double *Wvar, double *Wcov, double *Wld, cudaStream_t st) {
+    wrows_assemble_kernel<<<(D + 7) / 8, 256, 0, st>>>(D, q, stats, mu, gl, tau_d, WM, ldwm);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = launch_zsolve(D, q, WM, Wcov, Wld, gl, nullptr, st);
+    if (e != cudaSuccess) return e;
+    wrows_finish_kernel<<<(D * q + 255) / 256, 256, 0, st>>>(D, q, WM, ldwm, Wcov, Wbar, Wvar);
+    return cudaGetLastError();
+}
+
 // =============================================================== Mu, Gamma(s), ELBO: one CTA (+ helpers of its cluster)
 // The kernel is launched as ONE thread-block cluster: rank 0 does everything below; the other CTAs only take their share of the
 // D x P contraction  sum_d sum_p g_dp T1[d][p]  of the residual (0.3 of the kernel's 0.35 ms at D = 1024, q = 32 on a single SM),
@@ -730,14 +783,18 @@ __device__ __forceinline__ void gk_store_remote(const double *local_smem, uint32
 // done Mu, the per-dimension Gammas and their bound terms: this kernel skips its scalar Mu / Beta and the contraction, and adds
 // the per-dimension X and Beta terms in a fixed order (one CTA).
 // WT: weighted data (pyvb_global_w_f64): the X bound term also carries the data constant gl[PYVB_GL_LNS] = 1/2 sum ln s_nd.
+// WR: row-wise W posterior (pyvb_global_rows_f64): the contraction reads g = wbar_i wbar_j + Sigma_d,ij from the packed row
+// covariances Wcov [D][P], and the entropy part of the W term is that of D row nodes, sum_d [1/2 (0.5 / Wld_d) + q / 2]
+// (Wld_d = ln prod diag chol(Lambda_d), the reference's q_ln_det quirk per node) in place of the q column nodes'.
 constexpr int GK_CLUSTER = 8;
 
-template <bool WT>
+template <bool WT, bool WR = false>
 __global__ void __launch_bounds__(1024)
 global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__restrict__ stats, const double *__restrict__ Wbar,
               const double *__restrict__ Wvar, double *mu, double *muvar, double *gl,
               const double *__restrict__ P0, const double *__restrict__ h0, const pyvb_consts c,
-              double *elbo_out, const double *__restrict__ nd) {
+              double *elbo_out, const double *__restrict__ nd, const double *__restrict__ Wcov = nullptr,
+              const double *__restrict__ Wld = nullptr) {
     __shared__ double sh[33];
     __shared__ double cl_part[GK_CLUSTER];                              // the cluster's partial sums of the D x P contraction
     __shared__ unsigned short ijtab[PYVB_QMAX * (PYVB_QMAX + 1) / 2];   // packed index -> (i << 8) | j
@@ -806,7 +863,10 @@ global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__res
             for (long long idx = i0; idx < hi; idx += nt) {
                 const int ij = ijtab[pp], i = ij >> 8, j = ij & 255;
                 double g = Wbar[(size_t)d * q + i] * Wbar[(size_t)d * q + j];
-                if (i == j) g += Wvar[(size_t)d * q + i];
+                if (WR) {
+                    g += Wcov[idx];
+                    if (i != j) g *= 2.0;
+                } else if (i == j) g += Wvar[(size_t)d * q + i];
                 else g *= 2.0;
                 dot = fma(g, T1[idx], dot);
                 d += dstep;
@@ -859,7 +919,7 @@ global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__res
             for (int d = lane; d < D; d += 32) {
                 const double w = Wbar[(size_t)d * q + i], v = Wvar[(size_t)d * q + i];
                 pw += fma(w, w, v);
-                pl += log(v);
+                if (!WR) pl += log(v);
             }
             pw = warp_sum(pw);
             pl = warp_sum(pl);
@@ -874,7 +934,13 @@ global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__res
             const double qld = 0.5 / (-0.5 * lv);
             const double al = gl[PYVB_GL_ALPHA + i];
             const double lndet = c.ard ? D * (log(c.al_qa) - log(gl[PYVB_GL_ALQB + i])) : D * log(al);
-            eW += -0.5 * D * LN2PI + 0.5 * lndet - 0.5 * al * ww - (-0.5 * D * LN2PI - 0.5 * qld - 0.5 * D);
+            if (WR) eW += -0.5 * D * LN2PI + 0.5 * lndet - 0.5 * al * ww - (-0.5 * D * LN2PI - 0.5 * D);
+            else eW += -0.5 * D * LN2PI + 0.5 * lndet - 0.5 * al * ww - (-0.5 * D * LN2PI - 0.5 * qld - 0.5 * D);
+        }
+        if (WR) {
+            double pe = 0.0;
+            for (int d = tid; d < D; d += nt) pe += 0.5 / Wld[d];
+            eW += 0.5 * block_sum(pe, sh);
         }
         // ---- Mu
         double pm = 0.0, pl = 0.0;
@@ -952,7 +1018,8 @@ global_kernel(int D, int q, int ops, int col_lo, int col_hi, const double *__res
 
 cudaError_t launch_global(int D, int q, int ops, int col_lo, int col_hi, const double *stats, const double *Wbar, const double *Wvar,
                           double *mu, double *muvar, double *gl, const double *P0, const double *h0,
-                          const pyvb_consts &c, double *elbo_out, const double *nd, cudaStream_t st, bool weighted) {
+                          const pyvb_consts &c, double *elbo_out, const double *nd, cudaStream_t st, bool weighted,
+                          const double *Wcov, const double *Wld) {
     // one cluster; its size follows the work of the D x P contraction (small problems, or no contraction: one CTA)
     const long long work = nd ? 0 : (long long)D * q * (q + 1) / 2;
     const int cl = work >= (1LL << 17) ? GK_CLUSTER : work >= (1LL << 15) ? 2 : 1;
@@ -968,8 +1035,11 @@ cudaError_t launch_global(int D, int q, int ops, int col_lo, int col_hi, const d
     at[0].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
+    if (Wcov)
+        return cudaLaunchKernelEx(&cfg, weighted ? global_kernel<true, true> : global_kernel<false, true>, D, q, ops, col_lo,
+                                  col_hi, stats, Wbar, Wvar, mu, muvar, gl, P0, h0, c, elbo_out, nd, Wcov, Wld);
     return cudaLaunchKernelEx(&cfg, weighted ? global_kernel<true> : global_kernel<false>, D, q, ops, col_lo, col_hi, stats, Wbar,
-                              Wvar, mu, muvar, gl, P0, h0, c, elbo_out, nd);
+                              Wvar, mu, muvar, gl, P0, h0, c, elbo_out, nd, (const double *)nullptr, (const double *)nullptr);
 }
 
 // =============================================================== mode A imputation, warp per row

@@ -11,6 +11,7 @@
 // WT (per-entry observation weights): the statistics' cnt_d is the weight sum sum_n s_nd, which Mu and r_d read; the bound reads
 // the NUMBER of observed entries of column d from ncnt[d] instead.
 //          eB_d = the Gamma bound of entry d                                       (DiagonalGamma.log_lower_bound)
+// WR (row-wise W posterior): g = wbar_i wbar_j + Sigma_d,ij in r_d, from the packed row covariances Wcov [D][P].
 // global_kernel then adds eX_d and eB_d over d in a fixed order.  No atomics: replicas on several GPUs stay bit-identical.
 #include "common.cuh"
 #include "kernels.h"
@@ -19,11 +20,11 @@ namespace pyvb {
 
 constexpr int ND_WARPS = 8;
 
-template <bool WT>
+template <bool WT, bool WR = false>
 __global__ void __launch_bounds__(32 * ND_WARPS)
 noise_diag_kernel(int D, int q, int ops, const double *__restrict__ stats, const double *__restrict__ Wbar,
                   const double *__restrict__ Wvar, double *__restrict__ mu, double *__restrict__ muvar, double *__restrict__ nd,
-                  double alpha_mu, const double *__restrict__ ncnt) {
+                  double alpha_mu, const double *__restrict__ ncnt, const double *__restrict__ Wcov = nullptr) {
     __shared__ unsigned short ijtab[PYVB_QMAX * (PYVB_QMAX + 1) / 2];   // packed index -> (i << 8) | j
     const StatLayout L(D, q);
     const int P = L.P;
@@ -64,7 +65,10 @@ noise_diag_kernel(int D, int q, int ops, const double *__restrict__ stats, const
     for (int p = lane; p < P; p += 32) {
         const int ij = ijtab[p], i = ij >> 8, j = ij & 255;
         double g = w[i] * w[j];
-        if (i == j) g += v[i];
+        if (WR) {
+            g += Wcov[(size_t)d * P + p];
+            if (i != j) g *= 2.0;
+        } else if (i == j) g += v[i];
         else g *= 2.0;
         dot = fma(g, T1[p], dot);
     }
@@ -89,10 +93,17 @@ noise_diag_kernel(int D, int q, int ops, const double *__restrict__ stats, const
 }
 
 cudaError_t launch_noise_diag(int D, int q, int ops, const double *stats, const double *Wbar, const double *Wvar, double *mu,
-                              double *muvar, double *nd, double alpha_mu, cudaStream_t st, const double *ncnt) {
+                              double *muvar, double *nd, double alpha_mu, cudaStream_t st, const double *ncnt,
+                              const double *Wcov) {
     if (!(ops & (PYVB_OP_MU | PYVB_OP_BETA | PYVB_OP_ELBO))) return cudaSuccess;
     const unsigned blocks = (D + ND_WARPS - 1) / ND_WARPS;
-    if (ncnt)
+    if (Wcov && ncnt)
+        noise_diag_kernel<true, true><<<blocks, 32 * ND_WARPS, 0, st>>>(D, q, ops, stats, Wbar, Wvar, mu, muvar, nd, alpha_mu,
+                                                                        ncnt, Wcov);
+    else if (Wcov)
+        noise_diag_kernel<false, true><<<blocks, 32 * ND_WARPS, 0, st>>>(D, q, ops, stats, Wbar, Wvar, mu, muvar, nd, alpha_mu,
+                                                                         nullptr, Wcov);
+    else if (ncnt)
         noise_diag_kernel<true><<<blocks, 32 * ND_WARPS, 0, st>>>(D, q, ops, stats, Wbar, Wvar, mu, muvar, nd, alpha_mu, ncnt);
     else
         noise_diag_kernel<false><<<blocks, 32 * ND_WARPS, 0, st>>>(D, q, ops, stats, Wbar, Wvar, mu, muvar, nd, alpha_mu, nullptr);

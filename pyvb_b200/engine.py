@@ -81,12 +81,16 @@ class PlateEngine(object):
         or tensor storing exactly the entries X stores.  Mode "B", precision "f64", the DMMA, generic and sparse paths
         ("auto" picks DMMA where the shape allows it, else generic; "i8" is refused: its mask contraction is exact only for
         0/1 weights).  None (the default): every observed entry has weight 1, the unweighted model.
+    w_posterior : the factorisation of q(W).  "columns" (the default): the reference's q column nodes with diagonal
+        covariances, one Gauss-Seidel pass over the columns per update_W.  "rows": q(W) = prod_d N(w_d | wbar_d, Sigma_d), one
+        full q x q covariance per data dimension (the VB-PCA of Ilin & Raiko), solved outright per row by the batched q x q
+        solve of the Z step; get_state() then also returns "Wcov" (D, q, q).  Mode "B", precision "f64", q in {8, 16, 32, 64}.
     """
 
     def __init__(self, X, q, mode="B", alpha0=1e-3, alpha_mu=1e-3, a0=1e-3, b0=1e-3, ard=False,
                  ard_a0=1e-3, ard_b0=1e-3, P0=None, m0=None, device=None, algo="auto",
                  keep_sigma=True, distributed=False, row_offset=0, trace_len=4096, precision="f64", noise="scalar",
-                 weights=None):
+                 weights=None, w_posterior="columns"):
         if not torch.cuda.is_available():
             raise RuntimeError("pyvb_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         self.lib = _cabi.lib()
@@ -102,6 +106,19 @@ class PlateEngine(object):
         self.weighted = weights is not None
         if self.weighted and (mode != "B" or self.f32 or algo == "i8"):
             raise ValueError("weights need mode='B', precision='f64' and algo 'auto', 'dmma' or 'generic'")
+        if w_posterior not in ("columns", "rows"):
+            raise ValueError("w_posterior must be 'columns' or 'rows', got %r" % (w_posterior,))
+        self.wrows = (w_posterior == "rows")
+        if self.wrows:
+            if mode != "B":
+                raise ValueError("w_posterior='rows' needs mode='B': mode A is the reference-exact path, pinned against the "
+                                 "reference's column nodes of W")
+            if self.f32:
+                raise ValueError("w_posterior='rows' needs precision='f64': the FP32 variant builds its bf16 planes of G "
+                                 "from the column variances Wvar")
+            if int(q) not in (8, 16, 32, 64):
+                raise ValueError("w_posterior='rows' needs q in (8, 16, 32, 64), the q of the batched q x q solve that "
+                                 "solves the rows; got %d" % int(q))
         self.device = torch.device(device if device is not None else "cuda:%d" % torch.cuda.current_device())
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
@@ -297,6 +314,13 @@ class PlateEngine(object):
         self.muvar = torch.ones(D, dtype=f64, device=dev)
         self.ldg = int(self.lib.pyvb_gw_pitch(q))
         self.Gw = torch.zeros(D, self.ldg, dtype=f64, device=dev)
+        # row-wise W posterior: the K2 rows of the W step, packed Sigma_d and ln prod diag chol(Lambda_d)
+        self.WM = self.Wcov = self.Wld = None
+        if self.wrows:
+            self.WM = torch.zeros(D, self.ldmz, dtype=f64, device=dev)
+            ii, jj = tril_pack_index(q)
+            self.Wcov = torch.as_tensor((ii == jj).astype(np.float64), device=dev).repeat(D, 1).contiguous()
+            self.Wld = torch.zeros(D, dtype=f64, device=dev)
         self.stats = torch.zeros(self.L.len, dtype=f64, device=dev)
         assert self.L.len == int(self.lib.pyvb_stats_len(D, q))
         self.ws_bytes = int(self.lib.pyvb_stats_workspace_bytes(N, D, q, ALGO_F32 if self.f32 else self.algo))
@@ -429,9 +453,14 @@ class PlateEngine(object):
         def put(dst, src):
             dst.copy_(torch.as_tensor(np.ascontiguousarray(src), dtype=f64).reshape(dst.shape).to(dev))
 
+        if "Wcov" in st and not self.wrows:
+            raise ValueError("set_state: 'Wcov' is the state of w_posterior='rows'; this engine's W posterior has column "
+                             "variances only (Wvar)")
         for k in ("Wbar", "Wvar", "mu", "muvar", "Zbar"):
             if k in st:
                 put(getattr(self, k), st[k])
+        if self.wrows and ("Wcov" in st or "Wvar" in st):
+            self._set_wcov(st.get("Wcov"))
         if "Xhat" in st and self.mode == "A":
             put(self.X, st["Xhat"])
         if "V" in st and self.mode == "A":
@@ -479,6 +508,22 @@ class PlateEngine(object):
         self._gw_fresh = False
         self._zsums_valid = False
 
+    def _set_wcov(self, wcov):
+        """Row-wise W posterior: Wcov from a (D, q, q) array, or diag(Wvar) when None; Wvar = diag Wcov and Wld =
+        -1/2 ln det Sigma_d follow."""
+        q, dev = self.q, self.device
+        ii, jj = tril_pack_index(q)
+        if wcov is None:
+            S = torch.diag_embed(self.Wvar)
+        else:
+            S = torch.as_tensor(np.ascontiguousarray(wcov), dtype=torch.float64).reshape(self.D, q, q).to(dev)
+        L, info = torch.linalg.cholesky_ex(S)
+        if bool((info != 0).any()):
+            raise ValueError("set_state: every Wcov[d] must be symmetric positive definite")
+        self.Wcov.copy_(S[:, torch.as_tensor(ii, device=dev), torch.as_tensor(jj, device=dev)])
+        self.Wvar.copy_(torch.diagonal(S, dim1=1, dim2=2))
+        self.Wld.copy_(-torch.log(torch.diagonal(L, dim1=1, dim2=2)).sum(1))
+
     def _resplit(self, step=1 << 16):
         """FP32 variant: refresh the bf16 x 3 planes after the FP32 rows were written from outside the kernels."""
         for lo in range(0, self.N, step):
@@ -506,12 +551,14 @@ class PlateEngine(object):
     @_on_device
     def init_random(self, seed=1234, rank=0):
         """Scale-run initialisation on the device (SURVEY 8d): Wbar ~ N(0,1) (same on every rank),
-        Zbar ~ N(0,1) (per-rank stream), Wvar = 1, Sigma = I, mu = 0, qb = 0.5."""
+        Zbar ~ N(0,1) (per-rank stream), Wvar = 1 (Wcov = I), Sigma = I, mu = 0, qb = 0.5."""
         dev, q, P = self.device, self.q, self.P
         g = torch.Generator(device=dev)
         g.manual_seed(int(seed))
         self.Wbar.normal_(generator=g)
         self.Wvar.fill_(1.0)
+        if self.wrows:
+            self._set_wcov(None)
         self.mu.zero_()
         self.muvar.fill_(1.0)
         g.manual_seed(int(seed) + 1 + int(rank))
@@ -562,6 +609,8 @@ class PlateEngine(object):
         Sig[:, ii, jj] = sp
         Sig[:, jj, ii] = sp
         out["Sig"] = Sig
+        if self.wrows:
+            out["Wcov"] = self._wcov_host()
         if self.mode == "A":
             out["Xhat"] = self.X.cpu().numpy()
             out["V"] = self.V.cpu().numpy()
@@ -570,6 +619,15 @@ class PlateEngine(object):
         out["alpha"] = gl[GL_ALPHA:GL_ALPHA + q].copy()
         out["al_qb"] = gl[GL_ALQB:GL_ALQB + q].copy()
         return out
+
+    def _wcov_host(self):
+        """Row-wise W posterior: the packed Sigma_d as a (D, q, q) host array."""
+        ii, jj = tril_pack_index(self.q)
+        wp = self.Wcov.cpu().numpy()
+        Wc = np.zeros((self.D, self.q, self.q))
+        Wc[:, ii, jj] = wp
+        Wc[:, jj, ii] = wp
+        return Wc
 
     def _noise_state(self, gl):
         """qa, qb, tau: floats, or (D,) arrays with noise='diagonal'."""
@@ -603,6 +661,8 @@ class PlateEngine(object):
         out = {"Wbar": self.Wbar.cpu().numpy(), "Wvar": self.Wvar.cpu().numpy(), "mu": self.mu.cpu().numpy(),
                "muvar": self.muvar.cpu().numpy(), "alpha": gl[GL_ALPHA:GL_ALPHA + self.q].copy(),
                "al_qb": gl[GL_ALQB:GL_ALQB + self.q].copy()}
+        if self.wrows:
+            out["Wcov"] = self._wcov_host()
         out.update(self._noise_state(gl))
         return out
 
@@ -611,7 +671,8 @@ class PlateEngine(object):
         bad = float(self.gl[GL_NONPD].item())
         if bad > 0:
             self.gl[GL_NONPD] = 0.0             # reported once; a state injected afterwards starts clean
-            raise np.linalg.LinAlgError("posterior precision of %d row(s) is not positive definite" % int(bad))
+            what = "row(s) of Z or W" if self.wrows else "row(s)"
+            raise np.linalg.LinAlgError("posterior precision of %d %s is not positive definite" % (int(bad), what))
 
     def i8_fallbacks(self):
         """How often the accuracy guard of the INT8 path sent a step to the FP64 tensor cores: (Z steps, statistics passes)."""
@@ -628,6 +689,11 @@ class PlateEngine(object):
             rc = self.lib.pyvb_pack_gw_f32(self.D, self.q, self.Wbar.data_ptr(), self.Wvar.data_ptr(),
                                            self.mu.data_ptr(), self.GT.data_ptr(), self.WT.data_ptr(), self._stream())
             _cabi.check(rc, "pyvb_pack_gw_f32")
+            self._gw_fresh = True
+        if not self._gw_fresh and self.wrows:
+            rc = self.lib.pyvb_pack_gw_rows_f64(self.D, self.q, self.Wbar.data_ptr(), self.Wcov.data_ptr(), self.mu.data_ptr(),
+                                                self._p(self.nd), self.Gw.data_ptr(), self.ldg, self._stream())
+            _cabi.check(rc, "pyvb_pack_gw_rows_f64")
             self._gw_fresh = True
         if not self._gw_fresh and self.diag:
             rc = self.lib.pyvb_pack_gw_nd_f64(self.D, self.q, self.Wbar.data_ptr(), self.Wvar.data_ptr(), self.mu.data_ptr(),
@@ -718,7 +784,18 @@ class PlateEngine(object):
     @_on_device
     def update_W(self, col_lo=0, col_hi=None):
         col_hi = self.q if col_hi is None else col_hi
+        if self.wrows and (col_lo, col_hi) != (0, self.q):
+            raise ValueError("update_W: with w_posterior='rows' every row w_d is one block over all q columns; a column "
+                             "range [%d, %d) has no row update" % (col_lo, col_hi))
         self._ensure_stats()
+        if self.wrows:
+            rc = self.lib.pyvb_wupdate_rows_f64(self.D, self.q, self.stats.data_ptr(), self.mu.data_ptr(), self.gl.data_ptr(),
+                                                self._p(self.nd), self.WM.data_ptr(), self.ldmz, self.Wbar.data_ptr(),
+                                                self.Wvar.data_ptr(), self.Wcov.data_ptr(), self.Wld.data_ptr(),
+                                                self._stream())
+            _cabi.check(rc, "pyvb_wupdate_rows_f64")
+            self._gw_fresh = False
+            return
         if self.diag:
             rc = self.lib.pyvb_wupdate_nd_f64(self.D, self.q, col_lo, col_hi, self.stats.data_ptr(), self.mu.data_ptr(),
                                               self.nd.data_ptr(), self.gl.data_ptr(), self.Wbar.data_ptr(),
@@ -825,6 +902,16 @@ class PlateEngine(object):
     def _global(self, ops, elbo_out=0, col_lo=0, col_hi=None):
         self._ensure_stats()
         col_hi = self.q if col_hi is None else col_hi
+        if self.wrows:
+            rc = self.lib.pyvb_global_rows_f64(self.D, self.q, ops, col_lo, col_hi, self.stats.data_ptr(), self.Wbar.data_ptr(),
+                                               self.Wvar.data_ptr(), self.Wcov.data_ptr(), self.Wld.data_ptr(),
+                                               self.mu.data_ptr(), self.muvar.data_ptr(), self.gl.data_ptr(), self._p(self.nd),
+                                               self._p(self.ncnt), int(self.weighted), self.P0.data_ptr(), self.h0.data_ptr(),
+                                               _cabi.ctypes.byref(self.consts), elbo_out, self._stream())
+            _cabi.check(rc, "pyvb_global_rows_f64")
+            if ops & (OP_MU | (OP_BETA if self.diag else 0)):   # mu_d (and tau_d) live in the Gw rows
+                self._gw_fresh = False
+            return
         if self.weighted:
             rc = self.lib.pyvb_global_w_f64(self.D, self.q, ops, col_lo, col_hi, self.stats.data_ptr(), self.Wbar.data_ptr(),
                                             self.Wvar.data_ptr(), self.mu.data_ptr(), self.muvar.data_ptr(),
