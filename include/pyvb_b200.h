@@ -121,8 +121,8 @@ extern "C" {
 #define PYVB_ALGO_GENERIC 1  /* any D, q <= 64; FP64 FMA */
 #define PYVB_ALGO_DMMA 2     /* FP64 tensor-core (DMMA) + TMA staging; q in {8,16,32,64}, D % 16 == 0 */
 #define PYVB_ALGO_F32 4      /* FP32 variant (tcgen05): only for pyvb_stats_workspace_bytes */
-#define PYVB_ALGO_DMMA_K1 3  /* measurement only (zstep): the tensor-core contraction alone; the MZ rows are
-                                left as [qprec packed | eta] for pyvb_zsolve_f64 */
+#define PYVB_ALGO_DMMA_K1 3  /* zstep: the tensor-core contraction alone (measurements, and the K1 of pyvb_zstep_known_f64);
+                                the MZ rows are left as [qprec packed | eta] for pyvb_zsolve_f64 */
 
 typedef struct pyvb_consts {
     double alpha_mu;      /* prior precision of Mu (Constant alpha*I)                    */
@@ -435,6 +435,41 @@ int pyvb_stats_csr_w_f64(long long N, int D, int q, int nblk, const long long *c
                          const double *wts, const double *MZ, long long ldmz, const double *logdet, double *stats, void *ws,
                          size_t ws_bytes, const double *xcache, const double *zsums,
                          const pyvb_peers *peers /* host, nullable */, void *stream);
+
+/* ---- known row covariates: known trailing latent dimensions (mode B, FP64, DESIGN.md 5f) ----
+ * x_nd ~ N(w_d z_n + b_d c_n + mu_d, 1/tau) is the plate at q = q_free + k with z'_n = [z_n ; c_n] and W' = [W | B]: every
+ * statistic, the W step, Mu, the Gammas and the bound run unchanged at q, with the priors P0' = blockdiag(P0, 0) and
+ * h0' = [h0 ; 0].  Only the Z step changes: the Gaussian of z'_n conditioned on its known last k entries.
+ *   C [N][ldc]   c_n, the k known entries of every row (ldc >= k); 1 <= k < q <= 64
+ * pyvb_zknown_condition_f64: on MZ rows [qprec' packed | pad | eta'] (K1's output): eta_z -= qprec'_zc c, qprec'_zc = 0,
+ *   qprec'_cc = I, eta'_c = c.  pyvb_zsolve_f64 then solves blockdiag(A_n, I): the free block is the conditioned posterior, the
+ *   log-det is that of A_n (the identity pivots add ln 1 = 0).  Only the last k rows of the packed block and eta' are written.
+ * pyvb_zknown_finish_f64: on K2's rows: <z'z'^T>_cc = c c^T and zbar'_c = c.  Only those entries are written.
+ * The Z steps with covariates: K1 -> condition -> K2 -> finish on the DMMA path (S nullable: per-entry weights, as
+ * pyvb_zstep_w_f64; algo PYVB_ALGO_GENERIC, or AUTO where the DMMA path does not run: the generic kernel with the
+ * conditioning between its contraction and its factorisation, any q <= 64 and D), the INT8 path (K1-i8 -> condition -> K2 with the accuracy guard -> [K1-DMMA -> condition -> K2] as
+ * conditional launches -> finish; gl[PYVB_GL_I8BAD] and gl[PYVB_GL_I8FALL] as pyvb_zstep_i8_f64) and the CSR path (weights
+ * nullable).  The INT8 guard of a conditioned row compares against one scale, written to gmax [1] (device): the largest
+ * fixed-point scale of the free columns of qprec', and of its zc columns times max(1, cmax), cmax >= max_n sum_j |c_nj| over
+ * the rows of the call (the zc entries enter eta_z times c); the cc columns, which condition discards, do not count.
+ * They leave no K2 partials: K2's column sums and maxima are wrong on the cc entries, so the statistics are called
+ * with zsums = NULL and rebuild them from the finished rows.  Sig (nullable) receives Sigma'_n = blockdiag(Sigma_n, I). */
+int pyvb_zknown_condition_f64(long long N, int q, int k, const double *C, long long ldc, double *MZ, long long ldmz,
+                              void *stream);
+int pyvb_zknown_finish_f64(long long N, int q, int k, const double *C, long long ldc, double *MZ, long long ldmz,
+                           void *stream);
+int pyvb_zstep_known_f64(long long N, int D, int q, int k, const double *C, long long ldc, const double *X, long long ldx,
+                         const double *S /* nullable */, long long lds, const double *Gw, int ldg, const double *P0,
+                         const double *h0, double *gl, double *MZ, long long ldmz, double *Sig, double *logdet, int algo,
+                         void *stream);
+int pyvb_zstep_i8_known_f64(long long N, int D, int q, int k, const double *C, long long ldc, double cmax, const double *X,
+                            long long ldx, const void *mask, const double *Wbar, const double *Wvar, const double *Gw, int ldg,
+                            const double *P0, const double *h0, double *gl, double *MZ, long long ldmz, void *GI,
+                            double *gscale, double *gmax, double *Sig, double *logdet, void *stream);
+int pyvb_zstep_csr_known_f64(long long N, int D, int q, int k, const double *C, long long ldc, const long long *indptr,
+                             const int *indices, const double *values, const double *weights /* nullable */, const double *Gw,
+                             int ldg, const double *P0, const double *h0, double *gl, double *MZ, long long ldmz, double *Sig,
+                             double *logdet, void *stream);
 
 /* ---- VB smoother of a linear dynamic system, batched over B independent sequences (BASELINE config 5) ----
  * Replaces the sweep of examples/Linear_Dynamic_System.py:69-76 for every sequence: all X_t.update() forwards, all

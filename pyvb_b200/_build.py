@@ -11,7 +11,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libpyvb_b200.so")
 SOURCES = ["cabi.cu", "kernels_generic.cu", "kernels_dmma.cu", "kernels_k2.cu", "kernels_k2t.cu", "kernels_k2g.cu", "kernels_k2s.cu", "kernels_f32.cu",
-           "kernels_i8.cu", "kernels_lds.cu", "kernels_sparse.cu", "kernels_noise.cu"]
+           "kernels_i8.cu", "kernels_lds.cu", "kernels_sparse.cu", "kernels_noise.cu", "kernels_known.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-diag-suppress", "177",
     "-Xcompiler", "-fPIC",

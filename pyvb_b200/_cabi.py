@@ -88,6 +88,14 @@ SIGNATURES = {
                                      c_dp, c_dp, c_dp, c_dp]),
     "pyvb_stats_csr_w_f64": (c_int, [c_ll, c_int, c_int, c_int, c_dp, c_dp, c_dp, c_dp, c_dp, c_ll, c_dp, c_dp, c_dp, c_sz,
                                      c_dp, c_dp, ctypes.POINTER(Peers), c_dp]),
+    "pyvb_zknown_condition_f64": (c_int, [c_ll, c_int, c_int, c_dp, c_ll, c_dp, c_ll, c_dp]),
+    "pyvb_zknown_finish_f64": (c_int, [c_ll, c_int, c_int, c_dp, c_ll, c_dp, c_ll, c_dp]),
+    "pyvb_zstep_known_f64": (c_int, [c_ll, c_int, c_int, c_int, c_dp, c_ll, c_dp, c_ll, c_dp, c_ll, c_dp, c_int, c_dp, c_dp,
+                                     c_dp, c_dp, c_ll, c_dp, c_dp, c_int, c_dp]),
+    "pyvb_zstep_i8_known_f64": (c_int, [c_ll, c_int, c_int, c_int, c_dp, c_ll, ctypes.c_double, c_dp, c_ll, c_dp, c_dp, c_dp,
+                                        c_dp, c_int, c_dp, c_dp, c_dp, c_dp, c_ll, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp]),
+    "pyvb_zstep_csr_known_f64": (c_int, [c_ll, c_int, c_int, c_int, c_dp, c_ll, c_dp, c_dp, c_dp, c_dp, c_dp, c_int, c_dp,
+                                         c_dp, c_dp, c_dp, c_ll, c_dp, c_dp, c_dp]),
     "pyvb_lds_max_len": (c_int, []),
     "pyvb_lds_iterate_f64": (c_int, [c_int, c_int, c_int, c_int] + [c_dp] * 11 + [ctypes.c_double] * 3 + [c_int, c_dp, c_dp]),
     "pyvb_lds_iterate_known_f64": (c_int, [c_int, c_int, c_int, c_int] + [c_dp] * 12 + [ctypes.c_double] * 3 + [c_int, c_dp, c_dp]),

@@ -38,6 +38,15 @@ static bool i8_guard_forced() {
     return forced;
 }
 
+// the guard K2 applies to the INT8 qprec rows: the largest of the ncols scales in `gscale` against D * 2^-55 / I8_TOL
+static I8Check i8_check(int D, const double *gscale, int ncols) {
+    I8Check chk;
+    chk.gscale = gscale;
+    chk.ncols = ncols;
+    chk.fac = i8_guard_forced() ? 1e300 : (double)D * 2.7755575615628914e-17 / I8_TOL;     // D * 2^-55 / tol
+    return chk;
+}
+
 static int pick_algo(int algo, int D, int q) {
     if (algo == PYVB_ALGO_AUTO) return dmma_supported(D, q) ? PYVB_ALGO_DMMA : PYVB_ALGO_GENERIC;
     if (algo == PYVB_ALGO_DMMA_K1) return PYVB_ALGO_DMMA;
@@ -460,11 +469,7 @@ int pyvb_zstep_i8_f64(long long N, int D, int q, const double *X, long long ldx,
     if (e == cudaSuccess && !k1_only) {
         // K2 checks every finished qprec row against the fixed-point bound of K1-i8 (kernels.h: I8Check); when a row fails,
         // the whole step is redone on the FP64 tensor cores by two conditional launches that exit at once otherwise
-        I8Check chk;
-        chk.gscale = gscale;
-        chk.ncols = q * (q + 1) / 2;
-        chk.fac = i8_guard_forced() ? 1e300 : (double)D * 2.7755575615628914e-17 / I8_TOL;     // D * 2^-55 / tol
-        e = launch_zsolve(N, q, MZ, Sig, logdet, gl, zsums, st, nullptr, chk);
+        e = launch_zsolve(N, q, MZ, Sig, logdet, gl, zsums, st, nullptr, i8_check(D, gscale, q * (q + 1) / 2));
         if (e == cudaSuccess)
             e = launch_zstep_dmma(N, D, q, X, ldx, Gw, ldg, P0, h0, gl, MZ, Sig, logdet, zsums, 0, st, gl + PYVB_GL_I8BAD);
     }
@@ -703,6 +708,109 @@ int pyvb_stats_f32(long long N, long long nalloc, int D, int q, const void *plan
                             peers ? peers->bufs : NULL, peers ? peers->world : 1, peers ? peers->rank : 0,
                             peers ? peers->epoch : 0ULL, st);
     return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "stats_reduce");
+}
+
+static int known_args(long long N, int q, int k, const double *C, long long ldc, const double *MZ, long long ldmz) {
+    ARG(N >= 0 && k >= 1 && k < q && q <= PYVB_QMAX, "N, q, k (1 <= k < q <= 64)");
+    ARG(N == 0 || (C && MZ), "null pointer");
+    ARG(ldc >= k && ldmz >= gw_woff(q) + q, "ldc, ldmz");
+    return PYVB_OK;
+}
+
+int pyvb_zknown_condition_f64(long long N, int q, int k, const double *C, long long ldc, double *MZ, long long ldmz,
+                              void *stream) {
+    const int rc = known_args(N, q, k, C, ldc, MZ, ldmz);
+    if (rc != PYVB_OK) return rc;
+    cudaError_t e = launch_known_condition(N, q, k, C, ldc, MZ, ldmz, (cudaStream_t)stream);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zknown_condition");
+}
+
+int pyvb_zknown_finish_f64(long long N, int q, int k, const double *C, long long ldc, double *MZ, long long ldmz,
+                           void *stream) {
+    const int rc = known_args(N, q, k, C, ldc, MZ, ldmz);
+    if (rc != PYVB_OK) return rc;
+    cudaError_t e = launch_known_finish(N, q, k, C, ldc, MZ, ldmz, (cudaStream_t)stream);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zknown_finish");
+}
+
+int pyvb_zstep_known_f64(long long N, int D, int q, int k, const double *C, long long ldc, const double *X, long long ldx,
+                         const double *S, long long lds, const double *Gw, int ldg, const double *P0, const double *h0,
+                         double *gl, double *MZ, long long ldmz, double *Sig, double *logdet, int algo, void *stream) {
+    ARG(D >= 1, "D");
+    int rc = known_args(N, q, k, C, ldc, MZ, ldmz);
+    if (rc != PYVB_OK) return rc;
+    const int a = pick_algo(algo, D, q);
+    if (a == PYVB_ALGO_GENERIC) {
+        // K1 and K2 fused in one warp per row, the conditioning between them in shared memory
+        if (N == 0) return PYVB_OK;
+        ARG(X && Gw && P0 && h0 && gl && logdet, "null pointer");
+        ARG(ldx >= D && ldg >= gw_woff(q) + q + 1 && (S == NULL || lds >= D), "ldx, ldg, lds");
+        cudaError_t e = launch_zstep_generic(N, D, q, X, ldx, Gw, ldg, P0, h0, gl, MZ + gw_woff(q), ldmz, MZ, ldmz, Sig, logdet,
+                                             (cudaStream_t)stream, S, lds, C, ldc, k);
+        return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zstep_known (generic)");
+    }
+    if (a != PYVB_ALGO_DMMA) return fail(PYVB_EINVAL, "%s", "unknown algo");
+    if (!dmma_supported(D, q)) return fail(PYVB_ENOSUP, "%s", "DMMA path needs q in {8,16,32,64}, D % 16 == 0");
+    if (N == 0) return PYVB_OK;
+    ARG(ldmz == pyvb_mz_pitch(q), "ldmz must equal pyvb_mz_pitch(q)");
+    // K1 alone (PYVB_ALGO_DMMA_K1, with the checks of the plain entry point), then condition -> K2 -> finish
+    rc = zstep_impl(N, D, q, X, ldx, S, lds, Gw, ldg, P0, h0, gl, MZ + gw_woff(q), ldmz, MZ, ldmz, Sig, logdet, NULL,
+                    PYVB_ALGO_DMMA_K1, stream);
+    if (rc != PYVB_OK) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = launch_known_condition(N, q, k, C, ldc, MZ, ldmz, st);
+    if (e == cudaSuccess) e = launch_zsolve(N, q, MZ, Sig, logdet, gl, NULL, st);
+    if (e == cudaSuccess) e = launch_known_finish(N, q, k, C, ldc, MZ, ldmz, st);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zstep_known");
+}
+
+int pyvb_zstep_i8_known_f64(long long N, int D, int q, int k, const double *C, long long ldc, double cmax, const double *X,
+                            long long ldx, const void *mask, const double *Wbar, const double *Wvar, const double *Gw, int ldg,
+                            const double *P0, const double *h0, double *gl, double *MZ, long long ldmz, void *GI,
+                            double *gscale, double *gmax, double *Sig, double *logdet, void *stream) {
+    int rc = known_args(N, q, k, C, ldc, MZ, ldmz);
+    if (rc != PYVB_OK) return rc;
+    ARG(cmax >= 0.0 && (N == 0 || gmax), "cmax, gmax");
+    if (N == 0) return pyvb_i8_supported(D, q) ? PYVB_OK : fail(PYVB_ENOSUP, "%s", "the INT8 path needs q in {16, 32, 64}");
+    // K1 (INT8 qprec + DMMA eta, the checks of the plain entry point), condition, then K2 with the accuracy guard
+    rc = pyvb_zstep_i8_f64(N, D, q, X, ldx, mask, Wbar, Wvar, Gw, ldg, P0, h0, gl, MZ, ldmz, GI, gscale, Sig, logdet, NULL, 1,
+                           stream);
+    if (rc != PYVB_OK) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    // the guard's scale: the free columns of qprec' as they are, the zc columns times max(1, cmax) (they enter eta_z times c),
+    // the cc columns not at all (condition discards them)
+    cudaError_t e = launch_known_guard_scale(q, k, gscale, cmax, gmax, st);
+    if (e == cudaSuccess) e = launch_known_condition(N, q, k, C, ldc, MZ, ldmz, st);
+    if (e == cudaSuccess) e = launch_zsolve(N, q, MZ, Sig, logdet, gl, NULL, st, nullptr, i8_check(D, gmax, 1));
+    // the fall-back on the FP64 tensor cores, every launch conditional on the guard's counter: K1 -> condition -> K2
+    const double *cond = gl + PYVB_GL_I8BAD;
+    if (e == cudaSuccess)
+        e = launch_zstep_dmma(N, D, q, X, ldx, Gw, ldg, P0, h0, gl, MZ, Sig, logdet, NULL, 1, st, cond);
+    if (e == cudaSuccess) e = launch_known_condition(N, q, k, C, ldc, MZ, ldmz, st, cond);
+    if (e == cudaSuccess) e = launch_zsolve(N, q, MZ, Sig, logdet, gl, NULL, st, cond);
+    if (e == cudaSuccess) e = launch_known_finish(N, q, k, C, ldc, MZ, ldmz, st);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zstep_i8_known");
+}
+
+int pyvb_zstep_csr_known_f64(long long N, int D, int q, int k, const double *C, long long ldc, const long long *indptr,
+                             const int *indices, const double *values, const double *weights, const double *Gw, int ldg,
+                             const double *P0, const double *h0, double *gl, double *MZ, long long ldmz, double *Sig,
+                             double *logdet, void *stream) {
+    ARG(D >= 1, "D");
+    int rc = known_args(N, q, k, C, ldc, MZ, ldmz);
+    if (rc != PYVB_OK) return rc;
+    if (!csr_supported(q)) return fail(PYVB_ENOSUP, "%s", "the CSR path needs q in {8, 16, 32, 64}");
+    if (N == 0) return PYVB_OK;
+    ARG(indptr && indices && values && Gw && P0 && h0 && gl && logdet, "null pointer");
+    ARG(ldg == pyvb_gw_pitch(q) && ldmz == pyvb_mz_pitch(q), "ldg / ldmz must equal pyvb_gw_pitch(q) / pyvb_mz_pitch(q)");
+    ARG((reinterpret_cast<uintptr_t>(Gw) & 15) == 0 && (reinterpret_cast<uintptr_t>(MZ) & 15) == 0,
+        "Gw and MZ must be 16-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = launch_zstep_csr(N, q, indptr, indices, values, Gw, ldg, P0, h0, gl, MZ, (int)ldmz, st, weights);
+    if (e == cudaSuccess) e = launch_known_condition(N, q, k, C, ldc, MZ, ldmz, st);
+    if (e == cudaSuccess) e = launch_zsolve(N, q, MZ, Sig, logdet, gl, NULL, st);
+    if (e == cudaSuccess) e = launch_known_finish(N, q, k, C, ldc, MZ, ldmz, st);
+    return e == cudaSuccess ? PYVB_OK : cuda_fail(e, "zstep_csr_known");
 }
 
 int pyvb_lds_max_len(void) {

@@ -28,7 +28,9 @@ cudaError_t launch_pack_gw(int D, int q, const double *Wbar, const double *Wvar,
 cudaError_t launch_zstep_generic(long long N, int D, int q, const double *X, long long ldx, const double *Gw,
                                  int ldg, const double *P0, const double *h0, double *gl, double *Zbar,
                                  long long ldz, double *M2, long long ldm, double *Sig, double *logdet,
-                                 cudaStream_t st, const double *S = nullptr, long long lds = 0);
+                                 cudaStream_t st, const double *S = nullptr, long long lds = 0,
+                                 const double *Cv = nullptr, long long ldc = 0, int kn = 0);
+// (Cv, ldc, kn: the last kn dimensions known per row, c_n = Cv[n][0, kn), conditioned on inside the kernel: DESIGN.md 5f)
 // main statistics: partial sums for `nchunks` row chunks into ws_main[nchunks][statlen]
 int stats_generic_nchunks(long long N);
 cudaError_t launch_stats_generic(long long N, int D, int q, const double *X, long long ldx, const double *Zbar,
@@ -180,6 +182,17 @@ cudaError_t launch_zstep_csr(long long N, int q, const long long *indptr, const 
 // wts (nullable): per entry, in the order of vals
 cudaError_t launch_stats_csc(int D, int q, int nblk, const long long *colptr, const int *rows, const double *vals,
                              const double *MZ, int ldmz, double *ws_main, cudaStream_t st, const double *wts = nullptr);
+
+// ---- known trailing latent dimensions, the row covariates of the plate (kernels_known.cu) ----
+// MZ rows of width qt whose last k dimensions are known per row, c_n = C[n][0, k).  condition: on K1's rows, eta_z -= qprec_zc c,
+// qprec_zc = 0, qprec_cc = I, eta_c = c (cond as launch_zsolve's).  finish: on K2's rows, <z'z'^T>_cc = c c^T and zbar_c = c.
+cudaError_t launch_known_condition(long long N, int qt, int k, const double *C, long long ldc, double *MZ, long long ldmz,
+                                   cudaStream_t st, const double *cond = nullptr);
+// the INT8 guard's scale of a conditioned row, one double into *out: max(max of gscale over the free columns,
+// max(1, cmax) * max of gscale over the zc columns); the cc columns, which condition discards, are left out
+cudaError_t launch_known_guard_scale(int qt, int k, const double *gscale, double cmax, double *out, cudaStream_t st);
+cudaError_t launch_known_finish(long long N, int qt, int k, const double *C, long long ldc, double *MZ, long long ldmz,
+                                cudaStream_t st);
 
 // ---- LDS smoother, batched over sequences (kernels_lds.cu) ----
 size_t lds_smem_bytes(int T, int d);

@@ -65,13 +65,17 @@ cudaError_t launch_pack_gw(int D, int q, const double *Wbar, const double *Wvar,
 // qmu = qcov . (pprec.pmu + sum m2).  ln prod diag chol comes from the factor's diagonal.
 // WT: per-entry observation weights S [N][lds]: qprec_n = P0 + tau sum_d s_nd G_d, eta_n = h0 + tau sum_d s_nd (x_nd - mu_d) wbar_d
 // (an entry of weight 0 is skipped, as a NaN)
-template <int NT, int WPB, bool WT>
+// KN: the last kn of the q dimensions are known per row, c_n = Cv[n][0, kn) (row covariates, DESIGN.md 5f): between the
+// contraction and the factorisation the row is conditioned on them in shared memory (eta_z -= qprec_zc c, qprec_zc = 0,
+// qprec_cc = I, eta_c = c: kernels_known.cu's condition), and the finished row gets zbar_c = c, <z z^T>_cc = c_i c_j
+template <int NT, int WPB, bool WT, bool KN = false>
 __global__ void __launch_bounds__(32 * WPB)
 zstep_generic_kernel(long long N, int D, int q, const double *__restrict__ X, long long ldx,
                      const double *__restrict__ Gw, int ldg, const double *__restrict__ P0,
                      const double *__restrict__ h0, double *gl, double *__restrict__ Zbar, long long ldz,
                      double *__restrict__ M2, long long ldm, double *__restrict__ Sig,
-                     double *__restrict__ logdet, const double *__restrict__ S, long long lds) {
+                     double *__restrict__ logdet, const double *__restrict__ S, long long lds,
+                     const double *__restrict__ Cv, long long ldc, int kn) {
     extern __shared__ double smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int P = tri(q), Pp = gw_woff(q), C = P + q;
@@ -132,6 +136,21 @@ zstep_generic_kernel(long long N, int D, int q, const double *__restrict__ X, lo
             }
         }
         __syncwarp();
+        if (KN) {
+            const double *cn = Cv + n * ldc;
+            const int qf = q - kn;
+            for (int i = lane; i < qf; i += 32) {
+                double e = eta[i];
+                for (int j = 0; j < kn; ++j) e = fma(-a[(qf + j) * pitch + i], cn[j], e);
+                eta[i] = e;
+            }
+            __syncwarp();                           // every zc entry is read before the tail rows are overwritten
+            for (int r = qf + lane; r < q; r += 32) {
+                for (int m = 0; m <= r; ++m) a[r * pitch + m] = (m == r) ? 1.0 : 0.0;
+                eta[r] = cn[r - qf];
+            }
+            __syncwarp();
+        }
         // ---- left-looking Cholesky, lanes over rows
         double ld = 0.0;
         bool ok = true;
@@ -167,6 +186,7 @@ zstep_generic_kernel(long long N, int D, int q, const double *__restrict__ X, lo
         for (int r = lane; r < q; r += 32) {
             double z = 0.0;
             for (int j = 0; j < q; ++j) z = fma(sv[r * pitch + j], eta[j], z);
+            if (KN && r >= q - kn) z = Cv[n * ldc + r - (q - kn)];
             zb[r] = z;
             Zbar[n * ldz + r] = z;
         }
@@ -175,7 +195,8 @@ zstep_generic_kernel(long long N, int D, int q, const double *__restrict__ X, lo
             int i, j;
             unpack_p(p, i, j);
             const double sg = 0.5 * (sv[i * pitch + j] + sv[j * pitch + i]);
-            M2[n * ldm + p] = fma(zb[i], zb[j], sg);
+            if (KN && j >= q - kn) M2[n * ldm + p] = zb[i] * zb[j];      // <c c^T>: no variance
+            else M2[n * ldm + p] = fma(zb[i], zb[j], sg);
             if (Sig) Sig[n * P + p] = sg;
         }
         if (lane == 0) {
@@ -189,7 +210,7 @@ zstep_generic_kernel(long long N, int D, int q, const double *__restrict__ X, lo
 cudaError_t launch_zstep_generic(long long N, int D, int q, const double *X, long long ldx, const double *Gw,
                                  int ldg, const double *P0, const double *h0, double *gl, double *Zbar,
                                  long long ldz, double *M2, long long ldm, double *Sig, double *logdet,
-                                 cudaStream_t st, const double *S, long long lds) {
+                                 cudaStream_t st, const double *S, long long lds, const double *Cv, long long ldc, int kn) {
     if (N <= 0) return cudaSuccess;
     const int C = tri(q) + q;
     const int nt = (C + 31) / 32;
@@ -197,13 +218,18 @@ cudaError_t launch_zstep_generic(long long N, int D, int q, const double *X, lon
     const size_t smem = (size_t)wpb * (2 * q * (q + 1) + 2 * q) * sizeof(double);
     long long blocks = (N + wpb - 1) / wpb;
     if (blocks > 148 * 16) blocks = 148 * 16;
-#define PYVB_LAUNCH_ZW(NT, WPB, WT)                                                                            \
+#define PYVB_LAUNCH_ZK(NT, WPB, WT, KN)                                                                        \
     do {                                                                                                       \
-        cudaError_t e = cudaFuncSetAttribute(zstep_generic_kernel<NT, WPB, WT>,                                \
+        cudaError_t e = cudaFuncSetAttribute(zstep_generic_kernel<NT, WPB, WT, KN>,                            \
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);          \
         if (e != cudaSuccess) return e;                                                                        \
-        zstep_generic_kernel<NT, WPB, WT><<<(unsigned)blocks, 32 * WPB, smem, st>>>(                           \
-            N, D, q, X, ldx, Gw, ldg, P0, h0, gl, Zbar, ldz, M2, ldm, Sig, logdet, S, lds);                    \
+        zstep_generic_kernel<NT, WPB, WT, KN><<<(unsigned)blocks, 32 * WPB, smem, st>>>(                       \
+            N, D, q, X, ldx, Gw, ldg, P0, h0, gl, Zbar, ldz, M2, ldm, Sig, logdet, S, lds, Cv, ldc, kn);       \
+    } while (0)
+#define PYVB_LAUNCH_ZW(NT, WPB, WT)                                                                            \
+    do {                                                                                                       \
+        if (Cv) PYVB_LAUNCH_ZK(NT, WPB, WT, true);                                                             \
+        else PYVB_LAUNCH_ZK(NT, WPB, WT, false);                                                               \
     } while (0)
 #define PYVB_LAUNCH_Z(NT, WPB)                                                                                 \
     do {                                                                                                       \
@@ -217,6 +243,7 @@ cudaError_t launch_zstep_generic(long long N, int D, int q, const double *X, lon
     else PYVB_LAUNCH_Z(67, 2);
 #undef PYVB_LAUNCH_Z
 #undef PYVB_LAUNCH_ZW
+#undef PYVB_LAUNCH_ZK
     return cudaGetLastError();
 }
 

@@ -85,18 +85,31 @@ class PlateEngine(object):
         covariances, one Gauss-Seidel pass over the columns per update_W.  "rows": q(W) = prod_d N(w_d | wbar_d, Sigma_d), one
         full q x q covariance per data dimension (the VB-PCA of Ilin & Raiko), solved outright per row by the batched q x q
         solve of the Z step; get_state() then also returns "Wcov" (D, q, q).  Mode "B", precision "f64", q in {8, 16, 32, 64}.
+    covariates : known per-row covariates c_n of the local row shard, an (N, k) array or tensor (finite, k >= 1, q + k <= 64):
+        x_nd ~ N(w_d z_n + b_d c_n + mu_d, 1/tau), the fixed effects B (D, k) fitted jointly with the q free latent
+        dimensions.  The engine runs the plate at q' = q + k with z'_n = [z_n ; c_n] and W' = [W | B] (DESIGN 5f): the Z step
+        conditions on the known tail, everything else is unchanged at q'.  Mode "B", precision "f64"; q' selects the path
+        (INT8 where pyvb_i8_supported(D, q'), DMMA where q' in {8, 16, 32, 64} and D % 16 == 0, else generic; sparse X and
+        w_posterior="rows" need q' in {8, 16, 32, 64}).  P0, m0 describe the q free dimensions; the B columns share alpha0 or the ARD
+        Gammas with W (alpha and al_qb have q' entries).  get_state() returns Zbar (N, q), Sig (N, q, q), Wbar / Wvar (D, q),
+        Bbar / Bvar (D, k) and, with w_posterior="rows", Wcov (D, q', q'), the joint posterior covariance of [w_d ; b_d].
     """
 
     def __init__(self, X, q, mode="B", alpha0=1e-3, alpha_mu=1e-3, a0=1e-3, b0=1e-3, ard=False,
                  ard_a0=1e-3, ard_b0=1e-3, P0=None, m0=None, device=None, algo="auto",
                  keep_sigma=True, distributed=False, row_offset=0, trace_len=4096, precision="f64", noise="scalar",
-                 weights=None, w_posterior="columns"):
+                 weights=None, w_posterior="columns", covariates=None):
         if not torch.cuda.is_available():
             raise RuntimeError("pyvb_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         self.lib = _cabi.lib()
         assert mode in ("A", "B")
         assert 1 <= q <= QMAX, "latent dimension must be in [1, %d]" % QMAX
         assert precision in ("f64", "f32")
+        self.qz, self.k = int(q), 0
+        if covariates is not None:
+            covariates = self._check_covariates(covariates, int(q), mode, precision, algo)
+            self.k = int(covariates.shape[1])
+            q = self.qz + self.k
         self.f32 = (precision == "f32")
         if noise not in ("scalar", "diagonal"):
             raise ValueError("noise must be 'scalar' or 'diagonal', got %r" % (noise,))
@@ -124,10 +137,28 @@ class PlateEngine(object):
             self.device = torch.device("cuda", torch.cuda.current_device())
         with torch.cuda.device(self.device):
             self._construct(X, q, mode, alpha0, alpha_mu, a0, b0, ard, ard_a0, ard_b0, P0, m0, algo, keep_sigma,
-                            distributed, row_offset, trace_len, weights)
+                            distributed, row_offset, trace_len, weights, covariates)
+
+    @staticmethod
+    def _check_covariates(C, q, mode, precision, algo):
+        """The covariates as a host float64 (N, k) tensor; raises ValueError on what the covariate mode does not run."""
+        if _sparse.is_sparse(C):
+            raise ValueError("covariates must be a dense (N, k) array or tensor")
+        C = torch.as_tensor(C).detach().to(device="cpu", dtype=torch.float64)
+        if C.dim() != 2 or C.shape[1] < 1:
+            raise ValueError("covariates must have shape (N, k) with k >= 1, got %s" % (tuple(C.shape),))
+        if mode != "B":
+            raise ValueError("covariates need mode='B' (mode A is the reference-exact imputation path)")
+        if precision != "f64":
+            raise ValueError("covariates need precision='f64'")
+        if q + int(C.shape[1]) > QMAX:
+            raise ValueError("covariates: q + k must be <= %d, got q = %d, k = %d" % (QMAX, q, int(C.shape[1])))
+        if not bool(torch.isfinite(C).all()):
+            raise ValueError("covariates must be finite")
+        return C.contiguous()
 
     def _construct(self, X, q, mode, alpha0, alpha_mu, a0, b0, ard, ard_a0, ard_b0, P0, m0, algo, keep_sigma,
-                   distributed, row_offset, trace_len, weights):
+                   distributed, row_offset, trace_len, weights, covariates=None):
         self.mode, self.q, self.ard = mode, int(q), bool(ard)
         self.sparse = _sparse.is_sparse(X)
         if self.sparse:
@@ -160,6 +191,15 @@ class PlateEngine(object):
             Xt = Xt.to(device=dev, dtype=f64).contiguous()
             self.N, self.D = int(Xt.shape[0]), int(Xt.shape[1])
         N, D = self.N, self.D
+        # ---- known covariates: the last k latent columns of every row, c_n
+        self.C = None
+        if covariates is not None:
+            if int(covariates.shape[0]) != N:
+                raise ValueError("covariates must have one row per row of X: (%d, k), got %s" % (N, tuple(covariates.shape)))
+            self.C = covariates.to(dev)
+            # the INT8 guard weighs the zc columns of qprec' by the largest sum_j |c_nj| of the shard (they enter eta_z times c)
+            self.cmax = float(covariates.abs().sum(1).max()) if N > 0 else 0.0
+            self.gmax = torch.zeros(1, dtype=f64, device=dev)
         # ---- per-entry weights: S (dense, zero where x is missing) or the CSR-ordered `wcsr`; the NUMBER of observed entries of
         # positive weight (per column `ncnt`: the per-dimension Gammas) and 1/2 sum ln s, both constants of the data set
         self.S = self.wcsr = self.ncnt = None
@@ -376,10 +416,19 @@ class PlateEngine(object):
         self.trace_pos = 0
 
         # ---- priors
-        P0 = np.eye(q) if P0 is None else np.asarray(P0, dtype=np.float64).reshape(q, q)
-        m0 = np.zeros(q) if m0 is None else np.asarray(m0, dtype=np.float64).reshape(q)
-        self.P0 = torch.as_tensor(P0, dtype=f64).contiguous().to(dev)
-        self.h0 = torch.as_tensor(P0 @ m0, dtype=f64).contiguous().to(dev)
+        qz = self.qz if self.k else q
+        P0 = np.eye(qz) if P0 is None else np.asarray(P0, dtype=np.float64).reshape(qz, qz)
+        m0 = np.zeros(qz) if m0 is None else np.asarray(m0, dtype=np.float64).reshape(qz)
+        if self.k:
+            # the known dimensions have no prior: P0' = blockdiag(P0, 0), h0' = [h0 ; 0] (the bound's tr(P0' <z'z'^T>) and
+            # h0'^T zbar' are then those of the free block)
+            P0a = np.zeros((q, q))
+            P0a[:qz, :qz] = P0
+            self.P0 = torch.as_tensor(P0a, dtype=f64).contiguous().to(dev)
+            self.h0 = torch.as_tensor(np.concatenate([P0 @ m0, np.zeros(self.k)]), dtype=f64).contiguous().to(dev)
+        else:
+            self.P0 = torch.as_tensor(P0, dtype=f64).contiguous().to(dev)
+            self.h0 = torch.as_tensor(P0 @ m0, dtype=f64).contiguous().to(dev)
         qa = self.a0 + 0.5 * n_eff
         al_qa = self.ard_a0 + 0.5 * D
         c = _cabi.Consts()
@@ -389,6 +438,10 @@ class PlateEngine(object):
         c.psi_alqa, c.lgam_alqa, c.lgam_ard_a0 = _digamma(al_qa), math.lgamma(al_qa), math.lgamma(self.ard_a0)
         c.lndet_P0 = float(np.linalg.slogdet(P0)[1])
         c.m0P0m0 = float(m0 @ P0 @ m0)
+        if self.k:
+            # the Z term of the bound counts q/2 per row for the entropy of q(z_n); it is taken at q' = q + k, but only the
+            # q free dimensions have an entropy: -k is folded into ln det P0 (the term adds 1/2 ln det P0 per row)
+            c.lndet_P0 -= self.k
         c.ard, c.mode_a = int(self.ard), int(mode == "A")
         self.consts = c
         self.qa, self.al_qa = qa, al_qa
@@ -406,8 +459,23 @@ class PlateEngine(object):
 
         # deterministic stand-in initialisation (SURVEY 8d); parity runs call set_state()
         self.set_state({"qb": 0.5, "al_qb": np.ones(q)})
+        if self.k:
+            self._set_known_tail()
         self._stats_fresh = False
         self._gw_fresh = False
+
+    def _set_known_tail(self, step=1 << 16):
+        """Covariates: zbar'_c = c and the last k rows of <z'z'^T> packed, <z c^T> = zbar c^T and <c c^T> = c c^T (the
+        known dimensions have no variance), from the free columns of Zbar."""
+        qz, q = self.qz, self.q
+        ii, jj = tril_pack_index(q)
+        p0 = qz * (qz + 1) // 2
+        it, jt = torch.as_tensor(ii[p0:], device=self.device), torch.as_tensor(jj[p0:], device=self.device)
+        for lo in range(0, self.N, step):
+            z = self.Zbar[lo:lo + step]
+            z[:, qz:] = self.C[lo:lo + step]
+            self.M2[lo:lo + step, p0:] = z[:, it] * z[:, jt]
+        self._zsums_valid = False
 
     @_on_device
     def close(self):
@@ -456,6 +524,10 @@ class PlateEngine(object):
         if "Wcov" in st and not self.wrows:
             raise ValueError("set_state: 'Wcov' is the state of w_posterior='rows'; this engine's W posterior has column "
                              "variances only (Wvar)")
+        if self.k:
+            st = self._augment_state(st)
+        elif "Bbar" in st or "Bvar" in st:
+            raise ValueError("set_state: 'Bbar' / 'Bvar' are the covariate effects of an engine built with covariates=")
         for k in ("Wbar", "Wvar", "mu", "muvar", "Zbar"):
             if k in st:
                 put(getattr(self, k), st[k])
@@ -507,6 +579,50 @@ class PlateEngine(object):
         self._stats_fresh = False
         self._gw_fresh = False
         self._zsums_valid = False
+
+    def _augment_state(self, st):
+        """Covariates: a state in the user's layout (Zbar (N, q), Sig (N, q, q), Wbar / Wvar (D, q), Bbar / Bvar (D, k)) as
+        the engine's q' = q + k layout: Zbar' = [Zbar | C], Sig' = blockdiag(Sig, 0), W' = [W | B]."""
+        st = dict(st)
+        qz, q, N = self.qz, self.q, self.N
+        for a, b in (("Wbar", "Bbar"), ("Wvar", "Bvar")):
+            if a in st or b in st:
+                cur = getattr(self, a).cpu().numpy().copy()
+                if a in st:
+                    cur[:, :qz] = np.asarray(st[a], dtype=np.float64).reshape(self.D, qz)
+                if b in st:
+                    cur[:, qz:] = np.asarray(st.pop(b), dtype=np.float64).reshape(self.D, self.k)
+                st[a] = cur
+        if "Zbar" in st:
+            st["Zbar"] = np.concatenate([np.asarray(st["Zbar"], dtype=np.float64).reshape(N, qz), self.C.cpu().numpy()], 1)
+            if "Sig" not in st and self.Sig is not None:
+                st["Sig"] = self._sig_host(self.Sig.cpu().numpy(), None)
+        if "Sig" in st:
+            S = np.zeros((N, q, q))
+            S[:, :qz, :qz] = np.asarray(st["Sig"], dtype=np.float64).reshape(N, qz, qz)
+            st["Sig"] = S
+        return st
+
+    def _sig_host(self, sp, z):
+        """(n, q_free, q_free) covariances from packed rows at the engine's q: Sig rows (z None) or <zz^T> rows minus zbar zbar^T."""
+        ii, jj = tril_pack_index(self.q)
+        if z is not None:
+            sp = sp - z[:, ii] * z[:, jj]
+        S = np.zeros((sp.shape[0], self.q, self.q))
+        S[:, ii, jj] = sp
+        S[:, jj, ii] = sp
+        return S[:, :self.qz, :self.qz].copy()
+
+    def _split_state(self, out):
+        """Covariates: the engine's q' layout -> the user's (free columns; B apart)."""
+        qz = self.qz
+        for a, b in (("Wbar", "Bbar"), ("Wvar", "Bvar")):
+            if a in out:
+                out[b] = out[a][:, qz:].copy()
+                out[a] = out[a][:, :qz].copy()
+        if "Zbar" in out:
+            out["Zbar"] = out["Zbar"][..., :qz].copy()
+        return out
 
     def _set_wcov(self, wcov):
         """Row-wise W posterior: Wcov from a (D, q, q) array, or diag(Wvar) when None; Wvar = diag Wcov and Wld =
@@ -573,6 +689,8 @@ class PlateEngine(object):
             if self.Sig is not None:
                 self.Sig[lo:lo + step] = eye
         self.logdet.fill_(1.0)
+        if self.k:
+            self._set_known_tail()
         self.set_state({"qb": 0.5, "al_qb": np.ones(q)})
 
     @_on_device
@@ -586,6 +704,8 @@ class PlateEngine(object):
                                       "build a new engine for new data")
         if self.weighted:
             raise NotImplementedError("set_X: the weights belong to the data set; build a new engine for new data")
+        if self.k:
+            raise NotImplementedError("set_X: the covariates belong to the data set; build a new engine for new data")
         assert self.mode == "B" and not self.f32
         self.X.copy_(X, non_blocking=True)
         self._xcache_valid = False
@@ -600,15 +720,20 @@ class PlateEngine(object):
         out = {k: getattr(self, k).contiguous().to(torch.float64).cpu().numpy()
                for k in ("Wbar", "Wvar", "mu", "muvar", "Zbar")}
         N = self.N
-        if self.Sig is not None:
+        if self.k:
+            out["Sig"] = (self._sig_host(self.Sig.cpu().numpy(), None) if self.Sig is not None
+                          else self._sig_host(self.M2.contiguous().cpu().numpy(), out["Zbar"]))
+            self._split_state(out)
+        elif self.Sig is not None:
             sp = self.Sig.cpu().numpy()
         else:
             z = out["Zbar"]
             sp = self.M2.contiguous().to(torch.float64).cpu().numpy() - z[:, ii] * z[:, jj]
-        Sig = np.zeros((N, q, q))
-        Sig[:, ii, jj] = sp
-        Sig[:, jj, ii] = sp
-        out["Sig"] = Sig
+        if not self.k:
+            Sig = np.zeros((N, q, q))
+            Sig[:, ii, jj] = sp
+            Sig[:, jj, ii] = sp
+            out["Sig"] = Sig
         if self.wrows:
             out["Wcov"] = self._wcov_host()
         if self.mode == "A":
@@ -642,6 +767,9 @@ class PlateEngine(object):
         q = self.q
         ii, jj = tril_pack_index(q)
         z = self.Zbar[i].contiguous().to(torch.float64).cpu().numpy()
+        if self.k:
+            sp = self.Sig[i:i + 1].cpu().numpy() if self.Sig is not None else self.M2[i:i + 1].cpu().numpy()
+            return {"Zbar": z[:self.qz].copy(), "Sig": self._sig_host(sp, None if self.Sig is not None else z[None])[0]}
         if self.Sig is not None:
             sp = self.Sig[i].cpu().numpy()
         else:
@@ -664,6 +792,8 @@ class PlateEngine(object):
         if self.wrows:
             out["Wcov"] = self._wcov_host()
         out.update(self._noise_state(gl))
+        if self.k:
+            self._split_state(out)
         return out
 
     def check(self):
@@ -818,6 +948,9 @@ class PlateEngine(object):
         self._ensure_gw()
         q, P, D = self.q, self.P, self.D
         sig = 0 if self.Sig is None else self.Sig.data_ptr() + lo * P * 8
+        if self.k:
+            self._update_Z_known(lo, hi, sig)
+            return
         if self.sparse:
             # any row range: K1-csr owns whole rows, so [lo, hi) is a pointer offset into the row offsets
             full = (lo == 0 and hi == self.N and self.zsums is not None)
@@ -879,6 +1012,41 @@ class PlateEngine(object):
             _cabi.check(rc, "pyvb_zstep_f64")
         self._zsums_valid = full
         self._stats_fresh = False
+
+    def _update_Z_known(self, lo, hi, sig):
+        """Covariates: K1 at q' -> condition on c_n -> K2 -> finish (kernels_known.cu).  K2's partials are wrong on the known
+        entries, so none are kept: the next statistics pass rebuilds the column sums from the rows."""
+        q, D, k, ld = self.q, self.D, self.k, self.ldmz
+        self._zsums_valid = False
+        C = self.C.data_ptr() + lo * k * 8
+        MZ = self.MZ.data_ptr() + lo * ld * 8
+        if self.sparse:
+            rc = self.lib.pyvb_zstep_csr_known_f64(hi - lo, D, q, k, C, k, self.csr.indptr.data_ptr() + lo * 8,
+                                                   self.csr.indices.data_ptr(), self.csr.values.data_ptr(), self._p(self.wcsr),
+                                                   self.Gw.data_ptr(), self.ldg, self.P0.data_ptr(), self.h0.data_ptr(),
+                                                   self.gl.data_ptr(), MZ, ld, sig, self.logdet.data_ptr() + lo * 8,
+                                                   self._stream())
+            _cabi.check(rc, "pyvb_zstep_csr_known_f64")
+            return
+        if self.use_i8 and lo % 128 == 0:                   # (the int8 mask is tiled by 128 rows, as in update_Z)
+            if not self._mask_valid:
+                rc = self.lib.pyvb_prepare_mask_i8(hi - lo, D, self.X.data_ptr() + lo * D * 8, D,
+                                                   self.mask8.data_ptr() + lo * D, self._stream())
+                _cabi.check(rc, "pyvb_prepare_mask_i8")
+                self._mask_valid = (lo == 0 and hi == self.N)
+            rc = self.lib.pyvb_zstep_i8_known_f64(hi - lo, D, q, k, C, k, self.cmax, self.X.data_ptr() + lo * D * 8, D,
+                                                  self.mask8.data_ptr() + lo * D, self.Wbar.data_ptr(), self.Wvar.data_ptr(),
+                                                  self.Gw.data_ptr(), self.ldg, self.P0.data_ptr(), self.h0.data_ptr(),
+                                                  self.gl.data_ptr(), MZ, ld, self.GI.data_ptr(), self.gscale.data_ptr(),
+                                                  self.gmax.data_ptr(), sig,
+                                                  self.logdet.data_ptr() + lo * 8, self._stream())
+            _cabi.check(rc, "pyvb_zstep_i8_known_f64")
+            return
+        rc = self.lib.pyvb_zstep_known_f64(hi - lo, D, q, k, C, k, self.X.data_ptr() + lo * D * 8, D,
+                                           0 if self.S is None else self.S.data_ptr() + lo * D * 8, D, self.Gw.data_ptr(),
+                                           self.ldg, self.P0.data_ptr(), self.h0.data_ptr(), self.gl.data_ptr(), MZ, ld, sig,
+                                           self.logdet.data_ptr() + lo * 8, self.algo, self._stream())
+        _cabi.check(rc, "pyvb_zstep_known_f64")
 
     @_on_device
     def update_X(self, lo=0, hi=None):
@@ -996,6 +1164,8 @@ class PlateEngine(object):
                                       "the resident data set")
         if self.weighted:
             raise NotImplementedError("iterate_from_host: the weights are constants of the resident data set")
+        if self.k:
+            raise NotImplementedError("iterate_from_host: the covariates are constants of the resident data set")
         assert self.mode == "B"
         assert not self.f32, "iterate_from_host: the FP32 variant keeps X as bf16 planes; use precision='f64'"
         N = self.N
